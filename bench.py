@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            (torchrun for N > 1, one rank per GPU)
   python bench.py --impl reference --gpus N --steps K --warmup W
+  python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR     (writes the last timed step's outputs as .npy)
 
 Headline workload (config.workload): BASELINE.json config 4 -- an ensemble of 4096 independent
 reference-size (21, 21, 36) pose-cell networks IN TOTAL, float32, per-network global inhibition in
@@ -519,6 +520,18 @@ def check_sampled_networks(ens, odom_dev, gis, rank):
     return len(pick)
 
 
+def last_step_outputs(ens, n_sample=512):
+    """What a caller of the timed update_async holds after the last timed step, as host arrays in float32 / float64:
+    the arg-max cell (x, y, th), the total activity and the error flags of every network, and the whole state of a
+    fixed, seeded sample of ``n_sample`` networks (``networks``) in the reference's [x][y][th] layout (32.5 MB of the 260 MB ensemble)."""
+    import torch
+    pick = np.sort(np.random.default_rng(0).choice(ens.n_networks, min(n_sample, ens.n_networks), replace=False))
+    states = ens.state.index_select(0, torch.from_numpy(pick).to(ens.state.device)).permute(0, 2, 3, 1)
+    return {"argmax": ens._unravel(ens._argmax.cpu().numpy()).astype(np.float64),
+            "total": ens._total.cpu().numpy(), "err": ens._err.cpu().numpy().astype(np.float32),
+            "networks": pick.astype(np.float64), "posecells": states.cpu().numpy()}
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -579,6 +592,9 @@ def run_ours(args):
                 e.update_result()
 
     timed(torch, d, world, step_dev, W)
+    # The timed steps start from the state these W steps leave, whatever number of batches the clock warm-up below
+    # takes: with the same arguments they compute the same results from run to run
+    start = [e.state.clone() for e in ens]
     # The GPU idled while the host ran the oracle checks: keep warming up (untimed) until two consecutive batches of K
     # steps agree within 1 % -- SM clocks at their boost level -- at most ten batches
     prev = None
@@ -588,8 +604,12 @@ def run_ours(args):
         if prev is not None and abs(cur - prev) <= 0.01 * prev:
             break
         prev = cur
+    for e, s in zip(ens, start):
+        e.state.copy_(s)
+    del start
     with ClockSampler(local) as clk:
         ms = timed(torch, d, world, step_dev, K)
+        last = last_step_outputs(ens[(K - 1) % R]) if args.dump_outputs else None
         # keep the sampler alive for at least a few samples on very short runs
         if ms < 400:
             timed(torch, d, world, step_dev, max(K, int(400 / max(ms / K, 1e-3))))
@@ -698,6 +718,9 @@ def run_ours(args):
             line["extra_sharded"] = shard
     if rank == 0:
         emit(line)
+    if last is not None:
+        for name, a in last.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     if world > 1:
         dist.destroy_process_group()
 
@@ -730,7 +753,13 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-extra", action="store_true", help="skip the secondary workloads (profiling runs)")
     ap.add_argument("--no-parity", action="store_true", help="skip the in-run oracle checks (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step of the headline ensemble as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs:
+        if args.impl != "ours" or int(os.environ.get("WORLD_SIZE", "1")) > 1:
+            ap.error("--dump-outputs writes the outputs of one GPU: use it with --impl ours --gpus 1")
+        os.makedirs(args.dump_outputs, exist_ok=True)
     _claim_stdout()
     if args.impl == "reference":
         run_reference(args)
