@@ -345,6 +345,21 @@ PRS_API int prs_frame_run(prs_frame_plan* plan, int moved, void* stream);
  * frames back to back while the host prepares the next frame and digests the previous result. */
 PRS_API int prs_frame_launch(prs_frame_plan* plan, int moved, void* stream);
 
+/* View-template -> pose-cell injection inside the frame (ros_simulate.py:106-108, left commented out in the reference):
+ * after the create-or-match decision and the pose-cell update, one more node adds `energy` to the cell stored with the
+ * frame's template, posecells[loc_dev[template]] += energy, and keeps the plan's cached arg-max current (the injected
+ * cell becomes the arg-max if it now exceeds the old one, or equals it at a lower flat index: numpy.argmax's first
+ * maximum, exact for energy >= 0).  A created template's row is written on the device with the arg-max its match was
+ * made with; rows of templates appended outside the plans are the caller's to fill in.  A frame whose template has the
+ * row -1 leaves the state as it is and sets PRS_ERR_INJECT_LOC in its record's pc_err.  The record's arg-max stays the
+ * one the match was made with; the next frame sees the injected state.  With PRS_OPT_ACTIVE_SET the carried lists are
+ * invalidated, as prs_pc_inject does.
+ * loc_dev: device int64 [capacity], C-order flat cell of every template, -1 = invalid; NULL turns injection off.
+ *          Plans built on one library share it.
+ * energy: finite and >= 0 (PRS_E_INVALID otherwise).  Changing the setting drops the plan's captured graphs. */
+PRS_API int prs_frame_set_inject(prs_frame_plan* plan, double energy, long long* loc_dev);
+#define PRS_ERR_INJECT_LOC 8 /* prs_frame_result.pc_err: the matched template has no valid pose cell */
+
 /* The whole loop of ros_simulate.py:152-166 over recorded arrays in one call: frame t is staged into the pinned
  * buffers of plans[t % n_plans] and launched while earlier frames are still running; a plan is reused once its frame
  * has finished and its result has been copied to results[].  The plans must share pc / pc_state / pc_work / vt_packed /

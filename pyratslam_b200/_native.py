@@ -15,6 +15,7 @@ LIB_PATH = os.environ.get("PYRATSLAM_B200_LIB") or os.path.join(PKG, "_lib", "li
 
 PRS_F32, PRS_F64 = 0, 1
 ERR_LUT_KEY, ERR_RADIUS, ERR_THETA = 1, 2, 4
+ERR_INJECT_LOC = 8             # prs_frame_result.pc_err: the frame's template has no valid pose cell
 E_LUT_KEY, E_RADIUS = -4, -5   # return codes of prs_pc_update_host
 OG_RANGE = 8
 VT_MODE_REF, VT_MODE_CIRCULAR = 0, 1
@@ -91,6 +92,7 @@ _SIGNATURES["prs_frame_destroy"] = (c_int, [c_void_p])
 _SIGNATURES["prs_frame_set_count"] = (c_int, [c_void_p, c_int, c_void_p])
 _SIGNATURES["prs_frame_run"] = (c_int, [c_void_p, c_int, c_void_p])
 _SIGNATURES["prs_frame_launch"] = (c_int, [c_void_p, c_int, c_void_p])
+_SIGNATURES["prs_frame_set_inject"] = (c_int, [c_void_p, c_double, c_void_p])
 _SIGNATURES["prs_replay_run"] = (c_int, [POINTER(c_void_p), c_int, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p])
 
 

@@ -1246,10 +1246,13 @@ struct FrameScratch {               // device scratch layout (bytes)
   static constexpr size_t kBytes = kOdom + 64;
 };
 
+// dec (optional): a second, device-side copy of the decision (created, template_index, n_templates) for the frame's
+// injection node when `res` is the pinned host record
 __global__ void k_vt_decide_append(const unsigned long long* __restrict__ key, const uint8_t* __restrict__ tpl,
                                    uint4* __restrict__ packed, int n, unsigned threshold,
                                    const long long* __restrict__ argmax, const int* __restrict__ pc_err,
-                                   prs_frame_result* __restrict__ res, int* __restrict__ n_dev, int write_pc = 1) {
+                                   prs_frame_result* __restrict__ res, int* __restrict__ n_dev, int write_pc = 1,
+                                   prs_frame_result* __restrict__ dec = nullptr) {
   const int t = threadIdx.x;  // 32 threads, one per template row
   if (n_dev != nullptr) n = *n_dev;
   __syncwarp();
@@ -1267,7 +1270,59 @@ __global__ void k_vt_decide_append(const unsigned long long* __restrict__ key, c
     res->n_templates = n + (create ? 1 : 0);
     if (write_pc) res->pc_err = pc_err ? pc_err[0] : 0;
     if (n_dev != nullptr) *n_dev = n + (create ? 1 : 0);
+    if (dec != nullptr) {
+      dec->created = create ? 1 : 0;
+      dec->template_index = create ? n : (int)(k & 0xffffffffu);
+      dec->n_templates = n + (create ? 1 : 0);
+    }
   }
+}
+
+// View-template -> pose-cell injection at the tail of a frame (ros_simulate.py:106-108): posecells[location(template)]
+// += energy, where a created template's location is the arg-max its match was made with and a matched template's is
+// whatever its row of the location table holds (C-order flat index x*Y*Th + y*Th + th, -1 = not a valid cell).  One
+// thread does it all: one table row, one cell, one comparison.  The cached arg-max is kept current in O(1): no other
+// cell changed, so with energy >= 0 the first maximum (numpy.argmax) is either the old one or the injected cell.
+//   dec    : this frame's decision, device memory (never the pinned record: no read over the bus)
+//   argmax : the cached arg-max of pc_work, the one the match was made with; updated in place
+//   res    : the frame's record, receives PRS_ERR_INJECT_LOC (on top of pc_err, the pose-cell bits it already holds)
+// The node sits on the frame's critical path and is a chain of dependent loads: the arg-max cell is read alongside the
+// table row, a created template needs no row read at all, and the index arithmetic is 32-bit where the grid allows.
+template <typename I>
+__device__ __forceinline__ size_t pc_theta_major(I f, I X, I Y, I Th) {  // [x][y][th] flat index -> [th][x][y] offset
+  const I xy = f / Th, th = f - xy * Th, x = xy / Y, y = xy - x * Y;
+  return ((size_t)th * X + x) * Y + y;
+}
+
+template <typename T>
+__global__ void k_frame_inject(T* __restrict__ state, long long* __restrict__ loc, const prs_frame_result* dec,
+                               long long* __restrict__ argmax, const int* __restrict__ pc_err, prs_frame_result* res,
+                               int X, int Y, int Th, T energy) {
+  if (threadIdx.x != 0) return;
+  const long long N = (long long)X * Y * Th;
+  const bool narrow = N <= 0xffffffffLL;
+  auto offset = [&](long long f) {
+    return narrow ? pc_theta_major<unsigned>((unsigned)f, X, Y, Th) : pc_theta_major<long long>(f, X, Y, Th);
+  };
+  const long long a = *argmax;
+  const int ti = dec->template_index;
+  const bool created = dec->created != 0;
+  const bool a_ok = a >= 0 && a < N;
+  const size_t oa = a_ok ? offset(a) : 0;
+  const T m = state[oa];  // the arg-max's value; no other cell than the injected one changes
+  long long c = a;
+  if (created)
+    loc[ti] = a;
+  else
+    c = loc[ti];
+  if (c < 0 || c >= N) {  // the posecells of the frame stay as they are
+    res->pc_err = pc_err[0] | PRS_ERR_INJECT_LOC;
+    return;
+  }
+  const size_t oc = c == a ? oa : offset(c);
+  const T v = (c == a ? m : state[oc]) + energy;  // k_inject's arithmetic
+  state[oc] = v;
+  if (c != a && (!a_ok || v > m || (v == m && c < a))) *argmax = c;
 }
 
 extern "C" size_t prs_frame_scratch_bytes(void) { return FrameScratch::kBytes; }
@@ -1543,6 +1598,9 @@ struct prs_frame_plan {
   const double* odom_map;
   const uint8_t* frame_map;
   prs_frame_result* result_map;
+  // prs_frame_set_inject: the location table (null = no injection) and the energy of the frame's last node
+  long long* inj_loc;
+  double inj_energy;
 };
 
 static int frame_enqueue(prs_frame_plan* f, bool moved, cudaStream_t st) {
@@ -1600,10 +1658,22 @@ static int frame_enqueue(prs_frame_plan* f, bool moved, cudaStream_t st) {
     if (rc != PRS_OK) return rc;
   }
   if (moved && !pc_mirrored) PRS_CUDA(cudaStreamWaitEvent(st, f->ev_join, 0));  // the decision reports the new arg-max
-  k_vt_decide_append<<<1, 32, 0, st>>>(d_key, d_tpl, (uint4*)f->vt_packed, 0, f->threshold, d_argmax, d_err,
-                                       zero_copy ? f->result_map : d_res, f->d_n, pc_mirrored ? 0 : 1);
+  prs_frame_result* rec = zero_copy ? f->result_map : d_res;
+  k_vt_decide_append<<<1, 32, 0, st>>>(d_key, d_tpl, (uint4*)f->vt_packed, 0, f->threshold, d_argmax, d_err, rec, f->d_n,
+                                       pc_mirrored ? 0 : 1, (zero_copy && f->inj_loc) ? d_res : nullptr);
   PRS_CUDA(cudaGetLastError());
   if (moved && pc_mirrored) PRS_CUDA(cudaStreamWaitEvent(st, f->ev_join, 0));  // join: the frame ends with both branches
+  if (f->inj_loc) {  // behind both branches: the decision and the update (also the mirrored one the decision skips)
+    prs_pc_plan* pc = f->pc;
+    if (int rc_ = prs_pc_active_invalidate(pc, st)) return rc_;  // as prs_pc_inject: the carried lists are stale
+    if (pc->dtype == PRS_F32)
+      k_frame_inject<float><<<1, 32, 0, st>>>((float*)f->pc_state, f->inj_loc, d_res, d_argmax, d_err, rec, pc->X, pc->Y,
+                                              pc->Th, (float)f->inj_energy);
+    else
+      k_frame_inject<double><<<1, 32, 0, st>>>((double*)f->pc_state, f->inj_loc, d_res, d_argmax, d_err, rec, pc->X, pc->Y,
+                                               pc->Th, f->inj_energy);
+    PRS_CUDA(cudaGetLastError());
+  }
   if (!zero_copy)
     PRS_CUDA(cudaMemcpyAsync(f->result_host, d_res, sizeof(prs_frame_result), cudaMemcpyDeviceToHost, st));
   return PRS_OK;
@@ -1670,6 +1740,23 @@ extern "C" int prs_frame_set_count(prs_frame_plan* f, int n_templates, void* str
   PRS_REQUIRE(f && n_templates >= 0 && n_templates < f->capacity, "prs_frame_set_count: bad argument");
   PRS_CUDA(cudaMemcpyAsync(f->d_n, &n_templates, sizeof(int), cudaMemcpyHostToDevice, (cudaStream_t)stream));
   PRS_CUDA(cudaStreamSynchronize((cudaStream_t)stream));
+  return PRS_OK;
+}
+
+// Turning the injection on or off, or changing its energy or table, changes the frame's last node: the captured graphs
+// go, the next frame of each kind runs eagerly again and the one after it captures.
+extern "C" int prs_frame_set_inject(prs_frame_plan* f, double energy, long long* loc_dev) {
+  PRS_REQUIRE(f, "prs_frame_set_inject: null plan");
+  PRS_REQUIRE(energy >= 0.0 && energy <= 1.7976931348623157e308,
+              "prs_frame_set_inject: the energy must be finite and >= 0, got %g", energy);
+  if (f->inj_loc == loc_dev && (loc_dev == nullptr || f->inj_energy == energy)) return PRS_OK;
+  for (int i = 0; i < 2; ++i) {
+    if (f->ready[i]) cudaGraphExecDestroy(f->exec[i]);
+    f->ready[i] = false;
+    f->warm[i] = 0;
+  }
+  f->inj_loc = loc_dev;
+  f->inj_energy = energy;
   return PRS_OK;
 }
 

@@ -111,6 +111,7 @@ class RatslamRos(object):
         self._f_stream = torch.cuda.Stream(device=dev)
         self._f_plan = ctypes.c_void_p()
         self._f_plan_key = None
+        self._f_inj = self._NO_INJECT    # the injection setting of _f_plan
         self._f_gen = e._state_gen       # the pose-cell state the cached arg-max (_f_pcwork) was computed from
         self._f_n_dev = None             # the template count the plans' device-side counter holds
         torch.cuda.current_stream(dev).synchronize()
@@ -120,7 +121,8 @@ class RatslamRos(object):
         """Bring the device-side caches of the frame plans back in step with what happened OUTSIDE them: a pose-cell
         update / inject / assignment since the last fused frame invalidates the cached arg-max (it is recomputed on
         the frame stream, behind whatever the current stream still has queued), templates appended by
-        ``vts.match`` / ``create`` invalidate the device-side library size."""
+        ``vts.match`` / ``create`` invalidate the device-side library size and the rows of the device-side location
+        table that the injection node reads."""
         e, v = self.pcn._ens, self.vts
         if e._state_gen != self._f_gen:
             self._f_stream.wait_stream(torch.cuda.current_stream(e.device))
@@ -133,6 +135,38 @@ class RatslamRos(object):
             nat.check(nat.lib().prs_frame_set_count(plan, v._n, ctypes.c_void_p(self._f_stream.cuda_stream)),
                       "prs_frame_set_count")
         self._f_n_dev = v._n
+        v._cell_sync(self._f_stream)
+
+    # ------------------------------------------------------------------ injection inside the frame
+    _NO_INJECT = (None, None)
+
+    def _device_energy(self, strict=False):
+        """The energy the frame plans inject on the device (``prs_frame_set_inject``), None for no injection there.
+        The device node takes finite energies >= 0; another energy is injected by the host behind the frame
+        (``fused_frame``) or, ``strict``, refused (the pipelined and native replays)."""
+        en = self.inject_energy
+        if en is None:
+            return None
+        en = float(en)
+        if en >= 0 and math.isfinite(en):
+            return en
+        if strict:
+            raise ValueError("the pipelined and native replays inject on the device, which takes finite energies "
+                             ">= 0; got inject_energy=%r" % (self.inject_energy,))
+        return None
+
+    def _plan_inject(self, plan, current, energy):
+        """Point ``plan``'s injection node at ``energy`` and the library's location table (None: no node).  Returns
+        the setting, which the caller keeps beside the plan to skip the call while nothing changes."""
+        want = self._NO_INJECT if energy is None else (energy, self.vts._cell_table(self.pcn.shape).data_ptr())
+        if want != current:
+            nat.check(nat.lib().prs_frame_set_inject(plan, 0.0 if energy is None else energy, want[1]),
+                      "prs_frame_set_inject")
+        return want
+
+    def _inject_error(self, index):
+        loc = self.vts.templates[index].location()
+        return IndexError("index %r is out of bounds for shape %r" % (tuple(loc), self.pcn.shape))
 
     def _fused_plan(self):
         """(Re)create the CUDA-graph frame plan; needed again whenever the library buffer was reallocated."""
@@ -151,6 +185,7 @@ class RatslamRos(object):
             self._f_scratch.data_ptr(), self._f_odom.data_ptr(), self._f_frame.data_ptr(), self._f_res.data_ptr(),
             ctypes.byref(self._f_plan)), "prs_frame_create")
         self._f_plan_key = key
+        self._f_inj = self._NO_INJECT
         self._f_n_dev = v._n
 
     def __del__(self):
@@ -166,7 +201,9 @@ class RatslamRos(object):
         """``odom_callback(twist)`` + ``spin_once()`` + ``vis_callback(im)`` in one device round trip.
 
         Returns ``(template_index, created)``.  Same decisions as the three separate calls; a pose-cell
-        error (LUT hole, oversize shift) is raised after the frame instead of before it."""
+        error (LUT hole, oversize shift) is raised after the frame instead of before it.  With ``inject_energy >= 0``
+        the injection at the template's stored cell is the frame's last node on the device; a location outside the
+        grid raises ``IndexError`` after the frame, the pose cells untouched."""
         if not getattr(self, "_fused_ready", False):
             self._fused_setup()
         e, v = self.pcn._ens, self.vts
@@ -178,17 +215,21 @@ class RatslamRos(object):
             o[0], o[1] = vtrans, vrot
         v._grow(v._n + 2)
         self._fused_plan()
+        energy = self._device_energy()
+        self._f_inj = self._plan_inject(self._f_plan, self._f_inj, energy)
         self._fused_resync(self._f_plan)
         self._f_frame.numpy()[...] = im
         nat.check(nat.lib().prs_frame_run(self._f_plan, 1 if moved else 0, ctypes.c_void_p(self._f_stream.cuda_stream)),
                   "prs_frame_run")
         r = self._f_result
+        err = int(r.pc_err)
         if moved:
-            e._raise_on_err(np.array([r.pc_err], dtype=np.int32))
+            e._raise_on_err(np.array([err & ~nat.ERR_INJECT_LOC], dtype=np.int32))
         X, Y, Th = self.pcn.shape
         flat = int(r.argmax)
         pc_max = (flat // (Y * Th), (flat // Th) % Y, flat % Th)
-        self.pcn.max_pc, self.pcn._max_valid = pc_max, True
+        # the record holds the arg-max the match was made with; after an injection the state has moved on
+        self.pcn.max_pc, self.pcn._max_valid = pc_max, energy is None
         if moved:
             self._em_update(vtrans, vrot, pc_max)                                          # :136-137
             self.published_pose.append(self.em.get_current_point())
@@ -196,7 +237,12 @@ class RatslamRos(object):
             v._loc[v._n] = pc_max
         v._n = self._f_n_dev = int(r.n_templates)
         v.last_score = None if r.key == (1 << 64) - 1 else int(r.key >> 32)
-        if self.inject_energy is not None:
+        if energy is not None:
+            v._cell_n = v._n                 # the created template's row was written on the device
+            self._f_gen = e._state_gen       # the node kept the cached arg-max (_f_pcwork) current
+            if err & nat.ERR_INJECT_LOC:
+                raise self._inject_error(int(r.template_index))
+        elif self.inject_energy is not None:  # an energy the device node does not take: the host injects
             loc = tuple(int(c) for c in v._loc[int(r.template_index)])
             with torch.cuda.stream(self._f_stream):
                 self.pcn.inject(self.inject_energy, loc)
@@ -223,7 +269,8 @@ class RatslamRos(object):
             res = torch.zeros(32, dtype=torch.uint8).pin_memory()
             self._p_slots.append({"frame": frame, "frame_np": frame.numpy(), "odom": odom, "odom_np": odom.numpy(),
                                   "res": res, "result": nat.FrameResult.from_address(res.data_ptr()),
-                                  "plan": ctypes.c_void_p(), "event": torch.cuda.Event(), "meta": None})
+                                  "plan": ctypes.c_void_p(), "inj": self._NO_INJECT, "event": torch.cuda.Event(),
+                                  "meta": None})
         self._p_key = None
         self._p_inflight = 0
 
@@ -244,15 +291,19 @@ class RatslamRos(object):
                 v._capacity, thr, v.mode, v.im_x, v.im_y, v.y_range[0], v.y_range[1], v.y_step, v.x_range[0],
                 v.x_range[1], v.x_step, self._f_scratch.data_ptr(), sl["odom"].data_ptr(), sl["frame"].data_ptr(),
                 sl["res"].data_ptr(), ctypes.byref(sl["plan"])), "prs_frame_create")
+            sl["inj"] = self._NO_INJECT
         self._p_key = key
         self._f_n_dev = v._n
 
     def pipe_submit(self, slot, twist, im):
         """Stage and launch one frame in ``slot`` (0 or 1) without waiting for it; ``pipe_finish(slot)`` returns its
-        ``(template_index, created)``.  The previous frame of the same slot must have been finished."""
+        ``(template_index, created)``.  The previous frame of the same slot must have been finished.  ``inject_energy``
+        must be None or a finite energy >= 0 (``ValueError``): the injection is the frame's last node on the device."""
         v = self.vts
         sl = self._p_slots[slot]
         assert sl["meta"] is None, "slot still in flight"
+        energy = self._device_energy(strict=True)
+        sl["inj"] = self._plan_inject(sl["plan"], sl["inj"], energy)
         if v._n + self._p_inflight + 2 > v._capacity:   # growing reallocates the library: drain, grow, re-plan
             raise RuntimeError("pipe_submit: library full; finish the frames in flight and call pipe_grow()")
         moved = twist is not None and (abs(twist[0]) > 0.001 or abs(twist[1]) > 0.001)   # ros_simulate.py:128
@@ -266,7 +317,7 @@ class RatslamRos(object):
         nat.check(nat.lib().prs_frame_launch(sl["plan"], 1 if moved else 0, ctypes.c_void_p(self._f_stream.cuda_stream)),
                   "prs_frame_launch")
         sl["event"].record(self._f_stream)
-        sl["meta"] = (moved, vtrans, vrot)
+        sl["meta"] = (moved, vtrans, vrot, energy is not None)
         self._p_inflight += 1
 
     def pipe_needs_grow(self):
@@ -280,25 +331,30 @@ class RatslamRos(object):
     def pipe_finish(self, slot):
         e, v = self.pcn._ens, self.vts
         sl = self._p_slots[slot]
-        moved, vtrans, vrot = sl["meta"]
+        moved, vtrans, vrot, injected = sl["meta"]
         sl["event"].synchronize()
         sl["meta"] = None
         self._p_inflight -= 1
         r = sl["result"]
+        err = int(r.pc_err)
         if moved:
-            e._raise_on_err(np.array([r.pc_err], dtype=np.int32))
+            e._raise_on_err(np.array([err & ~nat.ERR_INJECT_LOC], dtype=np.int32))
         X, Y, Th = self.pcn.shape
         flat = int(r.argmax)
         pc_max = (flat // (Y * Th), (flat // Th) % Y, flat % Th)
-        self.pcn.max_pc, self.pcn._max_valid = pc_max, self._p_inflight == 0
+        self.pcn.max_pc, self.pcn._max_valid = pc_max, self._p_inflight == 0 and not injected
         if moved:
             self._em_update(vtrans, vrot, pc_max)                                          # :136-137
             self.published_pose.append(self.em.get_current_point())
         if r.created:
             v._loc[int(r.n_templates) - 1] = pc_max
         v._n = self._f_n_dev = int(r.n_templates)
+        if injected:
+            v._cell_n = v._n                 # the created template's row was written on the device
         self._f_gen = e._state_gen
         v.last_score = None if r.key == (1 << 64) - 1 else int(r.key >> 32)
+        if injected and err & nat.ERR_INJECT_LOC:
+            raise self._inject_error(int(r.template_index))
         self.published_index.append(int(r.template_index))
         return int(r.template_index), bool(r.created)
 
@@ -311,9 +367,10 @@ class RatslamRos(object):
         staging, graph launches and result collection happen in C with ``n_plans`` frames in flight (two already hide the host); the host-side
         bookkeeping (experience map, template locations) is replayed from the returned records afterwards.
         Returns the structured result array (one ``prs_frame_result`` per frame).  Same decisions as the
-        frame-by-frame calls; a pose-cell error is raised for the first offending frame after the batch."""
-        if self.inject_energy is not None:
-            raise ValueError("replay_native does not support inject_energy (the injection needs the match first)")
+        frame-by-frame calls; a pose-cell error is raised for the first offending frame after the batch, and so is the
+        ``IndexError`` of a template location outside the grid.  ``inject_energy`` must be None or a finite energy >= 0
+        (``ValueError``): the injection is every frame's last node on the device."""
+        energy = self._device_energy(strict=True)
         frames = np.ascontiguousarray(frames, dtype=np.uint8)
         odom = np.asarray(odom, dtype=np.float64)
         T = len(frames)
@@ -325,6 +382,8 @@ class RatslamRos(object):
         assert self._p_inflight == 0
         v._grow(v._n + T + 2)
         self._pipe_plans()
+        for sl in self._p_slots:
+            sl["inj"] = self._plan_inject(sl["plan"], sl["inj"], energy)
         self._fused_resync(self._p_slots[0]["plan"])
         moved = ((np.abs(odom[:, 0]) > 0.001) | (np.abs(odom[:, 1]) > 0.001)).astype(np.uint8)    # ros_simulate.py:128
         tw = np.ascontiguousarray(odom / float(self.odom_freq))                                    # :157-158
@@ -337,11 +396,15 @@ class RatslamRos(object):
         X, Y, Th = self.pcn.shape
         flat = res["argmax"]
         amax = np.stack([flat // (Y * Th), (flat // Th) % Y, flat % Th], axis=1)
-        bad = np.nonzero((res["pc_err"] != 0) & (moved != 0))[0]
+        pc_bad = ((res["pc_err"] & ~nat.ERR_INJECT_LOC) != 0) & (moved != 0)
+        inj_bad = (res["pc_err"] & nat.ERR_INJECT_LOC) != 0 if energy is not None else np.zeros(T, np.bool_)
+        bad = np.nonzero(pc_bad | inj_bad)[0]
         stop = int(bad[0]) if len(bad) else T
+        # a pose-cell error stops before its frame, a bad template location after its frame's match (vis_callback order)
+        booked = stop + 1 if len(bad) and not pc_bad[stop] else stop
         self._native_n_exp = np.zeros(T, np.int64)       # per-frame experience count / current point, for replay()
         self._native_em_xy = np.zeros((T, 2))
-        for t in range(stop):
+        for t in range(booked):
             pc_max = (int(amax[t, 0]), int(amax[t, 1]), int(amax[t, 2]))
             if moved[t]:
                 self._em_update(float(tw[t, 0]), float(tw[t, 1]), pc_max,
@@ -356,13 +419,17 @@ class RatslamRos(object):
         if T:
             last = T - 1
             v._n = self._f_n_dev = int(res["n_templates"][last])
+            if energy is not None:
+                v._cell_n = v._n             # the created templates' rows were written on the device
             self._f_gen = e._state_gen
             self.pcn.max_pc = tuple(int(c) for c in amax[last])
-            self.pcn._max_valid = True
+            self.pcn._max_valid = energy is None     # the record's arg-max precedes the last frame's injection
             k = int(res["key"][last])
             v.last_score = None if k == (1 << 64) - 1 else k >> 32
         if len(bad):
-            e._raise_on_err(np.array([res["pc_err"][stop]], dtype=np.int32))
+            if pc_bad[stop]:
+                e._raise_on_err(np.array([res["pc_err"][stop] & ~nat.ERR_INJECT_LOC], dtype=np.int32))
+            raise self._inject_error(int(res["template_index"][stop]))
         return res
 
     # ros_simulate.py:152-166, one pass of the loop body
@@ -399,8 +466,7 @@ def replay(frames, odom, fused=False, pipelined=False, native=False, **kwargs):
         rec["node"] = node
         return rec
     if pipelined:
-        if node.inject_energy is not None:
-            raise ValueError("pipelined replay does not support inject_energy (the injection needs the match first)")
+        node._device_energy(strict=True)
         node._pipe_setup()
         node.vts._grow(64)
         node._pipe_plans()
@@ -532,6 +598,8 @@ def main(argv=None):
     ap = argparse.ArgumentParser(description="Replay a ROS1 bag through the pose-cell / view-template loop")
     ap.add_argument("bag")
     ap.add_argument("--fused", action="store_true", help="one device round trip per frame")
+    ap.add_argument("--inject-energy", type=float, default=None, metavar="E",
+                    help="inject E at the matched template's pose cell after every frame (ros_simulate.py:106-108)")
     ap.add_argument("--record", default=None, help="write template matches and experience-map points to this bag")
     ap.add_argument("--npy", default=None, help="also save frames/odom arrays as <prefix>_frames.npy, <prefix>_odom.npy")
     ap.add_argument("--image-topic", default="navbot/camera/image")
@@ -543,7 +611,7 @@ def main(argv=None):
         frames, odom, _ = rb.events_to_arrays(events)
         np.save(a.npy + "_frames.npy", frames)
         np.save(a.npy + "_odom.npy", odom)
-    out = replay_events(events, fused=a.fused, record=a.record)
+    out = replay_events(events, fused=a.fused, record=a.record, inject_energy=a.inject_energy)
     print("frames %d  templates %d  experiences %d" % (len(out["template"]), out["n_templates"],
                                                       len(out["node"].em.experiences)))
 

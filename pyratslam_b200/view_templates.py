@@ -24,6 +24,21 @@ from .sharding import decide, reduce_packed_key, unpack_key
 _KEY_NONE = (1 << 64) - 1
 
 
+def flat_cell_index(locations, shape):
+    """Template locations ``[n, 3]`` -> the C-order flat pose cell ``x*Y*Th + y*Th + th`` each one injects into, or -1
+    where ``PoseCellEnsemble.inject`` raises ``IndexError``: coordinates are truncated the way ``int()`` does, a
+    coordinate in ``[-n, 0)`` wraps like a numpy index, anything else (out of range, not finite) is -1."""
+    loc = np.asarray(locations, dtype=np.float64).reshape(-1, 3)
+    dims = np.asarray(shape, dtype=np.int64).reshape(1, 3)
+    ok = np.isfinite(loc).all(axis=1)
+    v = np.trunc(np.where(np.isfinite(loc), loc, 0.0))
+    ok &= ((v >= -dims) & (v < dims)).all(axis=1)
+    c = np.where(ok[:, None], v, 0.0).astype(np.int64)
+    c = np.where(c < 0, c + dims, c)
+    X, Y, Th = (int(s) for s in shape)
+    return np.where(ok, c[:, 0] * (Y * Th) + c[:, 1] * Th + c[:, 2], -1).astype(np.int64)
+
+
 class ViewTemplate:
     """One stored view, tied to the pose cell that was most active when it was created
     (``view_templates.py:4-37``)."""
@@ -136,8 +151,13 @@ class ViewTemplates:
         self._capacity = int(capacity)
         self._loc = np.zeros((self._capacity, 3), dtype=np.float64)
         self._loc_is_int = True
+        # the device-side twin of _loc for the frame plans' injection node: int64 [capacity] flat pose cells
+        # (flat_cell_index of a grid of shape _cell_shape), rows [0, _cell_n) in step with _loc
+        self._cell_dev = None
+        self._cell_shape = None
+        self._cell_n = 0
         self.templates = _TemplateList(self)
-        self._key = torch.empty(1, dtype=torch.int64, device=self.device)
+        self._key =torch.empty(1, dtype=torch.int64, device=self.device)
         self._key_pin = torch.empty(1, dtype=torch.int64).pin_memory()
         self._frame_dev = torch.empty((self.im_x, self.im_y), dtype=torch.uint8, device=self.device)
         self._tpl_u8 = torch.empty(tuple(self.shape), dtype=torch.uint8, device=self.device)
@@ -201,7 +221,30 @@ class ViewTemplates:
         loc = np.zeros((cap, 3), dtype=np.float64)
         loc[: self._n] = self._loc[: self._n]
         self._loc = loc
+        if self._cell_dev is not None:
+            cells = torch.full((cap,), -1, dtype=torch.int64, device=self.device)
+            cells[: self._cell_dev.numel()].copy_(self._cell_dev)
+            self._cell_dev = cells
         self._capacity = cap
+
+    def _cell_table(self, shape):
+        """The device location table for a pose-cell grid of ``shape`` (created on first use, all rows -1)."""
+        shape = tuple(int(s) for s in shape)
+        if self._cell_dev is None or self._cell_shape != shape or self._cell_dev.numel() < self._capacity:
+            self._cell_dev = torch.full((self._capacity,), -1, dtype=torch.int64, device=self.device)
+            self._cell_shape, self._cell_n = shape, 0
+        return self._cell_dev
+
+    def _cell_sync(self, stream):
+        """Copy the rows of templates appended outside the frame plans (``match`` / ``create`` / ``load_library``) into
+        the device table, on ``stream``."""
+        if self._cell_dev is None or self._cell_n >= self._n:
+            self._cell_n = min(self._cell_n, self._n)
+            return
+        rows = torch.from_numpy(flat_cell_index(self._loc[self._cell_n: self._n], self._cell_shape))
+        with torch.cuda.stream(stream):
+            self._cell_dev[self._cell_n: self._n].copy_(rows)
+        self._cell_n = self._n
 
     def _store(self, tpl_dev, first, count):
         """Write ``count`` row-major templates into slots ``first..``."""
@@ -233,6 +276,7 @@ class ViewTemplates:
         self._loc = np.zeros((self._capacity, 3), dtype=np.float64)
         if locations is not None:
             self._loc[:n] = np.asarray(locations, np.float64)
+        self._cell_dev, self._cell_n = None, 0
         self.templates = _TemplateList(self)
 
     def _append(self, tpl_dev, pc_x, pc_y, pc_th):
