@@ -370,6 +370,44 @@ PRS_API int prs_frame_set_inject(prs_frame_plan* plan, double energy, long long*
 PRS_API int prs_replay_run(prs_frame_plan* const* plans, int n_plans, const uint8_t* frames, const double* odom,
                    const uint8_t* moved, int T, prs_frame_result* results, void* stream);
 
+/* ------------------------------------------------------------ ensemble replay */
+
+/* One recording through B independent agents in one pass (a parameter sweep of the ROS loop, ros_simulate.py:98-166):
+ * agent b is network b of the pose-cell plan `pc` (B = its network count, global inhibition gi[b]) with its own packed
+ * uint8 library, match threshold and injection energy.  Frames and odometry are shared: a frame is ONE graph for the
+ * whole ensemble -- the odometry broadcast and the pose-cell update of all B networks (moved frames only) on a side
+ * branch, the query prepared once, one sweep over every agent's library, then per agent the create-or-match decision
+ * (a created template goes into slot n_dev[b] of its library, its location row loc_dev[b][n] receives the agent's
+ * arg-max) and the injection of prs_frame_set_inject.  Agent b's records equal a single-agent frame plan's with
+ * threshold_dev[b], gi[b] and energy_dev[b].  Reference mode (PRS_VT_MODE_REF) only; PRS_E_INVALID otherwise.
+ *   pc_work       : device, B * 24 bytes: int64 arg-max [B], total [B] (8-byte slots), int32 err [B]; the arg-max must
+ *                   hold each network's current arg-max (prs_pc_argmax) before the first frame
+ *   libs          : device, B libraries of prs_vt_packed_bytes(capacity) bytes each, zero-filled once
+ *   capacity      : templates per library, at most 65536
+ *   n_dev         : device int32 [B], templates in each library; updated by every frame
+ *   threshold_dev : device uint32 [B], the match thresholds (clamped to [0, 2^32-1] by the caller)
+ *   energy_dev    : device double [B], energy injected at the frame template's cell; a value that is not >= 0 (e.g. -1)
+ *                   means no injection for that agent; NULL: no injection node at all
+ *   loc_dev       : device int64 [B][capacity], C-order flat cell of every template, -1 = invalid
+ *   scratch       : device, prs_ens_scratch_bytes(B, im_rows, im_cols); private to the plan
+ * The plan keeps pointers to all of these; they must outlive it. */
+typedef struct prs_ens_plan prs_ens_plan;
+PRS_API size_t prs_ens_scratch_bytes(int B, int im_rows, int im_cols);
+PRS_API int prs_ens_create(prs_pc_handle pc, void* pc_state, const void* gi, void* pc_work, void* libs, int capacity,
+                   int* n_dev, const unsigned* threshold_dev, const double* energy_dev, long long* loc_dev, int mode,
+                   int im_rows, int im_cols, int row_lo, int row_hi, int row_step, int col_lo, int col_hi,
+                   int col_step, void* scratch, prs_ens_plan** out);
+PRS_API int prs_ens_destroy(prs_ens_plan* plan);
+/* The loop of prs_replay_run for the ensemble.  Frames and odometry go to the device and the records come back in
+ * chunks of 256 frames; nothing per agent crosses the bus per frame.  Returns after one final synchronisation of
+ * `stream` (a non-default stream).  PRS_E_INVALID when the libraries have no room for T more templates.
+ *   frames : host uint8 [T][im_rows][im_cols]     odom : host double [T][2] = (vtrans, vrot) as given to update()
+ *   moved  : host uint8 [T], 0 = no pose-cell update for this frame (the 0.001 twist gate, ros_simulate.py:128)
+ *   results: host prs_frame_result [T][B]; pc_err holds the err bits of the last update (valid on moved frames) and
+ *            PRS_ERR_INJECT_LOC */
+PRS_API int prs_ens_replay_run(prs_ens_plan* plan, const uint8_t* frames, const double* odom, const uint8_t* moved, int T,
+                       prs_frame_result* results, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

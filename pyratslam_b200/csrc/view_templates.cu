@@ -1246,30 +1246,48 @@ struct FrameScratch {               // device scratch layout (bytes)
   static constexpr size_t kBytes = kOdom + 64;
 };
 
+// Per-agent layout of the ensemble frame (prs_ens_*): B agents share the query, each has its own library, template
+// count, threshold, location table and pose-cell network.  The default is the single-agent frame (B = 1, no strides).
+struct VtAgents {
+  int B = 1;
+  long long lib_u4 = 0;                 // uint4 per agent library
+  const unsigned* threshold = nullptr;  // [B]; null: the kernel's scalar threshold
+  long long* loc = nullptr;             // [B][loc_stride]: a created template's row receives the agent's arg-max
+  long long loc_stride = 0;
+  int* g_max = nullptr;                 // largest group count over the agents, raised by the decision (the sweep's grid)
+  const int* ctr = nullptr;             // frame index within the record chunk: the agent's record is res[*ctr * B + b]
+};
+
+// One warp per agent (b = global warp index), lane t packs row t of a created template.
 // dec (optional): a second, device-side copy of the decision (created, template_index, n_templates) for the frame's
 // injection node when `res` is the pinned host record
 __global__ void k_vt_decide_append(const unsigned long long* __restrict__ key, const uint8_t* __restrict__ tpl,
                                    uint4* __restrict__ packed, int n, unsigned threshold,
                                    const long long* __restrict__ argmax, const int* __restrict__ pc_err,
                                    prs_frame_result* __restrict__ res, int* __restrict__ n_dev, int write_pc = 1,
-                                   prs_frame_result* __restrict__ dec = nullptr) {
-  const int t = threadIdx.x;  // 32 threads, one per template row
-  if (n_dev != nullptr) n = *n_dev;
+                                   prs_frame_result* __restrict__ dec = nullptr, VtAgents ag = VtAgents()) {
+  const int b = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 5), t = threadIdx.x & 31;
+  if (b >= ag.B) return;  // whole warps
+  if (n_dev != nullptr) n = n_dev[b];
   __syncwarp();
-  const unsigned long long k = *key;
+  const unsigned long long k = key[b];
   const unsigned score = (unsigned)(k >> 32);
+  if (ag.threshold != nullptr) threshold = ag.threshold[b];
   const bool create = (n == 0) || (k == ~0ull) || (score > threshold);  // strict '>' (view_templates.py:67)
   if (create) {
-    vt_pack_row(tpl, packed, n, t);
+    vt_pack_row(tpl, packed + b * ag.lib_u4, n, t);
   }
   if (t == 0) {
-    if (write_pc) res->argmax = argmax ? argmax[0] : -1;  // else the pose-cell kernel writes both fields itself
+    res += (ag.ctr != nullptr ? (long long)*ag.ctr * ag.B : 0) + b;
+    if (write_pc) res->argmax = argmax ? argmax[b] : -1;  // else the pose-cell kernel writes both fields itself
     res->key = k;
     res->created = create ? 1 : 0;
     res->template_index = create ? n : (int)(k & 0xffffffffu);
     res->n_templates = n + (create ? 1 : 0);
-    if (write_pc) res->pc_err = pc_err ? pc_err[0] : 0;
-    if (n_dev != nullptr) *n_dev = n + (create ? 1 : 0);
+    if (write_pc) res->pc_err = pc_err ? pc_err[b] : 0;
+    if (n_dev != nullptr) n_dev[b] = n + (create ? 1 : 0);
+    if (create && ag.loc != nullptr) ag.loc[b * ag.loc_stride + n] = argmax[b];
+    if (create && ag.g_max != nullptr) atomicMax(ag.g_max, (n + 32) >> 5);  // groups of n + 1 templates
     if (dec != nullptr) {
       dec->created = create ? 1 : 0;
       dec->template_index = create ? n : (int)(k & 0xffffffffu);
@@ -1294,12 +1312,28 @@ __device__ __forceinline__ size_t pc_theta_major(I f, I X, I Y, I Th) {  // [x][
   return ((size_t)th * X + x) * Y + y;
 }
 
+// Ensemble frames (energies != null): one thread per agent b with its own network, table row stride, record and
+// energies[b]; an energy that is not >= 0 (the ensemble's "no injection") leaves agent b alone.
 template <typename T>
 __global__ void k_frame_inject(T* __restrict__ state, long long* __restrict__ loc, const prs_frame_result* dec,
                                long long* __restrict__ argmax, const int* __restrict__ pc_err, prs_frame_result* res,
-                               int X, int Y, int Th, T energy) {
-  if (threadIdx.x != 0) return;
+                               int X, int Y, int Th, T energy, const double* __restrict__ energies = nullptr,
+                               VtAgents ag = VtAgents()) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= ag.B) return;
   const long long N = (long long)X * Y * Th;
+  if (energies != nullptr) {
+    const double e = energies[b];
+    if (!(e >= 0.0)) return;
+    energy = (T)e;
+    const long long r = (ag.ctr != nullptr ? (long long)*ag.ctr * ag.B : 0) + b;
+    dec += r;
+    res += r;
+    state += b * N;
+    loc += b * ag.loc_stride;
+    argmax += b;
+    pc_err += b;
+  }
   const bool narrow = N <= 0xffffffffLL;
   auto offset = [&](long long f) {
     return narrow ? pc_theta_major<unsigned>((unsigned)f, X, Y, Th) : pc_theta_major<long long>(f, X, Y, Th);
@@ -1451,9 +1485,14 @@ constexpr int kSmallLibrary = 1 << 16;
 
 __global__ void __launch_bounds__(1024)
     k_vt_frame_prepare(const uint8_t* __restrict__ frame, int im_cols, int row_lo, int row_step, int col_lo, int col_step,
-                       uint8_t* __restrict__ tpl, uint32_t* __restrict__ planes, unsigned long long* __restrict__ key) {
+                       uint8_t* __restrict__ tpl, uint32_t* __restrict__ planes, unsigned long long* __restrict__ key,
+                       const int* __restrict__ ctr = nullptr, long long frame_bytes = 0, int n_keys = 1) {
+  // ctr (ensemble frames): the frame is number *ctr of a device-side chunk of frames `frame_bytes` apart; the n_keys
+  // agents' keys are reset
   __shared__ uint32_t s_sum[32];
   const int t = threadIdx.x >> 5, c = threadIdx.x & 31;  // template row, column
+  if (ctr != nullptr) frame += *ctr * frame_bytes;
+  for (int i = (int)threadIdx.x; i < n_keys; i += 1024) key[i] = ~0ull;
   const int rr = row_lo + (t / (row_step - 1)) * row_step + (t % (row_step - 1)) + 1;
   const int cc = col_lo + (c / (col_step - 1)) * col_step + (c % (col_step - 1)) + 1;
   const uint32_t px = frame[(size_t)rr * im_cols + cc];
@@ -1480,7 +1519,6 @@ __global__ void __launch_bounds__(1024)
     if (c == 0) {
       planes[256] = mid;
       planes[257] = all;
-      *key = ~0ull;
     }
   }
 }
@@ -1503,22 +1541,29 @@ __device__ __forceinline__ uint32_t lt_row_q(const uint4& lo, const uint4& hi, c
 // and the per-offset counts meet in shared memory (integer adds: exact, order-free).
 constexpr int kSmallThreads = 512;
 
+// Ensemble frames: n_agents libraries of lib_u4 uint4 each, agent b's live count n_dev[b] and key key_out[b].  The
+// blocks grid-stride over (agent, group) items, G = *g_max groups per agent (the largest live group count, kept by the
+// decision kernel); an item past its agent's live count is skipped, so the work follows sum_b n_b, not the capacity.
 __global__ void __launch_bounds__(kSmallThreads)
     k_vt_sweep_packed_ref_small(const uint4* __restrict__ packed, const uint32_t* __restrict__ qplanes,
-                                unsigned long long* __restrict__ key_out, const int* __restrict__ n_dev) {
+                                unsigned long long* __restrict__ key_out, const int* __restrict__ n_dev,
+                                int n_agents = 1, long long lib_u4 = 0, const int* __restrict__ g_max = nullptr) {
   __shared__ uint32_t q[32 * 8 + 8];
   __shared__ uint32_t s_cnt[15][32];
   __shared__ uint32_t s_A[15][32];
-  const long long n = *n_dev;
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-  const long long n_groups = (n + 31) >> 5;
-  if ((long long)blockIdx.x >= n_groups) return;  // the grid is laid out for the capacity, not the live count
+  const long long G = g_max != nullptr ? (long long)*g_max : ((long long)*n_dev + 31) >> 5;
+  const long long items = G * n_agents;
+  if ((long long)blockIdx.x >= items) return;  // the grid is laid out for the capacity, not the live count
   for (int i = threadIdx.x; i < 32 * 8 + 2; i += kSmallThreads) q[i] = qplanes[i];
-  unsigned long long best = ~0ull;
-  for (long long g = blockIdx.x; g < n_groups; g += gridDim.x) {
+  for (long long item = blockIdx.x; item < items; item += gridDim.x) {
+    const int b = (int)(item / G);
+    const long long g = item - b * G;
+    const long long n = n_dev[b];
+    if (g * 32 >= n) continue;  // block-uniform
     if (threadIdx.x < 15 * 32) s_cnt[wid][lane] = 0;
     __syncthreads();  // also publishes q on the first pass
-    const uint4* gp = packed + g * kGroupU4 + lane;
+    const uint4* gp = packed + b * lib_u4 + g * kGroupU4 + lane;
     if (wid < 15) {
       const int t0 = 2 * wid + 1;
       const uint4 lo0 = ld_stream_u4(gp + (t0 * 2 + 0) * 32), hi0 = ld_stream_u4(gp + (t0 * 2 + 1) * 32);
@@ -1559,16 +1604,11 @@ __global__ void __launch_bounds__(kSmallThreads)
 #pragma unroll
       for (int o = 0; o < 15; ++o) m = min(m, s_A[o][lane] + 256u * s_cnt[o][lane] - bq);
       const long long ti = g * 32 + lane;
-      if (ti < n) {
-        const unsigned long long key = ((unsigned long long)m << 32) | (unsigned long long)ti;
-        best = key < best ? key : best;
-      }
+      unsigned long long best = ti < n ? ((unsigned long long)m << 32) | (unsigned long long)ti : ~0ull;
+      best = warp_min_u64(best);
+      if (lane == 0) atomicMin(key_out + b, best);
     }
     __syncthreads();
-  }
-  if (wid == 0) {
-    best = warp_min_u64(best);
-    if (lane == 0 && best != ~0ull) atomicMin(key_out, best);
   }
 }
 
@@ -1847,6 +1887,255 @@ extern "C" int prs_replay_run(prs_frame_plan* const* plans, int n_plans, const u
       return PRS_E_CUDA;
     }
     results[t] = *f->result_host;
+  }
+  return rc;
+}
+
+// ---------------------------------------------------------------------------------------------
+// Ensemble replay: one recording through B agents, each with its own pose-cell network (the B networks of one plan),
+// view-template library, threshold and injection energy.  The frames and the odometry are shared, so a frame is ONE
+// graph for the whole ensemble:
+//   side branch (moved frames)  k_ens_odom broadcasts the frame's (vtrans, vrot) into odom[B][2] -> prs_pc_step
+//   template branch             k_vt_frame_prepare (once: the query is the same for every agent) ->
+//                               k_vt_sweep_packed_ref_small over every agent's library (grid-stride over (agent, group))
+//   join                        k_vt_decide_append, one warp per agent -> [k_frame_inject, one thread per agent] ->
+//                               k_ens_advance (the device-side frame counter)
+// Frames and odometry go to the device a chunk at a time, the records [chunk][B] come back a chunk at a time.
+constexpr int kEnsChunk = 256;
+
+struct EnsScratch {  // device scratch layout of an ensemble plan (bytes), every part 256-byte aligned
+  size_t frames, odom_chunk, rec, odom, key, tpl, planes, misc, bytes;
+  EnsScratch(int B, long long fbytes) {
+    auto up = [](size_t v) { return (v + 255) & ~(size_t)255; };
+    frames = 0;
+    odom_chunk = frames + up((size_t)kEnsChunk * fbytes);
+    rec = odom_chunk + up((size_t)kEnsChunk * 2 * sizeof(double));
+    odom = rec + up((size_t)kEnsChunk * B * sizeof(prs_frame_result));
+    key = odom + up((size_t)B * 2 * sizeof(double));
+    tpl = key + up((size_t)B * sizeof(unsigned long long));
+    planes = tpl + 1024;
+    misc = planes + 2048;  // int frame counter, int group maximum, int largest live count
+    bytes = misc + 256;
+  }
+};
+
+__global__ void k_ens_odom(const double* __restrict__ odom_chunk, const int* __restrict__ ctr, double* __restrict__ odom,
+                           int B) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  const int t = *ctr;
+  odom[2 * b] = odom_chunk[2 * t];
+  odom[2 * b + 1] = odom_chunk[2 * t + 1];
+}
+
+__global__ void k_ens_advance(int* ctr) { ++*ctr; }
+
+// group maximum and largest live count of the libraries a plan starts from
+__global__ void k_ens_init(const int* __restrict__ n_dev, int B, int* __restrict__ misc) {
+  for (int b = threadIdx.x; b < B; b += blockDim.x) {
+    atomicMax(misc + 1, (n_dev[b] + 31) >> 5);
+    atomicMax(misc + 2, n_dev[b]);
+  }
+}
+
+struct prs_ens_plan {
+  prs_pc_handle pc;
+  void *pc_state, *pc_work, *libs;
+  const void* gi;
+  int* n_dev;
+  const unsigned* thr_dev;
+  const double* energy_dev;
+  long long* loc_dev;
+  int B, capacity;
+  long long lib_u4, fbytes, room;  // room: frames the libraries can still take (one template per agent and frame)
+  int im_cols, row_lo, row_step, col_lo, col_step;
+  char* scratch;
+  EnsScratch lay;
+  cudaGraphExec_t exec[2];
+  bool ready[2];
+  int warm[2];
+  cudaStream_t side;
+  cudaEvent_t ev_fork, ev_join;
+};
+
+static int ens_enqueue(prs_ens_plan* e, bool moved, cudaStream_t st) {
+  char* sc = e->scratch;
+  const EnsScratch& L = e->lay;
+  long long* d_argmax = (long long*)e->pc_work;
+  void* d_total = (char*)e->pc_work + 8 * (size_t)e->B;
+  int* d_err = (int*)((char*)e->pc_work + 16 * (size_t)e->B);
+  int* d_ctr = (int*)(sc + L.misc);
+  int* d_gmax = d_ctr + 1;
+  double* d_odom = (double*)(sc + L.odom);
+  unsigned long long* d_key = (unsigned long long*)(sc + L.key);
+  prs_frame_result* d_rec = (prs_frame_result*)(sc + L.rec);
+  const int B = e->B;
+  int rc;
+  if (moved) {  // fork: the pose-cell update does not depend on the frame until the decision
+    PRS_CUDA(cudaEventRecord(e->ev_fork, st));
+    PRS_CUDA(cudaStreamWaitEvent(e->side, e->ev_fork, 0));
+    k_ens_odom<<<(B + 255) / 256, 256, 0, e->side>>>((const double*)(sc + L.odom_chunk), d_ctr, d_odom, B);
+    PRS_CUDA(cudaGetLastError());
+    rc = prs_pc_step(e->pc, e->pc_state, d_odom, e->gi, d_argmax, d_total, d_err, e->side);
+    if (rc != PRS_OK) return rc;
+    PRS_CUDA(cudaEventRecord(e->ev_join, e->side));
+  }
+  k_vt_frame_prepare<<<1, 1024, 0, st>>>((const uint8_t*)(sc + L.frames), e->im_cols, e->row_lo, e->row_step, e->col_lo,
+                                         e->col_step, (uint8_t*)(sc + L.tpl), (uint32_t*)(sc + L.planes), d_key, d_ctr,
+                                         e->fbytes, B);
+  long long blocks = (long long)B * ((e->capacity + 31) / 32);
+  if (blocks > 148LL * 4) blocks = 148LL * 4;
+  k_vt_sweep_packed_ref_small<<<(int)blocks, kSmallThreads, 0, st>>>((const uint4*)e->libs, (const uint32_t*)(sc + L.planes),
+                                                                     d_key, e->n_dev, B, e->lib_u4, d_gmax);
+  if (moved) PRS_CUDA(cudaStreamWaitEvent(st, e->ev_join, 0));  // the decision reports the new arg-max
+  VtAgents ag;
+  ag.B = B;
+  ag.lib_u4 = e->lib_u4;
+  ag.threshold = e->thr_dev;
+  ag.loc = e->loc_dev;
+  ag.loc_stride = e->capacity;
+  ag.g_max = d_gmax;
+  ag.ctr = d_ctr;
+  k_vt_decide_append<<<(B + 3) / 4, 128, 0, st>>>(d_key, (const uint8_t*)(sc + L.tpl), (uint4*)e->libs, 0, 0u, d_argmax,
+                                                  d_err, d_rec, e->n_dev, 1, nullptr, ag);
+  PRS_CUDA(cudaGetLastError());
+  if (e->energy_dev) {
+    prs_pc_plan* pc = e->pc;
+    if (int rc_ = prs_pc_active_invalidate(pc, st)) return rc_;  // as prs_pc_inject: the carried lists are stale
+    if (pc->dtype == PRS_F32)
+      k_frame_inject<float><<<(B + 127) / 128, 128, 0, st>>>((float*)e->pc_state, e->loc_dev, d_rec, d_argmax, d_err, d_rec,
+                                                             pc->X, pc->Y, pc->Th, 0.0f, e->energy_dev, ag);
+    else
+      k_frame_inject<double><<<(B + 127) / 128, 128, 0, st>>>((double*)e->pc_state, e->loc_dev, d_rec, d_argmax, d_err,
+                                                              d_rec, pc->X, pc->Y, pc->Th, 0.0, e->energy_dev, ag);
+    PRS_CUDA(cudaGetLastError());
+  }
+  k_ens_advance<<<1, 1, 0, st>>>(d_ctr);
+  PRS_CUDA(cudaGetLastError());
+  return PRS_OK;
+}
+
+extern "C" size_t prs_ens_scratch_bytes(int B, int im_rows, int im_cols) {
+  if (B < 1 || im_rows < 1 || im_cols < 1) return 0;
+  return EnsScratch(B, (long long)im_rows * im_cols).bytes;
+}
+
+extern "C" int prs_ens_create(prs_pc_handle pc, void* pc_state, const void* gi, void* pc_work, void* libs, int capacity,
+                              int* n_dev, const unsigned* threshold_dev, const double* energy_dev, long long* loc_dev,
+                              int mode, int im_rows, int im_cols, int row_lo, int row_hi, int row_step, int col_lo,
+                              int col_hi, int col_step, void* scratch, prs_ens_plan** out) {
+  PRS_REQUIRE(pc && pc_state && gi && pc_work && libs && n_dev && threshold_dev && loc_dev && scratch && out,
+              "prs_ens_create: null argument");
+  PRS_REQUIRE(mode == PRS_VT_MODE_REF, "prs_ens_create: only the reference mode (PRS_VT_MODE_REF) is supported, got %d",
+              mode);
+  PRS_REQUIRE(capacity >= 1 && capacity <= kSmallLibrary, "prs_ens_create: capacity %d outside [1, %d]", capacity,
+              kSmallLibrary);
+  PRS_REQUIRE(im_rows >= 1 && im_cols >= 1 && (size_t)im_rows * im_cols <= (1u << 20),
+              "prs_ens_create: frame must be 1 byte to 1 MiB");
+  if (int rc = check_mask(im_rows, im_cols, row_lo, row_hi, row_step, col_lo, col_hi, col_step, 32, 32)) return rc;
+  if (int rc = prs_pc_check_device(pc, "prs_ens_create")) return rc;
+  const int B = pc->B;
+  prs_ens_plan* e = new (std::nothrow) prs_ens_plan{pc, pc_state, pc_work, libs, gi, n_dev, threshold_dev, energy_dev,
+                                                     loc_dev, B, capacity, (long long)(prs_vt_packed_bytes(capacity) / 16),
+                                                     (long long)im_rows * im_cols, 0, im_cols, row_lo, row_step, col_lo,
+                                                     col_step, (char*)scratch, EnsScratch(B, (long long)im_rows * im_cols),
+                                                     {nullptr, nullptr}, {false, false}, {0, 0}, nullptr, nullptr, nullptr};
+  PRS_REQUIRE(e, "prs_ens_create: out of host memory");
+  int* misc = (int*)(e->scratch + e->lay.misc);
+  int init[3] = {0, 0, 0};
+  cudaError_t err = cudaStreamCreateWithFlags(&e->side, cudaStreamNonBlocking);
+  if (err == cudaSuccess) err = cudaEventCreateWithFlags(&e->ev_fork, cudaEventDisableTiming);
+  if (err == cudaSuccess) err = cudaEventCreateWithFlags(&e->ev_join, cudaEventDisableTiming);
+  if (err == cudaSuccess) err = cudaMemcpy(misc, init, sizeof(init), cudaMemcpyHostToDevice);
+  if (err == cudaSuccess) {
+    k_ens_init<<<1, 256>>>(n_dev, B, misc);
+    err = cudaGetLastError();
+  }
+  if (err == cudaSuccess) err = cudaMemcpy(init, misc, sizeof(init), cudaMemcpyDeviceToHost);
+  if (err != cudaSuccess) {
+    prs_set_error("prs_ens_create: %s", cudaGetErrorString(err));
+    prs_ens_destroy(e);
+    return PRS_E_CUDA;
+  }
+  e->room = (long long)capacity - init[2];
+  *out = e;
+  return PRS_OK;
+}
+
+extern "C" int prs_ens_destroy(prs_ens_plan* e) {
+  if (e) {
+    for (int i = 0; i < 2; ++i)
+      if (e->ready[i]) cudaGraphExecDestroy(e->exec[i]);
+    if (e->side) cudaStreamDestroy(e->side);
+    if (e->ev_fork) cudaEventDestroy(e->ev_fork);
+    if (e->ev_join) cudaEventDestroy(e->ev_join);
+    delete e;
+  }
+  return PRS_OK;
+}
+
+// One frame of the ensemble: the first call of each kind runs eagerly (lazily initialised kernel attributes), the
+// second captures the graph, later ones replay it.
+static int ens_launch(prs_ens_plan* e, int moved, cudaStream_t st) {
+  const int v = moved ? 1 : 0;
+  if (e->ready[v]) {
+    PRS_CUDA(cudaGraphLaunch(e->exec[v], st));
+    return PRS_OK;
+  }
+  if (e->warm[v] < 1) {
+    ++e->warm[v];
+    return ens_enqueue(e, moved != 0, st);
+  }
+  cudaGraph_t g = nullptr;
+  PRS_CUDA(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
+  int rc = ens_enqueue(e, moved != 0, st);
+  cudaError_t err = cudaStreamEndCapture(st, &g);
+  if (rc != PRS_OK || err != cudaSuccess) {
+    if (g) cudaGraphDestroy(g);
+    if (rc == PRS_OK) prs_set_error("prs_ens_replay_run: capture failed: %s", cudaGetErrorString(err));
+    return rc != PRS_OK ? rc : PRS_E_CUDA;
+  }
+  err = cudaGraphInstantiate(&e->exec[v], g, 0);
+  cudaGraphDestroy(g);
+  PRS_CUDA(err);
+  e->ready[v] = true;
+  PRS_CUDA(cudaGraphLaunch(e->exec[v], st));
+  return PRS_OK;
+}
+
+extern "C" int prs_ens_replay_run(prs_ens_plan* e, const uint8_t* frames, const double* odom, const uint8_t* moved, int T,
+                                  prs_frame_result* results, void* stream) {
+  PRS_REQUIRE(e && T >= 0 && (T == 0 || (frames && odom && moved && results)), "prs_ens_replay_run: bad argument");
+  PRS_REQUIRE(stream != nullptr, "prs_ens_replay_run: needs a non-default stream (the frames replay as CUDA graphs)");
+  PRS_REQUIRE(T <= e->room, "prs_ens_replay_run: %d frames do not fit the libraries (room for %lld more templates)", T,
+              e->room);
+  if (int rc = prs_pc_check_device(e->pc, "prs_ens_replay_run")) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  char* sc = e->scratch;
+  const EnsScratch& L = e->lay;
+  const size_t rec_bytes = (size_t)e->B * sizeof(prs_frame_result);
+  int rc = PRS_OK;
+  for (int c0 = 0; c0 < T && rc == PRS_OK; c0 += kEnsChunk) {
+    const int n = T - c0 < kEnsChunk ? T - c0 : kEnsChunk;
+    PRS_CUDA(cudaMemcpyAsync(sc + L.frames, frames + (size_t)c0 * e->fbytes, (size_t)n * e->fbytes,
+                             cudaMemcpyHostToDevice, st));
+    PRS_CUDA(cudaMemcpyAsync(sc + L.odom_chunk, odom + 2 * (size_t)c0, (size_t)n * 2 * sizeof(double),
+                             cudaMemcpyHostToDevice, st));
+    PRS_CUDA(cudaMemsetAsync(sc + L.misc, 0, sizeof(int), st));  // the frame counter
+    int done = 0;
+    for (; done < n; ++done) {
+      rc = ens_launch(e, moved[c0 + done], st);
+      if (rc != PRS_OK) break;
+    }
+    if (done > 0)
+      PRS_CUDA(cudaMemcpyAsync(results + (size_t)c0 * e->B, sc + L.rec, (size_t)done * rec_bytes, cudaMemcpyDeviceToHost,
+                               st));
+    e->room -= done;
+  }
+  const cudaError_t err = cudaStreamSynchronize(st);
+  if (rc == PRS_OK && err != cudaSuccess) {
+    prs_set_error("prs_ens_replay_run: %s", cudaGetErrorString(err));
+    return PRS_E_CUDA;
   }
   return rc;
 }

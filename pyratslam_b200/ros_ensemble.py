@@ -1,0 +1,266 @@
+"""One recording through B differently parameterised RatSLAM agents in one pass on the GPU.
+
+Tuning RatSLAM offline means replaying one recording under many settings -- the match threshold, the global inhibition,
+the view-template -> pose-cell injection energy -- and comparing the runs.  ``replay_ensemble`` runs all of them at
+once: agent ``b`` is the ROS loop of ``ros_simulate.replay(native=True, match_threshold=..., inject_energy=...)`` with
+``pcn.global_inhibition`` set to its own value, and it has its own pose-cell network, view-template library and
+experience map.  The frames and the odometry are shared, so a frame is one CUDA graph for the whole ensemble
+(``prs_ens_replay_run``, csrc/view_templates.cu): one pose-cell update of all B networks, one query, one sweep over
+every agent's library, then the per-agent create-or-match decision and injection.
+
+    python -m pyratslam_b200.ros_ensemble BAG --match-threshold 30000,45000,60000 --global-inhibition 0.1,0.2
+"""
+from __future__ import annotations
+
+import ctypes
+import itertools
+import math
+import numbers
+
+import numpy as np
+import torch
+
+from . import _native as nat
+from .experience_map import ExperienceMap
+from .kernels import PC_GLOBAL_INHIB
+from .posecell_network import PoseCellEnsemble, _as_np_dtype
+from .ros_simulate import IM_SIZE, MATCH_THRESHOLD, ODOM_FREQ, POSE_SIZE, X_RANGE, X_STEP, Y_RANGE, Y_STEP, RatslamRos
+
+MAX_CAPACITY = 1 << 16          # templates per agent the frame's library sweep takes (kSmallLibrary)
+
+
+def _real(v):
+    return isinstance(v, (numbers.Real, np.number)) and not isinstance(v, (bool, np.bool_))
+
+
+def agent_parameters(n_agents=None, match_threshold=MATCH_THRESHOLD, global_inhibition=PC_GLOBAL_INHIB,
+                     inject_energy=None):
+    """Broadcast the per-agent parameters to B agents and validate them (no CUDA involved).
+
+    Each parameter is a scalar or a length-B sequence; B is ``n_agents`` or the length of the sequences.  Returns
+    ``(B, thresholds uint32[B], gi float64[B], energies list of float-or-None)``; the thresholds are clamped the way the
+    single-agent frame plans clamp them.  ``ValueError`` for disagreeing lengths, non-finite thresholds or inhibitions,
+    and energies that are negative or not finite."""
+    params = {"match_threshold": match_threshold, "global_inhibition": global_inhibition, "inject_energy": inject_energy}
+    seqs = {}
+    for k, v in params.items():
+        if v is None or _real(v):
+            continue
+        try:
+            seqs[k] = list(v)
+        except TypeError:
+            raise ValueError("%s must be a scalar or a sequence, got %r" % (k, v)) from None
+    B = None if n_agents is None else int(n_agents)
+    if B is not None and B < 1:
+        raise ValueError("n_agents must be >= 1, got %r" % (n_agents,))
+    for k, v in seqs.items():
+        if B is None:
+            B = len(v)
+        if len(v) != B or B == 0:
+            raise ValueError("%s has %d values for %d agents" % (k, len(v), B))
+    B = 1 if B is None else B
+    out = {k: seqs[k] if k in seqs else [v] * B for k, v in params.items()}
+    thr = []
+    for v in out["match_threshold"]:
+        if not _real(v) or not math.isfinite(float(v)):
+            raise ValueError("match_threshold must be finite numbers, got %r" % (v,))
+        thr.append(int(min(max(math.floor(v), 0), 0xFFFFFFFF)))    # as RatslamRos._fused_plan
+    gi = []
+    for v in out["global_inhibition"]:
+        if not _real(v) or not math.isfinite(float(v)):
+            raise ValueError("global_inhibition must be finite numbers, got %r" % (v,))
+        gi.append(float(v))
+    energies = []
+    for v in out["inject_energy"]:
+        if v is not None and (not _real(v) or not math.isfinite(float(v)) or float(v) < 0):
+            raise ValueError("inject_energy must be None or a finite energy >= 0 (the injection runs on the device), "
+                             "got %r" % (v,))
+        energies.append(None if v is None else float(v))
+    return B, np.array(thr, dtype=np.uint32), np.array(gi, dtype=np.float64), energies
+
+
+def capacity_for(T):
+    """Templates per agent for a T-frame replay: one frame appends at most one template, whole groups of 32."""
+    return (int(T) + 1 + 31) // 32 * 32
+
+
+def _unravel(flat, shape):
+    X, Y, Th = shape
+    flat = np.asarray(flat, dtype=np.int64)
+    return np.stack([flat // (Y * Th), (flat // Th) % Y, flat % Th], axis=-1)
+
+
+class EnsembleAgents:
+    """What every agent holds after the replay: its library, the template locations and its pose cells."""
+
+    def __init__(self, ens, libs, loc, n_templates, shape):
+        self._ens, self._libs, self._loc = ens, libs, loc
+        self.n_templates = n_templates
+        self.shape = shape
+
+    def __len__(self):
+        return len(self.n_templates)
+
+    @property
+    def path(self):
+        """The pose-cell kernel family that updated the ensemble (``PoseCellEnsemble.path``)."""
+        return self._ens.path
+
+    @property
+    def state(self):
+        """The device tensor ``[B, Th, X, Y]`` of every agent's pose cells (theta-major)."""
+        return self._ens.state
+
+    def templates(self, b):
+        """uint8 ``[n_b, 32, 32]``: agent b's templates as ``ViewTemplate.template`` holds them."""
+        n = int(self.n_templates[b])
+        out = torch.empty((n, 32, 32), dtype=torch.uint8, device=self._libs.device)
+        with torch.cuda.device(self._libs.device):
+            for i in range(n):
+                nat.check(nat.lib().prs_vt_unpack_u8(self._libs[b].data_ptr(), i, out[i].data_ptr(), nat.stream_ptr()),
+                          "prs_vt_unpack_u8")
+            return out.cpu().numpy()
+
+    def locations(self, b):
+        """int64 ``[n_b, 3]``: the pose cell each of agent b's templates was created at (``ViewTemplate.location``)."""
+        return _unravel(self._loc[b, :int(self.n_templates[b])].cpu().numpy(), self.shape)
+
+    def posecells(self, b):
+        """Agent b's pose cells, float64 ``[X, Y, Th]`` (the reference's layout)."""
+        return self._ens.state[b].permute(1, 2, 0).cpu().numpy().astype(np.float64)
+
+
+def replay_ensemble(frames, odom, n_agents=None, match_threshold=MATCH_THRESHOLD, global_inhibition=PC_GLOBAL_INHIB,
+                    inject_energy=None, pose_size=POSE_SIZE, dtype=np.float32, active_set=0, experience_map=False,
+                    experience_links=False, mode="ref"):
+    """Replay ``frames[T,256,256]`` (uint8) and ``odom[T,2]`` = (linear.x, angular.z) through B agents.
+
+    ``match_threshold``, ``global_inhibition`` and ``inject_energy`` (None = no injection, else a finite energy >= 0)
+    are scalars or length-B sequences.  Every agent starts as ``RatslamRos`` does: energy 1 at the grid's midpoint,
+    an empty library.  Returns a dict with ``template [B,T]``, ``created [B,T]``, ``argmax [B,T,3]`` (the cell each
+    match was made with), ``n_templates [B]`` and ``agents`` (``EnsembleAgents``); with ``experience_map=True`` also
+    ``n_exp [B,T]`` and ``em_xy [B,T,2]``, replayed on the host from the records as ``RatslamRos.replay_native`` does
+    (O(B*T) Python, off by default).  A pose-cell error raises what ``replay(native=True)`` raises (``KeyError((5, 5))``
+    for the reference's LUT hole, ``ValueError`` for an oversize shift) for the first offending frame, which the shared
+    odometry makes the same frame for every agent."""
+    B, thr, gi, energies = agent_parameters(n_agents, match_threshold, global_inhibition, inject_energy)
+    if mode != "ref":
+        raise ValueError("replay_ensemble supports the reference matching mode only, got mode=%r" % (mode,))
+    frames = np.asarray(frames)
+    odom = np.asarray(odom, dtype=np.float64)
+    T = len(frames)
+    if frames.dtype != np.uint8 or frames.ndim != 3 or tuple(frames.shape[1:]) != IM_SIZE or odom.shape != (T, 2):
+        raise ValueError("replay_ensemble: frames must be uint8 [T,%d,%d] and odom [T,2], got %s %r and %r"
+                         % (IM_SIZE[0], IM_SIZE[1], frames.dtype, frames.shape, odom.shape))
+    pose_size = tuple(int(s) for s in pose_size)
+    np_dtype = _as_np_dtype(dtype)
+    cap = capacity_for(T)
+    if cap > MAX_CAPACITY:
+        raise ValueError("replay_ensemble: %d frames need %d templates per agent; the library sweep takes at most %d"
+                         % (T, cap, MAX_CAPACITY))
+    frames = np.ascontiguousarray(frames)
+    lib_bytes = (cap // 32) * 34816
+    need = B * (lib_bytes + cap * 8 + int(np.prod(pose_size)) * np.dtype(np_dtype).itemsize + 64)
+    nat.require_cuda()
+    dev = torch.device("cuda", torch.cuda.current_device())
+    free, _ = torch.cuda.mem_get_info(dev)
+    if need > free:
+        raise ValueError("replay_ensemble: %d agents x %d templates need %.2f GB of device memory, %.2f GB are free"
+                         % (B, cap, need / 1e9, free / 1e9))
+
+    ens = PoseCellEnsemble(pose_size, B, global_inhibition=gi, dtype=np_dtype, device=dev, active_set=active_set)
+    midpoint = tuple(math.floor(s / 2) for s in pose_size)
+    ens.inject(1, midpoint)                                             # RatslamRos.__init__
+    L = nat.lib()
+    assert int(L.prs_vt_packed_bytes(cap)) == lib_bytes
+    libs = torch.zeros((B, lib_bytes), dtype=torch.uint8, device=dev)
+    loc = torch.full((B, cap), -1, dtype=torch.int64, device=dev)
+    n_dev = torch.zeros(B, dtype=torch.int32, device=dev)
+    thr_dev = torch.from_numpy(thr.view(np.int32)).to(dev)
+    injecting = any(e is not None for e in energies)
+    energy_dev = torch.tensor([-1.0 if e is None else e for e in energies], dtype=torch.float64, device=dev)
+    pc_work = torch.zeros(3 * B, dtype=torch.int64, device=dev)
+    scratch = torch.empty(int(L.prs_ens_scratch_bytes(B, IM_SIZE[0], IM_SIZE[1])), dtype=torch.uint8, device=dev)
+    res = np.zeros((T, B), dtype=RatslamRos._RESULT_DTYPE)
+    stream = torch.cuda.Stream(device=dev)
+    plan = ctypes.c_void_p()
+    with torch.cuda.device(dev):
+        nat.check(L.prs_pc_argmax(ens._h, ens.state.data_ptr(), pc_work.data_ptr(), nat.stream_ptr()), "prs_pc_argmax")
+        torch.cuda.current_stream(dev).synchronize()
+        nat.check(L.prs_ens_create(
+            ens._h, ens.state.data_ptr(), ens._gi.data_ptr(), pc_work.data_ptr(), libs.data_ptr(), cap, n_dev.data_ptr(),
+            thr_dev.data_ptr(), energy_dev.data_ptr() if injecting else None, loc.data_ptr(), nat.VT_MODE_REF,
+            IM_SIZE[0], IM_SIZE[1], Y_RANGE[0], Y_RANGE[1], Y_STEP, X_RANGE[0], X_RANGE[1], X_STEP, scratch.data_ptr(),
+            ctypes.byref(plan)), "prs_ens_create")
+        try:
+            moved = ((np.abs(odom[:, 0]) > 0.001) | (np.abs(odom[:, 1]) > 0.001)).astype(np.uint8)   # ros_simulate.py:128
+            tw = np.ascontiguousarray(odom / float(ODOM_FREQ))                                         # :157-158
+            nat.check(L.prs_ens_replay_run(plan, frames.ctypes.data, tw.ctypes.data, moved.ctypes.data, T,
+                                           res.ctypes.data, ctypes.c_void_p(stream.cuda_stream)), "prs_ens_replay_run")
+        finally:
+            L.prs_ens_destroy(plan)
+    bad = np.nonzero((((res["pc_err"] & ~nat.ERR_INJECT_LOC) != 0) & (moved[:, None] != 0)).any(axis=1))[0]
+    if len(bad):
+        stop = int(bad[0])
+        ens._raise_on_err(np.asarray(res["pc_err"][stop] & ~nat.ERR_INJECT_LOC, dtype=np.int32))
+    n_templates = res["n_templates"][-1].astype(np.int64) if T else np.zeros(B, np.int64)
+    out = {"template": res["template_index"].T.astype(np.int64), "created": res["created"].T != 0,
+           "argmax": _unravel(res["argmax"].T, pose_size), "n_templates": n_templates,
+           "agents": EnsembleAgents(ens, libs, loc, n_templates, pose_size)}
+    if experience_map:
+        out["n_exp"], out["em_xy"] = _experience_maps(out, moved, tw, pose_size, experience_links)
+    return out
+
+
+def _experience_maps(out, moved, tw, pose_size, linked):
+    """Each agent's experience map replayed from its records (``RatslamRos.replay_native``'s bookkeeping)."""
+    B, T = out["template"].shape
+    n_exp = np.zeros((B, T), np.int64)
+    em_xy = np.zeros((B, T, 2))
+    for b in range(B):
+        em = ExperienceMap(linked=linked, pc_dims=pose_size)
+        tpl, amax = out["template"][b], out["argmax"][b]
+        for t in range(T):
+            if moved[t]:
+                vt = int(tpl[t - 1]) if t > 0 else None
+                em.update(float(tw[t, 0]), float(tw[t, 1]), tuple(int(c) for c in amax[t]), vt if linked else None)
+            n_exp[b, t] = len(em.experiences)
+            if em.current_exp is not None:
+                em_xy[b, t] = em.get_current_point()
+    return n_exp, em_xy
+
+
+def _list(text, parse):
+    return [parse(v.strip()) for v in text.split(",") if v.strip()]
+
+
+def main(argv=None):
+    import argparse
+    ap = argparse.ArgumentParser(description="Replay a ROS1 bag through an ensemble of RatSLAM agents: the cross "
+                                             "product of the given parameter lists, one agent per combination")
+    ap.add_argument("bag")
+    ap.add_argument("--match-threshold", default=str(MATCH_THRESHOLD), metavar="T1,T2,...")
+    ap.add_argument("--global-inhibition", default="0.2", metavar="G1,G2,...")
+    ap.add_argument("--inject-energy", default="none", metavar="E1,E2,...",
+                    help="energies injected at the matched template's pose cell; 'none' = no injection")
+    ap.add_argument("--image-topic", default="navbot/camera/image")
+    ap.add_argument("--odom-topic", default="navbot/odom")
+    a = ap.parse_args(argv)
+    from . import rosbag_io as rb
+    thr = _list(a.match_threshold, float)
+    gis = _list(a.global_inhibition, float)
+    ens = _list(a.inject_energy, lambda s: None if s.lower() == "none" else float(s))
+    combos = list(itertools.product(thr, gis, ens))
+    frames, odom, _ = rb.events_to_arrays(rb.read_events(a.bag, image_topic=a.image_topic, odom_topic=a.odom_topic))
+    out = replay_ensemble(frames, odom, n_agents=len(combos), match_threshold=[c[0] for c in combos],
+                          global_inhibition=[c[1] for c in combos], inject_energy=[c[2] for c in combos])
+    T = len(frames)
+    for b, (t, g, e) in enumerate(combos):
+        last = tuple(int(c) for c in out["argmax"][b, -1]) if T else None
+        print("agent %d  match_threshold %g  global_inhibition %g  inject_energy %s:  templates %d  created %d/%d  "
+              "final arg-max %s" % (b, t, g, "none" if e is None else "%g" % e, out["n_templates"][b],
+                                    int(out["created"][b].sum()), T, last))
+
+
+if __name__ == "__main__":
+    main()
