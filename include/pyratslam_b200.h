@@ -408,6 +408,40 @@ PRS_API int prs_ens_destroy(prs_ens_plan* plan);
 PRS_API int prs_ens_replay_run(prs_ens_plan* plan, const uint8_t* frames, const double* odom, const uint8_t* moved, int T,
                        prs_frame_result* results, void* stream);
 
+/* ------------------------------------------------------- ensemble experience maps */
+
+/* Every agent's linked experience map built from an ensemble's records (csrc/experience_map.cu): the per-frame update
+ * of ExperienceMap(linked=True) (pyratslam_b200/experience_map.py: update, _find, _add_link, _create_linked,
+ * _set_current) for B agents over T frames, one thread per agent.  Graph relaxation (ExperienceMap.iterate) stays on
+ * the host.  Creation, loop-closure and link decisions, experience cells, tags and headings `th` are bit-identical to
+ * the host class; positions, link lengths and link headings may differ by the ulps of the device's cos, sin, atan2 and
+ * hypot.  Inputs, all device memory:
+ *   argmax : int64 [T][B], the C-order flat arg-max cell of agent b at frame t
+ *   tag    : int32 [T][B], the view template the experience is tagged with (the template of frame t-1, -1 at t = 0);
+ *            a tag outside [0, n_templates) means no view template (the host's vt=None: no loop-closure search)
+ *   tw     : double [T][2], the shared (vtrans, vrot) given to update()   moved : uint8 [T], 0 = no update this frame
+ *   X, Y, Th : the pose-cell grid; delta_pc : the loop-closure radius in cells (sqrt(d2) <= delta_pc)
+ * Per-frame outputs, device memory: n_exp int32 [T][B] (experiences so far), exp_id int32 [T][B] (the current
+ * experience, -1 = none), em_xy double [T][B][2] (its position, 0 while there is none).
+ * work: device, prs_em_work_bytes(B, T, n_templates) bytes, no initialisation needed; the map is left there.  It holds
+ * these arrays, element [i][b] at index i*B + b, each starting at a multiple of 256 bytes, in this order:
+ *   double exp_x[T][B], exp_y[T][B], exp_th[T][B]             experiences: position and heading
+ *   double link_d[T][B], link_heading[T][B], link_facing[T][B] links, in creation order
+ *   double rel[3][B]                                           rel_x, rel_y, rel_th after the last frame
+ *   int64  exp_cell[T][B]                                      the experience's C-order flat cell
+ *   int32  exp_tag[T][B]                                       its view template, -1 = none
+ *   int32  exp_next[T][B], out_head[T][B]                      candidate lists (next experience with the same tag) and
+ *                                                              out-link lists (first link starting there), -1 = end
+ *   int32  link_from[T][B], link_to[T][B], link_next[T][B]     link ends; next link with the same start
+ *   int32  vt_head[n_templates][B]                             first experience of each template's candidate list
+ *   int32  counts[4][B]                                        experiences, links, current experience (-1 = none),
+ *                                                              loop closures
+ * Experience i and link l of agent b exist for i < counts[0][b] and l < counts[1][b].  Asynchronous on `stream`. */
+PRS_API size_t prs_em_work_bytes(int B, int T, int n_templates);
+PRS_API int prs_em_linked_run(int B, int T, int n_templates, const long long* argmax, const int* tag, const double* tw,
+                      const uint8_t* moved, int X, int Y, int Th, double delta_pc, void* work, int* n_exp, int* exp_id,
+                      double* em_xy, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

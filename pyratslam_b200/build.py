@@ -16,7 +16,7 @@ CSRC = os.path.join(PKG, "csrc")
 LIBDIR = os.path.join(PKG, "_lib")
 LIB = os.path.join(LIBDIR, "libpyratslam_b200.so")
 SOURCES = ["capi.cu", "posecell_generic.cu", "posecell_resident.cu", "posecell_tiled.cu", "posecell_cluster.cu", "posecell_pair.cu", "posecell_active.cu",
-           "view_templates.cu", "sharded.cu"]
+           "view_templates.cu", "sharded.cu", "experience_map.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden", "--expt-relaxed-constexpr"]
 

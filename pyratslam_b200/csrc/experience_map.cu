@@ -1,0 +1,190 @@
+// Linked experience maps of an ensemble on the device (prs_em_*, include/pyratslam_b200.h).
+//
+// The per-frame update of pyratslam_b200/experience_map.py (ExperienceMap.update with linked=True: _find, _add_link,
+// _create_linked, _set_current) for B agents over T recorded frames.  Each agent is a serial chain of T dependent
+// steps, so one thread runs one agent and the agents run in parallel; small blocks spread them over the SMs.
+//
+// Every decision -- create an experience, close a loop, do nothing, add a link or find it already there -- depends only
+// on integer cells, template tags and the IEEE-exact sqrt(d2) <= delta_pc test, so it is bit-identical to the host.
+// The double arithmetic is written with __dadd_rn / __dsub_rn / __dmul_rn / __ddiv_rn, which nvcc does not contract
+// into FMAs (Python does none), so clip_rad_180, signed_delta_rad and every heading sum are bit-identical as well.
+// Only cos, sin, atan2 and hypot may differ from glibc's by an ulp or two: they reach the positions, the link lengths
+// and the link headings, never a decision.
+#include <math.h>
+
+#include "common.cuh"
+
+namespace {
+
+constexpr int kEmBlock = 32;                    // one warp per block: B = 1024 agents spread over 32 SMs
+constexpr double kPi = 3.141592653589793;       // math.pi
+constexpr double kTwoPi = 6.283185307179586;    // 2 * math.pi (exact)
+
+// experience_map.py:clip_rad_180
+__device__ __forceinline__ double clip_rad_180(double a) {
+  if (a > kPi) return __dsub_rn(a, __dmul_rn(ceil(__ddiv_rn(a, kTwoPi)), kTwoPi));
+  if (a <= -kPi) return __dadd_rn(a, __dmul_rn(ceil(__ddiv_rn(fabs(a), kTwoPi)), kTwoPi));
+  return a;
+}
+
+// experience_map.py:signed_delta_rad
+__device__ __forceinline__ double signed_delta_rad(double a, double b) {
+  const double d = __dsub_rn(clip_rad_180(b), clip_rad_180(a));
+  if (d > kPi) return __dsub_rn(d, kTwoPi);
+  if (d <= -kPi) return __dadd_rn(d, kTwoPi);
+  return d;
+}
+
+// The workspace: structure-of-arrays, element [i][b] at i * B + b, each array at a multiple of 256 bytes, in the
+// order of the header's documentation (Python views the same offsets).
+struct EmLayout {
+  size_t exp_x, exp_y, exp_th, link_d, link_heading, link_facing, rel, exp_cell, exp_tag, exp_next, out_head, link_from,
+      link_to, link_next, vt_head, counts, bytes;
+  EmLayout(int B, int T, int N) {
+    size_t off = 0;
+    auto take = [&](size_t rows, size_t elem) {
+      const size_t o = off;
+      off += (rows * B * elem + 255) / 256 * 256;
+      return o;
+    };
+    exp_x = take(T, 8), exp_y = take(T, 8), exp_th = take(T, 8);
+    link_d = take(T, 8), link_heading = take(T, 8), link_facing = take(T, 8);
+    rel = take(3, 8);
+    exp_cell = take(T, 8);
+    exp_tag = take(T, 4), exp_next = take(T, 4), out_head = take(T, 4);
+    link_from = take(T, 4), link_to = take(T, 4), link_next = take(T, 4);
+    vt_head = take(N, 4);
+    counts = take(4, 4);
+    bytes = off;
+  }
+};
+
+struct EmWork {
+  double *exp_x, *exp_y, *exp_th, *link_d, *link_heading, *link_facing, *rel;
+  long long* exp_cell;
+  int *exp_tag, *exp_next, *out_head, *link_from, *link_to, *link_next, *vt_head, *counts;
+};
+
+__global__ void __launch_bounds__(kEmBlock)
+    k_em_linked(int B, int T, int N, const long long* __restrict__ argmax, const int* __restrict__ tag,
+                const double* __restrict__ tw, const uint8_t* __restrict__ moved, int X, int Y, int Th,
+                double delta_pc, EmWork w, int* __restrict__ n_exp_out, int* __restrict__ exp_id_out,
+                double* __restrict__ em_xy_out) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  const size_t sB = (size_t)B;
+  for (int v = 0; v < N; ++v) w.vt_head[v * sB + b] = -1;
+  int n_exp = 0, n_links = 0, cur = -1, n_loop = 0;
+  double rel_x = 0.0, rel_y = 0.0, rel_th = 0.0;
+  double cur_x = 0.0, cur_y = 0.0, cur_th = 0.0;   // the current experience's pose, kept in registers
+  const int YTh = Y * Th;
+
+  // _add_link(current, to) without the duplicate check, with the agent's rel_* at this point
+  auto link = [&](int to) {
+    const size_t l = n_links * sB + b;
+    w.link_from[l] = cur;
+    w.link_to[l] = to;
+    w.link_d[l] = hypot(rel_x, rel_y);
+    w.link_heading[l] = signed_delta_rad(cur_th, atan2(rel_y, rel_x));
+    w.link_facing[l] = signed_delta_rad(cur_th, rel_th);
+    w.link_next[l] = w.out_head[cur * sB + b];
+    w.out_head[cur * sB + b] = n_links;
+    ++n_links;
+  };
+  // _set_current
+  auto set_current = [&](int e, double x, double y, double th) {
+    cur = e, cur_x = x, cur_y = y, cur_th = th;
+    rel_x = 0.0, rel_y = 0.0, rel_th = th;
+  };
+
+  for (int t = 0; t < T; ++t) {
+    const size_t tb = t * sB + b;
+    if (moved[t]) {
+      // update(): the odometry since the current experience
+      const double vtrans = tw[2 * t], vrot = tw[2 * t + 1];
+      rel_th = clip_rad_180(__dadd_rn(rel_th, vrot));
+      rel_x = __dadd_rn(rel_x, __dmul_rn(vtrans, cos(rel_th)));
+      rel_y = __dadd_rn(rel_y, __dmul_rn(vtrans, sin(rel_th)));
+      const long long cell = argmax[tb];
+      const int px = (int)(cell / YTh), py = (int)(cell / Th % Y), pt = (int)(cell % Th);
+      const int vt = (unsigned)tag[tb] < (unsigned)N ? tag[tb] : -1;   // any tag outside [0, N): no view template
+      // _find: the nearest experience created with this view template within delta_pc cells (wrapped per axis);
+      // (distance, id) order, so the lowest id wins a tie whatever the order of the walk
+      int match = -1;
+      double best = 0.0;
+      if (vt >= 0 && cur >= 0) {
+        for (int e = w.vt_head[vt * sB + b]; e >= 0; e = w.exp_next[e * sB + b]) {
+          const long long c = w.exp_cell[e * sB + b];
+          int dx = abs((int)(c / YTh) - px) % X, dy = abs((int)(c / Th % Y) - py) % Y, dt = abs((int)(c % Th) - pt) % Th;
+          dx = min(dx, X - dx), dy = min(dy, Y - dy), dt = min(dt, Th - dt);
+          const double d = sqrt((double)(dx * dx + dy * dy + dt * dt));
+          if (d <= delta_pc && (match < 0 || d < best || (d == best && e < match))) match = e, best = d;
+        }
+      }
+      if (match < 0) {
+        // _create_linked: a new experience at the current one's position plus the odometry since, linked from it
+        const int e = n_exp++;
+        const size_t eb = e * sB + b;
+        const double x = __dadd_rn(cur >= 0 ? cur_x : 0.0, rel_x), y = __dadd_rn(cur >= 0 ? cur_y : 0.0, rel_y);
+        const double th = clip_rad_180(rel_th);
+        w.exp_x[eb] = x, w.exp_y[eb] = y, w.exp_th[eb] = th;
+        w.exp_cell[eb] = cell;
+        w.exp_tag[eb] = vt;
+        w.out_head[eb] = -1;
+        if (vt >= 0) {
+          w.exp_next[eb] = w.vt_head[vt * sB + b];
+          w.vt_head[vt * sB + b] = e;
+        } else {
+          w.exp_next[eb] = -1;
+        }
+        if (cur >= 0) link(e);          // e is new: no link current -> e exists yet
+        set_current(e, x, y, th);
+      } else if (match != cur) {
+        // a loop closure: link current -> match unless that pair is linked already, then move to match
+        bool linked = false;
+        for (int l = w.out_head[cur * sB + b]; l >= 0 && !linked; l = w.link_next[l * sB + b])
+          linked = w.link_to[l * sB + b] == match;
+        if (!linked) link(match);
+        ++n_loop;
+        const size_t mb = match * sB + b;
+        set_current(match, w.exp_x[mb], w.exp_y[mb], w.exp_th[mb]);
+      }
+    }
+    n_exp_out[tb] = n_exp;
+    exp_id_out[tb] = cur;
+    em_xy_out[2 * tb] = cur >= 0 ? cur_x : 0.0;
+    em_xy_out[2 * tb + 1] = cur >= 0 ? cur_y : 0.0;
+  }
+  w.rel[b] = rel_x, w.rel[sB + b] = rel_y, w.rel[2 * sB + b] = rel_th;
+  w.counts[b] = n_exp, w.counts[sB + b] = n_links, w.counts[2 * sB + b] = cur, w.counts[3 * sB + b] = n_loop;
+}
+
+}  // namespace
+
+extern "C" size_t prs_em_work_bytes(int B, int T, int n_templates) {
+  if (B < 1 || T < 0 || n_templates < 0) return 0;
+  return EmLayout(B, T, n_templates).bytes;
+}
+
+extern "C" int prs_em_linked_run(int B, int T, int n_templates, const long long* argmax, const int* tag, const double* tw,
+                                 const uint8_t* moved, int X, int Y, int Th, double delta_pc, void* work, int* n_exp,
+                                 int* exp_id, double* em_xy, void* stream) {
+  PRS_REQUIRE(B >= 1 && T >= 0 && n_templates >= 0, "prs_em_linked_run: bad size B=%d T=%d n_templates=%d", B, T,
+              n_templates);
+  PRS_REQUIRE(X >= 1 && Y >= 1 && Th >= 1 && (long long)X * Y * Th <= (1LL << 30),
+              "prs_em_linked_run: bad grid %d x %d x %d", X, Y, Th);
+  PRS_REQUIRE(work && (T == 0 || (argmax && tag && tw && moved && n_exp && exp_id && em_xy)),
+              "prs_em_linked_run: null argument");
+  const EmLayout L(B, T, n_templates);
+  char* p = (char*)work;
+  const EmWork w{(double*)(p + L.exp_x),     (double*)(p + L.exp_y),       (double*)(p + L.exp_th),
+                 (double*)(p + L.link_d),    (double*)(p + L.link_heading), (double*)(p + L.link_facing),
+                 (double*)(p + L.rel),       (long long*)(p + L.exp_cell), (int*)(p + L.exp_tag),
+                 (int*)(p + L.exp_next),     (int*)(p + L.out_head),      (int*)(p + L.link_from),
+                 (int*)(p + L.link_to),      (int*)(p + L.link_next),     (int*)(p + L.vt_head),
+                 (int*)(p + L.counts)};
+  k_em_linked<<<(B + kEmBlock - 1) / kEmBlock, kEmBlock, 0, (cudaStream_t)stream>>>(
+      B, T, n_templates, argmax, tag, tw, moved, X, Y, Th, delta_pc, w, n_exp, exp_id, em_xy);
+  PRS_CUDA(cudaGetLastError());
+  return PRS_OK;
+}

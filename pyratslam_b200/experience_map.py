@@ -1,8 +1,11 @@
 """Experience map -- host bookkeeping, as in the reference (``ratslam/experience_map.py``).
 
-O(1) per step and not part of the GPU path (BASELINE north_star: "ExperienceMap graph relaxation ... stay on the
-host as non-hot code").  By default it is the reference's class: it dead-reckons a 2-D pose from the odometry and
-records one experience per update, tagged with the arg-max pose cell (``experience_map.py:44-60``).
+Graph relaxation and the viewers stay on the host (BASELINE north_star: "ExperienceMap graph relaxation ... stay on
+the host as non-hot code"); so does this class's per-step update of a single agent.  For an ensemble replay, every
+agent's per-frame linked update runs on the device instead (``experience_ensemble``, csrc/experience_map.cu), and
+``ExperienceMap.from_arrays`` turns an agent's result back into this class.  By default it is the reference's class: it
+dead-reckons a 2-D pose from the odometry and records one experience per update, tagged with the arg-max pose cell
+(``experience_map.py:44-60``).
 
 ``ExperienceMap(linked=True)`` adds what the reference left as TODOs (``experience_map.py:49`` "linking will go here",
 ``:59`` "leaving vt stuff out"): experiences are linked by the odometry travelled between them, a revisit -- same view
@@ -65,6 +68,40 @@ class ExperienceMap:
         self._lfrom, self._lto, self._ld, self._lhead, self._lface = [], [], [], [], []   # links, creation order
         self._out = []            # per experience: indices of the links that start there
         self._by_vt = {}          # view template -> experience ids created with it
+
+    @classmethod
+    def from_arrays(cls, experiences, links, current, rel=(0.0, 0.0, 0.0), accum=(0.0, 0.0, 0.0), n_loop_closures=0,
+                    pc_dims=(21, 21, 36), delta_pc=1.0, correction=0.5):
+        """A linked map rebuilt from its arrays, e.g. one agent's map built on the device
+        (``experience_ensemble.EnsembleExperienceMaps.experience_map``).
+
+        ``experiences``: records with fields ``pc_x, pc_y, pc_th, vt`` (< 0: no view template), ``m_x, m_y, th``, in
+        index order; ``links``: records with fields ``from, to, d, heading, facing``, in creation order; ``current``:
+        the current experience's index (< 0: none); ``rel`` = (rel_x, rel_y, rel_th); ``accum`` = (accum_delta_x,
+        accum_delta_y, accum_delta_th).  The result relaxes (``iterate``) and updates as the original map would."""
+        em = cls(linked=True, pc_dims=pc_dims, delta_pc=delta_pc, correction=correction)
+        for i, r in enumerate(experiences):
+            vt = int(r["vt"])
+            vt = None if vt < 0 else vt
+            e = Experience((int(r["pc_x"]), int(r["pc_y"]), int(r["pc_th"])), (float(r["m_x"]), float(r["m_y"])), vt)
+            e.th = float(r["th"])
+            e.index = i
+            em.experiences.append(e)
+            em._out.append([])
+            if vt is not None:
+                em._by_vt.setdefault(vt, []).append(i)
+        for li, r in enumerate(links):
+            em._lfrom.append(int(r["from"]))
+            em._lto.append(int(r["to"]))
+            em._ld.append(float(r["d"]))
+            em._lhead.append(float(r["heading"]))
+            em._lface.append(float(r["facing"]))
+            em._out[int(r["from"])].append(li)
+        em.current_exp = em.experiences[int(current)] if int(current) >= 0 else None
+        em.rel_x, em.rel_y, em.rel_th = (float(v) for v in rel)
+        em.accum_delta_x, em.accum_delta_y, em.accum_delta_th = (float(v) for v in accum)
+        em.n_loop_closures = int(n_loop_closures)
+        return em
 
     # ------------------------------------------------------------------ the reference's class (experience_map.py:44-70)
     def create(self, pc_loc, vt=None):

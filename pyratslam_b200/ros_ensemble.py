@@ -21,10 +21,11 @@ import numpy as np
 import torch
 
 from . import _native as nat
+from . import experience_ensemble as xens
 from .experience_map import ExperienceMap
 from .kernels import PC_GLOBAL_INHIB
 from .posecell_network import PoseCellEnsemble, _as_np_dtype
-from .ros_simulate import IM_SIZE, MATCH_THRESHOLD, ODOM_FREQ, POSE_SIZE, X_RANGE, X_STEP, Y_RANGE, Y_STEP, RatslamRos
+from .ros_simulate import IM_SIZE, MATCH_THRESHOLD, POSE_SIZE, X_RANGE, X_STEP, Y_RANGE, Y_STEP, RatslamRos
 
 MAX_CAPACITY = 1 << 16          # templates per agent the frame's library sweep takes (kSmallLibrary)
 
@@ -142,7 +143,15 @@ def replay_ensemble(frames, odom, n_agents=None, match_threshold=MATCH_THRESHOLD
     ``n_exp [B,T]`` and ``em_xy [B,T,2]``, replayed on the host from the records as ``RatslamRos.replay_native`` does
     (O(B*T) Python, off by default).  A pose-cell error raises what ``replay(native=True)`` raises (``KeyError((5, 5))``
     for the reference's LUT hole, ``ValueError`` for an oversize shift) for the first offending frame, which the shared
-    odometry makes the same frame for every agent."""
+    odometry makes the same frame for every agent.
+
+    ``experience_map="device"`` builds the maps with ``experience_ensemble``: with ``experience_links=True`` every
+    agent's linked map on the device, next to ``n_exp`` and ``em_xy`` also ``exp_id [B,T]`` (the current experience),
+    ``n_loop_closures [B]`` and ``maps`` (``EnsembleExperienceMaps``); without links the shared dead reckoning once
+    (``maps`` None).  Any other value than False, True or "device" raises ``ValueError``."""
+    if not (isinstance(experience_map, (bool, np.bool_))
+            or (isinstance(experience_map, str) and experience_map == "device")):
+        raise ValueError("experience_map must be False, True or 'device', got %r" % (experience_map,))
     B, thr, gi, energies = agent_parameters(n_agents, match_threshold, global_inhibition, inject_energy)
     if mode != "ref":
         raise ValueError("replay_ensemble supports the reference matching mode only, got mode=%r" % (mode,))
@@ -161,6 +170,8 @@ def replay_ensemble(frames, odom, n_agents=None, match_threshold=MATCH_THRESHOLD
     frames = np.ascontiguousarray(frames)
     lib_bytes = (cap // 32) * 34816
     need = B * (lib_bytes + cap * 8 + int(np.prod(pose_size)) * np.dtype(np_dtype).itemsize + 64)
+    if experience_map == "device" and experience_links:
+        need += xens.work_bytes(B, T, cap) + xens.record_bytes(B, T)
     nat.require_cuda()
     dev = torch.device("cuda", torch.cuda.current_device())
     free, _ = torch.cuda.mem_get_info(dev)
@@ -193,8 +204,7 @@ def replay_ensemble(frames, odom, n_agents=None, match_threshold=MATCH_THRESHOLD
             IM_SIZE[0], IM_SIZE[1], Y_RANGE[0], Y_RANGE[1], Y_STEP, X_RANGE[0], X_RANGE[1], X_STEP, scratch.data_ptr(),
             ctypes.byref(plan)), "prs_ens_create")
         try:
-            moved = ((np.abs(odom[:, 0]) > 0.001) | (np.abs(odom[:, 1]) > 0.001)).astype(np.uint8)   # ros_simulate.py:128
-            tw = np.ascontiguousarray(odom / float(ODOM_FREQ))                                         # :157-158
+            moved, tw = xens.gate(odom)
             nat.check(L.prs_ens_replay_run(plan, frames.ctypes.data, tw.ctypes.data, moved.ctypes.data, T,
                                            res.ctypes.data, ctypes.c_void_p(stream.cuda_stream)), "prs_ens_replay_run")
         finally:
@@ -207,7 +217,10 @@ def replay_ensemble(frames, odom, n_agents=None, match_threshold=MATCH_THRESHOLD
     out = {"template": res["template_index"].T.astype(np.int64), "created": res["created"].T != 0,
            "argmax": _unravel(res["argmax"].T, pose_size), "n_templates": n_templates,
            "agents": EnsembleAgents(ens, libs, loc, n_templates, pose_size)}
-    if experience_map:
+    if experience_map == "device":
+        out.update(xens._maps(res["template_index"], np.ascontiguousarray(res["argmax"]), moved, tw, pose_size,
+                              experience_links, 1.0, 0.5, dev))
+    elif experience_map:
         out["n_exp"], out["em_xy"] = _experience_maps(out, moved, tw, pose_size, experience_links)
     return out
 
@@ -243,6 +256,9 @@ def main(argv=None):
     ap.add_argument("--global-inhibition", default="0.2", metavar="G1,G2,...")
     ap.add_argument("--inject-energy", default="none", metavar="E1,E2,...",
                     help="energies injected at the matched template's pose cell; 'none' = no injection")
+    ap.add_argument("--experience-links", action="store_true",
+                    help="build every agent's linked experience map on the device and print its experience and "
+                         "loop-closure counts")
     ap.add_argument("--image-topic", default="navbot/camera/image")
     ap.add_argument("--odom-topic", default="navbot/odom")
     a = ap.parse_args(argv)
@@ -253,13 +269,18 @@ def main(argv=None):
     combos = list(itertools.product(thr, gis, ens))
     frames, odom, _ = rb.events_to_arrays(rb.read_events(a.bag, image_topic=a.image_topic, odom_topic=a.odom_topic))
     out = replay_ensemble(frames, odom, n_agents=len(combos), match_threshold=[c[0] for c in combos],
-                          global_inhibition=[c[1] for c in combos], inject_energy=[c[2] for c in combos])
+                          global_inhibition=[c[1] for c in combos], inject_energy=[c[2] for c in combos],
+                          experience_map="device" if a.experience_links else False,
+                          experience_links=a.experience_links)
     T = len(frames)
     for b, (t, g, e) in enumerate(combos):
         last = tuple(int(c) for c in out["argmax"][b, -1]) if T else None
-        print("agent %d  match_threshold %g  global_inhibition %g  inject_energy %s:  templates %d  created %d/%d  "
-              "final arg-max %s" % (b, t, g, "none" if e is None else "%g" % e, out["n_templates"][b],
-                                    int(out["created"][b].sum()), T, last))
+        line = ("agent %d  match_threshold %g  global_inhibition %g  inject_energy %s:  templates %d  created %d/%d  "
+                "final arg-max %s" % (b, t, g, "none" if e is None else "%g" % e, out["n_templates"][b],
+                                      int(out["created"][b].sum()), T, last))
+        if a.experience_links:
+            line += "  experiences %d  loop closures %d" % (out["maps"].n_experiences[b], out["n_loop_closures"][b])
+        print(line)
 
 
 if __name__ == "__main__":
