@@ -408,6 +408,34 @@ PRS_API int prs_ens_destroy(prs_ens_plan* plan);
 PRS_API int prs_ens_replay_run(prs_ens_plan* plan, const uint8_t* frames, const double* odom, const uint8_t* moved, int T,
                        prs_frame_result* results, void* stream);
 
+/* Several recordings through one ensemble: agent b replays recording rec_of[b] of R, each with its own frames, odometry
+ * and length.  A frame is still ONE graph: one query per recording (a block each), one sweep in which agent b compares
+ * against its recording's query, the per-agent decision and injection.  The pose-cell update of all B networks runs
+ * when any recording moved; a network whose recording did not move, or has ended, gets the twist (0, 0), and on such a
+ * "mixed" frame its state slice and its pc_work slots are saved before the update and restored after it (the
+ * active-set lists are invalidated), so it ends the frame exactly as a skipped update leaves it.  Three graphs per plan:
+ * no recording moved, every recording has a frame and moved (no snapshot), mixed.  Past the end of its recording an
+ * agent appends and injects nothing; its record has template_index -1, created 0, key ~0 and n_templates unchanged.
+ * Agent b's records equal a single-recording plan's on recording rec_of[b]; the agents of one recording are best given
+ * contiguous indices (a sweep block reloads its query when the recording changes).
+ *   prs_ens_multi_scratch_bytes(plan, R): device bytes of multi_scratch, private to the plan.  It holds a chunk of
+ *            frames of every recording ([R][chunk][im_rows][im_cols], chunk = 256 MiB / (R * frame bytes), clamped to
+ *            [1, 256]), the per-recording queries and one snapshot of a network's state per agent.
+ *   prs_ens_set_recordings: rec_of_dev: device int32 [B] in [0, R); it and multi_scratch must outlive the plan's use.
+ *   prs_ens_multi_replay_run:
+ *     frames : host, R pointers; frames[r] is uint8 [lengths[r]][im_rows][im_cols] (may be NULL when lengths[r] = 0)
+ *     odom   : host double [T_max][R][2] = (vtrans, vrot) of recording r at frame t as given to update()
+ *     moved  : host uint8 [T_max][R], 0 = recording r makes no pose-cell update at frame t (entries past lengths[r] are
+ *              ignored)
+ *     lengths: host int32 [R], each in [0, T_max]; results: host prs_frame_result [T_max][B]
+ *   Frames go to the device one chunk at a time, one copy per recording.  PRS_E_INVALID when the libraries have no room
+ *   for T_max more templates. */
+PRS_API size_t prs_ens_multi_scratch_bytes(const prs_ens_plan* plan, int R);
+PRS_API int prs_ens_set_recordings(prs_ens_plan* plan, int R, const int* rec_of_dev, void* multi_scratch);
+PRS_API int prs_ens_multi_replay_run(prs_ens_plan* plan, const uint8_t* const* frames, const double* odom,
+                             const uint8_t* moved, const int* lengths, int T_max, prs_frame_result* results,
+                             void* stream);
+
 /* ------------------------------------------------------- ensemble experience maps */
 
 /* Every agent's linked experience map built from an ensemble's records (csrc/experience_map.cu): the per-frame update
@@ -441,6 +469,11 @@ PRS_API size_t prs_em_work_bytes(int B, int T, int n_templates);
 PRS_API int prs_em_linked_run(int B, int T, int n_templates, const long long* argmax, const int* tag, const double* tw,
                       const uint8_t* moved, int X, int Y, int Th, double delta_pc, void* work, int* n_exp, int* exp_id,
                       double* em_xy, void* stream);
+/* The same for agents that replayed different recordings: agent b follows recording rec_of[b] (device int32 [B], in
+ * [0, R)) of tw: device double [T][R][2] and moved: device uint8 [T][R] (frames past a recording's end: moved 0). */
+PRS_API int prs_em_linked_multi_run(int B, int T, int n_templates, const long long* argmax, const int* tag, int R,
+                            const double* tw, const uint8_t* moved, const int* rec_of, int X, int Y, int Th,
+                            double delta_pc, void* work, int* n_exp, int* exp_id, double* em_xy, void* stream);
 
 #ifdef __cplusplus
 }

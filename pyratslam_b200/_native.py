@@ -100,9 +100,16 @@ _SIGNATURES["prs_ens_create"] = (c_int, [c_void_p, c_void_p, c_void_p, c_void_p,
                                          c_void_p, POINTER(c_void_p)])
 _SIGNATURES["prs_ens_destroy"] = (c_int, [c_void_p])
 _SIGNATURES["prs_ens_replay_run"] = (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p])
+_SIGNATURES["prs_ens_multi_scratch_bytes"] = (c_size_t, [c_void_p, c_int])
+_SIGNATURES["prs_ens_set_recordings"] = (c_int, [c_void_p, c_int, c_void_p, c_void_p])
+_SIGNATURES["prs_ens_multi_replay_run"] = (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p,
+                                                   c_void_p])
 _SIGNATURES["prs_em_work_bytes"] = (c_size_t, [c_int, c_int, c_int])
 _SIGNATURES["prs_em_linked_run"] = (c_int, [c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int,
                                             c_int, c_double, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p])
+_SIGNATURES["prs_em_linked_multi_run"] = (c_int, [c_int, c_int, c_int, c_void_p, c_void_p, c_int, c_void_p, c_void_p,
+                                                  c_void_p, c_int, c_int, c_int, c_double, c_void_p, c_void_p, c_void_p,
+                                                  c_void_p, c_void_p])
 
 
 _SIGNATURES["prs_xchg_create"] = (c_int, [c_int, c_int, POINTER(c_void_p)])

@@ -69,9 +69,12 @@ __global__ void __launch_bounds__(kEmBlock)
     k_em_linked(int B, int T, int N, const long long* __restrict__ argmax, const int* __restrict__ tag,
                 const double* __restrict__ tw, const uint8_t* __restrict__ moved, int X, int Y, int Th,
                 double delta_pc, EmWork w, int* __restrict__ n_exp_out, int* __restrict__ exp_id_out,
-                double* __restrict__ em_xy_out) {
+                double* __restrict__ em_xy_out, int R = 1, const int* __restrict__ rec_of = nullptr) {
+  // rec_of (several recordings): agent b follows recording r = rec_of[b] of tw[T][R][2] and moved[T][R]
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
+  const int r = rec_of != nullptr ? rec_of[b] : 0;
+  if (rec_of == nullptr) R = 1;
   const size_t sB = (size_t)B;
   for (int v = 0; v < N; ++v) w.vt_head[v * sB + b] = -1;
   int n_exp = 0, n_links = 0, cur = -1, n_loop = 0;
@@ -99,9 +102,10 @@ __global__ void __launch_bounds__(kEmBlock)
 
   for (int t = 0; t < T; ++t) {
     const size_t tb = t * sB + b;
-    if (moved[t]) {
+    const size_t tr = (size_t)t * R + r;
+    if (moved[tr]) {
       // update(): the odometry since the current experience
-      const double vtrans = tw[2 * t], vrot = tw[2 * t + 1];
+      const double vtrans = tw[2 * tr], vrot = tw[2 * tr + 1];
       rel_th = clip_rad_180(__dadd_rn(rel_th, vrot));
       rel_x = __dadd_rn(rel_x, __dmul_rn(vtrans, cos(rel_th)));
       rel_y = __dadd_rn(rel_y, __dmul_rn(vtrans, sin(rel_th)));
@@ -166,15 +170,14 @@ extern "C" size_t prs_em_work_bytes(int B, int T, int n_templates) {
   return EmLayout(B, T, n_templates).bytes;
 }
 
-extern "C" int prs_em_linked_run(int B, int T, int n_templates, const long long* argmax, const int* tag, const double* tw,
-                                 const uint8_t* moved, int X, int Y, int Th, double delta_pc, void* work, int* n_exp,
-                                 int* exp_id, double* em_xy, void* stream) {
-  PRS_REQUIRE(B >= 1 && T >= 0 && n_templates >= 0, "prs_em_linked_run: bad size B=%d T=%d n_templates=%d", B, T,
-              n_templates);
-  PRS_REQUIRE(X >= 1 && Y >= 1 && Th >= 1 && (long long)X * Y * Th <= (1LL << 30),
-              "prs_em_linked_run: bad grid %d x %d x %d", X, Y, Th);
-  PRS_REQUIRE(work && (T == 0 || (argmax && tag && tw && moved && n_exp && exp_id && em_xy)),
-              "prs_em_linked_run: null argument");
+static int em_linked_launch(const char* who, int B, int T, int n_templates, const long long* argmax, const int* tag,
+                            int R, const double* tw, const uint8_t* moved, const int* rec_of, int X, int Y, int Th,
+                            double delta_pc, void* work, int* n_exp, int* exp_id, double* em_xy, void* stream) {
+  PRS_REQUIRE(B >= 1 && T >= 0 && n_templates >= 0 && R >= 1, "%s: bad size B=%d T=%d n_templates=%d R=%d", who, B, T,
+              n_templates, R);
+  PRS_REQUIRE(X >= 1 && Y >= 1 && Th >= 1 && (long long)X * Y * Th <= (1LL << 30), "%s: bad grid %d x %d x %d", who, X, Y,
+              Th);
+  PRS_REQUIRE(work && (T == 0 || (argmax && tag && tw && moved && n_exp && exp_id && em_xy)), "%s: null argument", who);
   const EmLayout L(B, T, n_templates);
   char* p = (char*)work;
   const EmWork w{(double*)(p + L.exp_x),     (double*)(p + L.exp_y),       (double*)(p + L.exp_th),
@@ -184,7 +187,23 @@ extern "C" int prs_em_linked_run(int B, int T, int n_templates, const long long*
                  (int*)(p + L.link_to),      (int*)(p + L.link_next),     (int*)(p + L.vt_head),
                  (int*)(p + L.counts)};
   k_em_linked<<<(B + kEmBlock - 1) / kEmBlock, kEmBlock, 0, (cudaStream_t)stream>>>(
-      B, T, n_templates, argmax, tag, tw, moved, X, Y, Th, delta_pc, w, n_exp, exp_id, em_xy);
+      B, T, n_templates, argmax, tag, tw, moved, X, Y, Th, delta_pc, w, n_exp, exp_id, em_xy, R, rec_of);
   PRS_CUDA(cudaGetLastError());
   return PRS_OK;
+}
+
+extern "C" int prs_em_linked_run(int B, int T, int n_templates, const long long* argmax, const int* tag, const double* tw,
+                                 const uint8_t* moved, int X, int Y, int Th, double delta_pc, void* work, int* n_exp,
+                                 int* exp_id, double* em_xy, void* stream) {
+  return em_linked_launch("prs_em_linked_run", B, T, n_templates, argmax, tag, 1, tw, moved, nullptr, X, Y, Th, delta_pc,
+                          work, n_exp, exp_id, em_xy, stream);
+}
+
+extern "C" int prs_em_linked_multi_run(int B, int T, int n_templates, const long long* argmax, const int* tag, int R,
+                                       const double* tw, const uint8_t* moved, const int* rec_of, int X, int Y, int Th,
+                                       double delta_pc, void* work, int* n_exp, int* exp_id, double* em_xy,
+                                       void* stream) {
+  PRS_REQUIRE(rec_of != nullptr || T == 0, "prs_em_linked_multi_run: null rec_of");
+  return em_linked_launch("prs_em_linked_multi_run", B, T, n_templates, argmax, tag, R, tw, moved, rec_of, X, Y, Th,
+                          delta_pc, work, n_exp, exp_id, em_xy, stream);
 }

@@ -32,6 +32,7 @@
 
 #include <atomic>
 #include <mutex>
+#include <vector>
 
 #include "common.cuh"
 #include "vt_pack.cuh"
@@ -1256,6 +1257,10 @@ struct VtAgents {
   long long loc_stride = 0;
   int* g_max = nullptr;                 // largest group count over the agents, raised by the decision (the sweep's grid)
   const int* ctr = nullptr;             // frame index within the record chunk: the agent's record is res[*ctr * B + b]
+  // multi-recording frames (prs_ens_set_recordings): agent b replays recording rec_of[b], whose template is
+  // tpl + rec_of[b] * 1024; present[r] = 0 past recording r's end, where its agents append and inject nothing
+  const int* rec_of = nullptr;          // [B]; null: one recording, one template
+  const uint8_t* present = nullptr;     // [R]
 };
 
 // One warp per agent (b = global warp index), lane t packs row t of a created template.
@@ -1270,6 +1275,22 @@ __global__ void k_vt_decide_append(const unsigned long long* __restrict__ key, c
   if (b >= ag.B) return;  // whole warps
   if (n_dev != nullptr) n = n_dev[b];
   __syncwarp();
+  if (ag.rec_of != nullptr) {
+    const int r = ag.rec_of[b];
+    if (!ag.present[r]) {  // the recording has ended: a "no frame" record, the library stays as it is
+      if (t == 0) {
+        res += (long long)*ag.ctr * ag.B + b;
+        res->argmax = argmax[b];
+        res->key = ~0ull;
+        res->created = 0;
+        res->template_index = -1;
+        res->n_templates = n;
+        res->pc_err = pc_err[b];
+      }
+      return;
+    }
+    tpl += (size_t)r * 1024;
+  }
   const unsigned long long k = key[b];
   const unsigned score = (unsigned)(k >> 32);
   if (ag.threshold != nullptr) threshold = ag.threshold[b];
@@ -1325,6 +1346,7 @@ __global__ void k_frame_inject(T* __restrict__ state, long long* __restrict__ lo
   if (energies != nullptr) {
     const double e = energies[b];
     if (!(e >= 0.0)) return;
+    if (ag.rec_of != nullptr && !ag.present[ag.rec_of[b]]) return;  // no frame, nothing to inject
     energy = (T)e;
     const long long r = (ag.ctr != nullptr ? (long long)*ag.ctr * ag.B : 0) + b;
     dec += r;
@@ -1523,6 +1545,62 @@ __global__ void __launch_bounds__(1024)
   }
 }
 
+// k_vt_frame_prepare's query (the template of `frame`, its bit planes and row sums) for one recording; kept as a
+// copy so that k_vt_frame_prepare itself compiles to the code it always had
+__device__ __forceinline__ void vt_prepare_query(const uint8_t* __restrict__ frame, int im_cols, int row_lo, int row_step,
+                                                 int col_lo, int col_step, uint8_t* __restrict__ tpl,
+                                                 uint32_t* __restrict__ planes, uint32_t* s_sum) {
+  const int t = threadIdx.x >> 5, c = threadIdx.x & 31;  // template row, column
+  const int rr = row_lo + (t / (row_step - 1)) * row_step + (t % (row_step - 1)) + 1;
+  const int cc = col_lo + (c / (col_step - 1)) * col_step + (c % (col_step - 1)) + 1;
+  const uint32_t px = frame[(size_t)rr * im_cols + cc];
+  tpl[t * 32 + c] = (uint8_t)px;
+  uint32_t mine = 0;
+#pragma unroll
+  for (int k = 0; k < 8; ++k) {
+    const uint32_t b = __ballot_sync(0xffffffffu, (px >> k) & 1u);
+    if (c == k) mine = b;
+  }
+  if (c < 8) planes[t * 8 + c] = mine;
+  uint32_t sum = px;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, o);
+  if (c == 0) s_sum[t] = sum;
+  __syncthreads();
+  if (t == 0) {
+    uint32_t all = s_sum[c], mid = (c >= 8 && c < 24) ? all : 0;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      all += __shfl_xor_sync(0xffffffffu, all, o);
+      mid += __shfl_xor_sync(0xffffffffu, mid, o);
+    }
+    if (c == 0) {
+      planes[256] = mid;
+      planes[257] = all;
+    }
+  }
+}
+
+// Multi-recording frames: block r prepares recording r's query from frame *ctr of its chunk, frames[r][chunk] (bytes
+// (r * chunk + *ctr) * frame_bytes), into tpl + r * 1024 and planes + r * kQueryStride, and sets present[r] from bit 0
+// of gate[*ctr][r] (0 past the recording's end: no query).  The blocks reset the n_keys agents' keys.
+constexpr int kQueryStride = 512;  // uint32 words between two recordings' query planes (258 used)
+
+__global__ void __launch_bounds__(1024)
+    k_vt_frame_prepare_multi(const uint8_t* __restrict__ frames, int chunk, long long frame_bytes, int im_cols, int row_lo,
+                             int row_step, int col_lo, int col_step, uint8_t* __restrict__ tpl,
+                             uint32_t* __restrict__ planes, unsigned long long* __restrict__ key, int n_keys,
+                             const int* __restrict__ ctr, const uint8_t* __restrict__ gate, uint8_t* __restrict__ present) {
+  __shared__ uint32_t s_sum[32];
+  const int r = blockIdx.x, R = gridDim.x, f = *ctr;
+  for (int i = r * 1024 + (int)threadIdx.x; i < n_keys; i += R * 1024) key[i] = ~0ull;
+  const bool here = (gate[(size_t)f * R + r] & 1) != 0;
+  if (threadIdx.x == 0) present[r] = here ? 1 : 0;
+  if (!here) return;  // block-uniform
+  vt_prepare_query(frames + ((size_t)r * chunk + f) * frame_bytes, im_cols, row_lo, row_step, col_lo, col_step,
+                   tpl + (size_t)r * 1024, planes + (size_t)r * kQueryStride, s_sum);
+}
+
 __device__ __forceinline__ uint32_t lt_row_q(const uint4& lo, const uint4& hi, const uint32_t* q) {
   uint32_t lt = ~lo.x & q[0];
   lt = (~lo.y & q[1]) | (~(lo.y ^ q[1]) & lt);
@@ -1544,10 +1622,16 @@ constexpr int kSmallThreads = 512;
 // Ensemble frames: n_agents libraries of lib_u4 uint4 each, agent b's live count n_dev[b] and key key_out[b].  The
 // blocks grid-stride over (agent, group) items, G = *g_max groups per agent (the largest live group count, kept by the
 // decision kernel); an item past its agent's live count is skipped, so the work follows sum_b n_b, not the capacity.
+// kMulti (multi-recording frames): agent b is compared with the query of its recording
+// rec_of[b], qplanes + rec_of[b] * kQueryStride, and skipped where present[rec_of[b]] = 0.  A block reloads q only
+// when its item's recording differs from the last one it loaded (the agents of a recording have contiguous indices).
+// k_vt_sweep_packed_ref_small is the <false> instantiation, whose code is that of the untemplated kernel it was.
+template <bool kMulti>
 __global__ void __launch_bounds__(kSmallThreads)
     k_vt_sweep_packed_ref_small(const uint4* __restrict__ packed, const uint32_t* __restrict__ qplanes,
                                 unsigned long long* __restrict__ key_out, const int* __restrict__ n_dev,
-                                int n_agents = 1, long long lib_u4 = 0, const int* __restrict__ g_max = nullptr) {
+                                int n_agents = 1, long long lib_u4 = 0, const int* __restrict__ g_max = nullptr,
+                                const int* __restrict__ rec_of = nullptr, const uint8_t* __restrict__ present = nullptr) {
   __shared__ uint32_t q[32 * 8 + 8];
   __shared__ uint32_t s_cnt[15][32];
   __shared__ uint32_t s_A[15][32];
@@ -1555,12 +1639,22 @@ __global__ void __launch_bounds__(kSmallThreads)
   const long long G = g_max != nullptr ? (long long)*g_max : ((long long)*n_dev + 31) >> 5;
   const long long items = G * n_agents;
   if ((long long)blockIdx.x >= items) return;  // the grid is laid out for the capacity, not the live count
-  for (int i = threadIdx.x; i < 32 * 8 + 2; i += kSmallThreads) q[i] = qplanes[i];
+  if (!kMulti)
+    for (int i = threadIdx.x; i < 32 * 8 + 2; i += kSmallThreads) q[i] = qplanes[i];
+  [[maybe_unused]] int q_rec = -1;
   for (long long item = blockIdx.x; item < items; item += gridDim.x) {
     const int b = (int)(item / G);
     const long long g = item - b * G;
     const long long n = n_dev[b];
     if (g * 32 >= n) continue;  // block-uniform
+    if (kMulti) {
+      const int r = rec_of[b];
+      if (!present[r]) continue;  // block-uniform: the recording has ended
+      if (r != q_rec) {           // block-uniform; the last item's final barrier retired every reader of q
+        for (int i = threadIdx.x; i < 32 * 8 + 2; i += kSmallThreads) q[i] = qplanes[(size_t)r * kQueryStride + i];
+        q_rec = r;
+      }
+    }
     if (threadIdx.x < 15 * 32) s_cnt[wid][lane] = 0;
     __syncthreads();  // also publishes q on the first pass
     const uint4* gp = packed + b * lib_u4 + g * kGroupU4 + lane;
@@ -1684,7 +1778,7 @@ static int frame_enqueue(prs_frame_plan* f, bool moved, cudaStream_t st) {
                                            d_tpl, d_planes, d_key);
     long long blocks = ((long long)f->capacity + 31) / 32;
     if (blocks > 148LL * 4) blocks = 148LL * 4;
-    k_vt_sweep_packed_ref_small<<<(int)blocks, kSmallThreads, 0, st>>>((const uint4*)f->vt_packed, d_planes, d_key, f->d_n);
+    k_vt_sweep_packed_ref_small<false><<<(int)blocks, kSmallThreads, 0, st>>>((const uint4*)f->vt_packed, d_planes, d_key, f->d_n);
   } else {
     PRS_CUDA(cudaMemcpyAsync(d_frame, f->frame_host, (size_t)f->im_rows * f->im_cols, cudaMemcpyHostToDevice, st));
     rc = prs_vt_extract_u8(d_frame, f->im_rows, f->im_cols, f->row_lo, f->row_hi, f->row_step, f->col_lo, f->col_hi,
@@ -1919,6 +2013,87 @@ struct EnsScratch {  // device scratch layout of an ensemble plan (bytes), every
   }
 };
 
+// Device scratch of the multi-recording frames (prs_ens_multi_scratch_bytes), every part 256-byte aligned.  The frame
+// counter and the group maximum stay in the plan's own scratch.  A chunk holds `chunk` frames of each of the R
+// recordings, as many as fit kEnsMultiFrameBytes (at least one, at most kEnsChunk).
+constexpr size_t kEnsMultiFrameBytes = 256u << 20;
+
+struct EnsMultiScratch {
+  int chunk = 0;
+  size_t frames = 0, odom_chunk = 0, gate = 0, rec = 0, odom = 0, key = 0, tpl = 0, planes = 0, present = 0, still = 0,
+         wsnap = 0, snap = 0, bytes = 0;
+  EnsMultiScratch() = default;
+  EnsMultiScratch(int B, int R, long long fbytes, size_t net_bytes) {
+    auto up = [](size_t v) { return (v + 255) & ~(size_t)255; };
+    const long long fit = (long long)(kEnsMultiFrameBytes / ((size_t)R * fbytes));
+    chunk = (int)(fit < 1 ? 1 : fit > kEnsChunk ? kEnsChunk : fit);
+    frames = 0;
+    odom_chunk = frames + up((size_t)R * chunk * fbytes);
+    gate = odom_chunk + up((size_t)chunk * R * 2 * sizeof(double));
+    rec = gate + up((size_t)chunk * R);
+    odom = rec + up((size_t)chunk * B * sizeof(prs_frame_result));
+    key = odom + up((size_t)B * 2 * sizeof(double));
+    tpl = key + up((size_t)B * sizeof(unsigned long long));
+    planes = tpl + up((size_t)R * 1024);
+    present = planes + up((size_t)R * kQueryStride * sizeof(uint32_t));
+    still = present + up((size_t)R);
+    wsnap = still + up((size_t)B);
+    snap = wsnap + up((size_t)B * 3 * sizeof(long long));
+    bytes = snap + up((size_t)B * net_bytes);
+  }
+};
+
+// Multi-recording frames: network b gets its recording's (vtrans, vrot) where that recording moved at this frame
+// (bit 1 of gate[*ctr][r]), else (0, 0), which no pose-cell kernel rejects; still[b] = 1 marks the network whose
+// update the mixed frame undoes.
+__global__ void k_ens_odom_multi(const double* __restrict__ odom_chunk, const uint8_t* __restrict__ gate,
+                                 const int* __restrict__ ctr, const int* __restrict__ rec_of, int R,
+                                 double* __restrict__ odom, uint8_t* __restrict__ still, int B) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  const size_t i = (size_t)*ctr * R + rec_of[b];
+  const bool mv = (gate[i] & 2) != 0;
+  odom[2 * b] = mv ? odom_chunk[2 * i] : 0.0;
+  odom[2 * b + 1] = mv ? odom_chunk[2 * i + 1] : 0.0;
+  still[b] = mv ? 0 : 1;
+}
+
+// The mixed frame's save (kRestore = false, before prs_pc_step) and restore (after it) of every still network: its
+// state slice of `words` W-words, and its pc_work slots (arg-max, total of total_bytes, err), to and from one snapshot per agent.
+// Blocks of other networks return at once.
+template <bool kRestore, typename W>
+__global__ void k_ens_snapshot(W* __restrict__ state, W* __restrict__ snap, long long words, int per_net,
+                               const uint8_t* __restrict__ still, long long* __restrict__ work,
+                               long long* __restrict__ wsnap, int B, int total_bytes) {
+  const int b = blockIdx.x / per_net;
+  if (!still[b]) return;
+  W* s = state + b * words;
+  W* d = snap + b * words;
+  for (long long i = (long long)(blockIdx.x % per_net) * blockDim.x + threadIdx.x; i < words;
+       i += (long long)per_net * blockDim.x) {
+    if (kRestore)
+      s[i] = d[i];
+    else
+      d[i] = s[i];
+  }
+  if (blockIdx.x % per_net == 0 && threadIdx.x == 0) {
+    int* err = (int*)(work + 2 * (size_t)B);
+    int* total32 = (int*)(work + B);  // a float32 plan's totals are 4-byte elements of the 8-byte slots' region
+    if (kRestore) {
+      work[b] = wsnap[3 * b];
+      if (total_bytes == 4)
+        total32[b] = (int)wsnap[3 * b + 1];
+      else
+        work[B + b] = wsnap[3 * b + 1];
+      err[b] = (int)wsnap[3 * b + 2];
+    } else {
+      wsnap[3 * b] = work[b];
+      wsnap[3 * b + 1] = total_bytes == 4 ? total32[b] : work[B + b];
+      wsnap[3 * b + 2] = err[b];
+    }
+  }
+}
+
 __global__ void k_ens_odom(const double* __restrict__ odom_chunk, const int* __restrict__ ctr, double* __restrict__ odom,
                            int B) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
@@ -1956,6 +2131,15 @@ struct prs_ens_plan {
   int warm[2];
   cudaStream_t side;
   cudaEvent_t ev_fork, ev_join;
+  // prs_ens_set_recordings (R = 0: not set): agent b replays recording rec_of[b]; the frame's three graphs are
+  // [0] no recording moved, [1] every recording has a frame and moved, [2] mixed
+  int R;
+  const int* rec_of;
+  char* mscratch;
+  EnsMultiScratch mlay;
+  cudaGraphExec_t mexec[3];
+  bool mready[3];
+  int mwarm[3];
 };
 
 static int ens_enqueue(prs_ens_plan* e, bool moved, cudaStream_t st) {
@@ -1985,7 +2169,7 @@ static int ens_enqueue(prs_ens_plan* e, bool moved, cudaStream_t st) {
                                          e->fbytes, B);
   long long blocks = (long long)B * ((e->capacity + 31) / 32);
   if (blocks > 148LL * 4) blocks = 148LL * 4;
-  k_vt_sweep_packed_ref_small<<<(int)blocks, kSmallThreads, 0, st>>>((const uint4*)e->libs, (const uint32_t*)(sc + L.planes),
+  k_vt_sweep_packed_ref_small<false><<<(int)blocks, kSmallThreads, 0, st>>>((const uint4*)e->libs, (const uint32_t*)(sc + L.planes),
                                                                      d_key, e->n_dev, B, e->lib_u4, d_gmax);
   if (moved) PRS_CUDA(cudaStreamWaitEvent(st, e->ev_join, 0));  // the decision reports the new arg-max
   VtAgents ag;
@@ -2039,7 +2223,8 @@ extern "C" int prs_ens_create(prs_pc_handle pc, void* pc_state, const void* gi, 
                                                      loc_dev, B, capacity, (long long)(prs_vt_packed_bytes(capacity) / 16),
                                                      (long long)im_rows * im_cols, 0, im_cols, row_lo, row_step, col_lo,
                                                      col_step, (char*)scratch, EnsScratch(B, (long long)im_rows * im_cols),
-                                                     {nullptr, nullptr}, {false, false}, {0, 0}, nullptr, nullptr, nullptr};
+                                                     {nullptr, nullptr}, {false, false}, {0, 0}, nullptr, nullptr, nullptr,
+                                                     0, nullptr, nullptr, EnsMultiScratch(), {}, {}, {}};
   PRS_REQUIRE(e, "prs_ens_create: out of host memory");
   int* misc = (int*)(e->scratch + e->lay.misc);
   int init[3] = {0, 0, 0};
@@ -2066,6 +2251,8 @@ extern "C" int prs_ens_destroy(prs_ens_plan* e) {
   if (e) {
     for (int i = 0; i < 2; ++i)
       if (e->ready[i]) cudaGraphExecDestroy(e->exec[i]);
+    for (int i = 0; i < 3; ++i)
+      if (e->mready[i]) cudaGraphExecDestroy(e->mexec[i]);
     if (e->side) cudaStreamDestroy(e->side);
     if (e->ev_fork) cudaEventDestroy(e->ev_fork);
     if (e->ev_join) cudaEventDestroy(e->ev_join);
@@ -2135,6 +2322,220 @@ extern "C" int prs_ens_replay_run(prs_ens_plan* e, const uint8_t* frames, const 
   const cudaError_t err = cudaStreamSynchronize(st);
   if (rc == PRS_OK && err != cudaSuccess) {
     prs_set_error("prs_ens_replay_run: %s", cudaGetErrorString(err));
+    return PRS_E_CUDA;
+  }
+  return rc;
+}
+
+// ---------------------------------------------------------------------------------------------
+// Multi-recording ensemble replay: agent b replays recording rec_of[b] (prs_ens_set_recordings).  The frame graph is
+// the one above with a query per recording and a per-agent gate:
+//   side branch  k_ens_odom_multi (each network its recording's twist, (0, 0) where that recording is still or has
+//                ended) -> [mixed: k_ens_snapshot save] -> prs_pc_step -> [mixed: k_ens_snapshot restore ->
+//                prs_pc_active_invalidate]
+//   template     k_vt_frame_prepare_multi (one block per recording) -> k_vt_sweep_packed_ref_small<true>
+//   join         k_vt_decide_append / k_frame_inject with VtAgents::rec_of and ::present -> k_ens_advance
+// The restore runs before the join, so the decision and the injection of a still network see its state, arg-max and
+// error bits as they were: what the single-recording frame leaves when it skips the update.  A frame where no recording
+// moved runs no update; one where every recording has a frame and moved needs no snapshot.
+static int ens_multi_enqueue(prs_ens_plan* e, int v, cudaStream_t st) {
+  char* sc = e->scratch;
+  char* ms = e->mscratch;
+  const EnsMultiScratch& M = e->mlay;
+  prs_pc_plan* pc = e->pc;
+  long long* d_argmax = (long long*)e->pc_work;
+  void* d_total = (char*)e->pc_work + 8 * (size_t)e->B;
+  int* d_err = (int*)((char*)e->pc_work + 16 * (size_t)e->B);
+  int* d_ctr = (int*)(sc + e->lay.misc);
+  int* d_gmax = d_ctr + 1;
+  double* d_odom = (double*)(ms + M.odom);
+  unsigned long long* d_key = (unsigned long long*)(ms + M.key);
+  prs_frame_result* d_rec = (prs_frame_result*)(ms + M.rec);
+  const uint8_t* d_gate = (const uint8_t*)(ms + M.gate);
+  uint8_t* d_present = (uint8_t*)(ms + M.present);
+  uint8_t* d_still = (uint8_t*)(ms + M.still);
+  const int B = e->B, R = e->R;
+  int rc;
+  if (v != 0) {
+    PRS_CUDA(cudaEventRecord(e->ev_fork, st));
+    PRS_CUDA(cudaStreamWaitEvent(e->side, e->ev_fork, 0));
+    k_ens_odom_multi<<<(B + 255) / 256, 256, 0, e->side>>>((const double*)(ms + M.odom_chunk), d_gate, d_ctr, e->rec_of, R,
+                                                           d_odom, d_still, B);
+    PRS_CUDA(cudaGetLastError());
+    const int es = pc->dtype == PRS_F32 ? 4 : 8;
+    const size_t net_bytes = (size_t)pc->N * es;
+    const bool wide = net_bytes % 16 == 0;
+    const long long words = (long long)(net_bytes / (wide ? 16 : 4));
+    const int per_net = (int)((words + 4095) / 4096);  // 256 threads x 16 words per block
+    auto snapshot = [&](bool restore) {
+      long long* ws = (long long*)(ms + M.wsnap);
+      long long* w = (long long*)e->pc_work;
+      const dim3 grid((unsigned)B * per_net);
+      if (wide) {
+        if (restore)
+          k_ens_snapshot<true, uint4><<<grid, 256, 0, e->side>>>((uint4*)e->pc_state, (uint4*)(ms + M.snap), words, per_net,
+                                                                 d_still, w, ws, B, es);
+        else
+          k_ens_snapshot<false, uint4><<<grid, 256, 0, e->side>>>((uint4*)e->pc_state, (uint4*)(ms + M.snap), words,
+                                                                  per_net, d_still, w, ws, B, es);
+      } else {
+        if (restore)
+          k_ens_snapshot<true, unsigned><<<grid, 256, 0, e->side>>>((unsigned*)e->pc_state, (unsigned*)(ms + M.snap), words,
+                                                                    per_net, d_still, w, ws, B, es);
+        else
+          k_ens_snapshot<false, unsigned><<<grid, 256, 0, e->side>>>((unsigned*)e->pc_state, (unsigned*)(ms + M.snap),
+                                                                     words, per_net, d_still, w, ws, B, es);
+      }
+      return cudaGetLastError();
+    };
+    if (v == 2) PRS_CUDA(snapshot(false));
+    rc = prs_pc_step(pc, e->pc_state, d_odom, e->gi, d_argmax, d_total, d_err, e->side);
+    if (rc != PRS_OK) return rc;
+    if (v == 2) {
+      PRS_CUDA(snapshot(true));
+      if (int rc_ = prs_pc_active_invalidate(pc, e->side)) return rc_;  // the carried lists describe the undone update
+    }
+    PRS_CUDA(cudaEventRecord(e->ev_join, e->side));
+  }
+  k_vt_frame_prepare_multi<<<R, 1024, 0, st>>>((const uint8_t*)(ms + M.frames), M.chunk, e->fbytes, e->im_cols, e->row_lo,
+                                               e->row_step, e->col_lo, e->col_step, (uint8_t*)(ms + M.tpl),
+                                               (uint32_t*)(ms + M.planes), d_key, B, d_ctr, d_gate, d_present);
+  long long blocks = (long long)B * ((e->capacity + 31) / 32);
+  if (blocks > 148LL * 4) blocks = 148LL * 4;
+  k_vt_sweep_packed_ref_small<true><<<(int)blocks, kSmallThreads, 0, st>>>(
+      (const uint4*)e->libs, (const uint32_t*)(ms + M.planes), d_key, e->n_dev, B, e->lib_u4, d_gmax, e->rec_of, d_present);
+  if (v != 0) PRS_CUDA(cudaStreamWaitEvent(st, e->ev_join, 0));
+  VtAgents ag;
+  ag.B = B;
+  ag.lib_u4 = e->lib_u4;
+  ag.threshold = e->thr_dev;
+  ag.loc = e->loc_dev;
+  ag.loc_stride = e->capacity;
+  ag.g_max = d_gmax;
+  ag.ctr = d_ctr;
+  ag.rec_of = e->rec_of;
+  ag.present = d_present;
+  k_vt_decide_append<<<(B + 3) / 4, 128, 0, st>>>(d_key, (const uint8_t*)(ms + M.tpl), (uint4*)e->libs, 0, 0u, d_argmax,
+                                                  d_err, d_rec, e->n_dev, 1, nullptr, ag);
+  PRS_CUDA(cudaGetLastError());
+  if (e->energy_dev) {
+    if (int rc_ = prs_pc_active_invalidate(pc, st)) return rc_;
+    if (pc->dtype == PRS_F32)
+      k_frame_inject<float><<<(B + 127) / 128, 128, 0, st>>>((float*)e->pc_state, e->loc_dev, d_rec, d_argmax, d_err, d_rec,
+                                                             pc->X, pc->Y, pc->Th, 0.0f, e->energy_dev, ag);
+    else
+      k_frame_inject<double><<<(B + 127) / 128, 128, 0, st>>>((double*)e->pc_state, e->loc_dev, d_rec, d_argmax, d_err,
+                                                              d_rec, pc->X, pc->Y, pc->Th, 0.0, e->energy_dev, ag);
+    PRS_CUDA(cudaGetLastError());
+  }
+  k_ens_advance<<<1, 1, 0, st>>>(d_ctr);
+  PRS_CUDA(cudaGetLastError());
+  return PRS_OK;
+}
+
+// as ens_launch: eager first call, capture on the second, replay after
+static int ens_multi_launch(prs_ens_plan* e, int v, cudaStream_t st) {
+  if (e->mready[v]) {
+    PRS_CUDA(cudaGraphLaunch(e->mexec[v], st));
+    return PRS_OK;
+  }
+  if (e->mwarm[v] < 1) {
+    ++e->mwarm[v];
+    return ens_multi_enqueue(e, v, st);
+  }
+  cudaGraph_t g = nullptr;
+  PRS_CUDA(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
+  int rc = ens_multi_enqueue(e, v, st);
+  cudaError_t err = cudaStreamEndCapture(st, &g);
+  if (rc != PRS_OK || err != cudaSuccess) {
+    if (g) cudaGraphDestroy(g);
+    if (rc == PRS_OK) prs_set_error("prs_ens_multi_replay_run: capture failed: %s", cudaGetErrorString(err));
+    return rc != PRS_OK ? rc : PRS_E_CUDA;
+  }
+  err = cudaGraphInstantiate(&e->mexec[v], g, 0);
+  cudaGraphDestroy(g);
+  PRS_CUDA(err);
+  e->mready[v] = true;
+  PRS_CUDA(cudaGraphLaunch(e->mexec[v], st));
+  return PRS_OK;
+}
+
+extern "C" size_t prs_ens_multi_scratch_bytes(const prs_ens_plan* e, int R) {
+  if (!e || R < 1) return 0;
+  return EnsMultiScratch(e->B, R, e->fbytes, (size_t)e->pc->N * (e->pc->dtype == PRS_F32 ? 4 : 8)).bytes;
+}
+
+extern "C" int prs_ens_set_recordings(prs_ens_plan* e, int R, const int* rec_of_dev, void* multi_scratch) {
+  PRS_REQUIRE(e && R >= 1 && rec_of_dev && multi_scratch, "prs_ens_set_recordings: bad argument");
+  for (int i = 0; i < 3; ++i) {
+    if (e->mready[i]) cudaGraphExecDestroy(e->mexec[i]);
+    e->mready[i] = false;
+    e->mwarm[i] = 0;
+  }
+  e->R = R;
+  e->rec_of = rec_of_dev;
+  e->mscratch = (char*)multi_scratch;
+  e->mlay = EnsMultiScratch(e->B, R, e->fbytes, (size_t)e->pc->N * (e->pc->dtype == PRS_F32 ? 4 : 8));
+  return PRS_OK;
+}
+
+extern "C" int prs_ens_multi_replay_run(prs_ens_plan* e, const uint8_t* const* frames, const double* odom,
+                                        const uint8_t* moved, const int* lengths, int T_max, prs_frame_result* results,
+                                        void* stream) {
+  PRS_REQUIRE(e && T_max >= 0 && lengths && (T_max == 0 || (frames && odom && moved && results)),
+              "prs_ens_multi_replay_run: bad argument");
+  PRS_REQUIRE(e->R >= 1, "prs_ens_multi_replay_run: no recordings set (prs_ens_set_recordings)");
+  PRS_REQUIRE(stream != nullptr, "prs_ens_multi_replay_run: needs a non-default stream (the frames replay as CUDA graphs)");
+  const int R = e->R;
+  for (int r = 0; r < R; ++r)
+    PRS_REQUIRE(lengths[r] >= 0 && lengths[r] <= T_max && (lengths[r] == 0 || frames[r]),
+                "prs_ens_multi_replay_run: recording %d has length %d outside [0, %d] or no frames", r, lengths[r], T_max);
+  PRS_REQUIRE(T_max <= e->room,
+              "prs_ens_multi_replay_run: %d frames do not fit the libraries (room for %lld more templates)", T_max, e->room);
+  if (int rc = prs_pc_check_device(e->pc, "prs_ens_multi_replay_run")) return rc;
+  // gate[t][r]: bit 0 = recording r has frame t, bit 1 = and it moved
+  std::vector<uint8_t> gate((size_t)T_max * R);
+  std::vector<uint8_t> variant(T_max);
+  for (int t = 0; t < T_max; ++t) {
+    bool any = false, all = true;
+    for (int r = 0; r < R; ++r) {
+      const bool here = t < lengths[r], mv = here && moved[(size_t)t * R + r] != 0;
+      gate[(size_t)t * R + r] = (uint8_t)((here ? 1 : 0) | (mv ? 2 : 0));
+      any |= mv;
+      all &= mv;
+    }
+    variant[t] = (uint8_t)(!any ? 0 : all ? 1 : 2);
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  char* ms = e->mscratch;
+  const EnsMultiScratch& M = e->mlay;
+  const size_t rec_bytes = (size_t)e->B * sizeof(prs_frame_result);
+  int rc = PRS_OK;
+  for (int c0 = 0; c0 < T_max && rc == PRS_OK; c0 += M.chunk) {
+    const int n = T_max - c0 < M.chunk ? T_max - c0 : M.chunk;
+    for (int r = 0; r < R; ++r) {
+      const int nr = lengths[r] - c0 < n ? lengths[r] - c0 : n;
+      if (nr > 0)
+        PRS_CUDA(cudaMemcpyAsync(ms + M.frames + (size_t)r * M.chunk * e->fbytes, frames[r] + (size_t)c0 * e->fbytes,
+                                 (size_t)nr * e->fbytes, cudaMemcpyHostToDevice, st));
+    }
+    PRS_CUDA(cudaMemcpyAsync(ms + M.odom_chunk, odom + (size_t)c0 * R * 2, (size_t)n * R * 2 * sizeof(double),
+                             cudaMemcpyHostToDevice, st));
+    PRS_CUDA(cudaMemcpyAsync(ms + M.gate, gate.data() + (size_t)c0 * R, (size_t)n * R, cudaMemcpyHostToDevice, st));
+    PRS_CUDA(cudaMemsetAsync(e->scratch + e->lay.misc, 0, sizeof(int), st));  // the frame counter
+    int done = 0;
+    for (; done < n; ++done) {
+      rc = ens_multi_launch(e, variant[c0 + done], st);
+      if (rc != PRS_OK) break;
+    }
+    if (done > 0)
+      PRS_CUDA(cudaMemcpyAsync(results + (size_t)c0 * e->B, ms + M.rec, (size_t)done * rec_bytes, cudaMemcpyDeviceToHost,
+                               st));
+    e->room -= done;
+  }
+  const cudaError_t err = cudaStreamSynchronize(st);
+  if (rc == PRS_OK && err != cudaSuccess) {
+    prs_set_error("prs_ens_multi_replay_run: %s", cudaGetErrorString(err));
     return PRS_E_CUDA;
   }
   return rc;

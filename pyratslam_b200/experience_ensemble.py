@@ -89,7 +89,7 @@ class EnsembleExperienceMaps:
     ``n_experiences``, ``n_links``, ``current`` (-1 = none) and ``n_loop_closures`` are int64 [B] on the host; an
     agent's experiences and links are copied from the device when asked for."""
 
-    def __init__(self, work, B, T, n_templates, moved, tw, pose_size, delta_pc, correction, vt_ids=None):
+    def __init__(self, work, B, T, n_templates, moved, tw, pose_size, delta_pc, correction, vt_ids=None, rec_of=None):
         lay, _ = _work_layout(B, T, n_templates)
         self._vt_ids = vt_ids       # per agent: the caller's template id of each tag, when the ids were renumbered
         self._v = {k: work[o:o + r * B * torch.empty((), dtype=dt).element_size()].view(dt).view(r, B)
@@ -97,7 +97,9 @@ class EnsembleExperienceMaps:
         counts = self._v["counts"].cpu().numpy().astype(np.int64)
         self.n_experiences, self.n_links, self.current, self.n_loop_closures = counts
         self._rel = self._v["rel"].cpu().numpy()
-        self._odom, self._accum = (moved, tw), None     # the shared dead reckoning, computed when a map is rebuilt
+        # the dead reckoning of each recording (rec_of: agent b's column of moved [T,R], tw [T,R,2]), computed when a map
+        # is rebuilt
+        self._odom, self._rec_of, self._accum = (moved, tw), rec_of, {}
         self.pose_size, self.delta_pc, self.correction = tuple(pose_size), delta_pc, correction
 
     def __len__(self):
@@ -133,23 +135,32 @@ class EnsembleExperienceMaps:
 
     def experience_map(self, b):
         """Agent b's map as a host ``ExperienceMap(linked=True)``: ``iterate`` relaxes it, ``update`` continues it."""
-        if self._accum is None:
-            self._accum = dead_reckoning(*self._odom)[2]
+        r = 0 if self._rec_of is None else int(self._rec_of[b])
+        if r not in self._accum:
+            moved, tw = self._odom
+            self._accum[r] = dead_reckoning(*((moved, tw) if self._rec_of is None else (moved[:, r], tw[:, r])))[2]
         return ExperienceMap.from_arrays(self.experiences(b), self.links(b), int(self.current[b]),
-                                         rel=self._rel[:, b], accum=self._accum,
+                                         rel=self._rel[:, b], accum=self._accum[r],
                                          n_loop_closures=int(self.n_loop_closures[b]), pc_dims=self.pose_size,
                                          delta_pc=self.delta_pc, correction=self.correction)
 
 
-def _maps(tpl, flat, moved, tw, pose_size, linked, delta_pc, correction, device=None, vt_ids=None):
+def _maps(tpl, flat, moved, tw, pose_size, linked, delta_pc, correction, device=None, vt_ids=None, rec_of=None):
     """The maps from records in frame-major layout: ``tpl`` int [T,B] (the template of each frame, < 0 = none; the
     kernel's workspace holds a candidate list per id up to the largest), ``flat`` int64 [T,B] (the C-order flat arg-max
-    cell); ``vt_ids``: per agent, the caller's template id of each of its ``tpl`` values, when they were renumbered."""
+    cell); ``vt_ids``: per agent, the caller's template id of each of its ``tpl`` values, when they were renumbered.
+    ``rec_of`` int [B] (several recordings): ``moved`` is [T,R], ``tw`` [T,R,2], and agent b follows ``rec_of[b]``."""
     T, B = tpl.shape
     if not linked:
-        n_exp, em_xy, _ = dead_reckoning(moved, tw)
-        return {"n_exp": np.tile(n_exp, (B, 1)), "em_xy": np.tile(em_xy, (B, 1, 1)),
-                "exp_id": np.tile(n_exp - 1, (B, 1)), "n_loop_closures": np.zeros(B, np.int64), "maps": None}
+        if rec_of is None:
+            n_exp, em_xy, _ = dead_reckoning(moved, tw)
+            return {"n_exp": np.tile(n_exp, (B, 1)), "em_xy": np.tile(em_xy, (B, 1, 1)),
+                    "exp_id": np.tile(n_exp - 1, (B, 1)), "n_loop_closures": np.zeros(B, np.int64), "maps": None}
+        per = [dead_reckoning(moved[:, r], tw[:, r])[:2] for r in range(moved.shape[1])]   # once per recording
+        n_exp = np.stack([per[r][0] for r in rec_of]) if B else np.zeros((0, T), np.int64)
+        em_xy = np.stack([per[r][1] for r in rec_of]) if B else np.zeros((0, T, 2))
+        return {"n_exp": n_exp, "em_xy": em_xy, "exp_id": n_exp - 1, "n_loop_closures": np.zeros(B, np.int64),
+                "maps": None}
     tag = np.full((T, B), -1, np.int32)
     if T > 1:
         tag[1:] = np.maximum(tpl[:-1], -1)
@@ -169,10 +180,19 @@ def _maps(tpl, flat, moved, tw, pose_size, linked, delta_pc, correction, device=
         id_d = torch.empty((T, B), dtype=torch.int32, device=dev)
         xy_d = torch.empty((T, B, 2), dtype=torch.float64, device=dev)
         X, Y, Th = pose_size
-        nat.check(L.prs_em_linked_run(B, T, n_templates, flat_d.data_ptr(), tag_d.data_ptr(), tw_d.data_ptr(),
-                                      moved_d.data_ptr(), X, Y, Th, float(delta_pc), work.data_ptr(), n_d.data_ptr(),
-                                      id_d.data_ptr(), xy_d.data_ptr(), nat.stream_ptr()), "prs_em_linked_run")
-        maps = EnsembleExperienceMaps(work, B, T, n_templates, moved, tw, pose_size, delta_pc, correction, vt_ids)
+        if rec_of is None:
+            nat.check(L.prs_em_linked_run(B, T, n_templates, flat_d.data_ptr(), tag_d.data_ptr(), tw_d.data_ptr(),
+                                          moved_d.data_ptr(), X, Y, Th, float(delta_pc), work.data_ptr(),
+                                          n_d.data_ptr(), id_d.data_ptr(), xy_d.data_ptr(), nat.stream_ptr()),
+                      "prs_em_linked_run")
+        else:
+            rec_d = torch.from_numpy(np.asarray(rec_of, dtype=np.int32)).to(dev)
+            nat.check(L.prs_em_linked_multi_run(B, T, n_templates, flat_d.data_ptr(), tag_d.data_ptr(), moved.shape[1],
+                                                tw_d.data_ptr(), moved_d.data_ptr(), rec_d.data_ptr(), X, Y, Th,
+                                                float(delta_pc), work.data_ptr(), n_d.data_ptr(), id_d.data_ptr(),
+                                                xy_d.data_ptr(), nat.stream_ptr()), "prs_em_linked_multi_run")
+        maps = EnsembleExperienceMaps(work, B, T, n_templates, moved, tw, pose_size, delta_pc, correction, vt_ids,
+                                      rec_of)
         out = {"n_exp": n_d.cpu().numpy().T.astype(np.int64), "exp_id": id_d.cpu().numpy().T.astype(np.int64),
                "em_xy": xy_d.cpu().numpy().transpose(1, 0, 2), "n_loop_closures": maps.n_loop_closures.copy(),
                "maps": maps}

@@ -8,7 +8,11 @@ experience map.  The frames and the odometry are shared, so a frame is one CUDA 
 (``prs_ens_replay_run``, csrc/view_templates.cu): one pose-cell update of all B networks, one query, one sweep over
 every agent's library, then the per-agent create-or-match decision and injection.
 
-    python -m pyratslam_b200.ros_ensemble BAG --match-threshold 30000,45000,60000 --global-inhibition 0.1,0.2
+Tuning on several recordings keeps the settings from fitting one route: with ``frames`` and ``odom`` given as lists of
+R recordings, agent ``b`` replays recording ``recording[b]`` (``prs_ens_multi_replay_run``), still in one graph per
+frame.
+
+    python -m pyratslam_b200.ros_ensemble BAG [BAG ...] --match-threshold 30000,45000,60000 --global-inhibition 0.1,0.2
 """
 from __future__ import annotations
 
@@ -85,6 +89,41 @@ def capacity_for(T):
     return (int(T) + 1 + 31) // 32 * 32
 
 
+def agent_recordings(recording, B, n_recordings):
+    """int64 [B]: the recording each agent replays, from ``recording`` = one index or a length-B sequence of indices into
+    the ``n_recordings`` recordings (no CUDA involved).  ``ValueError`` for a length other than B and for anything that is
+    not an integer in [0, n_recordings)."""
+    if isinstance(recording, (numbers.Integral, np.integer)) and not isinstance(recording, (bool, np.bool_)):
+        rec = [recording] * B
+    else:
+        try:
+            rec = list(recording)
+        except TypeError:
+            raise ValueError("recording must be an index or a sequence of indices, got %r" % (recording,)) from None
+        if len(rec) != B:
+            raise ValueError("recording has %d values for %d agents" % (len(rec), B))
+    for r in rec:
+        if (not isinstance(r, (numbers.Integral, np.integer)) or isinstance(r, (bool, np.bool_))
+                or not 0 <= int(r) < n_recordings):
+            raise ValueError("recording must be indices in [0, %d), got %r" % (n_recordings, r))
+    return np.array(rec, dtype=np.int64)
+
+
+def _recording_count(recording):
+    """The agent count a sequence ``recording`` implies, None for a scalar."""
+    if recording is None or isinstance(recording, (numbers.Number, np.number, str, bytes)):
+        return None
+    try:
+        return len(recording)
+    except TypeError:
+        return None
+
+
+def _multi_chunk(R, frame_bytes):
+    """Frames per recording in one device chunk (prs_ens_multi_scratch_bytes): 256 MiB over R recordings, in [1, 256]."""
+    return int(min(max((256 << 20) // (R * frame_bytes), 1), 256))
+
+
 def _unravel(flat, shape):
     X, Y, Th = shape
     flat = np.asarray(flat, dtype=np.int64)
@@ -133,7 +172,7 @@ class EnsembleAgents:
 
 def replay_ensemble(frames, odom, n_agents=None, match_threshold=MATCH_THRESHOLD, global_inhibition=PC_GLOBAL_INHIB,
                     inject_energy=None, pose_size=POSE_SIZE, dtype=np.float32, active_set=0, experience_map=False,
-                    experience_links=False, mode="ref"):
+                    experience_links=False, mode="ref", recording=0):
     """Replay ``frames[T,256,256]`` (uint8) and ``odom[T,2]`` = (linear.x, angular.z) through B agents.
 
     ``match_threshold``, ``global_inhibition`` and ``inject_energy`` (None = no injection, else a finite energy >= 0)
@@ -148,13 +187,26 @@ def replay_ensemble(frames, odom, n_agents=None, match_threshold=MATCH_THRESHOLD
     ``experience_map="device"`` builds the maps with ``experience_ensemble``: with ``experience_links=True`` every
     agent's linked map on the device, next to ``n_exp`` and ``em_xy`` also ``exp_id [B,T]`` (the current experience),
     ``n_loop_closures [B]`` and ``maps`` (``EnsembleExperienceMaps``); without links the shared dead reckoning once
-    (``maps`` None).  Any other value than False, True or "device" raises ``ValueError``."""
+    (``maps`` None).  Any other value than False, True or "device" raises ``ValueError``.
+
+    Several recordings: ``frames`` and ``odom`` are lists of R arrays ``[T_r,256,256]`` uint8 and ``[T_r,2]``, and
+    ``recording`` (an index or a length-B sequence, broadcast like the parameters) names the one each agent replays.
+    Agent b's outputs equal those of ``replay_ensemble`` on its own recording, or ``replay(native=True)``; the arrays are
+    ``[B, T_max]`` with ``length [B]`` (the agent's recording's frame count), and past an agent's length ``template`` and
+    ``argmax`` are -1, ``created`` False, ``n_exp`` and ``exp_id`` -1 and ``em_xy`` NaN.  A pose-cell error raises what
+    the native replay of that recording raises, for the earliest frame and, within it, the lowest agent.  With single
+    arrays ``recording`` can only be 0."""
     if not (isinstance(experience_map, (bool, np.bool_))
             or (isinstance(experience_map, str) and experience_map == "device")):
         raise ValueError("experience_map must be False, True or 'device', got %r" % (experience_map,))
-    B, thr, gi, energies = agent_parameters(n_agents, match_threshold, global_inhibition, inject_energy)
+    B, thr, gi, energies = agent_parameters(n_agents if n_agents is not None else _recording_count(recording),
+                                            match_threshold, global_inhibition, inject_energy)
     if mode != "ref":
         raise ValueError("replay_ensemble supports the reference matching mode only, got mode=%r" % (mode,))
+    if isinstance(frames, (list, tuple)) and (len(frames) == 0 or np.ndim(frames[0]) == 3):
+        return _replay_recordings(frames, odom, agent_recordings(recording, B, max(len(frames), 1)), thr, gi, energies,
+                                  pose_size, dtype, active_set, experience_map, experience_links)
+    agent_recordings(recording, B, 1)
     frames = np.asarray(frames)
     odom = np.asarray(odom, dtype=np.float64)
     T = len(frames)
@@ -225,22 +277,137 @@ def replay_ensemble(frames, odom, n_agents=None, match_threshold=MATCH_THRESHOLD
     return out
 
 
-def _experience_maps(out, moved, tw, pose_size, linked):
-    """Each agent's experience map replayed from its records (``RatslamRos.replay_native``'s bookkeeping)."""
+def _experience_maps(out, moved, tw, pose_size, linked, rec_of=None):
+    """Each agent's experience map replayed from its records (``RatslamRos.replay_native``'s bookkeeping); with
+    ``rec_of``, ``moved [T,R]`` and ``tw [T,R,2]`` hold every recording's odometry and agent b follows ``rec_of[b]``."""
     B, T = out["template"].shape
     n_exp = np.zeros((B, T), np.int64)
     em_xy = np.zeros((B, T, 2))
     for b in range(B):
         em = ExperienceMap(linked=linked, pc_dims=pose_size)
         tpl, amax = out["template"][b], out["argmax"][b]
+        mv, tws = (moved, tw) if rec_of is None else (moved[:, rec_of[b]], tw[:, rec_of[b]])
         for t in range(T):
-            if moved[t]:
+            if mv[t]:
                 vt = int(tpl[t - 1]) if t > 0 else None
-                em.update(float(tw[t, 0]), float(tw[t, 1]), tuple(int(c) for c in amax[t]), vt if linked else None)
+                em.update(float(tws[t, 0]), float(tws[t, 1]), tuple(int(c) for c in amax[t]), vt if linked else None)
             n_exp[b, t] = len(em.experiences)
             if em.current_exp is not None:
                 em_xy[b, t] = em.get_current_point()
     return n_exp, em_xy
+
+
+def _replay_recordings(frames, odom, rec_of, thr, gi, energies, pose_size, dtype, active_set, experience_map,
+                       experience_links):
+    """replay_ensemble over R recordings: agent b replays ``frames[rec_of[b]]``, ``odom[rec_of[b]]``."""
+    R = len(frames)
+    if not isinstance(odom, (list, tuple)) or len(odom) != R or R == 0:
+        raise ValueError("replay_ensemble: frames and odom must be lists of the same, non-zero number of recordings, "
+                         "got %d and %s" % (R, len(odom) if isinstance(odom, (list, tuple)) else type(odom).__name__))
+    fr, od = [], []
+    for r in range(R):
+        f, o = np.asarray(frames[r]), np.asarray(odom[r], dtype=np.float64)
+        if f.dtype != np.uint8 or f.ndim != 3 or tuple(f.shape[1:]) != IM_SIZE or o.shape != (len(f), 2):
+            raise ValueError("replay_ensemble: recording %d: frames must be uint8 [T,%d,%d] and odom [T,2], got %s %r "
+                             "and %r" % (r, IM_SIZE[0], IM_SIZE[1], f.dtype, f.shape, o.shape))
+        fr.append(np.ascontiguousarray(f))
+        od.append(o)
+    B = len(rec_of)
+    lengths = np.array([len(f) for f in fr], dtype=np.int32)
+    T = int(lengths.max())
+    pose_size = tuple(int(s) for s in pose_size)
+    np_dtype = _as_np_dtype(dtype)
+    cap = capacity_for(T)
+    if cap > MAX_CAPACITY:
+        raise ValueError("replay_ensemble: %d frames need %d templates per agent; the library sweep takes at most %d"
+                         % (T, cap, MAX_CAPACITY))
+    lib_bytes = (cap // 32) * 34816
+    net_bytes = int(np.prod(pose_size)) * np.dtype(np_dtype).itemsize
+    frame_bytes = IM_SIZE[0] * IM_SIZE[1]
+    # per agent: library, locations, network, its snapshot and the records; plus one chunk of every recording's frames
+    need = B * (lib_bytes + cap * 8 + 2 * net_bytes + 64) + R * _multi_chunk(R, frame_bytes) * frame_bytes
+    if experience_map == "device" and experience_links:
+        need += xens.work_bytes(B, T, cap) + xens.record_bytes(B, T)
+    nat.require_cuda()
+    dev = torch.device("cuda", torch.cuda.current_device())
+    free, _ = torch.cuda.mem_get_info(dev)
+    if need > free:
+        raise ValueError("replay_ensemble: %d agents x %d templates need %.2f GB of device memory, %.2f GB are free"
+                         % (B, cap, need / 1e9, free / 1e9))
+
+    # the agents of one recording get contiguous indices on the device (the sweep reloads a query per recording change)
+    order = np.argsort(rec_of, kind="stable")
+    inv = np.argsort(order)
+    ens = PoseCellEnsemble(pose_size, B, global_inhibition=gi[order], dtype=np_dtype, device=dev, active_set=active_set)
+    ens.inject(1, tuple(math.floor(s / 2) for s in pose_size))         # RatslamRos.__init__
+    L = nat.lib()
+    assert int(L.prs_vt_packed_bytes(cap)) == lib_bytes
+    libs = torch.zeros((B, lib_bytes), dtype=torch.uint8, device=dev)
+    loc = torch.full((B, cap), -1, dtype=torch.int64, device=dev)
+    n_dev = torch.zeros(B, dtype=torch.int32, device=dev)
+    thr_dev = torch.from_numpy(thr[order].view(np.int32)).to(dev)
+    injecting = any(e is not None for e in energies)
+    energy_dev = torch.tensor([-1.0 if energies[i] is None else energies[i] for i in order], dtype=torch.float64,
+                              device=dev)
+    rec_dev = torch.from_numpy(rec_of[order].astype(np.int32)).to(dev)
+    pc_work = torch.zeros(3 * B, dtype=torch.int64, device=dev)
+    scratch = torch.empty(int(L.prs_ens_scratch_bytes(B, IM_SIZE[0], IM_SIZE[1])), dtype=torch.uint8, device=dev)
+    moved = np.zeros((T, R), np.uint8)             # past a recording's end: not moved
+    tw = np.zeros((T, R, 2))
+    for r in range(R):
+        moved[:lengths[r], r], tw[:lengths[r], r] = xens.gate(od[r])
+    res = np.zeros((T, B), dtype=RatslamRos._RESULT_DTYPE)
+    stream = torch.cuda.Stream(device=dev)
+    plan = ctypes.c_void_p()
+    frame_ptrs = (ctypes.c_void_p * R)(*[f.ctypes.data if len(f) else None for f in fr])
+    with torch.cuda.device(dev):
+        nat.check(L.prs_pc_argmax(ens._h, ens.state.data_ptr(), pc_work.data_ptr(), nat.stream_ptr()), "prs_pc_argmax")
+        torch.cuda.current_stream(dev).synchronize()
+        nat.check(L.prs_ens_create(
+            ens._h, ens.state.data_ptr(), ens._gi.data_ptr(), pc_work.data_ptr(), libs.data_ptr(), cap, n_dev.data_ptr(),
+            thr_dev.data_ptr(), energy_dev.data_ptr() if injecting else None, loc.data_ptr(), nat.VT_MODE_REF,
+            IM_SIZE[0], IM_SIZE[1], Y_RANGE[0], Y_RANGE[1], Y_STEP, X_RANGE[0], X_RANGE[1], X_STEP, scratch.data_ptr(),
+            ctypes.byref(plan)), "prs_ens_create")
+        try:
+            mscratch = torch.empty(int(L.prs_ens_multi_scratch_bytes(plan, R)), dtype=torch.uint8, device=dev)
+            nat.check(L.prs_ens_set_recordings(plan, R, rec_dev.data_ptr(), mscratch.data_ptr()),
+                      "prs_ens_set_recordings")
+            nat.check(L.prs_ens_multi_replay_run(plan, frame_ptrs, tw.ctypes.data, moved.ctypes.data, lengths.ctypes.data,
+                                                 T, res.ctypes.data, ctypes.c_void_p(stream.cuda_stream)),
+                      "prs_ens_multi_replay_run")
+        finally:
+            L.prs_ens_destroy(plan)
+        # back to the caller's agent order
+        inv_d = torch.from_numpy(inv).to(dev)
+        ens.state.copy_(ens.state[inv_d])
+        ens.global_inhibition = gi
+        nat.check(L.prs_pc_invalidate_active(ens._h, nat.stream_ptr()), "prs_pc_invalidate_active")
+        libs, loc = libs[inv_d], loc[inv_d]
+    res = np.ascontiguousarray(res[:, inv])
+    agent_moved = moved[:, rec_of]                  # [T, B]
+    bad = ((res["pc_err"] & ~nat.ERR_INJECT_LOC) != 0) & (agent_moved != 0)
+    if bad.any():
+        t, b = np.argwhere(bad)[0]                  # frame-major: the earliest frame, then the lowest agent
+        ens._raise_on_err(np.array([res["pc_err"][t, b] & ~nat.ERR_INJECT_LOC], dtype=np.int32))
+    length = lengths[rec_of].astype(np.int64)
+    past = np.arange(T)[None, :] >= length[:, None]  # [B, T]
+    n_templates = res["n_templates"][-1].astype(np.int64) if T else np.zeros(B, np.int64)
+    argmax = _unravel(res["argmax"].T, pose_size)
+    argmax[past] = -1
+    out = {"template": res["template_index"].T.astype(np.int64), "created": res["created"].T != 0, "argmax": argmax,
+           "n_templates": n_templates, "length": length,
+           "agents": EnsembleAgents(ens, libs, loc, n_templates, pose_size)}
+    if experience_map == "device":
+        out.update(xens._maps(res["template_index"], np.ascontiguousarray(res["argmax"]), moved, tw, pose_size,
+                              experience_links, 1.0, 0.5, dev, rec_of=rec_of))
+    elif experience_map:
+        out["n_exp"], out["em_xy"] = _experience_maps(out, moved, tw, pose_size, experience_links, rec_of)
+    if experience_map:
+        for k in ("n_exp", "exp_id"):
+            if k in out:
+                out[k][past] = -1
+        out["em_xy"][past] = np.nan
+    return out
 
 
 def _list(text, parse):
@@ -249,9 +416,9 @@ def _list(text, parse):
 
 def main(argv=None):
     import argparse
-    ap = argparse.ArgumentParser(description="Replay a ROS1 bag through an ensemble of RatSLAM agents: the cross "
-                                             "product of the given parameter lists, one agent per combination")
-    ap.add_argument("bag")
+    ap = argparse.ArgumentParser(description="Replay ROS1 bags through an ensemble of RatSLAM agents: the cross product "
+                                             "of the bags and the given parameter lists, one agent per combination")
+    ap.add_argument("bag", nargs="+")
     ap.add_argument("--match-threshold", default=str(MATCH_THRESHOLD), metavar="T1,T2,...")
     ap.add_argument("--global-inhibition", default="0.2", metavar="G1,G2,...")
     ap.add_argument("--inject-energy", default="none", metavar="E1,E2,...",
@@ -267,17 +434,25 @@ def main(argv=None):
     gis = _list(a.global_inhibition, float)
     ens = _list(a.inject_energy, lambda s: None if s.lower() == "none" else float(s))
     combos = list(itertools.product(thr, gis, ens))
-    frames, odom, _ = rb.events_to_arrays(rb.read_events(a.bag, image_topic=a.image_topic, odom_topic=a.odom_topic))
-    out = replay_ensemble(frames, odom, n_agents=len(combos), match_threshold=[c[0] for c in combos],
-                          global_inhibition=[c[1] for c in combos], inject_energy=[c[2] for c in combos],
-                          experience_map="device" if a.experience_links else False,
-                          experience_links=a.experience_links)
-    T = len(frames)
-    for b, (t, g, e) in enumerate(combos):
-        last = tuple(int(c) for c in out["argmax"][b, -1]) if T else None
+    recs = [rb.events_to_arrays(rb.read_events(bag, image_topic=a.image_topic, odom_topic=a.odom_topic))[:2]
+            for bag in a.bag]
+    several = len(a.bag) > 1
+    agents = list(itertools.product(range(len(a.bag)), combos))     # bag-major
+    kw = dict(n_agents=len(agents), match_threshold=[c[0] for _, c in agents],
+              global_inhibition=[c[1] for _, c in agents], inject_energy=[c[2] for _, c in agents],
+              experience_map="device" if a.experience_links else False, experience_links=a.experience_links)
+    if several:
+        out = replay_ensemble([f for f, _ in recs], [o for _, o in recs], recording=[r for r, _ in agents], **kw)
+    else:
+        out = replay_ensemble(recs[0][0], recs[0][1], **kw)
+    for b, (r, (t, g, e)) in enumerate(agents):
+        T = len(recs[r][0])
+        last = tuple(int(c) for c in out["argmax"][b, T - 1]) if T else None
         line = ("agent %d  match_threshold %g  global_inhibition %g  inject_energy %s:  templates %d  created %d/%d  "
                 "final arg-max %s" % (b, t, g, "none" if e is None else "%g" % e, out["n_templates"][b],
                                       int(out["created"][b].sum()), T, last))
+        if several:
+            line = "bag %s  %s" % (a.bag[r], line)
         if a.experience_links:
             line += "  experiences %d  loop closures %d" % (out["maps"].n_experiences[b], out["n_loop_closures"][b])
         print(line)
