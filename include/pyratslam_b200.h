@@ -398,6 +398,10 @@ PRS_API int prs_ens_create(prs_pc_handle pc, void* pc_state, const void* gi, voi
                    int im_rows, int im_cols, int row_lo, int row_hi, int row_step, int col_lo, int col_hi,
                    int col_step, void* scratch, prs_ens_plan** out);
 PRS_API int prs_ens_destroy(prs_ens_plan* plan);
+/* The room for T more frames that the runs below check is counted in frames (one template per agent and frame at most)
+ * and decremented by every run.  prs_ens_refresh_room recounts it from n_dev as the libraries are now, so a plan fed in
+ * pieces whose agents match more than they create keeps going without a new plan.  Synchronises `stream`. */
+PRS_API int prs_ens_refresh_room(prs_ens_plan* plan, void* stream);
 /* The loop of prs_replay_run for the ensemble.  Frames and odometry go to the device and the records come back in
  * chunks of 256 frames; nothing per agent crosses the bus per frame.  Returns after one final synchronisation of
  * `stream` (a non-default stream).  PRS_E_INVALID when the libraries have no room for T more templates.
@@ -474,6 +478,26 @@ PRS_API int prs_em_linked_run(int B, int T, int n_templates, const long long* ar
 PRS_API int prs_em_linked_multi_run(int B, int T, int n_templates, const long long* argmax, const int* tag, int R,
                             const double* tw, const uint8_t* moved, const int* rec_of, int X, int Y, int Th,
                             double delta_pc, void* work, int* n_exp, int* exp_id, double* em_xy, void* stream);
+
+/* Maps that continue across calls (an ensemble session fed in pieces).  The session workspace is the layout above with
+ * the rows keyed by capacities instead of T -- E rows for each experience and link array, N rows of vt_head -- followed
+ * by one int32 error word at byte offset prs_em_work_bytes(B, E, N).  Each moved frame adds at most one experience and
+ * one link, so the caller keeps E >= max(experiences, links) so far + the frames of the next call, and N above every tag.
+ *   prs_em_session_bytes(B, E, N): device bytes of such a workspace.
+ *   prs_em_session_init: an empty map for every agent (vt_head -1, counts (0, 0, -1, 0), rel 0, error word 0).
+ *   prs_em_session_grow: copies the maps of `src` (layout B, E0, N0) into `dst` (B, E1, N1; E1 >= E0, N1 >= N0, not
+ *            overlapping src) and fills the new vt_head rows with -1; asynchronous on `stream`.
+ *   prs_em_linked_resume_run: prs_em_linked_multi_run continued over T more frames: the counts, rel and the current
+ *            experience's pose come from the workspace and go back to it, vt_head is not reset.  rec_of may be NULL for
+ *            R = 1.  A moved frame of an agent that has no room for one more experience and link, or whose tag is >= N,
+ *            sets the error word to 1 and stops that agent: nothing is written past E or N, and the caller reads the
+ *            word after the call. */
+PRS_API size_t prs_em_session_bytes(int B, int E, int N);
+PRS_API int prs_em_session_init(int B, int E, int N, void* work, void* stream);
+PRS_API int prs_em_session_grow(int B, int E0, int N0, int E1, int N1, const void* src, void* dst, void* stream);
+PRS_API int prs_em_linked_resume_run(int B, int T, int E, int N, const long long* argmax, const int* tag, int R,
+                             const double* tw, const uint8_t* moved, const int* rec_of, int X, int Y, int Th,
+                             double delta_pc, void* work, int* n_exp, int* exp_id, double* em_xy, void* stream);
 
 #ifdef __cplusplus
 }

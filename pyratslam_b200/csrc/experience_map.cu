@@ -65,21 +65,33 @@ struct EmWork {
   int *exp_tag, *exp_next, *out_head, *link_from, *link_to, *link_next, *vt_head, *counts;
 };
 
+// kResume = false: T frames from an empty map (prs_em_linked_run).  kResume = true (prs_em_linked_resume_run): the map
+// the workspace holds -- counts, rel and the current experience's pose -- continues over T more frames; the workspace has
+// E rows for the experiences and links and N template heads, and a moved frame that finds no room for one more of each,
+// or a tag at or beyond N, sets *err and stops the agent instead of writing past them.
+template <bool kResume>
 __global__ void __launch_bounds__(kEmBlock)
     k_em_linked(int B, int T, int N, const long long* __restrict__ argmax, const int* __restrict__ tag,
                 const double* __restrict__ tw, const uint8_t* __restrict__ moved, int X, int Y, int Th,
                 double delta_pc, EmWork w, int* __restrict__ n_exp_out, int* __restrict__ exp_id_out,
-                double* __restrict__ em_xy_out, int R = 1, const int* __restrict__ rec_of = nullptr) {
+                double* __restrict__ em_xy_out, int R = 1, const int* __restrict__ rec_of = nullptr, int E = 0,
+                int* __restrict__ err = nullptr) {
   // rec_of (several recordings): agent b follows recording r = rec_of[b] of tw[T][R][2] and moved[T][R]
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
   const int r = rec_of != nullptr ? rec_of[b] : 0;
   if (rec_of == nullptr) R = 1;
   const size_t sB = (size_t)B;
-  for (int v = 0; v < N; ++v) w.vt_head[v * sB + b] = -1;
+  if (!kResume)
+    for (int v = 0; v < N; ++v) w.vt_head[v * sB + b] = -1;
   int n_exp = 0, n_links = 0, cur = -1, n_loop = 0;
   double rel_x = 0.0, rel_y = 0.0, rel_th = 0.0;
   double cur_x = 0.0, cur_y = 0.0, cur_th = 0.0;   // the current experience's pose, kept in registers
+  if (kResume) {
+    n_exp = w.counts[b], n_links = w.counts[sB + b], cur = w.counts[2 * sB + b], n_loop = w.counts[3 * sB + b];
+    rel_x = w.rel[b], rel_y = w.rel[sB + b], rel_th = w.rel[2 * sB + b];
+    if (cur >= 0) cur_x = w.exp_x[cur * sB + b], cur_y = w.exp_y[cur * sB + b], cur_th = w.exp_th[cur * sB + b];
+  }
   const int YTh = Y * Th;
 
   // _add_link(current, to) without the duplicate check, with the agent's rel_* at this point
@@ -104,6 +116,10 @@ __global__ void __launch_bounds__(kEmBlock)
     const size_t tb = t * sB + b;
     const size_t tr = (size_t)t * R + r;
     if (moved[tr]) {
+      if (kResume && (n_exp >= E || n_links >= E || tag[tb] >= N)) {
+        atomicOr(err, 1);
+        break;
+      }
       // update(): the odometry since the current experience
       const double vtrans = tw[2 * tr], vrot = tw[2 * tr + 1];
       rel_th = clip_rad_180(__dadd_rn(rel_th, vrot));
@@ -170,6 +186,16 @@ extern "C" size_t prs_em_work_bytes(int B, int T, int n_templates) {
   return EmLayout(B, T, n_templates).bytes;
 }
 
+static EmWork em_work(void* work, const EmLayout& L) {
+  char* p = (char*)work;
+  return EmWork{(double*)(p + L.exp_x),     (double*)(p + L.exp_y),       (double*)(p + L.exp_th),
+                (double*)(p + L.link_d),    (double*)(p + L.link_heading), (double*)(p + L.link_facing),
+                (double*)(p + L.rel),       (long long*)(p + L.exp_cell), (int*)(p + L.exp_tag),
+                (int*)(p + L.exp_next),     (int*)(p + L.out_head),      (int*)(p + L.link_from),
+                (int*)(p + L.link_to),      (int*)(p + L.link_next),     (int*)(p + L.vt_head),
+                (int*)(p + L.counts)};
+}
+
 static int em_linked_launch(const char* who, int B, int T, int n_templates, const long long* argmax, const int* tag,
                             int R, const double* tw, const uint8_t* moved, const int* rec_of, int X, int Y, int Th,
                             double delta_pc, void* work, int* n_exp, int* exp_id, double* em_xy, void* stream) {
@@ -178,15 +204,8 @@ static int em_linked_launch(const char* who, int B, int T, int n_templates, cons
   PRS_REQUIRE(X >= 1 && Y >= 1 && Th >= 1 && (long long)X * Y * Th <= (1LL << 30), "%s: bad grid %d x %d x %d", who, X, Y,
               Th);
   PRS_REQUIRE(work && (T == 0 || (argmax && tag && tw && moved && n_exp && exp_id && em_xy)), "%s: null argument", who);
-  const EmLayout L(B, T, n_templates);
-  char* p = (char*)work;
-  const EmWork w{(double*)(p + L.exp_x),     (double*)(p + L.exp_y),       (double*)(p + L.exp_th),
-                 (double*)(p + L.link_d),    (double*)(p + L.link_heading), (double*)(p + L.link_facing),
-                 (double*)(p + L.rel),       (long long*)(p + L.exp_cell), (int*)(p + L.exp_tag),
-                 (int*)(p + L.exp_next),     (int*)(p + L.out_head),      (int*)(p + L.link_from),
-                 (int*)(p + L.link_to),      (int*)(p + L.link_next),     (int*)(p + L.vt_head),
-                 (int*)(p + L.counts)};
-  k_em_linked<<<(B + kEmBlock - 1) / kEmBlock, kEmBlock, 0, (cudaStream_t)stream>>>(
+  const EmWork w = em_work(work, EmLayout(B, T, n_templates));
+  k_em_linked<false><<<(B + kEmBlock - 1) / kEmBlock, kEmBlock, 0, (cudaStream_t)stream>>>(
       B, T, n_templates, argmax, tag, tw, moved, X, Y, Th, delta_pc, w, n_exp, exp_id, em_xy, R, rec_of);
   PRS_CUDA(cudaGetLastError());
   return PRS_OK;
@@ -206,4 +225,71 @@ extern "C" int prs_em_linked_multi_run(int B, int T, int n_templates, const long
   PRS_REQUIRE(rec_of != nullptr || T == 0, "prs_em_linked_multi_run: null rec_of");
   return em_linked_launch("prs_em_linked_multi_run", B, T, n_templates, argmax, tag, R, tw, moved, rec_of, X, Y, Th,
                           delta_pc, work, n_exp, exp_id, em_xy, stream);
+}
+
+// ---------------------------------------------------------------------------------------------
+// Sessions: a map workspace that lives across calls (prs_em_session_*, prs_em_linked_resume_run).  The layout is
+// EmLayout(B, E, N) -- E rows of experiences and links, N template heads -- followed by one int32 error word.
+
+extern "C" size_t prs_em_session_bytes(int B, int E, int N) {
+  if (B < 1 || E < 0 || N < 0) return 0;
+  return EmLayout(B, E, N).bytes + 256;
+}
+
+extern "C" int prs_em_session_init(int B, int E, int N, void* work, void* stream) {
+  PRS_REQUIRE(B >= 1 && E >= 0 && N >= 0 && work, "prs_em_session_init: bad argument B=%d E=%d N=%d", B, E, N);
+  const EmLayout L(B, E, N);
+  char* p = (char*)work;
+  const cudaStream_t st = (cudaStream_t)stream;
+  const size_t sB = (size_t)B;
+  PRS_CUDA(cudaMemsetAsync(p + L.vt_head, 0xFF, (size_t)N * sB * 4, st));          // -1: no experience yet
+  PRS_CUDA(cudaMemsetAsync(p + L.rel, 0, 3 * sB * 8, st));
+  PRS_CUDA(cudaMemsetAsync(p + L.counts, 0, 4 * sB * 4, st));
+  PRS_CUDA(cudaMemsetAsync(p + L.counts + 2 * sB * 4, 0xFF, sB * 4, st));        // current experience: none
+  PRS_CUDA(cudaMemsetAsync(p + L.bytes, 0, 4, st));                                // the error word
+  return PRS_OK;
+}
+
+extern "C" int prs_em_session_grow(int B, int E0, int N0, int E1, int N1, const void* src, void* dst, void* stream) {
+  PRS_REQUIRE(B >= 1 && E0 >= 0 && N0 >= 0 && E1 >= E0 && N1 >= N0 && src && dst && src != dst,
+              "prs_em_session_grow: bad argument B=%d E %d -> %d N %d -> %d", B, E0, E1, N0, N1);
+  const EmLayout A(B, E0, N0), Z(B, E1, N1);
+  const char* s = (const char*)src;
+  char* d = (char*)dst;
+  const cudaStream_t st = (cudaStream_t)stream;
+  const size_t sB = (size_t)B;
+  // element [i][b] is at i * B + b in both layouts, so each array's old rows are one contiguous prefix
+  const struct { size_t from, to, bytes; } arrays[] = {
+      {A.exp_x, Z.exp_x, E0 * sB * 8},         {A.exp_y, Z.exp_y, E0 * sB * 8},
+      {A.exp_th, Z.exp_th, E0 * sB * 8},       {A.link_d, Z.link_d, E0 * sB * 8},
+      {A.link_heading, Z.link_heading, E0 * sB * 8}, {A.link_facing, Z.link_facing, E0 * sB * 8},
+      {A.rel, Z.rel, 3 * sB * 8},              {A.exp_cell, Z.exp_cell, E0 * sB * 8},
+      {A.exp_tag, Z.exp_tag, E0 * sB * 4},     {A.exp_next, Z.exp_next, E0 * sB * 4},
+      {A.out_head, Z.out_head, E0 * sB * 4},   {A.link_from, Z.link_from, E0 * sB * 4},
+      {A.link_to, Z.link_to, E0 * sB * 4},     {A.link_next, Z.link_next, E0 * sB * 4},
+      {A.vt_head, Z.vt_head, N0 * sB * 4},     {A.counts, Z.counts, 4 * sB * 4},
+      {A.bytes, Z.bytes, 4}};
+  for (const auto& a : arrays)
+    if (a.bytes) PRS_CUDA(cudaMemcpyAsync(d + a.to, s + a.from, a.bytes, cudaMemcpyDeviceToDevice, st));
+  if (N1 > N0) PRS_CUDA(cudaMemsetAsync(d + Z.vt_head + N0 * sB * 4, 0xFF, (size_t)(N1 - N0) * sB * 4, st));
+  return PRS_OK;
+}
+
+extern "C" int prs_em_linked_resume_run(int B, int T, int E, int N, const long long* argmax, const int* tag, int R,
+                                        const double* tw, const uint8_t* moved, const int* rec_of, int X, int Y, int Th,
+                                        double delta_pc, void* work, int* n_exp, int* exp_id, double* em_xy,
+                                        void* stream) {
+  PRS_REQUIRE(B >= 1 && T >= 0 && E >= 0 && N >= 0 && R >= 1 && (R == 1 || rec_of || T == 0),
+              "prs_em_linked_resume_run: bad size B=%d T=%d E=%d N=%d R=%d (rec_of is needed for R > 1)", B, T, E, N, R);
+  PRS_REQUIRE(X >= 1 && Y >= 1 && Th >= 1 && (long long)X * Y * Th <= (1LL << 30),
+              "prs_em_linked_resume_run: bad grid %d x %d x %d", X, Y, Th);
+  PRS_REQUIRE(work && (T == 0 || (argmax && tag && tw && moved && n_exp && exp_id && em_xy)),
+              "prs_em_linked_resume_run: null argument");
+  if (T == 0) return PRS_OK;
+  const EmLayout L(B, E, N);
+  k_em_linked<true><<<(B + kEmBlock - 1) / kEmBlock, kEmBlock, 0, (cudaStream_t)stream>>>(
+      B, T, N, argmax, tag, tw, moved, X, Y, Th, delta_pc, em_work(work, L), n_exp, exp_id, em_xy, R, rec_of, E,
+      (int*)((char*)work + L.bytes));
+  PRS_CUDA(cudaGetLastError());
+  return PRS_OK;
 }

@@ -2247,6 +2247,22 @@ extern "C" int prs_ens_create(prs_pc_handle pc, void* pc_state, const void* gi, 
   return PRS_OK;
 }
 
+// Room counts frames, not templates (a run may append one per frame); a session that feeds a plan in pieces recounts
+// it from the libraries as they are after the earlier runs.
+extern "C" int prs_ens_refresh_room(prs_ens_plan* e, void* stream) {
+  PRS_REQUIRE(e && stream, "prs_ens_refresh_room: bad argument");
+  const cudaStream_t st = (cudaStream_t)stream;
+  int* misc = (int*)(e->scratch + e->lay.misc);
+  int n = 0;
+  PRS_CUDA(cudaMemsetAsync(misc + 2, 0, sizeof(int), st));
+  k_ens_init<<<1, 256, 0, st>>>(e->n_dev, e->B, misc);  // the group maximum it raises is already at least as high
+  PRS_CUDA(cudaGetLastError());
+  PRS_CUDA(cudaMemcpyAsync(&n, misc + 2, sizeof(int), cudaMemcpyDeviceToHost, st));
+  PRS_CUDA(cudaStreamSynchronize(st));
+  e->room = (long long)e->capacity - n;
+  return PRS_OK;
+}
+
 extern "C" int prs_ens_destroy(prs_ens_plan* e) {
   if (e) {
     for (int i = 0; i < 2; ++i)

@@ -67,19 +67,26 @@ def gate(odom):
     return moved, np.ascontiguousarray(odom / float(ODOM_FREQ))
 
 
-def dead_reckoning(moved, tw):
+def dead_reckoning(moved, tw, start=None):
     """The reference's unlinked map over the shared odometry, which is every agent's: ``(n_exp int64[T],
-    em_xy float64[T,2], accum)`` with accum = the final (accum_delta_x, accum_delta_y, accum_delta_th)."""
+    em_xy float64[T,2], accum)`` with accum = the final (accum_delta_x, accum_delta_y, accum_delta_th).  ``start`` =
+    ``(n_exp, accum)`` after earlier frames of the same recording continues that map (an experience is created at the
+    accumulated position, so the last one sits at accum's (x, y))."""
     T = len(moved)
     em = ExperienceMap()
+    n0 = 0
+    if start is not None:
+        n0, (em.accum_delta_x, em.accum_delta_y, em.accum_delta_th) = int(start[0]), start[1]
     n_exp = np.zeros(T, np.int64)
     em_xy = np.zeros((T, 2))
     for t in range(T):
         if moved[t]:
             em.update(float(tw[t, 0]), float(tw[t, 1]), (0, 0, 0))    # the cell tags the experience, nothing else
-        n_exp[t] = len(em.experiences)
+        n_exp[t] = n0 + len(em.experiences)
         if em.current_exp is not None:
             em_xy[t] = em.get_current_point()
+        elif n0:
+            em_xy[t] = (em.accum_delta_x, em.accum_delta_y)
     return n_exp, em_xy, (em.accum_delta_x, em.accum_delta_y, em.accum_delta_th)
 
 
@@ -89,24 +96,27 @@ class EnsembleExperienceMaps:
     ``n_experiences``, ``n_links``, ``current`` (-1 = none) and ``n_loop_closures`` are int64 [B] on the host; an
     agent's experiences and links are copied from the device when asked for."""
 
-    def __init__(self, work, B, T, n_templates, moved, tw, pose_size, delta_pc, correction, vt_ids=None, rec_of=None):
+    def __init__(self, work, B, T, n_templates, moved, tw, pose_size, delta_pc, correction, vt_ids=None, rec_of=None,
+                 accum=None, cols=None):
         lay, _ = _work_layout(B, T, n_templates)
         self._vt_ids = vt_ids       # per agent: the caller's template id of each tag, when the ids were renumbered
+        # cols: the workspace column of each agent, when the workspace holds them in another order (EnsembleSession)
+        self._cols = np.arange(B) if cols is None else np.asarray(cols)
         self._v = {k: work[o:o + r * B * torch.empty((), dtype=dt).element_size()].view(dt).view(r, B)
                    for k, (o, dt, r) in lay.items()}
-        counts = self._v["counts"].cpu().numpy().astype(np.int64)
+        counts = self._v["counts"].cpu().numpy().astype(np.int64)[:, self._cols]
         self.n_experiences, self.n_links, self.current, self.n_loop_closures = counts
-        self._rel = self._v["rel"].cpu().numpy()
+        self._rel = self._v["rel"].cpu().numpy()[:, self._cols]
         # the dead reckoning of each recording (rec_of: agent b's column of moved [T,R], tw [T,R,2]), computed when a map
-        # is rebuilt
-        self._odom, self._rec_of, self._accum = (moved, tw), rec_of, {}
+        # is rebuilt unless ``accum`` ({recording: accum}) gives it
+        self._odom, self._rec_of, self._accum = (moved, tw), rec_of, {} if accum is None else dict(accum)
         self.pose_size, self.delta_pc, self.correction = tuple(pose_size), delta_pc, correction
 
     def __len__(self):
         return len(self.n_experiences)
 
     def _col(self, name, n, b):
-        return self._v[name][:n, b].cpu().numpy()
+        return self._v[name][:n, int(self._cols[b])].cpu().numpy()
 
     def experiences(self, b):
         """Agent b's experiences in index order, ``EXPERIENCE_DTYPE`` [n]: cell, view template (-1 = none), position

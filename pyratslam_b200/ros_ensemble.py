@@ -12,6 +12,9 @@ Tuning on several recordings keeps the settings from fitting one route: with ``f
 R recordings, agent ``b`` replays recording ``recording[b]`` (``prs_ens_multi_replay_run``), still in one graph per
 frame.
 
+``EnsembleSession`` keeps the agents on the device between calls and feeds them recordings in pieces: bags streamed
+in chunks, recordings longer than 65535 frames, or a second run of a route continuing the maps of the first.
+
     python -m pyratslam_b200.ros_ensemble BAG [BAG ...] --match-threshold 30000,45000,60000 --global-inhibition 0.1,0.2
 """
 from __future__ import annotations
@@ -133,13 +136,17 @@ def _unravel(flat, shape):
 class EnsembleAgents:
     """What every agent holds after the replay: its library, the template locations and its pose cells."""
 
-    def __init__(self, ens, libs, loc, n_templates, shape):
+    def __init__(self, ens, libs, loc, n_templates, shape, rows=None):
         self._ens, self._libs, self._loc = ens, libs, loc
+        self._rows = rows           # the ensemble's row of each agent, when it holds them in another order
         self.n_templates = n_templates
         self.shape = shape
 
     def __len__(self):
         return len(self.n_templates)
+
+    def _row(self, b):
+        return b if self._rows is None else int(self._rows[b])
 
     @property
     def path(self):
@@ -149,25 +156,389 @@ class EnsembleAgents:
     @property
     def state(self):
         """The device tensor ``[B, Th, X, Y]`` of every agent's pose cells (theta-major)."""
-        return self._ens.state
+        if self._rows is None:
+            return self._ens.state
+        return self._ens.state[torch.from_numpy(np.asarray(self._rows)).to(self._ens.state.device)]
 
     def templates(self, b):
         """uint8 ``[n_b, 32, 32]``: agent b's templates as ``ViewTemplate.template`` holds them."""
         n = int(self.n_templates[b])
+        lib = self._libs[self._row(b)]
         out = torch.empty((n, 32, 32), dtype=torch.uint8, device=self._libs.device)
         with torch.cuda.device(self._libs.device):
             for i in range(n):
-                nat.check(nat.lib().prs_vt_unpack_u8(self._libs[b].data_ptr(), i, out[i].data_ptr(), nat.stream_ptr()),
+                nat.check(nat.lib().prs_vt_unpack_u8(lib.data_ptr(), i, out[i].data_ptr(), nat.stream_ptr()),
                           "prs_vt_unpack_u8")
             return out.cpu().numpy()
 
     def locations(self, b):
         """int64 ``[n_b, 3]``: the pose cell each of agent b's templates was created at (``ViewTemplate.location``)."""
-        return _unravel(self._loc[b, :int(self.n_templates[b])].cpu().numpy(), self.shape)
+        return _unravel(self._loc[self._row(b), :int(self.n_templates[b])].cpu().numpy(), self.shape)
 
     def posecells(self, b):
         """Agent b's pose cells, float64 ``[X, Y, Th]`` (the reference's layout)."""
-        return self._ens.state[b].permute(1, 2, 0).cpu().numpy().astype(np.float64)
+        return self._ens.state[self._row(b)].permute(1, 2, 0).cpu().numpy().astype(np.float64)
+
+
+def grow_capacity(capacity, n_max, t):
+    """A session's library growth rule (no CUDA involved): ``(capacity', frames)`` before t more frames when the
+    fullest library holds ``n_max`` templates.  capacity' is ``capacity`` while n_max + t fits it, else
+    ``min(65536, max(2 * capacity, capacity_for(n_max + t)))``: doubling keeps the growths O(log) per session.  A frame
+    appends at most one template, so ``frames = min(t, capacity' - n_max)`` of them fit; fewer than t only at 65536,
+    where the rest goes in later sub-runs, and 0 when a library is full."""
+    cap = int(capacity)
+    if n_max + t > cap:
+        cap = min(MAX_CAPACITY, max(2 * cap, capacity_for(n_max + t)))
+    return cap, max(min(int(t), cap - int(n_max)), 0)
+
+
+def _grow_rows(rows, need):
+    """Experience-map workspace rows for ``need``: unchanged while they suffice, else doubled (at least ``need``)."""
+    return rows if need <= rows else max(2 * rows, need)
+
+
+def feed_inputs(frames, odom, n_recordings):
+    """Validate one feed of a session of ``n_recordings`` recordings (no CUDA involved): with one recording ``frames``
+    uint8 [t,256,256] and ``odom`` [t,2]; with R > 1 lists of R such arrays, of any lengths (0 allowed).  Returns lists
+    of R contiguous uint8 frame arrays and R float64 odometry arrays; ``ValueError`` otherwise."""
+    R = int(n_recordings)
+    if R == 1:
+        if isinstance(frames, (list, tuple)) or isinstance(odom, (list, tuple)):
+            raise ValueError("EnsembleSession.feed: a session of one recording takes arrays, not lists")
+        frames, odom = [frames], [odom]
+    elif (not isinstance(frames, (list, tuple)) or not isinstance(odom, (list, tuple)) or len(frames) != R
+          or len(odom) != R):
+        raise ValueError("EnsembleSession.feed: a session of %d recordings takes lists of %d frame and %d odometry "
+                         "arrays" % (R, R, R))
+    fr, od = [], []
+    for r in range(R):
+        f = np.asarray(frames[r])
+        try:
+            o = np.asarray(odom[r], dtype=np.float64)
+        except (TypeError, ValueError):
+            raise ValueError("EnsembleSession.feed: recording %d: odometry must be numbers" % r) from None
+        if f.dtype != np.uint8 or f.ndim != 3 or tuple(f.shape[1:]) != IM_SIZE or o.shape != (len(f), 2):
+            raise ValueError("EnsembleSession.feed: recording %d: frames must be uint8 [t,%d,%d] and odom [t,2], got %s "
+                             "%r and %r" % (r, IM_SIZE[0], IM_SIZE[1], f.dtype, f.shape, o.shape))
+        fr.append(np.ascontiguousarray(f))
+        od.append(o)
+    return fr, od
+
+
+class EnsembleSession:
+    """B RatSLAM agents that stay on the device between calls: ``feed`` replays the next frames of every recording.
+
+    The parameters are those of ``replay_ensemble`` and are validated and broadcast the same way; ``n_recordings`` R
+    and ``recording`` (an index or a length-B sequence) say which recording each agent replays, ``capacity`` is the
+    initial templates per agent (default 32, rounded up to whole groups of 32).  ``experience_map`` is False or
+    "device"; the host replay (True) needs whole recordings and is refused.
+
+    ``feed(frames, odom)`` takes uint8 [t,256,256] and [t,2] (R = 1) or lists of R such arrays of any lengths, 0
+    allowed, and continues each recording where the previous feed left it.  It returns what ``replay_ensemble``'s
+    several-recordings form returns for the fed frames: ``template``, ``created``, ``argmax`` ``[B, t_max]``, ``length
+    [B]`` (the agent's recording's frames in this feed, -1 / False past it), ``n_templates [B]``, and with
+    ``experience_map="device"`` ``n_exp``, ``exp_id``, ``em_xy`` and ``n_loop_closures``.  Template and experience ids
+    are global to the session: concatenating agent b's first ``length[b]`` columns over the feeds gives what
+    ``replay_ensemble`` returns on the concatenation of its recording's feeds.  The libraries grow when a feed could
+    overfill them (``grow_capacity``), so a session replays any number of frames while no agent holds more than 65536
+    templates.  A pose-cell error raises what ``replay_ensemble`` raises and closes the session; a closed session's
+    ``feed`` raises ``RuntimeError``."""
+
+    def __init__(self, n_agents=None, match_threshold=MATCH_THRESHOLD, global_inhibition=PC_GLOBAL_INHIB,
+                 inject_energy=None, pose_size=POSE_SIZE, dtype=np.float32, active_set=0, experience_map=False,
+                 experience_links=False, n_recordings=1, recording=0, capacity=None):
+        self._plan, self._ens, self._work = None, None, None
+        self._closed = True
+        if isinstance(experience_map, (bool, np.bool_)) and experience_map:
+            raise ValueError("EnsembleSession: experience_map=True replays the maps on the host from whole recordings; "
+                             "a session builds them on the device (experience_map='device')")
+        if not (isinstance(experience_map, (bool, np.bool_))
+                or (isinstance(experience_map, str) and experience_map == "device")):
+            raise ValueError("experience_map must be False or 'device', got %r" % (experience_map,))
+        if (not isinstance(n_recordings, (numbers.Integral, np.integer)) or isinstance(n_recordings, (bool, np.bool_))
+                or n_recordings < 1):
+            raise ValueError("n_recordings must be an integer >= 1, got %r" % (n_recordings,))
+        R = int(n_recordings)
+        B, thr, gi, energies = agent_parameters(n_agents if n_agents is not None else _recording_count(recording),
+                                                match_threshold, global_inhibition, inject_energy)
+        rec_of = agent_recordings(recording, B, R)
+        cap = 32 if capacity is None else capacity
+        if not _real(cap) or not 1 <= cap <= MAX_CAPACITY or cap != int(cap):
+            raise ValueError("capacity must be an integer in [1, %d], got %r" % (MAX_CAPACITY, capacity))
+        cap = (int(cap) + 31) // 32 * 32
+        pose_size = tuple(int(s) for s in pose_size)
+        np_dtype = _as_np_dtype(dtype)
+        nat.require_cuda()
+        dev = torch.device("cuda", torch.cuda.current_device())
+        self.B, self.R, self.pose_size, self.capacity = B, R, pose_size, cap
+        self._dev, self._rec_of = dev, rec_of
+        self._map = isinstance(experience_map, str)
+        self._linked = self._map and bool(experience_links)
+        # the agents of one recording get contiguous indices on the device (the sweep reloads a query per recording
+        # change); _order[d] is the agent at device row d, _rows[b] the device row of agent b
+        self._order = np.argsort(rec_of, kind="stable")
+        self._rows = np.argsort(self._order)
+        self._ens = ens = PoseCellEnsemble(pose_size, B, global_inhibition=gi[self._order], dtype=np_dtype, device=dev,
+                                           active_set=active_set)
+        ens.inject(1, tuple(math.floor(s / 2) for s in pose_size))         # RatslamRos.__init__
+        L = nat.lib()
+        self._libs = torch.zeros((B, int(L.prs_vt_packed_bytes(cap))), dtype=torch.uint8, device=dev)
+        self._loc = torch.full((B, cap), -1, dtype=torch.int64, device=dev)
+        self._n_dev = torch.zeros(B, dtype=torch.int32, device=dev)
+        self._thr_dev = torch.from_numpy(thr[self._order].view(np.int32)).to(dev)
+        injecting = any(e is not None for e in energies)
+        self._energy_dev = torch.tensor([-1.0 if energies[i] is None else energies[i] for i in self._order],
+                                        dtype=torch.float64, device=dev) if injecting else None
+        self._rec_dev = torch.from_numpy(rec_of[self._order].astype(np.int32)).to(dev)
+        self._pc_work = torch.zeros(3 * B, dtype=torch.int64, device=dev)
+        self._scratch = torch.empty(int(L.prs_ens_scratch_bytes(B, IM_SIZE[0], IM_SIZE[1])), dtype=torch.uint8,
+                                    device=dev)
+        self._mscratch = None
+        self._stream = torch.cuda.Stream(device=dev)
+        self.frames_fed = np.zeros(R, np.int64)
+        self._n = np.zeros(B, np.int64)                       # templates per device row
+        self._prev_tpl = np.full(B, -1, np.int32)             # per device row: the template of its last frame
+        self._dr = [(0, (0, 0, 0))] * R                       # per recording: the dead reckoning's (n_exp, accum)
+        self._counts = np.zeros((4, B), np.int64)             # per device row: the linked map's counts
+        self._counts[2] = -1
+        with torch.cuda.device(dev):
+            nat.check(L.prs_pc_argmax(ens._h, ens.state.data_ptr(), self._pc_work.data_ptr(), nat.stream_ptr()),
+                      "prs_pc_argmax")
+            torch.cuda.current_stream(dev).synchronize()
+            self._create_plan()
+            self._closed = False
+            if self._linked:
+                self._E, self._N = cap, cap
+                self._work = torch.empty(int(L.prs_em_session_bytes(B, self._E, self._N)), dtype=torch.uint8,
+                                         device=dev)
+                nat.check(L.prs_em_session_init(B, self._E, self._N, self._work.data_ptr(), nat.stream_ptr()),
+                          "prs_em_session_init")
+
+    # ------------------------------------------------------------------ the plan and its growth
+    def _create_plan(self):
+        L = nat.lib()
+        plan = ctypes.c_void_p()
+        e = self._ens
+        nat.check(L.prs_ens_create(
+            e._h, e.state.data_ptr(), e._gi.data_ptr(), self._pc_work.data_ptr(), self._libs.data_ptr(), self.capacity,
+            self._n_dev.data_ptr(), self._thr_dev.data_ptr(),
+            None if self._energy_dev is None else self._energy_dev.data_ptr(), self._loc.data_ptr(), nat.VT_MODE_REF,
+            IM_SIZE[0], IM_SIZE[1], Y_RANGE[0], Y_RANGE[1], Y_STEP, X_RANGE[0], X_RANGE[1], X_STEP,
+            self._scratch.data_ptr(), ctypes.byref(plan)), "prs_ens_create")
+        self._plan = plan
+        self._room = self.capacity - int(self._n.max())
+        if self.R > 1:
+            if self._mscratch is None:
+                self._mscratch = torch.empty(int(L.prs_ens_multi_scratch_bytes(plan, self.R)), dtype=torch.uint8,
+                                             device=self._dev)
+            nat.check(L.prs_ens_set_recordings(plan, self.R, self._rec_dev.data_ptr(), self._mscratch.data_ptr()),
+                      "prs_ens_set_recordings")
+
+    def _grow(self, cap):
+        """Libraries of ``cap`` templates: a larger library is the old one with groups appended, so each agent's row is
+        copied as a prefix; the plan is made again on the new buffers (its graphs are captured again)."""
+        L = nat.lib()
+        libs = torch.zeros((self.B, int(L.prs_vt_packed_bytes(cap))), dtype=torch.uint8, device=self._dev)
+        libs[:, :self._libs.shape[1]].copy_(self._libs)
+        loc = torch.full((self.B, cap), -1, dtype=torch.int64, device=self._dev)
+        loc[:, :self.capacity].copy_(self._loc)
+        torch.cuda.current_stream(self._dev).synchronize()
+        L.prs_ens_destroy(self._plan)
+        self._plan = None
+        self._libs, self._loc, self.capacity = libs, loc, cap
+        self._create_plan()
+
+    def _grow_maps(self, E, N):
+        L = nat.lib()
+        work = torch.empty(int(L.prs_em_session_bytes(self.B, E, N)), dtype=torch.uint8, device=self._dev)
+        nat.check(L.prs_em_session_grow(self.B, self._E, self._N, E, N, self._work.data_ptr(), work.data_ptr(),
+                                        nat.stream_ptr()), "prs_em_session_grow")
+        self._work, self._E, self._N = work, E, N
+
+    # ------------------------------------------------------------------ feeding
+    def feed(self, frames, odom):
+        """Replay the next frames of every recording; see the class documentation for the inputs and the result."""
+        if self._closed:
+            raise RuntimeError("EnsembleSession: the session is closed")
+        fr, od = feed_inputs(frames, odom, self.R)
+        R, B = self.R, self.B
+        lengths = np.array([len(f) for f in fr], dtype=np.int64)
+        T = int(lengths.max())
+        moved = np.zeros((T, R), np.uint8)             # past a recording's end: not moved
+        tw = np.zeros((T, R, 2))
+        for r in range(R):
+            moved[:lengths[r], r], tw[:lengths[r], r] = xens.gate(od[r])
+        res = np.zeros((T, B), dtype=RatslamRos._RESULT_DTYPE)     # device rows
+        if self._linked:
+            n_exp = np.zeros((T, B), np.int32)
+            exp_id = np.zeros((T, B), np.int32)
+            em_xy = np.zeros((T, B, 2))
+        try:
+            with torch.cuda.device(self._dev):
+                s0 = 0
+                while s0 < T:
+                    cap, run = grow_capacity(self.capacity, int(self._n.max()), T - s0)
+                    if run == 0:
+                        d = int(np.argmax(self._n))
+                        raise ValueError("EnsembleSession: agent %d holds %d templates, the most the library sweep "
+                                         "takes, and frame %d of its recording remains"
+                                         % (self._order[d], self._n[d],
+                                            self.frames_fed[self._rec_of[self._order[d]]] + s0))
+                    if cap != self.capacity:
+                        self._grow(cap)
+                    if self._room < run:     # the plan counted earlier runs' frames, not their templates
+                        nat.check(nat.lib().prs_ens_refresh_room(self._plan, ctypes.c_void_p(self._stream.cuda_stream)),
+                                  "prs_ens_refresh_room")
+                        self._room = self.capacity - int(self._n.max())
+                    sub = slice(s0, s0 + run)
+                    self._replay(fr, tw[sub], moved[sub], lengths, s0, run, res[sub])
+                    self._room -= run
+                    self._n = res["n_templates"][s0 + run - 1].astype(np.int64)
+                    if self._linked:
+                        self._maps(res[sub], tw[sub], moved[sub], np.clip(lengths - s0, 0, run), n_exp[sub],
+                                   exp_id[sub], em_xy[sub])
+                    s0 += run
+        except BaseException:
+            self.close()
+            raise
+        self.frames_fed += lengths
+        inv = self._rows
+        res = res[:, inv]
+        length = lengths[self._rec_of]
+        past = np.arange(T)[None, :] >= length[:, None]  # [B, T]
+        argmax = _unravel(res["argmax"].T, self.pose_size)
+        argmax[past] = -1
+        out = {"template": res["template_index"].T.astype(np.int64), "created": res["created"].T != 0,
+               "argmax": argmax, "n_templates": self.n_templates, "length": length}
+        if self._map:
+            if self._linked:
+                out["n_exp"] = n_exp[:, inv].T.astype(np.int64)
+                out["exp_id"] = exp_id[:, inv].T.astype(np.int64)
+                out["em_xy"] = em_xy[:, inv].transpose(1, 0, 2)
+                for r in range(R):       # the recording's accumulators, for maps.experience_map(b)
+                    self._dead_reckoning(r, moved[:, r], tw[:, r], lengths[r])
+            else:
+                per = [self._dead_reckoning(r, moved[:, r], tw[:, r], lengths[r]) for r in range(R)]
+                out["n_exp"] = np.stack([per[r][0] for r in self._rec_of])
+                out["em_xy"] = np.stack([per[r][1] for r in self._rec_of])
+                out["exp_id"] = out["n_exp"] - 1
+            out["n_loop_closures"] = self.n_loop_closures
+            out["n_exp"][past] = -1
+            out["exp_id"][past] = -1
+            out["em_xy"][past] = np.nan
+        return out
+
+    def _replay(self, fr, tw, moved, lengths, s0, run, res):
+        """Frames [s0, s0 + run) of the feed through the plan; raises a pose-cell error as replay_ensemble does."""
+        L = nat.lib()
+        stream = ctypes.c_void_p(self._stream.cuda_stream)
+        if self.R == 1:
+            tw1, mv1 = np.ascontiguousarray(tw[:, 0]), np.ascontiguousarray(moved[:, 0])
+            nat.check(L.prs_ens_replay_run(self._plan, fr[0].ctypes.data + s0 * IM_SIZE[0] * IM_SIZE[1], tw1.ctypes.data,
+                                           mv1.ctypes.data, run, res.ctypes.data, stream), "prs_ens_replay_run")
+            bad = np.nonzero((((res["pc_err"] & ~nat.ERR_INJECT_LOC) != 0) & (mv1[:, None] != 0)).any(axis=1))[0]
+            if len(bad):
+                self._ens._raise_on_err(np.asarray(res["pc_err"][int(bad[0])] & ~nat.ERR_INJECT_LOC, dtype=np.int32))
+            return
+        sub_len = np.clip(lengths - s0, 0, run).astype(np.int32)
+        ptrs = (ctypes.c_void_p * self.R)(*[fr[r].ctypes.data + s0 * IM_SIZE[0] * IM_SIZE[1] if sub_len[r] else None
+                                            for r in range(self.R)])
+        tw, moved = np.ascontiguousarray(tw), np.ascontiguousarray(moved)
+        nat.check(L.prs_ens_multi_replay_run(self._plan, ptrs, tw.ctypes.data, moved.ctypes.data, sub_len.ctypes.data,
+                                             run, res.ctypes.data, stream), "prs_ens_multi_replay_run")
+        rc = res[:, self._rows]
+        bad = ((rc["pc_err"] & ~nat.ERR_INJECT_LOC) != 0) & (moved[:, self._rec_of] != 0)
+        if bad.any():
+            t, b = np.argwhere(bad)[0]                  # frame-major: the earliest frame, then the lowest agent
+            self._ens._raise_on_err(np.array([rc["pc_err"][t, b] & ~nat.ERR_INJECT_LOC], dtype=np.int32))
+
+    def _maps(self, res, tw, moved, sub_len, n_exp, exp_id, em_xy):
+        """The linked maps continued over one sub-run's records (device rows)."""
+        L = nat.lib()
+        T, B = res.shape
+        tpl = res["template_index"]
+        tag = np.empty((T, B), np.int32)
+        tag[0] = self._prev_tpl
+        tag[1:] = np.maximum(tpl[:-1], -1)
+        mine = sub_len[self._rec_of[self._order]]        # per device row: its frames in this sub-run
+        here = mine > 0
+        self._prev_tpl[here] = tpl[mine[here] - 1, np.nonzero(here)[0]]
+        E = _grow_rows(self._E, int(self._counts[:2].max()) + T)
+        if E != self._E or self.capacity != self._N:
+            self._grow_maps(E, self.capacity)
+        X, Y, Th = self.pose_size
+        dev = self._dev
+        flat_d = torch.from_numpy(np.ascontiguousarray(res["argmax"])).to(dev)
+        tag_d = torch.from_numpy(tag).to(dev)
+        tw_d = torch.from_numpy(np.ascontiguousarray(tw)).to(dev)
+        moved_d = torch.from_numpy(np.ascontiguousarray(moved)).to(dev)
+        n_d = torch.empty((T, B), dtype=torch.int32, device=dev)
+        id_d = torch.empty((T, B), dtype=torch.int32, device=dev)
+        xy_d = torch.empty((T, B, 2), dtype=torch.float64, device=dev)
+        nat.check(L.prs_em_linked_resume_run(B, T, self._E, self._N, flat_d.data_ptr(), tag_d.data_ptr(), self.R,
+                                             tw_d.data_ptr(), moved_d.data_ptr(),
+                                             self._rec_dev.data_ptr() if self.R > 1 else None, X, Y, Th, 1.0,
+                                             self._work.data_ptr(), n_d.data_ptr(), id_d.data_ptr(), xy_d.data_ptr(),
+                                             nat.stream_ptr()), "prs_em_linked_resume_run")
+        lay, end = xens._work_layout(B, self._E, self._N)
+        if int(self._work[end:end + 4].view(torch.int32).item()):
+            raise RuntimeError("EnsembleSession: the experience-map workspace (%d rows, %d template heads) was too small"
+                               % (self._E, self._N))
+        o = lay["counts"][0]
+        self._counts = self._work[o:o + 16 * B].view(torch.int32).view(4, B).cpu().numpy().astype(np.int64)
+        n_exp[:] = n_d.cpu().numpy()
+        exp_id[:] = id_d.cpu().numpy()
+        em_xy[:] = xy_d.cpu().numpy()
+
+    def _dead_reckoning(self, r, moved, tw, length):
+        """Recording r's unlinked map continued over its frames of this feed: ``(n_exp [T], em_xy [T,2])``."""
+        n, xy, accum = xens.dead_reckoning(moved, tw, start=self._dr[r])
+        if length:
+            self._dr[r] = (int(n[length - 1]), accum)
+        return n, xy
+
+    # ------------------------------------------------------------------ what the agents hold
+    @property
+    def n_templates(self):
+        """int64 [B]: templates in each agent's library."""
+        return self._n[self._rows].copy()
+
+    @property
+    def n_loop_closures(self):
+        """int64 [B]: loop closures of each agent's linked map (0 without one)."""
+        return self._counts[3][self._rows].copy() if self._linked else np.zeros(self.B, np.int64)
+
+    @property
+    def agents(self):
+        """``EnsembleAgents``, in the caller's agent order (the libraries as they are now)."""
+        if self._ens is None:
+            raise RuntimeError("EnsembleSession: the session is closed")
+        identity = bool((self._order == np.arange(self.B)).all())
+        return EnsembleAgents(self._ens, self._libs, self._loc, self.n_templates, self.pose_size,
+                              None if identity else self._rows)
+
+    @property
+    def maps(self):
+        """``EnsembleExperienceMaps`` of the linked device maps, in the caller's agent order; None without them."""
+        if not self._linked or self._work is None:
+            return None
+        return xens.EnsembleExperienceMaps(self._work, self.B, self._E, self._N, None, None, self.pose_size, 1.0, 0.5,
+                                           rec_of=self._rec_of, accum={r: dr[1] for r, dr in enumerate(self._dr)},
+                                           cols=self._rows)
+
+    def close(self):
+        """Destroy the frame plan; a closed session's ``feed`` raises ``RuntimeError``.  What ``agents`` and ``maps``
+        returned before stays readable."""
+        if self._plan is not None:
+            nat.lib().prs_ens_destroy(self._plan)
+            self._plan = None
+        self._closed = True
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
 
 
 def replay_ensemble(frames, odom, n_agents=None, match_threshold=MATCH_THRESHOLD, global_inhibition=PC_GLOBAL_INHIB,
@@ -195,7 +566,10 @@ def replay_ensemble(frames, odom, n_agents=None, match_threshold=MATCH_THRESHOLD
     ``[B, T_max]`` with ``length [B]`` (the agent's recording's frame count), and past an agent's length ``template`` and
     ``argmax`` are -1, ``created`` False, ``n_exp`` and ``exp_id`` -1 and ``em_xy`` NaN.  A pose-cell error raises what
     the native replay of that recording raises, for the earliest frame and, within it, the lowest agent.  With single
-    arrays ``recording`` can only be 0."""
+    arrays ``recording`` can only be 0.
+
+    This is one ``EnsembleSession`` fed once, with libraries reserved for every frame up front; a session fed in
+    pieces replays recordings that do not fit in host memory, or longer than 65535 frames."""
     if not (isinstance(experience_map, (bool, np.bool_))
             or (isinstance(experience_map, str) and experience_map == "device")):
         raise ValueError("experience_map must be False, True or 'device', got %r" % (experience_map,))
@@ -203,25 +577,46 @@ def replay_ensemble(frames, odom, n_agents=None, match_threshold=MATCH_THRESHOLD
                                             match_threshold, global_inhibition, inject_energy)
     if mode != "ref":
         raise ValueError("replay_ensemble supports the reference matching mode only, got mode=%r" % (mode,))
-    if isinstance(frames, (list, tuple)) and (len(frames) == 0 or np.ndim(frames[0]) == 3):
-        return _replay_recordings(frames, odom, agent_recordings(recording, B, max(len(frames), 1)), thr, gi, energies,
-                                  pose_size, dtype, active_set, experience_map, experience_links)
-    agent_recordings(recording, B, 1)
-    frames = np.asarray(frames)
-    odom = np.asarray(odom, dtype=np.float64)
-    T = len(frames)
-    if frames.dtype != np.uint8 or frames.ndim != 3 or tuple(frames.shape[1:]) != IM_SIZE or odom.shape != (T, 2):
-        raise ValueError("replay_ensemble: frames must be uint8 [T,%d,%d] and odom [T,2], got %s %r and %r"
-                         % (IM_SIZE[0], IM_SIZE[1], frames.dtype, frames.shape, odom.shape))
+    several = isinstance(frames, (list, tuple)) and (len(frames) == 0 or np.ndim(frames[0]) == 3)
+    if several:
+        R = len(frames)
+        rec_of = agent_recordings(recording, B, max(R, 1))
+        if not isinstance(odom, (list, tuple)) or len(odom) != R or R == 0:
+            raise ValueError("replay_ensemble: frames and odom must be lists of the same, non-zero number of "
+                             "recordings, got %d and %s"
+                             % (R, len(odom) if isinstance(odom, (list, tuple)) else type(odom).__name__))
+        fr, od = [], []
+        for r in range(R):
+            f, o = np.asarray(frames[r]), np.asarray(odom[r], dtype=np.float64)
+            if f.dtype != np.uint8 or f.ndim != 3 or tuple(f.shape[1:]) != IM_SIZE or o.shape != (len(f), 2):
+                raise ValueError("replay_ensemble: recording %d: frames must be uint8 [T,%d,%d] and odom [T,2], got %s "
+                                 "%r and %r" % (r, IM_SIZE[0], IM_SIZE[1], f.dtype, f.shape, o.shape))
+            fr.append(np.ascontiguousarray(f))
+            od.append(o)
+        T = max(len(f) for f in fr)
+    else:
+        rec_of = agent_recordings(recording, B, 1)
+        fr, od = [np.asarray(frames)], [np.asarray(odom, dtype=np.float64)]
+        T = len(fr[0])
+        if fr[0].dtype != np.uint8 or fr[0].ndim != 3 or tuple(fr[0].shape[1:]) != IM_SIZE or od[0].shape != (T, 2):
+            raise ValueError("replay_ensemble: frames must be uint8 [T,%d,%d] and odom [T,2], got %s %r and %r"
+                             % (IM_SIZE[0], IM_SIZE[1], fr[0].dtype, fr[0].shape, od[0].shape))
+        R = 1
     pose_size = tuple(int(s) for s in pose_size)
     np_dtype = _as_np_dtype(dtype)
     cap = capacity_for(T)
     if cap > MAX_CAPACITY:
         raise ValueError("replay_ensemble: %d frames need %d templates per agent; the library sweep takes at most %d"
                          % (T, cap, MAX_CAPACITY))
-    frames = np.ascontiguousarray(frames)
     lib_bytes = (cap // 32) * 34816
-    need = B * (lib_bytes + cap * 8 + int(np.prod(pose_size)) * np.dtype(np_dtype).itemsize + 64)
+    net_bytes = int(np.prod(pose_size)) * np.dtype(np_dtype).itemsize
+    if several:
+        frame_bytes = IM_SIZE[0] * IM_SIZE[1]
+        # per agent: library, locations, network, its snapshot and the records; plus one chunk of every recording's
+        # frames
+        need = B * (lib_bytes + cap * 8 + 2 * net_bytes + 64) + R * _multi_chunk(R, frame_bytes) * frame_bytes
+    else:
+        need = B * (lib_bytes + cap * 8 + net_bytes + 64)
     if experience_map == "device" and experience_links:
         need += xens.work_bytes(B, T, cap) + xens.record_bytes(B, T)
     nat.require_cuda()
@@ -231,49 +626,28 @@ def replay_ensemble(frames, odom, n_agents=None, match_threshold=MATCH_THRESHOLD
         raise ValueError("replay_ensemble: %d agents x %d templates need %.2f GB of device memory, %.2f GB are free"
                          % (B, cap, need / 1e9, free / 1e9))
 
-    ens = PoseCellEnsemble(pose_size, B, global_inhibition=gi, dtype=np_dtype, device=dev, active_set=active_set)
-    midpoint = tuple(math.floor(s / 2) for s in pose_size)
-    ens.inject(1, midpoint)                                             # RatslamRos.__init__
-    L = nat.lib()
-    assert int(L.prs_vt_packed_bytes(cap)) == lib_bytes
-    libs = torch.zeros((B, lib_bytes), dtype=torch.uint8, device=dev)
-    loc = torch.full((B, cap), -1, dtype=torch.int64, device=dev)
-    n_dev = torch.zeros(B, dtype=torch.int32, device=dev)
-    thr_dev = torch.from_numpy(thr.view(np.int32)).to(dev)
-    injecting = any(e is not None for e in energies)
-    energy_dev = torch.tensor([-1.0 if e is None else e for e in energies], dtype=torch.float64, device=dev)
-    pc_work = torch.zeros(3 * B, dtype=torch.int64, device=dev)
-    scratch = torch.empty(int(L.prs_ens_scratch_bytes(B, IM_SIZE[0], IM_SIZE[1])), dtype=torch.uint8, device=dev)
-    res = np.zeros((T, B), dtype=RatslamRos._RESULT_DTYPE)
-    stream = torch.cuda.Stream(device=dev)
-    plan = ctypes.c_void_p()
-    with torch.cuda.device(dev):
-        nat.check(L.prs_pc_argmax(ens._h, ens.state.data_ptr(), pc_work.data_ptr(), nat.stream_ptr()), "prs_pc_argmax")
-        torch.cuda.current_stream(dev).synchronize()
-        nat.check(L.prs_ens_create(
-            ens._h, ens.state.data_ptr(), ens._gi.data_ptr(), pc_work.data_ptr(), libs.data_ptr(), cap, n_dev.data_ptr(),
-            thr_dev.data_ptr(), energy_dev.data_ptr() if injecting else None, loc.data_ptr(), nat.VT_MODE_REF,
-            IM_SIZE[0], IM_SIZE[1], Y_RANGE[0], Y_RANGE[1], Y_STEP, X_RANGE[0], X_RANGE[1], X_STEP, scratch.data_ptr(),
-            ctypes.byref(plan)), "prs_ens_create")
-        try:
-            moved, tw = xens.gate(odom)
-            nat.check(L.prs_ens_replay_run(plan, frames.ctypes.data, tw.ctypes.data, moved.ctypes.data, T,
-                                           res.ctypes.data, ctypes.c_void_p(stream.cuda_stream)), "prs_ens_replay_run")
-        finally:
-            L.prs_ens_destroy(plan)
-    bad = np.nonzero((((res["pc_err"] & ~nat.ERR_INJECT_LOC) != 0) & (moved[:, None] != 0)).any(axis=1))[0]
-    if len(bad):
-        stop = int(bad[0])
-        ens._raise_on_err(np.asarray(res["pc_err"][stop] & ~nat.ERR_INJECT_LOC, dtype=np.int32))
-    n_templates = res["n_templates"][-1].astype(np.int64) if T else np.zeros(B, np.int64)
-    out = {"template": res["template_index"].T.astype(np.int64), "created": res["created"].T != 0,
-           "argmax": _unravel(res["argmax"].T, pose_size), "n_templates": n_templates,
-           "agents": EnsembleAgents(ens, libs, loc, n_templates, pose_size)}
-    if experience_map == "device":
-        out.update(xens._maps(res["template_index"], np.ascontiguousarray(res["argmax"]), moved, tw, pose_size,
-                              experience_links, 1.0, 0.5, dev))
-    elif experience_map:
-        out["n_exp"], out["em_xy"] = _experience_maps(out, moved, tw, pose_size, experience_links)
+    session = EnsembleSession(B, thr, gi, energies, pose_size, np_dtype, active_set,
+                              "device" if experience_map == "device" else False, experience_links, R, rec_of, cap)
+    try:
+        out = session.feed(fr if R > 1 else fr[0], od if R > 1 else od[0])
+        out["agents"] = session.agents
+        if experience_map == "device":
+            out["maps"] = session.maps
+    finally:
+        session.close()
+    if isinstance(experience_map, (bool, np.bool_)) and experience_map:
+        moved, tw = np.zeros((T, R), np.uint8), np.zeros((T, R, 2))
+        for r in range(R):
+            moved[:len(fr[r]), r], tw[:len(fr[r]), r] = xens.gate(od[r])
+        if several:
+            out["n_exp"], out["em_xy"] = _experience_maps(out, moved, tw, pose_size, experience_links, rec_of)
+            past = np.arange(T)[None, :] >= out["length"][:, None]
+            out["n_exp"][past] = -1
+            out["em_xy"][past] = np.nan
+        else:
+            out["n_exp"], out["em_xy"] = _experience_maps(out, moved[:, 0], tw[:, 0], pose_size, experience_links)
+    if not several:
+        del out["length"]
     return out
 
 
@@ -297,121 +671,46 @@ def _experience_maps(out, moved, tw, pose_size, linked, rec_of=None):
     return n_exp, em_xy
 
 
-def _replay_recordings(frames, odom, rec_of, thr, gi, energies, pose_size, dtype, active_set, experience_map,
-                       experience_links):
-    """replay_ensemble over R recordings: agent b replays ``frames[rec_of[b]]``, ``odom[rec_of[b]]``."""
-    R = len(frames)
-    if not isinstance(odom, (list, tuple)) or len(odom) != R or R == 0:
-        raise ValueError("replay_ensemble: frames and odom must be lists of the same, non-zero number of recordings, "
-                         "got %d and %s" % (R, len(odom) if isinstance(odom, (list, tuple)) else type(odom).__name__))
-    fr, od = [], []
-    for r in range(R):
-        f, o = np.asarray(frames[r]), np.asarray(odom[r], dtype=np.float64)
-        if f.dtype != np.uint8 or f.ndim != 3 or tuple(f.shape[1:]) != IM_SIZE or o.shape != (len(f), 2):
-            raise ValueError("replay_ensemble: recording %d: frames must be uint8 [T,%d,%d] and odom [T,2], got %s %r "
-                             "and %r" % (r, IM_SIZE[0], IM_SIZE[1], f.dtype, f.shape, o.shape))
-        fr.append(np.ascontiguousarray(f))
-        od.append(o)
-    B = len(rec_of)
-    lengths = np.array([len(f) for f in fr], dtype=np.int32)
-    T = int(lengths.max())
-    pose_size = tuple(int(s) for s in pose_size)
-    np_dtype = _as_np_dtype(dtype)
-    cap = capacity_for(T)
-    if cap > MAX_CAPACITY:
-        raise ValueError("replay_ensemble: %d frames need %d templates per agent; the library sweep takes at most %d"
-                         % (T, cap, MAX_CAPACITY))
-    lib_bytes = (cap // 32) * 34816
-    net_bytes = int(np.prod(pose_size)) * np.dtype(np_dtype).itemsize
-    frame_bytes = IM_SIZE[0] * IM_SIZE[1]
-    # per agent: library, locations, network, its snapshot and the records; plus one chunk of every recording's frames
-    need = B * (lib_bytes + cap * 8 + 2 * net_bytes + 64) + R * _multi_chunk(R, frame_bytes) * frame_bytes
-    if experience_map == "device" and experience_links:
-        need += xens.work_bytes(B, T, cap) + xens.record_bytes(B, T)
-    nat.require_cuda()
-    dev = torch.device("cuda", torch.cuda.current_device())
-    free, _ = torch.cuda.mem_get_info(dev)
-    if need > free:
-        raise ValueError("replay_ensemble: %d agents x %d templates need %.2f GB of device memory, %.2f GB are free"
-                         % (B, cap, need / 1e9, free / 1e9))
-
-    # the agents of one recording get contiguous indices on the device (the sweep reloads a query per recording change)
-    order = np.argsort(rec_of, kind="stable")
-    inv = np.argsort(order)
-    ens = PoseCellEnsemble(pose_size, B, global_inhibition=gi[order], dtype=np_dtype, device=dev, active_set=active_set)
-    ens.inject(1, tuple(math.floor(s / 2) for s in pose_size))         # RatslamRos.__init__
-    L = nat.lib()
-    assert int(L.prs_vt_packed_bytes(cap)) == lib_bytes
-    libs = torch.zeros((B, lib_bytes), dtype=torch.uint8, device=dev)
-    loc = torch.full((B, cap), -1, dtype=torch.int64, device=dev)
-    n_dev = torch.zeros(B, dtype=torch.int32, device=dev)
-    thr_dev = torch.from_numpy(thr[order].view(np.int32)).to(dev)
-    injecting = any(e is not None for e in energies)
-    energy_dev = torch.tensor([-1.0 if energies[i] is None else energies[i] for i in order], dtype=torch.float64,
-                              device=dev)
-    rec_dev = torch.from_numpy(rec_of[order].astype(np.int32)).to(dev)
-    pc_work = torch.zeros(3 * B, dtype=torch.int64, device=dev)
-    scratch = torch.empty(int(L.prs_ens_scratch_bytes(B, IM_SIZE[0], IM_SIZE[1])), dtype=torch.uint8, device=dev)
-    moved = np.zeros((T, R), np.uint8)             # past a recording's end: not moved
-    tw = np.zeros((T, R, 2))
-    for r in range(R):
-        moved[:lengths[r], r], tw[:lengths[r], r] = xens.gate(od[r])
-    res = np.zeros((T, B), dtype=RatslamRos._RESULT_DTYPE)
-    stream = torch.cuda.Stream(device=dev)
-    plan = ctypes.c_void_p()
-    frame_ptrs = (ctypes.c_void_p * R)(*[f.ctypes.data if len(f) else None for f in fr])
-    with torch.cuda.device(dev):
-        nat.check(L.prs_pc_argmax(ens._h, ens.state.data_ptr(), pc_work.data_ptr(), nat.stream_ptr()), "prs_pc_argmax")
-        torch.cuda.current_stream(dev).synchronize()
-        nat.check(L.prs_ens_create(
-            ens._h, ens.state.data_ptr(), ens._gi.data_ptr(), pc_work.data_ptr(), libs.data_ptr(), cap, n_dev.data_ptr(),
-            thr_dev.data_ptr(), energy_dev.data_ptr() if injecting else None, loc.data_ptr(), nat.VT_MODE_REF,
-            IM_SIZE[0], IM_SIZE[1], Y_RANGE[0], Y_RANGE[1], Y_STEP, X_RANGE[0], X_RANGE[1], X_STEP, scratch.data_ptr(),
-            ctypes.byref(plan)), "prs_ens_create")
-        try:
-            mscratch = torch.empty(int(L.prs_ens_multi_scratch_bytes(plan, R)), dtype=torch.uint8, device=dev)
-            nat.check(L.prs_ens_set_recordings(plan, R, rec_dev.data_ptr(), mscratch.data_ptr()),
-                      "prs_ens_set_recordings")
-            nat.check(L.prs_ens_multi_replay_run(plan, frame_ptrs, tw.ctypes.data, moved.ctypes.data, lengths.ctypes.data,
-                                                 T, res.ctypes.data, ctypes.c_void_p(stream.cuda_stream)),
-                      "prs_ens_multi_replay_run")
-        finally:
-            L.prs_ens_destroy(plan)
-        # back to the caller's agent order
-        inv_d = torch.from_numpy(inv).to(dev)
-        ens.state.copy_(ens.state[inv_d])
-        ens.global_inhibition = gi
-        nat.check(L.prs_pc_invalidate_active(ens._h, nat.stream_ptr()), "prs_pc_invalidate_active")
-        libs, loc = libs[inv_d], loc[inv_d]
-    res = np.ascontiguousarray(res[:, inv])
-    agent_moved = moved[:, rec_of]                  # [T, B]
-    bad = ((res["pc_err"] & ~nat.ERR_INJECT_LOC) != 0) & (agent_moved != 0)
-    if bad.any():
-        t, b = np.argwhere(bad)[0]                  # frame-major: the earliest frame, then the lowest agent
-        ens._raise_on_err(np.array([res["pc_err"][t, b] & ~nat.ERR_INJECT_LOC], dtype=np.int32))
-    length = lengths[rec_of].astype(np.int64)
-    past = np.arange(T)[None, :] >= length[:, None]  # [B, T]
-    n_templates = res["n_templates"][-1].astype(np.int64) if T else np.zeros(B, np.int64)
-    argmax = _unravel(res["argmax"].T, pose_size)
-    argmax[past] = -1
-    out = {"template": res["template_index"].T.astype(np.int64), "created": res["created"].T != 0, "argmax": argmax,
-           "n_templates": n_templates, "length": length,
-           "agents": EnsembleAgents(ens, libs, loc, n_templates, pose_size)}
-    if experience_map == "device":
-        out.update(xens._maps(res["template_index"], np.ascontiguousarray(res["argmax"]), moved, tw, pose_size,
-                              experience_links, 1.0, 0.5, dev, rec_of=rec_of))
-    elif experience_map:
-        out["n_exp"], out["em_xy"] = _experience_maps(out, moved, tw, pose_size, experience_links, rec_of)
-    if experience_map:
-        for k in ("n_exp", "exp_id"):
-            if k in out:
-                out[k][past] = -1
-        out["em_xy"][past] = np.nan
-    return out
-
-
 def _list(text, parse):
     return [parse(v.strip()) for v in text.split(",") if v.strip()]
+
+
+def _chunk_arg(text):
+    import argparse
+    try:
+        n = int(text)
+    except ValueError:
+        n = 0
+    if n < 1:
+        raise argparse.ArgumentTypeError("--chunk takes a number of frames >= 1, got %r" % (text,))
+    return n
+
+
+def _replay_chunked(bags, chunk, image_topic, odom_topic, recording, **kw):
+    """The bags fed through one ``EnsembleSession`` ``chunk`` frames per bag at a time: per agent the templates, the
+    frames created on, its bag's frame count and final arg-max (None for an empty bag), and the session's maps."""
+    from . import rosbag_io as rb
+    R = len(bags)
+    its = [rb.iter_frames(bag, chunk, image_topic=image_topic, odom_topic=odom_topic) for bag in bags]
+    s = EnsembleSession(n_recordings=R, recording=recording if R > 1 else 0, capacity=capacity_for(chunk), **kw)
+    try:
+        B = len(s.n_templates)
+        created = np.zeros(B, np.int64)
+        last = [None] * B
+        while True:
+            pieces = [next(it, None) for it in its]
+            if all(p is None for p in pieces):
+                break
+            fr = [p[0] if p is not None else np.zeros((0,) + IM_SIZE, np.uint8) for p in pieces]
+            od = [p[1] if p is not None else np.zeros((0, 2)) for p in pieces]
+            out = s.feed(fr if R > 1 else fr[0], od if R > 1 else od[0])
+            created += out["created"].sum(axis=1)
+            for b in range(B):
+                if out["length"][b]:
+                    last[b] = tuple(int(c) for c in out["argmax"][b, out["length"][b] - 1])
+        return s.n_templates, created, s.frames_fed, last, s.maps
+    finally:
+        s.close()
 
 
 def main(argv=None):
@@ -428,33 +727,44 @@ def main(argv=None):
                          "loop-closure counts")
     ap.add_argument("--image-topic", default="navbot/camera/image")
     ap.add_argument("--odom-topic", default="navbot/odom")
+    ap.add_argument("--chunk", type=_chunk_arg, metavar="FRAMES",
+                    help="feed the bags through one session this many frames per bag at a time, decoding only those "
+                         "frames (the output is the same as without it)")
     a = ap.parse_args(argv)
     from . import rosbag_io as rb
     thr = _list(a.match_threshold, float)
     gis = _list(a.global_inhibition, float)
     ens = _list(a.inject_energy, lambda s: None if s.lower() == "none" else float(s))
     combos = list(itertools.product(thr, gis, ens))
-    recs = [rb.events_to_arrays(rb.read_events(bag, image_topic=a.image_topic, odom_topic=a.odom_topic))[:2]
-            for bag in a.bag]
     several = len(a.bag) > 1
     agents = list(itertools.product(range(len(a.bag)), combos))     # bag-major
     kw = dict(n_agents=len(agents), match_threshold=[c[0] for _, c in agents],
               global_inhibition=[c[1] for _, c in agents], inject_energy=[c[2] for _, c in agents],
               experience_map="device" if a.experience_links else False, experience_links=a.experience_links)
-    if several:
-        out = replay_ensemble([f for f, _ in recs], [o for _, o in recs], recording=[r for r, _ in agents], **kw)
+    if a.chunk is not None:
+        n_templates, created, fed, last, maps = _replay_chunked(a.bag, a.chunk, a.image_topic, a.odom_topic,
+                                                                [r for r, _ in agents], **kw)
+        frames = [int(fed[r if several else 0]) for r, _ in agents]
+        loops = maps.n_loop_closures if maps is not None else None
     else:
-        out = replay_ensemble(recs[0][0], recs[0][1], **kw)
+        recs = [rb.events_to_arrays(rb.read_events(bag, image_topic=a.image_topic, odom_topic=a.odom_topic))[:2]
+                for bag in a.bag]
+        if several:
+            out = replay_ensemble([f for f, _ in recs], [o for _, o in recs], recording=[r for r, _ in agents], **kw)
+        else:
+            out = replay_ensemble(recs[0][0], recs[0][1], **kw)
+        n_templates, maps, loops = out["n_templates"], out.get("maps"), out.get("n_loop_closures")
+        frames = [len(recs[r][0]) for r, _ in agents]
+        created = [int(out["created"][b].sum()) for b in range(len(agents))]
+        last = [tuple(int(c) for c in out["argmax"][b, T - 1]) if T else None for b, T in enumerate(frames)]
     for b, (r, (t, g, e)) in enumerate(agents):
-        T = len(recs[r][0])
-        last = tuple(int(c) for c in out["argmax"][b, T - 1]) if T else None
         line = ("agent %d  match_threshold %g  global_inhibition %g  inject_energy %s:  templates %d  created %d/%d  "
-                "final arg-max %s" % (b, t, g, "none" if e is None else "%g" % e, out["n_templates"][b],
-                                      int(out["created"][b].sum()), T, last))
+                "final arg-max %s" % (b, t, g, "none" if e is None else "%g" % e, n_templates[b],
+                                      int(created[b]), frames[b], last[b]))
         if several:
             line = "bag %s  %s" % (a.bag[r], line)
         if a.experience_links:
-            line += "  experiences %d  loop closures %d" % (out["maps"].n_experiences[b], out["n_loop_closures"][b])
+            line += "  experiences %d  loop closures %d" % (maps.n_experiences[b], loops[b])
         print(line)
 
 

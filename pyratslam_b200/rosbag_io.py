@@ -429,6 +429,33 @@ def events_to_arrays(events):
     return np.stack(frames), np.asarray(odom, dtype=np.float64).reshape(-1, 2), np.asarray(stamps)
 
 
+def iter_frames(path, chunk, image_topic=IMAGE_TOPIC, odom_topic=ODOM_TOPIC):
+    """``events_to_arrays(read_events(path, ...))[:2]`` in pieces: yields ``(frames[n, H, W] uint8, odom[n, 2])`` with
+    n <= ``chunk`` (n < chunk only for the last piece), paired by the same rule.  Images are decoded only for the piece
+    being yielded, so the decoded frames in memory stay at one piece; ``BagReader`` still reads the file whole."""
+    chunk = int(chunk)
+    if chunk < 1:
+        raise ValueError("iter_frames: chunk must be >= 1, got %r" % (chunk,))
+    bag = BagReader(path)
+    want = {image_topic.lstrip("/"): "image", odom_topic.lstrip("/"): "odom"}
+    raw, odom = [], []
+    last = (0.0, 0.0)
+    for m in bag.messages():
+        kind = want.get(m.topic.lstrip("/"))
+        if kind == "odom":
+            o = decode_odometry(m.data)
+            last = (o.linear[0], o.angular[2])
+        elif kind == "image":
+            raw.append(m.data)
+            odom.append(last)
+            last = (0.0, 0.0)
+            if len(raw) == chunk:
+                yield np.stack([decode_image(d).image for d in raw]), np.asarray(odom, dtype=np.float64)
+                raw, odom = [], []
+    if raw:
+        yield np.stack([decode_image(d).image for d in raw]), np.asarray(odom, dtype=np.float64).reshape(-1, 2)
+
+
 def write_run(path, frames, odom, rate_hz=10.0, compression="none", image_topic=IMAGE_TOPIC, odom_topic=ODOM_TOPIC,
               chunk_threshold=768 * 1024):
     """Write ``frames[T,H,W]`` / ``odom[T,2]`` as the bag the node would have been fed: per time step one
