@@ -440,6 +440,27 @@ PRS_API int prs_ens_multi_replay_run(prs_ens_plan* plan, const uint8_t* const* f
                              const uint8_t* moved, const int* lengths, int T_max, prs_frame_result* results,
                              void* stream);
 
+/* Several recordings as message streams: every gated odometry message is its own pose-cell update, as in the node's
+ * message loop (ros_simulate.replay_events), instead of one twist per frame.  The caller compacts each recording into
+ * ticks of (optional gated twist, optional image), odometry before image: an odometry message directly followed by an
+ * image shares its tick, gated-out odometry makes no tick, an image with no twist before it is an image-only tick,
+ * other odometry an odometry-only tick.  Tick t is the frame of prs_ens_multi_replay_run for the recordings with an
+ * image at t; an agent whose recording has no image at t (an odometry-only tick, or past the recording's end) gets
+ * the "no frame" record: template_index -1, created 0, key ~0, n_templates unchanged, and the arg-max and pc_err its
+ * update left.  A tick at which no recording has an image runs only the update (lean: no query, sweep, decision or
+ * injection).  Needs prs_ens_set_recordings first; R = 1 is allowed.
+ *   frames  : host, R pointers; frames[r] is uint8 [n_images[r]][im_rows][im_cols], recording r's images only, in
+ *             order (may be NULL when n_images[r] = 0)
+ *   odom    : host double [T][R][2] = (vtrans, vrot) of recording r's twist at tick t as given to update()
+ *   gate    : host uint8 [T][R]: bit 0 = recording r has an image at tick t, bit 1 = it moved (a gated twist); 0 past
+ *             the end of recording r's ticks
+ *   n_images: host int32 [R], must equal the number of bit-0 ticks of each recording
+ *   results : host prs_frame_result [T][B], one record per tick and agent
+ *   Frames go to the device one chunk of ticks at a time, one copy per recording.  The room check and its decrement
+ *   count ticks with an image (only they can append): PRS_E_INVALID when the libraries have no room for them. */
+PRS_API int prs_ens_events_run(prs_ens_plan* plan, const uint8_t* const* frames, const double* odom, const uint8_t* gate,
+                       const int* n_images, int T, prs_frame_result* results, void* stream);
+
 /* ------------------------------------------------------- ensemble experience maps */
 
 /* Every agent's linked experience map built from an ensemble's records (csrc/experience_map.cu): the per-frame update

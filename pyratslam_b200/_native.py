@@ -105,6 +105,8 @@ _SIGNATURES["prs_ens_multi_scratch_bytes"] = (c_size_t, [c_void_p, c_int])
 _SIGNATURES["prs_ens_set_recordings"] = (c_int, [c_void_p, c_int, c_void_p, c_void_p])
 _SIGNATURES["prs_ens_multi_replay_run"] = (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p,
                                                    c_void_p])
+_SIGNATURES["prs_ens_events_run"] = (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p,
+                                             c_void_p])
 _SIGNATURES["prs_em_work_bytes"] = (c_size_t, [c_int, c_int, c_int])
 _SIGNATURES["prs_em_linked_run"] = (c_int, [c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int,
                                             c_int, c_double, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p])

@@ -30,6 +30,7 @@
 #include <new>
 #include <string.h>
 
+#include <algorithm>
 #include <atomic>
 #include <mutex>
 #include <vector>
@@ -1584,20 +1585,32 @@ __device__ __forceinline__ void vt_prepare_query(const uint8_t* __restrict__ fra
 // Multi-recording frames: block r prepares recording r's query from frame *ctr of its chunk, frames[r][chunk] (bytes
 // (r * chunk + *ctr) * frame_bytes), into tpl + r * 1024 and planes + r * kQueryStride, and sets present[r] from bit 0
 // of gate[*ctr][r] (0 past the recording's end: no query).  The blocks reset the n_keys agents' keys.
+// kSlots (message-stream ticks, prs_ens_events_run): a recording's images sit contiguously in its chunk but not at the
+// tick index, so the image is slot slots[*ctr][r] of the chunk, and -1 (no image at this tick) clears present[r].
+// The <false> instantiation is the kernel as it was.
 constexpr int kQueryStride = 512;  // uint32 words between two recordings' query planes (258 used)
 
+template <bool kSlots>
 __global__ void __launch_bounds__(1024)
     k_vt_frame_prepare_multi(const uint8_t* __restrict__ frames, int chunk, long long frame_bytes, int im_cols, int row_lo,
                              int row_step, int col_lo, int col_step, uint8_t* __restrict__ tpl,
                              uint32_t* __restrict__ planes, unsigned long long* __restrict__ key, int n_keys,
-                             const int* __restrict__ ctr, const uint8_t* __restrict__ gate, uint8_t* __restrict__ present) {
+                             const int* __restrict__ ctr, const uint8_t* __restrict__ gate, uint8_t* __restrict__ present,
+                             const int* __restrict__ slots = nullptr) {
   __shared__ uint32_t s_sum[32];
   const int r = blockIdx.x, R = gridDim.x, f = *ctr;
   for (int i = r * 1024 + (int)threadIdx.x; i < n_keys; i += R * 1024) key[i] = ~0ull;
-  const bool here = (gate[(size_t)f * R + r] & 1) != 0;
+  int s = f;
+  bool here;
+  if constexpr (kSlots) {
+    s = slots[(size_t)f * R + r];
+    here = s >= 0;
+  } else {
+    here = (gate[(size_t)f * R + r] & 1) != 0;
+  }
   if (threadIdx.x == 0) present[r] = here ? 1 : 0;
   if (!here) return;  // block-uniform
-  vt_prepare_query(frames + ((size_t)r * chunk + f) * frame_bytes, im_cols, row_lo, row_step, col_lo, col_step,
+  vt_prepare_query(frames + ((size_t)r * chunk + s) * frame_bytes, im_cols, row_lo, row_step, col_lo, col_step,
                    tpl + (size_t)r * 1024, planes + (size_t)r * kQueryStride, s_sum);
 }
 
@@ -2021,7 +2034,7 @@ constexpr size_t kEnsMultiFrameBytes = 256u << 20;
 struct EnsMultiScratch {
   int chunk = 0;
   size_t frames = 0, odom_chunk = 0, gate = 0, rec = 0, odom = 0, key = 0, tpl = 0, planes = 0, present = 0, still = 0,
-         wsnap = 0, snap = 0, bytes = 0;
+         wsnap = 0, snap = 0, slots = 0, bytes = 0;
   EnsMultiScratch() = default;
   EnsMultiScratch(int B, int R, long long fbytes, size_t net_bytes) {
     auto up = [](size_t v) { return (v + 255) & ~(size_t)255; };
@@ -2039,7 +2052,8 @@ struct EnsMultiScratch {
     still = present + up((size_t)R);
     wsnap = still + up((size_t)B);
     snap = wsnap + up((size_t)B * 3 * sizeof(long long));
-    bytes = snap + up((size_t)B * net_bytes);
+    slots = snap + up((size_t)B * net_bytes);  // int32 [chunk][R], message-stream ticks only
+    bytes = slots + up((size_t)chunk * R * sizeof(int));
   }
 };
 
@@ -2105,6 +2119,27 @@ __global__ void k_ens_odom(const double* __restrict__ odom_chunk, const int* __r
 
 __global__ void k_ens_advance(int* ctr) { ++*ctr; }
 
+// The odometry-only tick of a message-stream replay (prs_ens_events_run) in place of the decision: every agent's
+// "no image" record -- the arg-max, error bits and template count as the tick's update left them, template -1, as
+// k_vt_decide_append writes for an agent whose recording has no frame -- then the tick counter advances.  One block,
+// one thread per agent (strided past 1024).
+__global__ void __launch_bounds__(1024)
+    k_ens_no_image(const long long* __restrict__ argmax, const int* __restrict__ pc_err, const int* __restrict__ n_dev,
+                   prs_frame_result* __restrict__ rec, int* __restrict__ ctr, int B) {
+  prs_frame_result* row = rec + (long long)*ctr * B;
+  for (int b = threadIdx.x; b < B; b += blockDim.x) {
+    prs_frame_result* r = row + b;
+    r->argmax = argmax[b];
+    r->key = ~0ull;
+    r->created = 0;
+    r->template_index = -1;
+    r->n_templates = n_dev[b];
+    r->pc_err = pc_err[b];
+  }
+  __syncthreads();  // every thread has read the counter
+  if (threadIdx.x == 0) ++*ctr;
+}
+
 // group maximum and largest live count of the libraries a plan starts from
 __global__ void k_ens_init(const int* __restrict__ n_dev, int B, int* __restrict__ misc) {
   for (int b = threadIdx.x; b < B; b += blockDim.x) {
@@ -2140,6 +2175,10 @@ struct prs_ens_plan {
   cudaGraphExec_t mexec[3];
   bool mready[3];
   int mwarm[3];
+  // prs_ens_events_run's ticks: [v] with an image in some recording, [3 + v] odometry only, v as above
+  cudaGraphExec_t eexec[6];
+  bool eready[6];
+  int ewarm[6];
 };
 
 static int ens_enqueue(prs_ens_plan* e, bool moved, cudaStream_t st) {
@@ -2224,7 +2263,7 @@ extern "C" int prs_ens_create(prs_pc_handle pc, void* pc_state, const void* gi, 
                                                      (long long)im_rows * im_cols, 0, im_cols, row_lo, row_step, col_lo,
                                                      col_step, (char*)scratch, EnsScratch(B, (long long)im_rows * im_cols),
                                                      {nullptr, nullptr}, {false, false}, {0, 0}, nullptr, nullptr, nullptr,
-                                                     0, nullptr, nullptr, EnsMultiScratch(), {}, {}, {}};
+                                                     0, nullptr, nullptr, EnsMultiScratch(), {}, {}, {}, {}, {}, {}};
   PRS_REQUIRE(e, "prs_ens_create: out of host memory");
   int* misc = (int*)(e->scratch + e->lay.misc);
   int init[3] = {0, 0, 0};
@@ -2269,6 +2308,8 @@ extern "C" int prs_ens_destroy(prs_ens_plan* e) {
       if (e->ready[i]) cudaGraphExecDestroy(e->exec[i]);
     for (int i = 0; i < 3; ++i)
       if (e->mready[i]) cudaGraphExecDestroy(e->mexec[i]);
+    for (int i = 0; i < 6; ++i)
+      if (e->eready[i]) cudaGraphExecDestroy(e->eexec[i]);
     if (e->side) cudaStreamDestroy(e->side);
     if (e->ev_fork) cudaEventDestroy(e->ev_fork);
     if (e->ev_join) cudaEventDestroy(e->ev_join);
@@ -2354,7 +2395,11 @@ extern "C" int prs_ens_replay_run(prs_ens_plan* e, const uint8_t* frames, const 
 // The restore runs before the join, so the decision and the injection of a still network see its state, arg-max and
 // error bits as they were: what the single-recording frame leaves when it skips the update.  A frame where no recording
 // moved runs no update; one where every recording has a frame and moved needs no snapshot.
-static int ens_multi_enqueue(prs_ens_plan* e, int v, cudaStream_t st) {
+// events (message-stream ticks, prs_ens_events_run): the query reads its image through the chunk's slot table
+// (k_vt_frame_prepare_multi<true>).  A tick without an image in any recording (!image) is lean: the side branch's
+// nodes run on `st` itself, then k_ens_no_image writes the records and advances the counter -- no query, sweep,
+// decision or injection.
+static int ens_multi_enqueue(prs_ens_plan* e, int v, cudaStream_t st, bool events = false, bool image = true) {
   char* sc = e->scratch;
   char* ms = e->mscratch;
   const EnsMultiScratch& M = e->mlay;
@@ -2371,12 +2416,15 @@ static int ens_multi_enqueue(prs_ens_plan* e, int v, cudaStream_t st) {
   uint8_t* d_present = (uint8_t*)(ms + M.present);
   uint8_t* d_still = (uint8_t*)(ms + M.still);
   const int B = e->B, R = e->R;
+  const cudaStream_t side = image ? e->side : st;
   int rc;
   if (v != 0) {
-    PRS_CUDA(cudaEventRecord(e->ev_fork, st));
-    PRS_CUDA(cudaStreamWaitEvent(e->side, e->ev_fork, 0));
-    k_ens_odom_multi<<<(B + 255) / 256, 256, 0, e->side>>>((const double*)(ms + M.odom_chunk), d_gate, d_ctr, e->rec_of, R,
-                                                           d_odom, d_still, B);
+    if (image) {
+      PRS_CUDA(cudaEventRecord(e->ev_fork, st));
+      PRS_CUDA(cudaStreamWaitEvent(e->side, e->ev_fork, 0));
+    }
+    k_ens_odom_multi<<<(B + 255) / 256, 256, 0, side>>>((const double*)(ms + M.odom_chunk), d_gate, d_ctr, e->rec_of, R,
+                                                        d_odom, d_still, B);
     PRS_CUDA(cudaGetLastError());
     const int es = pc->dtype == PRS_F32 ? 4 : 8;
     const size_t net_bytes = (size_t)pc->N * es;
@@ -2389,33 +2437,45 @@ static int ens_multi_enqueue(prs_ens_plan* e, int v, cudaStream_t st) {
       const dim3 grid((unsigned)B * per_net);
       if (wide) {
         if (restore)
-          k_ens_snapshot<true, uint4><<<grid, 256, 0, e->side>>>((uint4*)e->pc_state, (uint4*)(ms + M.snap), words, per_net,
+          k_ens_snapshot<true, uint4><<<grid, 256, 0, side>>>((uint4*)e->pc_state, (uint4*)(ms + M.snap), words, per_net,
                                                                  d_still, w, ws, B, es);
         else
-          k_ens_snapshot<false, uint4><<<grid, 256, 0, e->side>>>((uint4*)e->pc_state, (uint4*)(ms + M.snap), words,
+          k_ens_snapshot<false, uint4><<<grid, 256, 0, side>>>((uint4*)e->pc_state, (uint4*)(ms + M.snap), words,
                                                                   per_net, d_still, w, ws, B, es);
       } else {
         if (restore)
-          k_ens_snapshot<true, unsigned><<<grid, 256, 0, e->side>>>((unsigned*)e->pc_state, (unsigned*)(ms + M.snap), words,
+          k_ens_snapshot<true, unsigned><<<grid, 256, 0, side>>>((unsigned*)e->pc_state, (unsigned*)(ms + M.snap), words,
                                                                     per_net, d_still, w, ws, B, es);
         else
-          k_ens_snapshot<false, unsigned><<<grid, 256, 0, e->side>>>((unsigned*)e->pc_state, (unsigned*)(ms + M.snap),
+          k_ens_snapshot<false, unsigned><<<grid, 256, 0, side>>>((unsigned*)e->pc_state, (unsigned*)(ms + M.snap),
                                                                      words, per_net, d_still, w, ws, B, es);
       }
       return cudaGetLastError();
     };
     if (v == 2) PRS_CUDA(snapshot(false));
-    rc = prs_pc_step(pc, e->pc_state, d_odom, e->gi, d_argmax, d_total, d_err, e->side);
+    rc = prs_pc_step(pc, e->pc_state, d_odom, e->gi, d_argmax, d_total, d_err, side);
     if (rc != PRS_OK) return rc;
     if (v == 2) {
       PRS_CUDA(snapshot(true));
-      if (int rc_ = prs_pc_active_invalidate(pc, e->side)) return rc_;  // the carried lists describe the undone update
+      if (int rc_ = prs_pc_active_invalidate(pc, side)) return rc_;  // the carried lists describe the undone update
     }
-    PRS_CUDA(cudaEventRecord(e->ev_join, e->side));
+    if (image) PRS_CUDA(cudaEventRecord(e->ev_join, e->side));
   }
-  k_vt_frame_prepare_multi<<<R, 1024, 0, st>>>((const uint8_t*)(ms + M.frames), M.chunk, e->fbytes, e->im_cols, e->row_lo,
-                                               e->row_step, e->col_lo, e->col_step, (uint8_t*)(ms + M.tpl),
-                                               (uint32_t*)(ms + M.planes), d_key, B, d_ctr, d_gate, d_present);
+  if (!image) {
+    k_ens_no_image<<<1, B < 1024 ? (B + 31) / 32 * 32 : 1024, 0, st>>>(d_argmax, d_err, e->n_dev, d_rec, d_ctr, B);
+    PRS_CUDA(cudaGetLastError());
+    return PRS_OK;
+  }
+  if (events)
+    k_vt_frame_prepare_multi<true><<<R, 1024, 0, st>>>((const uint8_t*)(ms + M.frames), M.chunk, e->fbytes, e->im_cols,
+                                                       e->row_lo, e->row_step, e->col_lo, e->col_step,
+                                                       (uint8_t*)(ms + M.tpl), (uint32_t*)(ms + M.planes), d_key, B, d_ctr,
+                                                       d_gate, d_present, (const int*)(ms + M.slots));
+  else
+    k_vt_frame_prepare_multi<false><<<R, 1024, 0, st>>>((const uint8_t*)(ms + M.frames), M.chunk, e->fbytes, e->im_cols,
+                                                        e->row_lo, e->row_step, e->col_lo, e->col_step,
+                                                        (uint8_t*)(ms + M.tpl), (uint32_t*)(ms + M.planes), d_key, B,
+                                                        d_ctr, d_gate, d_present);
   long long blocks = (long long)B * ((e->capacity + 31) / 32);
   if (blocks > 148LL * 4) blocks = 148LL * 4;
   k_vt_sweep_packed_ref_small<true><<<(int)blocks, kSmallThreads, 0, st>>>(
@@ -2449,30 +2509,35 @@ static int ens_multi_enqueue(prs_ens_plan* e, int v, cudaStream_t st) {
   return PRS_OK;
 }
 
-// as ens_launch: eager first call, capture on the second, replay after
-static int ens_multi_launch(prs_ens_plan* e, int v, cudaStream_t st) {
-  if (e->mready[v]) {
-    PRS_CUDA(cudaGraphLaunch(e->mexec[v], st));
+// as ens_launch: eager first call, capture on the second, replay after.  kind 0: a frame of prs_ens_multi_replay_run
+// (graphs mexec[v]); 1 / 2: a tick of prs_ens_events_run with / without an image (eexec[v] / eexec[3 + v])
+static int ens_multi_launch(prs_ens_plan* e, int v, cudaStream_t st, int kind = 0) {
+  cudaGraphExec_t* exec = kind == 0 ? &e->mexec[v] : &e->eexec[kind == 1 ? v : 3 + v];
+  bool* ready = kind == 0 ? &e->mready[v] : &e->eready[kind == 1 ? v : 3 + v];
+  int* warm = kind == 0 ? &e->mwarm[v] : &e->ewarm[kind == 1 ? v : 3 + v];
+  const char* who = kind == 0 ? "prs_ens_multi_replay_run" : "prs_ens_events_run";
+  if (*ready) {
+    PRS_CUDA(cudaGraphLaunch(*exec, st));
     return PRS_OK;
   }
-  if (e->mwarm[v] < 1) {
-    ++e->mwarm[v];
-    return ens_multi_enqueue(e, v, st);
+  if (*warm < 1) {
+    ++*warm;
+    return ens_multi_enqueue(e, v, st, kind != 0, kind != 2);
   }
   cudaGraph_t g = nullptr;
   PRS_CUDA(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
-  int rc = ens_multi_enqueue(e, v, st);
+  int rc = ens_multi_enqueue(e, v, st, kind != 0, kind != 2);
   cudaError_t err = cudaStreamEndCapture(st, &g);
   if (rc != PRS_OK || err != cudaSuccess) {
     if (g) cudaGraphDestroy(g);
-    if (rc == PRS_OK) prs_set_error("prs_ens_multi_replay_run: capture failed: %s", cudaGetErrorString(err));
+    if (rc == PRS_OK) prs_set_error("%s: capture failed: %s", who, cudaGetErrorString(err));
     return rc != PRS_OK ? rc : PRS_E_CUDA;
   }
-  err = cudaGraphInstantiate(&e->mexec[v], g, 0);
+  err = cudaGraphInstantiate(exec, g, 0);
   cudaGraphDestroy(g);
   PRS_CUDA(err);
-  e->mready[v] = true;
-  PRS_CUDA(cudaGraphLaunch(e->mexec[v], st));
+  *ready = true;
+  PRS_CUDA(cudaGraphLaunch(*exec, st));
   return PRS_OK;
 }
 
@@ -2487,6 +2552,11 @@ extern "C" int prs_ens_set_recordings(prs_ens_plan* e, int R, const int* rec_of_
     if (e->mready[i]) cudaGraphExecDestroy(e->mexec[i]);
     e->mready[i] = false;
     e->mwarm[i] = 0;
+  }
+  for (int i = 0; i < 6; ++i) {
+    if (e->eready[i]) cudaGraphExecDestroy(e->eexec[i]);
+    e->eready[i] = false;
+    e->ewarm[i] = 0;
   }
   e->R = R;
   e->rec_of = rec_of_dev;
@@ -2552,6 +2622,91 @@ extern "C" int prs_ens_multi_replay_run(prs_ens_plan* e, const uint8_t* const* f
   const cudaError_t err = cudaStreamSynchronize(st);
   if (rc == PRS_OK && err != cudaSuccess) {
     prs_set_error("prs_ens_multi_replay_run: %s", cudaGetErrorString(err));
+    return PRS_E_CUDA;
+  }
+  return rc;
+}
+
+// ---------------------------------------------------------------------------------------------
+// Message-stream ensemble replay: the node's message loop (ros_simulate.replay_events) for every agent, one pose-cell
+// update per gated odometry message.  The caller compacts each recording's stream into ticks of (optional gated twist,
+// optional image), odometry before image; tick t of recording r has gate[t][r] bit 0 = image, bit 1 = moved.  A tick
+// is the multi-recording frame graph with two differences: the query of recording r is its image at slot
+// slots[t][r] of the chunk (images are contiguous per recording, not one per tick), and a tick with no image in any
+// recording runs the side branch alone, then k_ens_no_image.  Six graphs: {no update, all moved, mixed} x {image, none}.
+extern "C" int prs_ens_events_run(prs_ens_plan* e, const uint8_t* const* frames, const double* odom, const uint8_t* gate,
+                                  const int* n_images, int T, prs_frame_result* results, void* stream) {
+  PRS_REQUIRE(e && T >= 0 && n_images && (T == 0 || (frames && odom && gate && results)),
+              "prs_ens_events_run: bad argument");
+  PRS_REQUIRE(e->R >= 1, "prs_ens_events_run: no recordings set (prs_ens_set_recordings)");
+  PRS_REQUIRE(stream != nullptr, "prs_ens_events_run: needs a non-default stream (the ticks replay as CUDA graphs)");
+  const int R = e->R;
+  // slots[t][r]: recording r's image at tick t, counted from the first image of t's chunk; -1 = none
+  const EnsMultiScratch& M = e->mlay;
+  std::vector<int> slots((size_t)T * R);
+  std::vector<uint8_t> variant(T), has_image(T);
+  std::vector<int> seen(R, 0), in_chunk(R, 0);
+  long long image_ticks = 0;
+  for (int t = 0; t < T; ++t) {
+    if (t % M.chunk == 0) std::fill(in_chunk.begin(), in_chunk.end(), 0);
+    bool any = false, all = true, img = false;
+    for (int r = 0; r < R; ++r) {
+      const uint8_t g = gate[(size_t)t * R + r];
+      const bool here = (g & 1) != 0, mv = (g & 2) != 0;
+      slots[(size_t)t * R + r] = here ? in_chunk[r]++ : -1;
+      seen[r] += here ? 1 : 0;
+      img |= here;
+      any |= mv;
+      all &= mv;
+    }
+    variant[t] = (uint8_t)(!any ? 0 : all ? 1 : 2);
+    has_image[t] = img ? 1 : 0;
+    image_ticks += img ? 1 : 0;
+  }
+  for (int r = 0; r < R; ++r)
+    PRS_REQUIRE(n_images[r] == seen[r] && (seen[r] == 0 || frames[r]),
+                "prs_ens_events_run: recording %d has %d images in its gate, n_images says %d (or no frames)", r, seen[r],
+                n_images[r]);
+  PRS_REQUIRE(image_ticks <= e->room,
+              "prs_ens_events_run: %lld ticks with images do not fit the libraries (room for %lld more templates)",
+              image_ticks, e->room);
+  if (int rc = prs_pc_check_device(e->pc, "prs_ens_events_run")) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  char* ms = e->mscratch;
+  const size_t rec_bytes = (size_t)e->B * sizeof(prs_frame_result);
+  std::vector<long long> first(R, 0);  // each recording's first image of the chunk
+  int rc = PRS_OK;
+  for (int c0 = 0; c0 < T && rc == PRS_OK; c0 += M.chunk) {
+    const int n = T - c0 < M.chunk ? T - c0 : M.chunk;
+    long long img_ticks = 0;
+    for (int t = c0; t < c0 + n; ++t) img_ticks += has_image[t];
+    for (int r = 0; r < R; ++r) {
+      int nr = 0;
+      for (int t = c0; t < c0 + n; ++t) nr += slots[(size_t)t * R + r] >= 0 ? 1 : 0;
+      if (nr > 0)
+        PRS_CUDA(cudaMemcpyAsync(ms + M.frames + (size_t)r * M.chunk * e->fbytes, frames[r] + first[r] * e->fbytes,
+                                 (size_t)nr * e->fbytes, cudaMemcpyHostToDevice, st));
+      first[r] += nr;
+    }
+    PRS_CUDA(cudaMemcpyAsync(ms + M.odom_chunk, odom + (size_t)c0 * R * 2, (size_t)n * R * 2 * sizeof(double),
+                             cudaMemcpyHostToDevice, st));
+    PRS_CUDA(cudaMemcpyAsync(ms + M.gate, gate + (size_t)c0 * R, (size_t)n * R, cudaMemcpyHostToDevice, st));
+    PRS_CUDA(cudaMemcpyAsync(ms + M.slots, slots.data() + (size_t)c0 * R, (size_t)n * R * sizeof(int),
+                             cudaMemcpyHostToDevice, st));
+    PRS_CUDA(cudaMemsetAsync(e->scratch + e->lay.misc, 0, sizeof(int), st));  // the tick counter
+    int done = 0;
+    for (; done < n; ++done) {
+      rc = ens_multi_launch(e, variant[c0 + done], st, has_image[c0 + done] ? 1 : 2);
+      if (rc != PRS_OK) break;
+    }
+    if (done > 0)
+      PRS_CUDA(cudaMemcpyAsync(results + (size_t)c0 * e->B, ms + M.rec, (size_t)done * rec_bytes, cudaMemcpyDeviceToHost,
+                               st));
+    e->room -= img_ticks;
+  }
+  const cudaError_t err = cudaStreamSynchronize(st);
+  if (rc == PRS_OK && err != cudaSuccess) {
+    prs_set_error("prs_ens_events_run: %s", cudaGetErrorString(err));
     return PRS_E_CUDA;
   }
   return rc;

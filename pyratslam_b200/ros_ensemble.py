@@ -225,6 +225,74 @@ def feed_inputs(frames, odom, n_recordings):
     return fr, od
 
 
+def _is_event(x):
+    return isinstance(x, (tuple, list)) and len(x) == 3 and isinstance(x[0], str)
+
+
+def event_ticks(events):
+    """Compact one message stream (``rosbag_io.read_events``) into ticks of (optional gated twist, optional image),
+    odometry before image, as ``ros_simulate.replay_events(fused=True)`` folds it (no CUDA involved): an odometry message
+    directly followed by an image shares that image's tick, odometry the 0.001 gate drops makes no tick, an image with
+    no twist before it is an image-only tick and any other odometry an odometry-only tick.  Returns ``(frames uint8
+    [I,256,256], odom float64 [K,2], moved uint8 [K], image bool [K])``: the stream's images in order, and per tick the
+    (linear.x, angular.z) twist (0 where it does not move), the gate and whether it has an image.  ``ValueError`` for
+    anything that is not such a stream."""
+    if isinstance(events, (str, bytes)) or not hasattr(events, "__iter__"):
+        raise ValueError("a message stream is a sequence of (kind, stamp, payload) events, got %r" % (events,))
+    events = list(events)
+    frames, odom, moved, image = [], [], [], []
+    i, n = 0, len(events)
+    while i < n:
+        ev = events[i]
+        if not _is_event(ev):
+            raise ValueError("event %d is not a (kind, stamp, payload) tuple: %r" % (i, ev))
+        kind, _, payload = ev
+        if kind == "odom":
+            try:
+                x, z = float(payload[0]), float(payload[1])
+            except (TypeError, ValueError, IndexError):
+                raise ValueError("event %d: odometry must be a (linear.x, angular.z) pair, got %r" % (i, payload)) from None
+            mv = abs(x) > 0.001 or abs(z) > 0.001                                  # ros_simulate.py:128
+            paired = i + 1 < n and _is_event(events[i + 1]) and events[i + 1][0] == "image"
+            if mv or paired:
+                odom.append((x, z) if mv else (0.0, 0.0))
+                moved.append(mv)
+                image.append(paired)
+                if paired:
+                    i += 1
+                    frames.append(events[i][2])
+            i += 1
+            continue
+        if kind != "image":
+            raise ValueError("event %d: unknown event kind %r" % (i, kind))
+        odom.append((0.0, 0.0))
+        moved.append(False)
+        image.append(True)
+        frames.append(payload)
+        i += 1
+    for j, f in enumerate(frames):
+        f = np.asarray(f)
+        if f.dtype != np.uint8 or f.shape != IM_SIZE:
+            raise ValueError("image %d of the stream must be uint8 %r, got %s %r" % (j, IM_SIZE, f.dtype, f.shape))
+        frames[j] = f
+    fr = np.stack(frames) if frames else np.zeros((0,) + IM_SIZE, np.uint8)
+    return (fr, np.asarray(odom, dtype=np.float64).reshape(-1, 2), np.asarray(moved, dtype=np.uint8),
+            np.asarray(image, dtype=np.bool_))
+
+
+def event_streams(events, n_recordings):
+    """One feed of message streams for a session of ``n_recordings`` recordings: a stream for R = 1, a list of R streams
+    otherwise.  Returns the R compacted streams (``event_ticks``); ``ValueError`` for anything else."""
+    R = int(n_recordings)
+    if R == 1:
+        return [event_ticks(events)]
+    if (isinstance(events, (str, bytes)) or not isinstance(events, (list, tuple)) or len(events) != R
+            or any(_is_event(s) for s in events)):
+        raise ValueError("EnsembleSession.feed_events: a session of %d recordings takes a list of %d message streams"
+                         % (R, R))
+    return [event_ticks(s) for s in events]
+
+
 class EnsembleSession:
     """B RatSLAM agents that stay on the device between calls: ``feed`` replays the next frames of every recording.
 
@@ -294,6 +362,7 @@ class EnsembleSession:
         self._scratch = torch.empty(int(L.prs_ens_scratch_bytes(B, IM_SIZE[0], IM_SIZE[1])), dtype=torch.uint8,
                                     device=dev)
         self._mscratch = None
+        self._multi = R > 1          # the several-recordings machinery is attached (always for R > 1)
         self._stream = torch.cuda.Stream(device=dev)
         self.frames_fed = np.zeros(R, np.int64)
         self._n = np.zeros(B, np.int64)                       # templates per device row
@@ -327,7 +396,7 @@ class EnsembleSession:
             self._scratch.data_ptr(), ctypes.byref(plan)), "prs_ens_create")
         self._plan = plan
         self._room = self.capacity - int(self._n.max())
-        if self.R > 1:
+        if self._multi:
             if self._mscratch is None:
                 self._mscratch = torch.empty(int(L.prs_ens_multi_scratch_bytes(plan, self.R)), dtype=torch.uint8,
                                              device=self._dev)
@@ -395,8 +464,15 @@ class EnsembleSession:
                     self._room -= run
                     self._n = res["n_templates"][s0 + run - 1].astype(np.int64)
                     if self._linked:
-                        self._maps(res[sub], tw[sub], moved[sub], np.clip(lengths - s0, 0, run), n_exp[sub],
-                                   exp_id[sub], em_xy[sub])
+                        sub_len = np.clip(lengths - s0, 0, run)
+                        tpl = res["template_index"][sub]
+                        tag = np.empty((run, B), np.int32)
+                        tag[0] = self._prev_tpl
+                        tag[1:] = np.maximum(tpl[:-1], -1)
+                        mine = sub_len[self._rec_of[self._order]]        # per device row: its frames in this sub-run
+                        here = mine > 0
+                        self._prev_tpl[here] = tpl[mine[here] - 1, np.nonzero(here)[0]]
+                        self._maps(res[sub], tag, run, tw[sub], moved[sub], n_exp[sub], exp_id[sub], em_xy[sub])
                     s0 += run
         except BaseException:
             self.close()
@@ -452,18 +528,155 @@ class EnsembleSession:
             t, b = np.argwhere(bad)[0]                  # frame-major: the earliest frame, then the lowest agent
             self._ens._raise_on_err(np.array([rc["pc_err"][t, b] & ~nat.ERR_INJECT_LOC], dtype=np.int32))
 
-    def _maps(self, res, tw, moved, sub_len, n_exp, exp_id, em_xy):
-        """The linked maps continued over one sub-run's records (device rows)."""
+    def _attach_multi(self):
+        """The several-recordings machinery for a session of one recording, at its first ``feed_events``; ``feed`` keeps
+        using the single-recording frames."""
+        L = nat.lib()
+        self._multi = True
+        self._mscratch = torch.empty(int(L.prs_ens_multi_scratch_bytes(self._plan, self.R)), dtype=torch.uint8,
+                                     device=self._dev)
+        nat.check(L.prs_ens_set_recordings(self._plan, self.R, self._rec_dev.data_ptr(), self._mscratch.data_ptr()),
+                  "prs_ens_set_recordings")
+
+    def feed_events(self, events):
+        """Replay the next messages of every recording the way the node's message loop does
+        (``ros_simulate.replay_events``): one pose-cell update and one experience-map update per gated odometry message,
+        one match per image.  ``events`` is a message stream (``rosbag_io.read_events``, or a piece of ``iter_events``)
+        for R = 1 and a list of R streams otherwise, any of them empty; a piece may end anywhere, inside a run of
+        odometry too.  The streams are compacted into ticks (``event_ticks``) and replayed with
+        ``prs_ens_events_run``.  Returns per image: ``template``, ``created``, ``argmax`` ``[B, i_max]``, ``length [B]``
+        (the images of the agent's recording in this feed; -1 / False past it), ``n_templates [B]``, and with
+        ``experience_map="device"`` ``n_exp``, ``exp_id``, ``em_xy`` at each image (-1 / NaN past the length) and
+        ``n_loop_closures``.  ``feed`` and ``feed_events`` continue the same agents, libraries and maps."""
+        if self._closed:
+            raise RuntimeError("EnsembleSession: the session is closed")
+        return self._feed_ticks(event_streams(events, self.R))
+
+    def _feed_ticks(self, streams):
+        R, B = self.R, self.B
+        n_ticks = np.array([len(st[2]) for st in streams], dtype=np.int64)
+        n_img = np.array([len(st[0]) for st in streams], dtype=np.int64)
+        K = int(n_ticks.max())
+        moved = np.zeros((K, R), np.uint8)             # past a recording's ticks: no update, no image
+        tw = np.zeros((K, R, 2))
+        img = np.zeros((K, R), np.bool_)
+        for r, (_, od, _, im) in enumerate(streams):
+            moved[:n_ticks[r], r], tw[:n_ticks[r], r] = xens.gate(od)
+            img[:n_ticks[r], r] = im
+        gate = np.ascontiguousarray(img.astype(np.uint8) | (moved << 1))
+        img_tick = img.any(axis=1)
+        res = np.empty((K, B), dtype=RatslamRos._RESULT_DTYPE)    # device rows; every tick's records are written
+        rec_rows = self._rec_of[self._order]                        # per device row: its recording
+        if self._linked:
+            n_exp = np.zeros((K, B), np.int32)
+            exp_id = np.zeros((K, B), np.int32)
+            em_xy = np.zeros((K, B, 2))
+        first = np.zeros(R, np.int64)                  # per recording: its first image of the sub-run
+        try:
+            with torch.cuda.device(self._dev):
+                if not self._multi:
+                    self._attach_multi()
+                k0 = 0
+                while k0 < K:
+                    left = int(img_tick[k0:].sum())
+                    cap, run = grow_capacity(self.capacity, int(self._n.max()), left)
+                    if run == 0 and left:
+                        d = int(np.argmax(self._n))
+                        raise ValueError("EnsembleSession: agent %d holds %d templates, the most the library sweep "
+                                         "takes, and image %d of its recording remains"
+                                         % (self._order[d], self._n[d], self.frames_fed[rec_rows[d]] + first[rec_rows[d]]))
+                    if cap != self.capacity:
+                        self._grow(cap)
+                    # ticks [k0, k1) hold `run` ticks with images; the last sub-run takes the trailing odometry
+                    k1 = K if run >= left else k0 + int(np.nonzero(img_tick[k0:])[0][run])
+                    if self._room < min(run, left):
+                        nat.check(nat.lib().prs_ens_refresh_room(self._plan, ctypes.c_void_p(self._stream.cuda_stream)),
+                                  "prs_ens_refresh_room")
+                        self._room = self.capacity - int(self._n.max())
+                    sub = slice(k0, k1)
+                    sub_img = img[sub].sum(axis=0)
+                    self._replay_events(streams, first, sub_img, tw[sub], moved[sub], gate[sub], res[sub])
+                    self._room -= int(img_tick[sub].sum())
+                    self._n = res["n_templates"][k1 - 1].astype(np.int64)
+                    if self._linked:
+                        self._maps(res[sub], self._event_tags(res[sub], img[sub][:, rec_rows]),
+                                   int(moved[sub].sum(axis=0).max()), tw[sub], moved[sub], n_exp[sub], exp_id[sub],
+                                   em_xy[sub])
+                    first += sub_img
+                    k0 = k1
+        except BaseException:
+            self.close()
+            raise
+        self.frames_fed += n_img
+        length = n_img[self._rec_of]
+        i_max = int(n_img.max())
+        out = {"template": np.full((B, i_max), -1, np.int64), "created": np.zeros((B, i_max), np.bool_),
+               "argmax": np.full((B, i_max, 3), -1, np.int64), "n_templates": self.n_templates, "length": length}
+        if self._map:
+            out["n_exp"] = np.full((B, i_max), -1, np.int64)
+            out["exp_id"] = np.full((B, i_max), -1, np.int64)
+            out["em_xy"] = np.full((B, i_max, 2), np.nan)
+        for r in range(R):
+            ticks = np.nonzero(img[:, r])[0]
+            agents = np.nonzero(self._rec_of == r)[0]
+            cols = self._rows[agents]
+            m = len(ticks)
+            out["template"][agents, :m] = res["template_index"][ticks][:, cols].T
+            out["created"][agents, :m] = res["created"][ticks][:, cols].T != 0
+            out["argmax"][agents, :m] = _unravel(res["argmax"][ticks][:, cols].T, self.pose_size)
+            if self._linked:
+                out["n_exp"][agents, :m] = n_exp[ticks][:, cols].T
+                out["exp_id"][agents, :m] = exp_id[ticks][:, cols].T
+                out["em_xy"][agents, :m] = em_xy[ticks][:, cols].transpose(1, 0, 2)
+            if self._map:
+                n_r, xy_r = self._dead_reckoning(r, moved[:, r], tw[:, r], n_ticks[r])
+                if not self._linked:
+                    out["n_exp"][agents, :m] = n_r[ticks]
+                    out["exp_id"][agents, :m] = n_r[ticks] - 1
+                    out["em_xy"][agents, :m] = xy_r[ticks]
+        if self._map:
+            out["n_loop_closures"] = self.n_loop_closures
+        return out
+
+    def _replay_events(self, streams, first, sub_img, tw, moved, gate, res):
+        """One sub-run of ticks through ``prs_ens_events_run``; raises a pose-cell error as ``replay_events`` does, for
+        the earliest tick and, within it, the lowest agent."""
+        L = nat.lib()
+        fb = IM_SIZE[0] * IM_SIZE[1]
+        ptrs = (ctypes.c_void_p * self.R)(*[streams[r][0].ctypes.data + int(first[r]) * fb if sub_img[r] else None
+                                            for r in range(self.R)])
+        tw, n_images = np.ascontiguousarray(tw), np.ascontiguousarray(sub_img, dtype=np.int32)
+        nat.check(L.prs_ens_events_run(self._plan, ptrs, tw.ctypes.data, gate.ctypes.data, n_images.ctypes.data,
+                                       len(gate), res.ctypes.data, ctypes.c_void_p(self._stream.cuda_stream)),
+                  "prs_ens_events_run")
+        if not (((res["pc_err"] & ~nat.ERR_INJECT_LOC) != 0) & (moved[:, self._rec_of[self._order]] != 0)).any():
+            return
+        rc = res[:, self._rows]
+        bad = ((rc["pc_err"] & ~nat.ERR_INJECT_LOC) != 0) & (moved[:, self._rec_of] != 0)
+        t, b = np.argwhere(bad)[0]
+        self._ens._raise_on_err(np.array([rc["pc_err"][t, b] & ~nat.ERR_INJECT_LOC], dtype=np.int32))
+
+    def _event_tags(self, res, img):
+        """``tag [K,B]`` of one sub-run of ticks (device rows): the template of the agent's most recent image before
+        each tick (``RatslamRos._em_update``'s ``published_index[-1]``), carried across sub-runs and feeds."""
+        K, B = res.shape
+        last = np.where(img, np.arange(K)[:, None], -1)
+        np.maximum.accumulate(last, axis=0, out=last)
+        filled = np.where(last >= 0, res["template_index"][np.maximum(last, 0), np.arange(B)[None, :]],
+                          self._prev_tpl[None, :]).astype(np.int32)
+        tag = np.empty((K, B), np.int32)
+        tag[0] = self._prev_tpl
+        tag[1:] = filled[:-1]
+        if K:
+            self._prev_tpl = filled[-1].copy()
+        return tag
+
+    def _maps(self, res, tag, updates, tw, moved, n_exp, exp_id, em_xy):
+        """The linked maps continued over one sub-run's records (device rows): ``tag [T,B]`` is the view each step's
+        experience is tagged with, ``updates`` bounds the moved steps of any agent (one experience and one link each)."""
         L = nat.lib()
         T, B = res.shape
-        tpl = res["template_index"]
-        tag = np.empty((T, B), np.int32)
-        tag[0] = self._prev_tpl
-        tag[1:] = np.maximum(tpl[:-1], -1)
-        mine = sub_len[self._rec_of[self._order]]        # per device row: its frames in this sub-run
-        here = mine > 0
-        self._prev_tpl[here] = tpl[mine[here] - 1, np.nonzero(here)[0]]
-        E = _grow_rows(self._E, int(self._counts[:2].max()) + T)
+        E = _grow_rows(self._E, int(self._counts[:2].max()) + int(updates))
         if E != self._E or self.capacity != self._N:
             self._grow_maps(E, self.capacity)
         X, Y, Th = self.pose_size
@@ -502,6 +715,15 @@ class EnsembleSession:
     def n_templates(self):
         """int64 [B]: templates in each agent's library."""
         return self._n[self._rows].copy()
+
+    @property
+    def n_experiences(self):
+        """int64 [B]: experiences in each agent's map so far (0 without ``experience_map``)."""
+        if self._linked:
+            return self._counts[0][self._rows].copy()
+        if self._map:
+            return np.array([self._dr[r][0] for r in self._rec_of], dtype=np.int64)
+        return np.zeros(self.B, np.int64)
 
     @property
     def n_loop_closures(self):
@@ -651,6 +873,63 @@ def replay_ensemble(frames, odom, n_agents=None, match_threshold=MATCH_THRESHOLD
     return out
 
 
+def replay_ensemble_events(events, n_agents=None, match_threshold=MATCH_THRESHOLD, global_inhibition=PC_GLOBAL_INHIB,
+                           inject_energy=None, pose_size=POSE_SIZE, dtype=np.float32, active_set=0, experience_map=False,
+                           experience_links=False, mode="ref", recording=0):
+    """``replay_ensemble`` over message streams (``rosbag_io.read_events``) instead of paired frames and twists: agent b
+    is the node's message loop, ``ros_simulate.replay_events(events, match_threshold=..., inject_energy=...,
+    experience_links=...)`` with ``pcn.global_inhibition`` set to its own value, so every gated odometry message is its
+    own pose-cell update and experience-map update.  ``events`` is one stream, or a list of R streams with
+    ``recording`` naming each agent's.  The parameters and their validation are ``replay_ensemble``'s;
+    ``experience_map`` is False or "device" (the host maps, True, are refused).  Returns what
+    ``EnsembleSession.feed_events`` returns -- per image ``template``, ``created``, ``argmax`` ``[B, i_max]`` and
+    ``length [B]``, the maps' ``n_exp``, ``exp_id``, ``em_xy`` and ``n_loop_closures`` -- plus ``agents`` and, with
+    ``experience_map="device"``, ``maps``.  On a stream in which odometry and images alternate it equals
+    ``replay_ensemble`` on ``rosbag_io.events_to_arrays(events)[:2]``.  This is one ``EnsembleSession`` fed once."""
+    if not (isinstance(experience_map, (bool, np.bool_)) and not experience_map
+            or (isinstance(experience_map, str) and experience_map == "device")):
+        raise ValueError("replay_ensemble_events: experience_map must be False or 'device' (the host maps need the "
+                         "paired frames of replay_ensemble), got %r" % (experience_map,))
+    B, thr, gi, energies = agent_parameters(n_agents if n_agents is not None else _recording_count(recording),
+                                            match_threshold, global_inhibition, inject_energy)
+    if mode != "ref":
+        raise ValueError("replay_ensemble_events supports the reference matching mode only, got mode=%r" % (mode,))
+    several = (isinstance(events, (list, tuple)) and len(events) > 0 and not _is_event(events[0]))
+    R = len(events) if several else 1
+    rec_of = agent_recordings(recording, B, R)
+    streams = [event_ticks(st) for st in events] if several else [event_ticks(events)]
+    pose_size = tuple(int(s) for s in pose_size)
+    np_dtype = _as_np_dtype(dtype)
+    K = max(len(st[2]) for st in streams)
+    img = np.zeros((K, R), np.bool_)
+    for r, st in enumerate(streams):
+        img[:len(st[3]), r] = st[3]
+    cap = min(capacity_for(int(img.any(axis=1).sum())), MAX_CAPACITY)
+    lib_bytes = (cap // 32) * 34816
+    net_bytes = int(np.prod(pose_size)) * np.dtype(np_dtype).itemsize
+    # per agent: library, locations, network, its snapshot and the records; plus one chunk of every recording's images
+    frame_bytes = IM_SIZE[0] * IM_SIZE[1]
+    need = B * (lib_bytes + cap * 8 + 2 * net_bytes + 64) + R * _multi_chunk(R, frame_bytes) * frame_bytes
+    if experience_map == "device" and experience_links:
+        need += xens.work_bytes(B, K, cap) + xens.record_bytes(B, K)
+    nat.require_cuda()
+    dev = torch.device("cuda", torch.cuda.current_device())
+    free, _ = torch.cuda.mem_get_info(dev)
+    if need > free:
+        raise ValueError("replay_ensemble_events: %d agents x %d templates need %.2f GB of device memory, %.2f GB are "
+                         "free" % (B, cap, need / 1e9, free / 1e9))
+    session = EnsembleSession(B, thr, gi, energies, pose_size, np_dtype, active_set, experience_map, experience_links,
+                              R, rec_of, cap)
+    try:
+        out = session._feed_ticks(streams)
+        out["agents"] = session.agents
+        if experience_map == "device":
+            out["maps"] = session.maps
+    finally:
+        session.close()
+    return out
+
+
 def _experience_maps(out, moved, tw, pose_size, linked, rec_of=None):
     """Each agent's experience map replayed from its records (``RatslamRos.replay_native``'s bookkeeping); with
     ``rec_of``, ``moved [T,R]`` and ``tw [T,R,2]`` hold every recording's odometry and agent b follows ``rec_of[b]``."""
@@ -713,6 +992,37 @@ def _replay_chunked(bags, chunk, image_topic, odom_topic, recording, **kw):
         s.close()
 
 
+def _replay_all_messages(bags, chunk, image_topic, odom_topic, recording, **kw):
+    """``--all-messages``: the bags' message streams fed through one ``EnsembleSession`` with ``feed_events``, ``chunk``
+    images per bag at a time (each bag whole without it): per agent the templates, the images created on, its bag's
+    image count and final arg-max, and the experience and loop-closure counts of its map."""
+    from . import rosbag_io as rb
+    R = len(bags)
+    if chunk is None:
+        its = [iter([rb.read_events(bag, image_topic=image_topic, odom_topic=odom_topic)]) for bag in bags]
+    else:
+        its = [rb.iter_events(bag, chunk, image_topic=image_topic, odom_topic=odom_topic) for bag in bags]
+    s = EnsembleSession(n_recordings=R, recording=recording if R > 1 else 0,
+                        capacity=capacity_for(chunk) if chunk is not None else None, **kw)
+    try:
+        B = len(s.n_templates)
+        created = np.zeros(B, np.int64)
+        last = [None] * B
+        while True:
+            pieces = [next(it, None) for it in its]
+            if all(p is None for p in pieces):
+                break
+            ev = [p if p is not None else [] for p in pieces]
+            out = s.feed_events(ev if R > 1 else ev[0])
+            created += out["created"].sum(axis=1)
+            for b in range(B):
+                if out["length"][b]:
+                    last[b] = tuple(int(c) for c in out["argmax"][b, out["length"][b] - 1])
+        return s.n_templates, created, s.frames_fed, last, s.n_experiences, s.n_loop_closures
+    finally:
+        s.close()
+
+
 def main(argv=None):
     import argparse
     ap = argparse.ArgumentParser(description="Replay ROS1 bags through an ensemble of RatSLAM agents: the cross product "
@@ -729,7 +1039,11 @@ def main(argv=None):
     ap.add_argument("--odom-topic", default="navbot/odom")
     ap.add_argument("--chunk", type=_chunk_arg, metavar="FRAMES",
                     help="feed the bags through one session this many frames per bag at a time, decoding only those "
-                         "frames (the output is the same as without it)")
+                         "frames (the output is the same as without it); with --all-messages, this many images")
+    ap.add_argument("--all-messages", action="store_true",
+                    help="replay every odometry message as its own pose-cell update, as the node's message loop does "
+                         "(ros_simulate), instead of pairing each image with the last twist before it; also prints "
+                         "every agent's experience count")
     a = ap.parse_args(argv)
     from . import rosbag_io as rb
     thr = _list(a.match_threshold, float)
@@ -740,8 +1054,14 @@ def main(argv=None):
     agents = list(itertools.product(range(len(a.bag)), combos))     # bag-major
     kw = dict(n_agents=len(agents), match_threshold=[c[0] for _, c in agents],
               global_inhibition=[c[1] for _, c in agents], inject_energy=[c[2] for _, c in agents],
-              experience_map="device" if a.experience_links else False, experience_links=a.experience_links)
-    if a.chunk is not None:
+              experience_map="device" if a.experience_links or a.all_messages else False,
+              experience_links=a.experience_links)
+    n_exp = None
+    if a.all_messages:
+        n_templates, created, fed, last, n_exp, loops = _replay_all_messages(a.bag, a.chunk, a.image_topic,
+                                                                             a.odom_topic, [r for r, _ in agents], **kw)
+        frames = [int(fed[r if several else 0]) for r, _ in agents]
+    elif a.chunk is not None:
         n_templates, created, fed, last, maps = _replay_chunked(a.bag, a.chunk, a.image_topic, a.odom_topic,
                                                                 [r for r, _ in agents], **kw)
         frames = [int(fed[r if several else 0]) for r, _ in agents]
@@ -763,7 +1083,11 @@ def main(argv=None):
                                       int(created[b]), frames[b], last[b]))
         if several:
             line = "bag %s  %s" % (a.bag[r], line)
-        if a.experience_links:
+        if n_exp is not None:
+            line += "  experiences %d" % n_exp[b]
+            if a.experience_links:
+                line += "  loop closures %d" % loops[b]
+        elif a.experience_links:
             line += "  experiences %d  loop closures %d" % (maps.n_experiences[b], loops[b])
         print(line)
 

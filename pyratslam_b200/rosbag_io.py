@@ -468,3 +468,49 @@ def write_run(path, frames, odom, rate_hz=10.0, compression="none", image_topic=
             w.write(odom_topic, "nav_msgs/Odometry", s_odom,
                     encode_odometry(odom[t][0], odom[t][1], stamp=s_odom, seq=t))
             w.write(image_topic, "sensor_msgs/Image", s_img, encode_image(frames[t], stamp=s_img, seq=t))
+
+
+def iter_events(path, chunk, image_topic=IMAGE_TOPIC, odom_topic=ODOM_TOPIC):
+    """``read_events(path, ...)`` in pieces: yields lists of events holding at most ``chunk`` images each.  A piece ends
+    right after its ``chunk``-th image, wherever that falls (the odometry after it opens the next piece), and the last
+    piece holds what remains, trailing odometry included; concatenated, the pieces are ``read_events``.  Images are
+    decoded only for the piece being yielded; ``BagReader`` still reads the file whole."""
+    chunk = int(chunk)
+    if chunk < 1:
+        raise ValueError("iter_events: chunk must be >= 1, got %r" % (chunk,))
+    bag = BagReader(path)
+    want = {image_topic.lstrip("/"): "image", odom_topic.lstrip("/"): "odom"}
+    piece, n_img = [], 0
+    for m in bag.messages():
+        kind = want.get(m.topic.lstrip("/"))
+        if kind == "odom":
+            o = decode_odometry(m.data)
+            piece.append(("odom", m.stamp, (o.linear[0], o.angular[2])))
+        elif kind == "image":
+            piece.append(("image", m.stamp, m.data))
+            n_img += 1
+            if n_img == chunk:
+                yield [(k, s, decode_image(p).image if k == "image" else p) for k, s, p in piece]
+                piece, n_img = [], 0
+    if piece:
+        yield [(k, s, decode_image(p).image if k == "image" else p) for k, s, p in piece]
+
+
+def write_events(path, events, compression="none", image_topic=IMAGE_TOPIC, odom_topic=ODOM_TOPIC,
+                 chunk_threshold=768 * 1024):
+    """Write a message stream as ``read_events`` returns it -- ``("odom", stamp, (linear.x, angular.z))`` and
+    ``("image", stamp, uint8[H, W])`` -- as a bag, each message at its own stamp, so that ``read_events`` gives the
+    stream back."""
+    with BagWriter(path, compression=compression, chunk_threshold=chunk_threshold) as w:
+        n_odom = n_img = 0
+        for kind, stamp, payload in events:
+            stamp = (int(stamp[0]), int(stamp[1]))
+            if kind == "odom":
+                w.write(odom_topic, "nav_msgs/Odometry", stamp,
+                        encode_odometry(payload[0], payload[1], stamp=stamp, seq=n_odom))
+                n_odom += 1
+            elif kind == "image":
+                w.write(image_topic, "sensor_msgs/Image", stamp, encode_image(payload, stamp=stamp, seq=n_img))
+                n_img += 1
+            else:
+                raise ValueError("write_events: unknown event kind %r" % (kind,))
