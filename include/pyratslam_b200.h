@@ -320,7 +320,7 @@ PRS_API size_t prs_frame_scratch_bytes(void);
  *   scratch : device, prs_frame_scratch_bytes()
  *   frame_host / odom_host / result_host : host (pinned for asynchronous copies) */
 PRS_API int prs_frame_host(prs_pc_handle pc, void* pc_state, const void* gi, void* pc_work, const double* odom_host,
-                   void* vt_packed, int n_templates, unsigned threshold, int mode, const uint8_t* frame_host,
+                   void* vt_packed, int n_templates, double threshold, int mode, const uint8_t* frame_host,
                    int im_rows, int im_cols, int row_lo, int row_hi, int row_step, int col_lo, int col_hi,
                    int col_step, void* scratch, prs_frame_result* result_host, void* stream);
 
@@ -331,7 +331,7 @@ PRS_API int prs_frame_host(prs_pc_handle pc, void* pc_state, const void* gi, voi
  * `stream` must be a non-default stream for the graph to be captured (otherwise every frame is enqueued eagerly). */
 typedef struct prs_frame_plan prs_frame_plan;
 PRS_API int prs_frame_create(prs_pc_handle pc, void* pc_state, const void* gi, void* pc_work, void* vt_packed,
-                     int n_templates, int capacity, unsigned threshold, int mode, int im_rows, int im_cols,
+                     int n_templates, int capacity, double threshold, int mode, int im_rows, int im_cols,
                      int row_lo, int row_hi, int row_step, int col_lo, int col_hi, int col_step, void* scratch,
                      double* odom_host, uint8_t* frame_host, prs_frame_result* result_host, prs_frame_plan** out);
 PRS_API int prs_frame_destroy(prs_frame_plan* plan);
@@ -385,7 +385,8 @@ PRS_API int prs_replay_run(prs_frame_plan* const* plans, int n_plans, const uint
  *   libs          : device, B libraries of prs_vt_packed_bytes(capacity) bytes each, zero-filled once
  *   capacity      : templates per library, at most 65536
  *   n_dev         : device int32 [B], templates in each library; updated by every frame
- *   threshold_dev : device uint32 [B], the match thresholds (clamped to [0, 2^32-1] by the caller)
+ *   threshold_dev : device double [B], the match thresholds as the caller gives them (create when score > threshold,
+ *                   so a negative threshold creates on every frame)
  *   energy_dev    : device double [B], energy injected at the frame template's cell; a value that is not >= 0 (e.g. -1)
  *                   means no injection for that agent; NULL: no injection node at all
  *   loc_dev       : device int64 [B][capacity], C-order flat cell of every template, -1 = invalid
@@ -394,7 +395,7 @@ PRS_API int prs_replay_run(prs_frame_plan* const* plans, int n_plans, const uint
 typedef struct prs_ens_plan prs_ens_plan;
 PRS_API size_t prs_ens_scratch_bytes(int B, int im_rows, int im_cols);
 PRS_API int prs_ens_create(prs_pc_handle pc, void* pc_state, const void* gi, void* pc_work, void* libs, int capacity,
-                   int* n_dev, const unsigned* threshold_dev, const double* energy_dev, long long* loc_dev, int mode,
+                   int* n_dev, const double* threshold_dev, const double* energy_dev, long long* loc_dev, int mode,
                    int im_rows, int im_cols, int row_lo, int row_hi, int row_step, int col_lo, int col_hi,
                    int col_step, void* scratch, prs_ens_plan** out);
 PRS_API int prs_ens_destroy(prs_ens_plan* plan);

@@ -82,10 +82,10 @@ _SIGNATURES = {
 }
 
 _SIGNATURES["prs_frame_scratch_bytes"] = (c_size_t, [])
-_SIGNATURES["prs_frame_host"] = (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, ctypes.c_uint,
+_SIGNATURES["prs_frame_host"] = (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_double,
                                          c_int, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p,
                                          c_void_p, c_void_p])
-_SIGNATURES["prs_frame_create"] = (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, ctypes.c_uint,
+_SIGNATURES["prs_frame_create"] = (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_double,
                                            c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p,
                                            c_void_p, c_void_p, c_void_p, POINTER(c_void_p)])
 _SIGNATURES["prs_frame_destroy"] = (c_int, [c_void_p])

@@ -1253,7 +1253,7 @@ struct FrameScratch {               // device scratch layout (bytes)
 struct VtAgents {
   int B = 1;
   long long lib_u4 = 0;                 // uint4 per agent library
-  const unsigned* threshold = nullptr;  // [B]; null: the kernel's scalar threshold
+  const double* threshold = nullptr;    // [B]; null: the kernel's scalar threshold
   long long* loc = nullptr;             // [B][loc_stride]: a created template's row receives the agent's arg-max
   long long loc_stride = 0;
   int* g_max = nullptr;                 // largest group count over the agents, raised by the decision (the sweep's grid)
@@ -1268,7 +1268,7 @@ struct VtAgents {
 // dec (optional): a second, device-side copy of the decision (created, template_index, n_templates) for the frame's
 // injection node when `res` is the pinned host record
 __global__ void k_vt_decide_append(const unsigned long long* __restrict__ key, const uint8_t* __restrict__ tpl,
-                                   uint4* __restrict__ packed, int n, unsigned threshold,
+                                   uint4* __restrict__ packed, int n, double threshold,
                                    const long long* __restrict__ argmax, const int* __restrict__ pc_err,
                                    prs_frame_result* __restrict__ res, int* __restrict__ n_dev, int write_pc = 1,
                                    prs_frame_result* __restrict__ dec = nullptr, VtAgents ag = VtAgents()) {
@@ -1295,7 +1295,9 @@ __global__ void k_vt_decide_append(const unsigned long long* __restrict__ key, c
   const unsigned long long k = key[b];
   const unsigned score = (unsigned)(k >> 32);
   if (ag.threshold != nullptr) threshold = ag.threshold[b];
-  const bool create = (n == 0) || (k == ~0ull) || (score > threshold);  // strict '>' (view_templates.py:67)
+  // strict '>' (view_templates.py:67) on the caller's number: a score is an integer <= 130560, exact in a double, so a
+  // negative threshold creates on every frame and a fractional or huge one means what it means to the reference
+  const bool create = (n == 0) || (k == ~0ull) || ((double)score > threshold);
   if (create) {
     vt_pack_row(tpl, packed + b * ag.lib_u4, n, t);
   }
@@ -1385,7 +1387,7 @@ __global__ void k_frame_inject(T* __restrict__ state, long long* __restrict__ lo
 extern "C" size_t prs_frame_scratch_bytes(void) { return FrameScratch::kBytes; }
 
 extern "C" int prs_frame_host(prs_pc_handle pc, void* pc_state, const void* gi, void* pc_work, const double* odom_host,
-                              void* vt_packed, int n_templates, unsigned threshold, int mode,
+                              void* vt_packed, int n_templates, double threshold, int mode,
                               const uint8_t* frame_host, int im_rows, int im_cols, int row_lo, int row_hi, int row_step,
                               int col_lo, int col_hi, int col_step, void* scratch, prs_frame_result* result_host,
                               void* stream) {
@@ -1731,7 +1733,7 @@ struct prs_frame_plan {
   double* odom_host;
   uint8_t* frame_host;
   prs_frame_result* result_host;
-  unsigned threshold;
+  double threshold;
   int mode, capacity;
   int im_rows, im_cols, row_lo, row_hi, row_step, col_lo, col_hi, col_step;
   cudaGraphExec_t exec[2];
@@ -1827,7 +1829,7 @@ static int frame_enqueue(prs_frame_plan* f, bool moved, cudaStream_t st) {
 }
 
 extern "C" int prs_frame_create(prs_pc_handle pc, void* pc_state, const void* gi, void* pc_work, void* vt_packed,
-                                int n_templates, int capacity, unsigned threshold, int mode, int im_rows, int im_cols,
+                                int n_templates, int capacity, double threshold, int mode, int im_rows, int im_cols,
                                 int row_lo, int row_hi, int row_step, int col_lo, int col_hi, int col_step,
                                 void* scratch, double* odom_host, uint8_t* frame_host, prs_frame_result* result_host,
                                 prs_frame_plan** out) {
@@ -2153,7 +2155,7 @@ struct prs_ens_plan {
   void *pc_state, *pc_work, *libs;
   const void* gi;
   int* n_dev;
-  const unsigned* thr_dev;
+  const double* thr_dev;
   const double* energy_dev;
   long long* loc_dev;
   int B, capacity;
@@ -2219,7 +2221,7 @@ static int ens_enqueue(prs_ens_plan* e, bool moved, cudaStream_t st) {
   ag.loc_stride = e->capacity;
   ag.g_max = d_gmax;
   ag.ctr = d_ctr;
-  k_vt_decide_append<<<(B + 3) / 4, 128, 0, st>>>(d_key, (const uint8_t*)(sc + L.tpl), (uint4*)e->libs, 0, 0u, d_argmax,
+  k_vt_decide_append<<<(B + 3) / 4, 128, 0, st>>>(d_key, (const uint8_t*)(sc + L.tpl), (uint4*)e->libs, 0, 0.0, d_argmax,
                                                   d_err, d_rec, e->n_dev, 1, nullptr, ag);
   PRS_CUDA(cudaGetLastError());
   if (e->energy_dev) {
@@ -2244,7 +2246,7 @@ extern "C" size_t prs_ens_scratch_bytes(int B, int im_rows, int im_cols) {
 }
 
 extern "C" int prs_ens_create(prs_pc_handle pc, void* pc_state, const void* gi, void* pc_work, void* libs, int capacity,
-                              int* n_dev, const unsigned* threshold_dev, const double* energy_dev, long long* loc_dev,
+                              int* n_dev, const double* threshold_dev, const double* energy_dev, long long* loc_dev,
                               int mode, int im_rows, int im_cols, int row_lo, int row_hi, int row_step, int col_lo,
                               int col_hi, int col_step, void* scratch, prs_ens_plan** out) {
   PRS_REQUIRE(pc && pc_state && gi && pc_work && libs && n_dev && threshold_dev && loc_dev && scratch && out,
@@ -2491,7 +2493,7 @@ static int ens_multi_enqueue(prs_ens_plan* e, int v, cudaStream_t st, bool event
   ag.ctr = d_ctr;
   ag.rec_of = e->rec_of;
   ag.present = d_present;
-  k_vt_decide_append<<<(B + 3) / 4, 128, 0, st>>>(d_key, (const uint8_t*)(ms + M.tpl), (uint4*)e->libs, 0, 0u, d_argmax,
+  k_vt_decide_append<<<(B + 3) / 4, 128, 0, st>>>(d_key, (const uint8_t*)(ms + M.tpl), (uint4*)e->libs, 0, 0.0, d_argmax,
                                                   d_err, d_rec, e->n_dev, 1, nullptr, ag);
   PRS_CUDA(cudaGetLastError());
   if (e->energy_dev) {

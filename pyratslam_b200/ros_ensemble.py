@@ -32,7 +32,8 @@ from . import experience_ensemble as xens
 from .experience_map import ExperienceMap
 from .kernels import PC_GLOBAL_INHIB
 from .posecell_network import PoseCellEnsemble, _as_np_dtype
-from .ros_simulate import IM_SIZE, MATCH_THRESHOLD, POSE_SIZE, X_RANGE, X_STEP, Y_RANGE, Y_STEP, RatslamRos
+from .ros_simulate import (IM_SIZE, MATCH_THRESHOLD, POSE_SIZE, X_RANGE, X_STEP, Y_RANGE, Y_STEP, RatslamRos,
+                           key_scores)
 
 MAX_CAPACITY = 1 << 16          # templates per agent the frame's library sweep takes (kSmallLibrary)
 
@@ -46,9 +47,10 @@ def agent_parameters(n_agents=None, match_threshold=MATCH_THRESHOLD, global_inhi
     """Broadcast the per-agent parameters to B agents and validate them (no CUDA involved).
 
     Each parameter is a scalar or a length-B sequence; B is ``n_agents`` or the length of the sequences.  Returns
-    ``(B, thresholds uint32[B], gi float64[B], energies list of float-or-None)``; the thresholds are clamped the way the
-    single-agent frame plans clamp them.  ``ValueError`` for disagreeing lengths, non-finite thresholds or inhibitions,
-    and energies that are negative or not finite."""
+    ``(B, thresholds float64[B], gi float64[B], energies list of float-or-None)``; a threshold is the caller's number, as
+    ``ViewTemplates`` compares it: a frame creates a template when its best score is strictly above it, so a negative
+    threshold creates on every frame.  ``ValueError`` for disagreeing lengths, non-finite thresholds or inhibitions, and
+    energies that are negative or not finite."""
     params = {"match_threshold": match_threshold, "global_inhibition": global_inhibition, "inject_energy": inject_energy}
     seqs = {}
     for k, v in params.items():
@@ -72,7 +74,7 @@ def agent_parameters(n_agents=None, match_threshold=MATCH_THRESHOLD, global_inhi
     for v in out["match_threshold"]:
         if not _real(v) or not math.isfinite(float(v)):
             raise ValueError("match_threshold must be finite numbers, got %r" % (v,))
-        thr.append(int(min(max(math.floor(v), 0), 0xFFFFFFFF)))    # as RatslamRos._fused_plan
+        thr.append(float(v))
     gi = []
     for v in out["global_inhibition"]:
         if not _real(v) or not math.isfinite(float(v)):
@@ -84,7 +86,7 @@ def agent_parameters(n_agents=None, match_threshold=MATCH_THRESHOLD, global_inhi
             raise ValueError("inject_energy must be None or a finite energy >= 0 (the injection runs on the device), "
                              "got %r" % (v,))
         energies.append(None if v is None else float(v))
-    return B, np.array(thr, dtype=np.uint32), np.array(gi, dtype=np.float64), energies
+    return B, np.array(thr, dtype=np.float64), np.array(gi, dtype=np.float64), energies
 
 
 def capacity_for(T):
@@ -303,8 +305,8 @@ class EnsembleSession:
 
     ``feed(frames, odom)`` takes uint8 [t,256,256] and [t,2] (R = 1) or lists of R such arrays of any lengths, 0
     allowed, and continues each recording where the previous feed left it.  It returns what ``replay_ensemble``'s
-    several-recordings form returns for the fed frames: ``template``, ``created``, ``argmax`` ``[B, t_max]``, ``length
-    [B]`` (the agent's recording's frames in this feed, -1 / False past it), ``n_templates [B]``, and with
+    several-recordings form returns for the fed frames: ``template``, ``created``, ``score``, ``argmax`` ``[B, t_max]``,
+    ``length [B]`` (the agent's recording's frames in this feed, -1 / False past it), ``n_templates [B]``, and with
     ``experience_map="device"`` ``n_exp``, ``exp_id``, ``em_xy`` and ``n_loop_closures``.  Template and experience ids
     are global to the session: concatenating agent b's first ``length[b]`` columns over the feeds gives what
     ``replay_ensemble`` returns on the concatenation of its recording's feeds.  The libraries grow when a feed could
@@ -353,7 +355,7 @@ class EnsembleSession:
         self._libs = torch.zeros((B, int(L.prs_vt_packed_bytes(cap))), dtype=torch.uint8, device=dev)
         self._loc = torch.full((B, cap), -1, dtype=torch.int64, device=dev)
         self._n_dev = torch.zeros(B, dtype=torch.int32, device=dev)
-        self._thr_dev = torch.from_numpy(thr[self._order].view(np.int32)).to(dev)
+        self._thr_dev = torch.from_numpy(thr[self._order]).to(dev)
         injecting = any(e is not None for e in energies)
         self._energy_dev = torch.tensor([-1.0 if energies[i] is None else energies[i] for i in self._order],
                                         dtype=torch.float64, device=dev) if injecting else None
@@ -484,8 +486,10 @@ class EnsembleSession:
         past = np.arange(T)[None, :] >= length[:, None]  # [B, T]
         argmax = _unravel(res["argmax"].T, self.pose_size)
         argmax[past] = -1
+        score = key_scores(res["key"].T)
+        score[past] = -1
         out = {"template": res["template_index"].T.astype(np.int64), "created": res["created"].T != 0,
-               "argmax": argmax, "n_templates": self.n_templates, "length": length}
+               "score": score, "argmax": argmax, "n_templates": self.n_templates, "length": length}
         if self._map:
             if self._linked:
                 out["n_exp"] = n_exp[:, inv].T.astype(np.int64)
@@ -544,9 +548,9 @@ class EnsembleSession:
         one match per image.  ``events`` is a message stream (``rosbag_io.read_events``, or a piece of ``iter_events``)
         for R = 1 and a list of R streams otherwise, any of them empty; a piece may end anywhere, inside a run of
         odometry too.  The streams are compacted into ticks (``event_ticks``) and replayed with
-        ``prs_ens_events_run``.  Returns per image: ``template``, ``created``, ``argmax`` ``[B, i_max]``, ``length [B]``
-        (the images of the agent's recording in this feed; -1 / False past it), ``n_templates [B]``, and with
-        ``experience_map="device"`` ``n_exp``, ``exp_id``, ``em_xy`` at each image (-1 / NaN past the length) and
+        ``prs_ens_events_run``.  Returns per image: ``template``, ``created``, ``score``, ``argmax`` ``[B, i_max]``,
+        ``length [B]`` (the images of the agent's recording in this feed; -1 / False past it), ``n_templates [B]``, and
+        with ``experience_map="device"`` ``n_exp``, ``exp_id``, ``em_xy`` at each image (-1 / NaN past the length) and
         ``n_loop_closures``.  ``feed`` and ``feed_events`` continue the same agents, libraries and maps."""
         if self._closed:
             raise RuntimeError("EnsembleSession: the session is closed")
@@ -611,7 +615,8 @@ class EnsembleSession:
         length = n_img[self._rec_of]
         i_max = int(n_img.max())
         out = {"template": np.full((B, i_max), -1, np.int64), "created": np.zeros((B, i_max), np.bool_),
-               "argmax": np.full((B, i_max, 3), -1, np.int64), "n_templates": self.n_templates, "length": length}
+               "score": np.full((B, i_max), -1, np.int64), "argmax": np.full((B, i_max, 3), -1, np.int64),
+               "n_templates": self.n_templates, "length": length}
         if self._map:
             out["n_exp"] = np.full((B, i_max), -1, np.int64)
             out["exp_id"] = np.full((B, i_max), -1, np.int64)
@@ -623,6 +628,7 @@ class EnsembleSession:
             m = len(ticks)
             out["template"][agents, :m] = res["template_index"][ticks][:, cols].T
             out["created"][agents, :m] = res["created"][ticks][:, cols].T != 0
+            out["score"][agents, :m] = key_scores(res["key"][ticks][:, cols].T)
             out["argmax"][agents, :m] = _unravel(res["argmax"][ticks][:, cols].T, self.pose_size)
             if self._linked:
                 out["n_exp"][agents, :m] = n_exp[ticks][:, cols].T
@@ -770,12 +776,13 @@ def replay_ensemble(frames, odom, n_agents=None, match_threshold=MATCH_THRESHOLD
 
     ``match_threshold``, ``global_inhibition`` and ``inject_energy`` (None = no injection, else a finite energy >= 0)
     are scalars or length-B sequences.  Every agent starts as ``RatslamRos`` does: energy 1 at the grid's midpoint,
-    an empty library.  Returns a dict with ``template [B,T]``, ``created [B,T]``, ``argmax [B,T,3]`` (the cell each
-    match was made with), ``n_templates [B]`` and ``agents`` (``EnsembleAgents``); with ``experience_map=True`` also
-    ``n_exp [B,T]`` and ``em_xy [B,T,2]``, replayed on the host from the records as ``RatslamRos.replay_native`` does
-    (O(B*T) Python, off by default).  A pose-cell error raises what ``replay(native=True)`` raises (``KeyError((5, 5))``
-    for the reference's LUT hole, ``ValueError`` for an oversize shift) for the first offending frame, which the shared
-    odometry makes the same frame for every agent.
+    an empty library.  Returns a dict with ``template [B,T]``, ``created [B,T]``, ``score [B,T]`` (int64: the best score
+    each match was made with, -1 where nothing was compared -- an empty library, past the agent's ``length``),
+    ``argmax [B,T,3]`` (the cell each match was made with), ``n_templates [B]`` and ``agents`` (``EnsembleAgents``); with
+    ``experience_map=True`` also ``n_exp [B,T]`` and ``em_xy [B,T,2]``, replayed on the host from the records as
+    ``RatslamRos.replay_native`` does (O(B*T) Python, off by default).  A pose-cell error raises what
+    ``replay(native=True)`` raises (``KeyError((5, 5))`` for the reference's LUT hole, ``ValueError`` for an oversize
+    shift) for the first offending frame, which the shared odometry makes the same frame for every agent.
 
     ``experience_map="device"`` builds the maps with ``experience_ensemble``: with ``experience_links=True`` every
     agent's linked map on the device, next to ``n_exp`` and ``em_xy`` also ``exp_id [B,T]`` (the current experience),
@@ -882,9 +889,9 @@ def replay_ensemble_events(events, n_agents=None, match_threshold=MATCH_THRESHOL
     own pose-cell update and experience-map update.  ``events`` is one stream, or a list of R streams with
     ``recording`` naming each agent's.  The parameters and their validation are ``replay_ensemble``'s;
     ``experience_map`` is False or "device" (the host maps, True, are refused).  Returns what
-    ``EnsembleSession.feed_events`` returns -- per image ``template``, ``created``, ``argmax`` ``[B, i_max]`` and
-    ``length [B]``, the maps' ``n_exp``, ``exp_id``, ``em_xy`` and ``n_loop_closures`` -- plus ``agents`` and, with
-    ``experience_map="device"``, ``maps``.  On a stream in which odometry and images alternate it equals
+    ``EnsembleSession.feed_events`` returns -- per image ``template``, ``created``, ``score``, ``argmax``
+    ``[B, i_max]`` and ``length [B]``, the maps' ``n_exp``, ``exp_id``, ``em_xy`` and ``n_loop_closures`` -- plus
+    ``agents`` and, with ``experience_map="device"``, ``maps``.  On a stream in which odometry and images alternate it equals
     ``replay_ensemble`` on ``rosbag_io.events_to_arrays(events)[:2]``.  This is one ``EnsembleSession`` fed once."""
     if not (isinstance(experience_map, (bool, np.bool_)) and not experience_map
             or (isinstance(experience_map, str) and experience_map == "device")):

@@ -36,6 +36,13 @@ MATCH_THRESHOLD = 45000
 ODOM_FREQ = 10
 
 
+def key_scores(key):
+    """int64 scores of packed ``(score << 32 | index)`` record keys, -1 where the key is ``UINT64_MAX`` (nothing was
+    compared: an empty library, or no frame)."""
+    k = np.asarray(key, dtype=np.uint64)
+    return np.where(k == np.uint64(0xFFFFFFFFFFFFFFFF), -1, (k >> np.uint64(32)).astype(np.int64))
+
+
 class RatslamRos(object):
     """The node's state and callbacks, fed from arrays instead of ROS topics."""
 
@@ -178,12 +185,11 @@ class RatslamRos(object):
             nat.lib().prs_frame_destroy(self._f_plan)
             self._f_plan = ctypes.c_void_p()
         torch.cuda.synchronize(e.device)
-        thr = int(min(max(math.floor(v.match_threshold), 0), 0xFFFFFFFF))
         nat.check(nat.lib().prs_frame_create(
             e._h, e._state.data_ptr(), e._gi.data_ptr(), self._f_pcwork.data_ptr(), v._lib.data_ptr(), v._n, v._capacity,
-            thr, v.mode, v.im_x, v.im_y, v.y_range[0], v.y_range[1], v.y_step, v.x_range[0], v.x_range[1], v.x_step,
-            self._f_scratch.data_ptr(), self._f_odom.data_ptr(), self._f_frame.data_ptr(), self._f_res.data_ptr(),
-            ctypes.byref(self._f_plan)), "prs_frame_create")
+            float(v.match_threshold), v.mode, v.im_x, v.im_y, v.y_range[0], v.y_range[1], v.y_step, v.x_range[0],
+            v.x_range[1], v.x_step, self._f_scratch.data_ptr(), self._f_odom.data_ptr(), self._f_frame.data_ptr(),
+            self._f_res.data_ptr(), ctypes.byref(self._f_plan)), "prs_frame_create")
         self._f_plan_key = key
         self._f_inj = self._NO_INJECT
         self._f_n_dev = v._n
@@ -281,16 +287,15 @@ class RatslamRos(object):
             return
         assert self._p_inflight == 0
         torch.cuda.synchronize(e.device)
-        thr = int(min(max(math.floor(v.match_threshold), 0), 0xFFFFFFFF))
         for sl in self._p_slots:
             if sl["plan"]:
                 nat.lib().prs_frame_destroy(sl["plan"])
                 sl["plan"] = ctypes.c_void_p()
             nat.check(nat.lib().prs_frame_create(
                 e._h, e._state.data_ptr(), e._gi.data_ptr(), self._f_pcwork.data_ptr(), v._lib.data_ptr(), v._n,
-                v._capacity, thr, v.mode, v.im_x, v.im_y, v.y_range[0], v.y_range[1], v.y_step, v.x_range[0],
-                v.x_range[1], v.x_step, self._f_scratch.data_ptr(), sl["odom"].data_ptr(), sl["frame"].data_ptr(),
-                sl["res"].data_ptr(), ctypes.byref(sl["plan"])), "prs_frame_create")
+                v._capacity, float(v.match_threshold), v.mode, v.im_x, v.im_y, v.y_range[0], v.y_range[1], v.y_step,
+                v.x_range[0], v.x_range[1], v.x_step, self._f_scratch.data_ptr(), sl["odom"].data_ptr(),
+                sl["frame"].data_ptr(), sl["res"].data_ptr(), ctypes.byref(sl["plan"])), "prs_frame_create")
             sl["inj"] = self._NO_INJECT
         self._p_key = key
         self._f_n_dev = v._n
@@ -448,11 +453,18 @@ def replay(frames, odom, fused=False, pipelined=False, native=False, **kwargs):
     reference-shaped calls; ``pipelined=True`` additionally overlaps the host's staging and bookkeeping of
     neighbouring frames with the device work (two alternating frame plans); ``native=True`` runs the whole loop in
     one library call (``prs_replay_run``, two frames in flight) and replays the host bookkeeping from its records.
-    The records are identical."""
+    The records are identical: ``template``, ``created``, ``argmax [T,3]`` (the cell each match was made with),
+    ``score [T]`` (the best score the frame's match was made with, -1 where the library was empty), ``n_exp`` and
+    ``em_xy``."""
     node = RatslamRos(**kwargs)
     T = len(frames)
-    rec = {"template": np.zeros(T, np.int64), "created": np.zeros(T, np.bool_),
+    rec = {"template": np.zeros(T, np.int64), "created": np.zeros(T, np.bool_), "score": np.full(T, -1, np.int64),
            "argmax": np.zeros((T, 3), np.int64), "n_exp": np.zeros(T, np.int64), "em_xy": np.zeros((T, 2))}
+
+    def note_score(t):
+        if node.vts.last_score is not None:
+            rec["score"][t] = node.vts.last_score
+
     if native:
         odom = np.asarray(odom, dtype=np.float64)
         res = node.replay_native(frames, odom)
@@ -461,6 +473,7 @@ def replay(frames, odom, fused=False, pipelined=False, native=False, **kwargs):
         rec["argmax"] = np.stack([flat // (Y * Th), (flat // Th) % Y, flat % Th], axis=1).astype(np.int64)
         rec["template"] = res["template_index"].astype(np.int64)
         rec["created"] = res["created"] != 0
+        rec["score"] = key_scores(res["key"])
         rec["n_exp"], rec["em_xy"] = node._native_n_exp, node._native_em_xy
         rec["n_templates"] = len(node.vts.templates)
         rec["node"] = node
@@ -476,6 +489,7 @@ def replay(frames, odom, fused=False, pipelined=False, native=False, **kwargs):
             rec["argmax"][t] = node.pcn.max_pc
             rec["template"][t] = idx
             rec["created"][t] = created
+            note_score(t)
             rec["n_exp"][t] = len(node.em.experiences)
             if node.em.current_exp is not None:
                 rec["em_xy"][t] = node.em.get_current_point()
@@ -506,6 +520,7 @@ def replay(frames, odom, fused=False, pipelined=False, native=False, **kwargs):
             idx, created = node.vis_callback(frames[t])
         rec["template"][t] = idx
         rec["created"][t] = created
+        note_score(t)
         rec["n_exp"][t] = len(node.em.experiences)
         if node.em.current_exp is not None:
             rec["em_xy"][t] = node.em.get_current_point()

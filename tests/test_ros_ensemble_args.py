@@ -8,18 +8,19 @@ import pytest
 from pyratslam_b200 import ros_ensemble
 
 
-def test_broadcasting():
+def test_broadcasting_keeps_thresholds():
     B, thr, gi, en = ros_ensemble.agent_parameters()
     assert B == 1 and thr.tolist() == [45000] and gi.tolist() == [0.2] and en == [None]
     B, thr, gi, en = ros_ensemble.agent_parameters(n_agents=3, match_threshold=30000.7, inject_energy=0.3)
-    assert B == 3 and thr.tolist() == [30000] * 3 and gi.tolist() == [0.2] * 3 and en == [0.3] * 3
-    B, thr, gi, en = ros_ensemble.agent_parameters(match_threshold=[0, -5, 2.0 ** 40, 45000],
-                                                   global_inhibition=np.linspace(0.05, 0.25, 4),
-                                                   inject_energy=[None, 0, 0.02, np.float32(0.5)])
-    assert B == 4
-    assert thr.dtype == np.uint32 and thr.tolist() == [0, 0, 2 ** 32 - 1, 45000]     # the frame plans' clamp
-    assert np.array_equal(gi, np.linspace(0.05, 0.25, 4))
-    assert en == [None, 0.0, 0.02, 0.5]
+    assert B == 3 and thr.tolist() == [30000.7] * 3 and gi.tolist() == [0.2] * 3 and en == [0.3] * 3
+    B, thr, gi, en = ros_ensemble.agent_parameters(match_threshold=[0, -5, 2.0 ** 40, 45000, -0.5, np.int64(7)],
+                                                   global_inhibition=np.linspace(0.05, 0.25, 6),
+                                                   inject_energy=[None, 0, 0.02, np.float32(0.5), None, None])
+    assert B == 6
+    # the caller's numbers, unclamped: a negative threshold creates on every frame, as ViewTemplates.match does
+    assert thr.dtype == np.float64 and thr.tolist() == [0, -5, 2.0 ** 40, 45000, -0.5, 7]
+    assert np.array_equal(gi, np.linspace(0.05, 0.25, 6))
+    assert en == [None, 0.0, 0.02, 0.5, None, None]
     assert ros_ensemble.agent_parameters(n_agents=2, global_inhibition=(0.1, 0.3))[0] == 2
 
 
@@ -40,6 +41,8 @@ def test_capacity():
     {"inject_energy": [0.1, math.nan]},
     {"inject_energy": "0.1"},
     {"match_threshold": math.nan},
+    {"match_threshold": [0, -math.inf]},
+    {"match_threshold": [0, math.inf]},
     {"global_inhibition": [0.1, math.inf]},
     {"global_inhibition": True},
 ])
