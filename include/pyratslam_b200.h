@@ -372,95 +372,67 @@ PRS_API int prs_replay_run(prs_frame_plan* const* plans, int n_plans, const uint
 
 /* ------------------------------------------------------------ ensemble replay */
 
-/* One recording through B independent agents in one pass (a parameter sweep of the ROS loop, ros_simulate.py:98-166):
- * agent b is network b of the pose-cell plan `pc` (B = its network count, global inhibition gi[b]) with its own packed
- * uint8 library, match threshold and injection energy.  Frames and odometry are shared: a frame is ONE graph for the
- * whole ensemble -- the odometry broadcast and the pose-cell update of all B networks (moved frames only) on a side
- * branch, the query prepared once, one sweep over every agent's library, then per agent the create-or-match decision
- * (a created template goes into slot n_dev[b] of its library, its location row loc_dev[b][n] receives the agent's
- * arg-max) and the injection of prs_frame_set_inject.  Agent b's records equal a single-agent frame plan's with
- * threshold_dev[b], gi[b] and energy_dev[b].  Reference mode (PRS_VT_MODE_REF) only; PRS_E_INVALID otherwise.
+/* B independent agents in one pass (a parameter sweep of the ROS loop, ros_simulate.py:98-166): agent b is network b
+ * of the pose-cell plan `pc` (B = its network count, global inhibition gi[b]) with its own packed uint8 library, match
+ * threshold and injection energy, and it replays recording rec_of_dev[b] of R.  A recording is a stream of ticks, each
+ * an optional gated twist and an optional image; a frame replay is the stream in which every tick has an image.  A
+ * tick is ONE graph for the whole ensemble: the pose-cell update of all B networks on a side branch, one query per
+ * recording, one sweep in which agent b compares against its recording's query, then per agent the create-or-match
+ * decision (a created template goes into slot n_dev[b] of its library, its location row loc_dev[b][n] receives the
+ * agent's arg-max) and the injection of prs_frame_set_inject.  Agent b's records equal a single-agent frame plan's on
+ * its recording with threshold_dev[b], gi[b] and energy_dev[b].  Reference mode (PRS_VT_MODE_REF) only; PRS_E_INVALID
+ * otherwise.
  *   pc_work       : device, B * 24 bytes: int64 arg-max [B], total [B] (8-byte slots), int32 err [B]; the arg-max must
- *                   hold each network's current arg-max (prs_pc_argmax) before the first frame
+ *                   hold each network's current arg-max (prs_pc_argmax) before the first tick
  *   libs          : device, B libraries of prs_vt_packed_bytes(capacity) bytes each, zero-filled once
  *   capacity      : templates per library, at most 65536
- *   n_dev         : device int32 [B], templates in each library; updated by every frame
+ *   n_dev         : device int32 [B], templates in each library; updated by every tick with an image
  *   threshold_dev : device double [B], the match thresholds as the caller gives them (create when score > threshold,
  *                   so a negative threshold creates on every frame)
  *   energy_dev    : device double [B], energy injected at the frame template's cell; a value that is not >= 0 (e.g. -1)
  *                   means no injection for that agent; NULL: no injection node at all
  *   loc_dev       : device int64 [B][capacity], C-order flat cell of every template, -1 = invalid
- *   scratch       : device, prs_ens_scratch_bytes(B, im_rows, im_cols); private to the plan
+ *   rec_of_dev    : device int32 [B] in [0, R); the agents of one recording are best given contiguous indices (a sweep
+ *                   block reloads its query when the recording changes)
+ *   scratch       : device, prs_ens_scratch_bytes(pc, R, im_rows, im_cols); private to the plan.  It holds a chunk of
+ *                   images of every recording ([R][chunk][im_rows][im_cols], chunk = 256 MiB / (R * frame bytes),
+ *                   clamped to [1, 256]), the per-recording queries and, for R > 1, one snapshot of a network's state
+ *                   per agent
  * The plan keeps pointers to all of these; they must outlive it. */
 typedef struct prs_ens_plan prs_ens_plan;
-PRS_API size_t prs_ens_scratch_bytes(int B, int im_rows, int im_cols);
+PRS_API size_t prs_ens_scratch_bytes(prs_pc_handle pc, int R, int im_rows, int im_cols);
 PRS_API int prs_ens_create(prs_pc_handle pc, void* pc_state, const void* gi, void* pc_work, void* libs, int capacity,
-                   int* n_dev, const double* threshold_dev, const double* energy_dev, long long* loc_dev, int mode,
-                   int im_rows, int im_cols, int row_lo, int row_hi, int row_step, int col_lo, int col_hi,
-                   int col_step, void* scratch, prs_ens_plan** out);
+                   int* n_dev, const double* threshold_dev, const double* energy_dev, long long* loc_dev, int R,
+                   const int* rec_of_dev, int mode, int im_rows, int im_cols, int row_lo, int row_hi, int row_step,
+                   int col_lo, int col_hi, int col_step, void* scratch, prs_ens_plan** out);
 PRS_API int prs_ens_destroy(prs_ens_plan* plan);
-/* The room for T more frames that the runs below check is counted in frames (one template per agent and frame at most)
- * and decremented by every run.  prs_ens_refresh_room recounts it from n_dev as the libraries are now, so a plan fed in
+/* The room that prs_ens_run checks is counted in ticks with an image (one template per agent and image at most) and
+ * decremented by every run.  prs_ens_refresh_room recounts it from n_dev as the libraries are now, so a plan fed in
  * pieces whose agents match more than they create keeps going without a new plan.  Synchronises `stream`. */
 PRS_API int prs_ens_refresh_room(prs_ens_plan* plan, void* stream);
-/* The loop of prs_replay_run for the ensemble.  Frames and odometry go to the device and the records come back in
- * chunks of 256 frames; nothing per agent crosses the bus per frame.  Returns after one final synchronisation of
- * `stream` (a non-default stream).  PRS_E_INVALID when the libraries have no room for T more templates.
- *   frames : host uint8 [T][im_rows][im_cols]     odom : host double [T][2] = (vtrans, vrot) as given to update()
- *   moved  : host uint8 [T], 0 = no pose-cell update for this frame (the 0.001 twist gate, ros_simulate.py:128)
- *   results: host prs_frame_result [T][B]; pc_err holds the err bits of the last update (valid on moved frames) and
- *            PRS_ERR_INJECT_LOC */
-PRS_API int prs_ens_replay_run(prs_ens_plan* plan, const uint8_t* frames, const double* odom, const uint8_t* moved, int T,
-                       prs_frame_result* results, void* stream);
-
-/* Several recordings through one ensemble: agent b replays recording rec_of[b] of R, each with its own frames, odometry
- * and length.  A frame is still ONE graph: one query per recording (a block each), one sweep in which agent b compares
- * against its recording's query, the per-agent decision and injection.  The pose-cell update of all B networks runs
- * when any recording moved; a network whose recording did not move, or has ended, gets the twist (0, 0), and on such a
- * "mixed" frame its state slice and its pc_work slots are saved before the update and restored after it (the
- * active-set lists are invalidated), so it ends the frame exactly as a skipped update leaves it.  Three graphs per plan:
- * no recording moved, every recording has a frame and moved (no snapshot), mixed.  Past the end of its recording an
- * agent appends and injects nothing; its record has template_index -1, created 0, key ~0 and n_templates unchanged.
- * Agent b's records equal a single-recording plan's on recording rec_of[b]; the agents of one recording are best given
- * contiguous indices (a sweep block reloads its query when the recording changes).
- *   prs_ens_multi_scratch_bytes(plan, R): device bytes of multi_scratch, private to the plan.  It holds a chunk of
- *            frames of every recording ([R][chunk][im_rows][im_cols], chunk = 256 MiB / (R * frame bytes), clamped to
- *            [1, 256]), the per-recording queries and one snapshot of a network's state per agent.
- *   prs_ens_set_recordings: rec_of_dev: device int32 [B] in [0, R); it and multi_scratch must outlive the plan's use.
- *   prs_ens_multi_replay_run:
- *     frames : host, R pointers; frames[r] is uint8 [lengths[r]][im_rows][im_cols] (may be NULL when lengths[r] = 0)
- *     odom   : host double [T_max][R][2] = (vtrans, vrot) of recording r at frame t as given to update()
- *     moved  : host uint8 [T_max][R], 0 = recording r makes no pose-cell update at frame t (entries past lengths[r] are
- *              ignored)
- *     lengths: host int32 [R], each in [0, T_max]; results: host prs_frame_result [T_max][B]
- *   Frames go to the device one chunk at a time, one copy per recording.  PRS_E_INVALID when the libraries have no room
- *   for T_max more templates. */
-PRS_API size_t prs_ens_multi_scratch_bytes(const prs_ens_plan* plan, int R);
-PRS_API int prs_ens_set_recordings(prs_ens_plan* plan, int R, const int* rec_of_dev, void* multi_scratch);
-PRS_API int prs_ens_multi_replay_run(prs_ens_plan* plan, const uint8_t* const* frames, const double* odom,
-                             const uint8_t* moved, const int* lengths, int T_max, prs_frame_result* results,
-                             void* stream);
-
-/* Several recordings as message streams: every gated odometry message is its own pose-cell update, as in the node's
- * message loop (ros_simulate.replay_events), instead of one twist per frame.  The caller compacts each recording into
- * ticks of (optional gated twist, optional image), odometry before image: an odometry message directly followed by an
- * image shares its tick, gated-out odometry makes no tick, an image with no twist before it is an image-only tick,
- * other odometry an odometry-only tick.  Tick t is the frame of prs_ens_multi_replay_run for the recordings with an
- * image at t; an agent whose recording has no image at t (an odometry-only tick, or past the recording's end) gets
- * the "no frame" record: template_index -1, created 0, key ~0, n_templates unchanged, and the arg-max and pc_err its
- * update left.  A tick at which no recording has an image runs only the update (lean: no query, sweep, decision or
- * injection).  Needs prs_ens_set_recordings first; R = 1 is allowed.
+/* T ticks of every recording.  The caller compacts a message stream into ticks, odometry before image: an odometry
+ * message directly followed by an image shares its tick, gated-out odometry makes no tick, an image with no twist
+ * before it is an image-only tick, other odometry an odometry-only tick.  The pose-cell update of all B networks runs
+ * when any recording moved at the tick; a network whose recording did not move, or has ended, gets the twist (0, 0),
+ * and on such a "mixed" tick its state slice and its pc_work slots are saved before the update and restored after it
+ * (the active-set lists are invalidated), so it ends the tick exactly as a skipped update leaves it.  An agent whose
+ * recording has no image at the tick (an odometry-only tick, or past the recording's end) appends and injects nothing
+ * and gets the "no frame" record: template_index -1, created 0, key ~0, n_templates unchanged, and the arg-max and
+ * pc_err its update left.  A tick at which no recording has an image runs only the update (no query, sweep, decision
+ * or injection).  Six graphs per plan: {no recording moved, every recording moved, mixed} x {image, none}.
  *   frames  : host, R pointers; frames[r] is uint8 [n_images[r]][im_rows][im_cols], recording r's images only, in
  *             order (may be NULL when n_images[r] = 0)
  *   odom    : host double [T][R][2] = (vtrans, vrot) of recording r's twist at tick t as given to update()
- *   gate    : host uint8 [T][R]: bit 0 = recording r has an image at tick t, bit 1 = it moved (a gated twist); 0 past
- *             the end of recording r's ticks
+ *   gate    : host uint8 [T][R]: bit 0 = recording r has an image at tick t, bit 1 = it moved (the 0.001 twist gate,
+ *             ros_simulate.py:128); 0 past the end of recording r's ticks
  *   n_images: host int32 [R], must equal the number of bit-0 ticks of each recording
- *   results : host prs_frame_result [T][B], one record per tick and agent
- *   Frames go to the device one chunk of ticks at a time, one copy per recording.  The room check and its decrement
- *   count ticks with an image (only they can append): PRS_E_INVALID when the libraries have no room for them. */
-PRS_API int prs_ens_events_run(prs_ens_plan* plan, const uint8_t* const* frames, const double* odom, const uint8_t* gate,
-                       const int* n_images, int T, prs_frame_result* results, void* stream);
+ *   results : host prs_frame_result [T][B], one record per tick and agent; pc_err holds the err bits of the last
+ *             update (valid where the agent's recording moved) and PRS_ERR_INJECT_LOC
+ * Images, odometry and gates go to the device and the records come back one chunk of ticks at a time, one image copy
+ * per recording; nothing per agent crosses the bus per tick.  Returns after one final synchronisation of `stream` (a
+ * non-default stream).  PRS_E_INVALID when the libraries have no room for the ticks with an image. */
+PRS_API int prs_ens_run(prs_ens_plan* plan, const uint8_t* const* frames, const double* odom, const uint8_t* gate,
+                const int* n_images, int T, prs_frame_result* results, void* stream);
 
 /* ------------------------------------------------------- ensemble experience maps */
 

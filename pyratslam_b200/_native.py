@@ -94,19 +94,13 @@ _SIGNATURES["prs_frame_run"] = (c_int, [c_void_p, c_int, c_void_p])
 _SIGNATURES["prs_frame_launch"] = (c_int, [c_void_p, c_int, c_void_p])
 _SIGNATURES["prs_frame_set_inject"] = (c_int, [c_void_p, c_double, c_void_p])
 _SIGNATURES["prs_replay_run"] = (c_int, [POINTER(c_void_p), c_int, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p])
-_SIGNATURES["prs_ens_scratch_bytes"] = (c_size_t, [c_int, c_int, c_int])
+_SIGNATURES["prs_ens_scratch_bytes"] = (c_size_t, [c_void_p, c_int, c_int, c_int])
 _SIGNATURES["prs_ens_create"] = (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p,
-                                         c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
-                                         c_void_p, POINTER(c_void_p)])
+                                         c_void_p, c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int,
+                                         c_int, c_int, c_int, c_void_p, POINTER(c_void_p)])
 _SIGNATURES["prs_ens_destroy"] = (c_int, [c_void_p])
 _SIGNATURES["prs_ens_refresh_room"] = (c_int, [c_void_p, c_void_p])
-_SIGNATURES["prs_ens_replay_run"] = (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p])
-_SIGNATURES["prs_ens_multi_scratch_bytes"] = (c_size_t, [c_void_p, c_int])
-_SIGNATURES["prs_ens_set_recordings"] = (c_int, [c_void_p, c_int, c_void_p, c_void_p])
-_SIGNATURES["prs_ens_multi_replay_run"] = (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p,
-                                                   c_void_p])
-_SIGNATURES["prs_ens_events_run"] = (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p,
-                                             c_void_p])
+_SIGNATURES["prs_ens_run"] = (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p])
 _SIGNATURES["prs_em_work_bytes"] = (c_size_t, [c_int, c_int, c_int])
 _SIGNATURES["prs_em_linked_run"] = (c_int, [c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int,
                                             c_int, c_double, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p])

@@ -1258,9 +1258,9 @@ struct VtAgents {
   long long loc_stride = 0;
   int* g_max = nullptr;                 // largest group count over the agents, raised by the decision (the sweep's grid)
   const int* ctr = nullptr;             // frame index within the record chunk: the agent's record is res[*ctr * B + b]
-  // multi-recording frames (prs_ens_set_recordings): agent b replays recording rec_of[b], whose template is
-  // tpl + rec_of[b] * 1024; present[r] = 0 past recording r's end, where its agents append and inject nothing
-  const int* rec_of = nullptr;          // [B]; null: one recording, one template
+  // ensemble ticks: agent b replays recording rec_of[b], whose template is tpl + rec_of[b] * 1024; present[r] = 0 where
+  // recording r has no image at this tick, and there its agents append and inject nothing
+  const int* rec_of = nullptr;          // [B]; null: one template
   const uint8_t* present = nullptr;     // [R]
 };
 
@@ -1508,48 +1508,7 @@ extern "C" int prs_vt_sweep_any_f32(const float* lib, long long n, const float* 
 // and the pose-cell kernel reads its two doubles of odometry from the pinned buffer as well.
 constexpr int kSmallLibrary = 1 << 16;
 
-__global__ void __launch_bounds__(1024)
-    k_vt_frame_prepare(const uint8_t* __restrict__ frame, int im_cols, int row_lo, int row_step, int col_lo, int col_step,
-                       uint8_t* __restrict__ tpl, uint32_t* __restrict__ planes, unsigned long long* __restrict__ key,
-                       const int* __restrict__ ctr = nullptr, long long frame_bytes = 0, int n_keys = 1) {
-  // ctr (ensemble frames): the frame is number *ctr of a device-side chunk of frames `frame_bytes` apart; the n_keys
-  // agents' keys are reset
-  __shared__ uint32_t s_sum[32];
-  const int t = threadIdx.x >> 5, c = threadIdx.x & 31;  // template row, column
-  if (ctr != nullptr) frame += *ctr * frame_bytes;
-  for (int i = (int)threadIdx.x; i < n_keys; i += 1024) key[i] = ~0ull;
-  const int rr = row_lo + (t / (row_step - 1)) * row_step + (t % (row_step - 1)) + 1;
-  const int cc = col_lo + (c / (col_step - 1)) * col_step + (c % (col_step - 1)) + 1;
-  const uint32_t px = frame[(size_t)rr * im_cols + cc];
-  tpl[t * 32 + c] = (uint8_t)px;
-  uint32_t mine = 0;
-#pragma unroll
-  for (int k = 0; k < 8; ++k) {
-    const uint32_t b = __ballot_sync(0xffffffffu, (px >> k) & 1u);
-    if (c == k) mine = b;
-  }
-  if (c < 8) planes[t * 8 + c] = mine;
-  uint32_t sum = px;
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, o);
-  if (c == 0) s_sum[t] = sum;
-  __syncthreads();
-  if (t == 0) {
-    uint32_t all = s_sum[c], mid = (c >= 8 && c < 24) ? all : 0;
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-      all += __shfl_xor_sync(0xffffffffu, all, o);
-      mid += __shfl_xor_sync(0xffffffffu, mid, o);
-    }
-    if (c == 0) {
-      planes[256] = mid;
-      planes[257] = all;
-    }
-  }
-}
-
-// k_vt_frame_prepare's query (the template of `frame`, its bit planes and row sums) for one recording; kept as a
-// copy so that k_vt_frame_prepare itself compiles to the code it always had
+// The query of `frame`: the template, its bit planes and row sums.  A block of 1024 threads, one per template pixel.
 __device__ __forceinline__ void vt_prepare_query(const uint8_t* __restrict__ frame, int im_cols, int row_lo, int row_step,
                                                  int col_lo, int col_step, uint8_t* __restrict__ tpl,
                                                  uint32_t* __restrict__ planes, uint32_t* s_sum) {
@@ -1584,32 +1543,30 @@ __device__ __forceinline__ void vt_prepare_query(const uint8_t* __restrict__ fra
   }
 }
 
-// Multi-recording frames: block r prepares recording r's query from frame *ctr of its chunk, frames[r][chunk] (bytes
-// (r * chunk + *ctr) * frame_bytes), into tpl + r * 1024 and planes + r * kQueryStride, and sets present[r] from bit 0
-// of gate[*ctr][r] (0 past the recording's end: no query).  The blocks reset the n_keys agents' keys.
-// kSlots (message-stream ticks, prs_ens_events_run): a recording's images sit contiguously in its chunk but not at the
-// tick index, so the image is slot slots[*ctr][r] of the chunk, and -1 (no image at this tick) clears present[r].
-// The <false> instantiation is the kernel as it was.
+__global__ void __launch_bounds__(1024)
+    k_vt_frame_prepare(const uint8_t* __restrict__ frame, int im_cols, int row_lo, int row_step, int col_lo, int col_step,
+                       uint8_t* __restrict__ tpl, uint32_t* __restrict__ planes, unsigned long long* __restrict__ key) {
+  __shared__ uint32_t s_sum[32];
+  if (threadIdx.x == 0) *key = ~0ull;
+  vt_prepare_query(frame, im_cols, row_lo, row_step, col_lo, col_step, tpl, planes, s_sum);
+}
+
+// Ensemble ticks: block r prepares recording r's query into tpl + r * 1024 and planes + r * kQueryStride.  A recording's
+// images sit contiguously in its chunk, frames[r][chunk] (bytes (r * chunk + s) * frame_bytes), but not at the tick
+// index: its image at tick *ctr is slot s = slots[*ctr][r] of the chunk, and s = -1 (no image at this tick, or past
+// the recording's end) clears present[r].  The blocks reset the n_keys agents' keys.
 constexpr int kQueryStride = 512;  // uint32 words between two recordings' query planes (258 used)
 
-template <bool kSlots>
 __global__ void __launch_bounds__(1024)
     k_vt_frame_prepare_multi(const uint8_t* __restrict__ frames, int chunk, long long frame_bytes, int im_cols, int row_lo,
                              int row_step, int col_lo, int col_step, uint8_t* __restrict__ tpl,
                              uint32_t* __restrict__ planes, unsigned long long* __restrict__ key, int n_keys,
-                             const int* __restrict__ ctr, const uint8_t* __restrict__ gate, uint8_t* __restrict__ present,
-                             const int* __restrict__ slots = nullptr) {
+                             const int* __restrict__ ctr, uint8_t* __restrict__ present, const int* __restrict__ slots) {
   __shared__ uint32_t s_sum[32];
   const int r = blockIdx.x, R = gridDim.x, f = *ctr;
   for (int i = r * 1024 + (int)threadIdx.x; i < n_keys; i += R * 1024) key[i] = ~0ull;
-  int s = f;
-  bool here;
-  if constexpr (kSlots) {
-    s = slots[(size_t)f * R + r];
-    here = s >= 0;
-  } else {
-    here = (gate[(size_t)f * R + r] & 1) != 0;
-  }
+  const int s = slots[(size_t)f * R + r];
+  const bool here = s >= 0;
   if (threadIdx.x == 0) present[r] = here ? 1 : 0;
   if (!here) return;  // block-uniform
   vt_prepare_query(frames + ((size_t)r * chunk + s) * frame_bytes, im_cols, row_lo, row_step, col_lo, col_step,
@@ -1634,13 +1591,13 @@ __device__ __forceinline__ uint32_t lt_row_q(const uint4& lo, const uint4& hi, c
 // and the per-offset counts meet in shared memory (integer adds: exact, order-free).
 constexpr int kSmallThreads = 512;
 
-// Ensemble frames: n_agents libraries of lib_u4 uint4 each, agent b's live count n_dev[b] and key key_out[b].  The
-// blocks grid-stride over (agent, group) items, G = *g_max groups per agent (the largest live group count, kept by the
-// decision kernel); an item past its agent's live count is skipped, so the work follows sum_b n_b, not the capacity.
-// kMulti (multi-recording frames): agent b is compared with the query of its recording
-// rec_of[b], qplanes + rec_of[b] * kQueryStride, and skipped where present[rec_of[b]] = 0.  A block reloads q only
-// when its item's recording differs from the last one it loaded (the agents of a recording have contiguous indices).
-// k_vt_sweep_packed_ref_small is the <false> instantiation, whose code is that of the untemplated kernel it was.
+// <false>: the single-agent frame's sweep of one library against one query.
+// <true> (ensemble ticks): n_agents libraries of lib_u4 uint4 each, agent b's live count n_dev[b] and key key_out[b].
+// The blocks grid-stride over (agent, group) items, G = *g_max groups per agent (the largest live group count, kept by
+// the decision kernel); an item past its agent's live count is skipped, so the work follows sum_b n_b, not the
+// capacity.  Agent b is compared with the query of its recording rec_of[b], qplanes + rec_of[b] * kQueryStride, and
+// skipped where present[rec_of[b]] = 0.  A block reloads q only when its item's recording differs from the last one it
+// loaded (the agents of a recording have contiguous indices).
 template <bool kMulti>
 __global__ void __launch_bounds__(kSmallThreads)
     k_vt_sweep_packed_ref_small(const uint4* __restrict__ packed, const uint32_t* __restrict__ qplanes,
@@ -2001,51 +1958,46 @@ extern "C" int prs_replay_run(prs_frame_plan* const* plans, int n_plans, const u
 }
 
 // ---------------------------------------------------------------------------------------------
-// Ensemble replay: one recording through B agents, each with its own pose-cell network (the B networks of one plan),
-// view-template library, threshold and injection energy.  The frames and the odometry are shared, so a frame is ONE
-// graph for the whole ensemble:
-//   side branch (moved frames)  k_ens_odom broadcasts the frame's (vtrans, vrot) into odom[B][2] -> prs_pc_step
-//   template branch             k_vt_frame_prepare (once: the query is the same for every agent) ->
-//                               k_vt_sweep_packed_ref_small over every agent's library (grid-stride over (agent, group))
-//   join                        k_vt_decide_append, one warp per agent -> [k_frame_inject, one thread per agent] ->
-//                               k_ens_advance (the device-side frame counter)
-// Frames and odometry go to the device a chunk at a time, the records [chunk][B] come back a chunk at a time.
+// Ensemble replay: B agents, each with its own pose-cell network (the B networks of one plan), view-template library,
+// threshold and injection energy; agent b replays recording rec_of[b] of R.  A recording is a stream of ticks, each an
+// optional gated twist and an optional image (a frame replay is the stream in which every tick has an image), and a
+// tick is ONE graph for the whole ensemble:
+//   side branch  k_ens_odom_multi (each network its recording's twist, (0, 0) where that recording did not move or has
+//                ended) -> [mixed: k_ens_snapshot save] -> prs_pc_step -> [mixed: k_ens_snapshot restore ->
+//                prs_pc_active_invalidate]
+//   template     k_vt_frame_prepare_multi (one block per recording) -> k_vt_sweep_packed_ref_small<true> over every
+//                agent's library (grid-stride over (agent, group))
+//   join         k_vt_decide_append, one warp per agent -> [k_frame_inject, one thread per agent] -> k_ens_advance (the
+//                device-side tick counter)
+// The restore runs before the join, so the decision and the injection of a still network see its state, arg-max and
+// error bits as they were: what a skipped update leaves.  A tick where no recording moved runs no update; one where
+// every recording moved needs no snapshot, so with R = 1 no tick is mixed.  A tick without an image in any recording
+// is lean: the side branch's nodes run on the tick's stream itself, then k_ens_no_image writes the records and advances
+// the counter -- no query, sweep, decision or injection.  Six graphs: {no update, all moved, mixed} x {image, none}.
+// Images, odometry, gates and image slots go to the device a chunk of ticks at a time, the records [chunk][B] come
+// back a chunk at a time.
 constexpr int kEnsChunk = 256;
 
-struct EnsScratch {  // device scratch layout of an ensemble plan (bytes), every part 256-byte aligned
-  size_t frames, odom_chunk, rec, odom, key, tpl, planes, misc, bytes;
-  EnsScratch(int B, long long fbytes) {
-    auto up = [](size_t v) { return (v + 255) & ~(size_t)255; };
-    frames = 0;
-    odom_chunk = frames + up((size_t)kEnsChunk * fbytes);
-    rec = odom_chunk + up((size_t)kEnsChunk * 2 * sizeof(double));
-    odom = rec + up((size_t)kEnsChunk * B * sizeof(prs_frame_result));
-    key = odom + up((size_t)B * 2 * sizeof(double));
-    tpl = key + up((size_t)B * sizeof(unsigned long long));
-    planes = tpl + 1024;
-    misc = planes + 2048;  // int frame counter, int group maximum, int largest live count
-    bytes = misc + 256;
-  }
-};
+// Device scratch of an ensemble plan (prs_ens_scratch_bytes), every part 256-byte aligned.  A chunk holds `chunk` ticks
+// of each of the R recordings, as many as fit kEnsFrameBytes of images (at least one, at most kEnsChunk).  The
+// per-agent snapshot of a mixed tick is empty when R = 1.
+constexpr size_t kEnsFrameBytes = 256u << 20;
 
-// Device scratch of the multi-recording frames (prs_ens_multi_scratch_bytes), every part 256-byte aligned.  The frame
-// counter and the group maximum stay in the plan's own scratch.  A chunk holds `chunk` frames of each of the R
-// recordings, as many as fit kEnsMultiFrameBytes (at least one, at most kEnsChunk).
-constexpr size_t kEnsMultiFrameBytes = 256u << 20;
-
-struct EnsMultiScratch {
+struct EnsScratch {
   int chunk = 0;
-  size_t frames = 0, odom_chunk = 0, gate = 0, rec = 0, odom = 0, key = 0, tpl = 0, planes = 0, present = 0, still = 0,
-         wsnap = 0, snap = 0, slots = 0, bytes = 0;
-  EnsMultiScratch() = default;
-  EnsMultiScratch(int B, int R, long long fbytes, size_t net_bytes) {
+  size_t frames = 0, odom_chunk = 0, gate = 0, slots = 0, rec = 0, odom = 0, key = 0, tpl = 0, planes = 0, present = 0,
+         still = 0, wsnap = 0, snap = 0, misc = 0, bytes = 0;
+  EnsScratch() = default;
+  EnsScratch(int B, int R, long long fbytes, size_t net_bytes) {
     auto up = [](size_t v) { return (v + 255) & ~(size_t)255; };
-    const long long fit = (long long)(kEnsMultiFrameBytes / ((size_t)R * fbytes));
+    const long long fit = (long long)(kEnsFrameBytes / ((size_t)R * fbytes));
     chunk = (int)(fit < 1 ? 1 : fit > kEnsChunk ? kEnsChunk : fit);
+    const size_t snaps = R > 1 ? (size_t)B : 0;
     frames = 0;
     odom_chunk = frames + up((size_t)R * chunk * fbytes);
     gate = odom_chunk + up((size_t)chunk * R * 2 * sizeof(double));
-    rec = gate + up((size_t)chunk * R);
+    slots = gate + up((size_t)chunk * R);
+    rec = slots + up((size_t)chunk * R * sizeof(int));
     odom = rec + up((size_t)chunk * B * sizeof(prs_frame_result));
     key = odom + up((size_t)B * 2 * sizeof(double));
     tpl = key + up((size_t)B * sizeof(unsigned long long));
@@ -2053,15 +2005,14 @@ struct EnsMultiScratch {
     present = planes + up((size_t)R * kQueryStride * sizeof(uint32_t));
     still = present + up((size_t)R);
     wsnap = still + up((size_t)B);
-    snap = wsnap + up((size_t)B * 3 * sizeof(long long));
-    slots = snap + up((size_t)B * net_bytes);  // int32 [chunk][R], message-stream ticks only
-    bytes = slots + up((size_t)chunk * R * sizeof(int));
+    snap = wsnap + up(snaps * 3 * sizeof(long long));
+    misc = snap + up(snaps * net_bytes);  // int tick counter, int group maximum, int largest live count
+    bytes = misc + 256;
   }
 };
 
-// Multi-recording frames: network b gets its recording's (vtrans, vrot) where that recording moved at this frame
-// (bit 1 of gate[*ctr][r]), else (0, 0), which no pose-cell kernel rejects; still[b] = 1 marks the network whose
-// update the mixed frame undoes.
+// Network b gets its recording's (vtrans, vrot) where that recording moved at this tick (bit 1 of gate[*ctr][r]), else
+// (0, 0), which no pose-cell kernel rejects; still[b] = 1 marks the network whose update the mixed tick undoes.
 __global__ void k_ens_odom_multi(const double* __restrict__ odom_chunk, const uint8_t* __restrict__ gate,
                                  const int* __restrict__ ctr, const int* __restrict__ rec_of, int R,
                                  double* __restrict__ odom, uint8_t* __restrict__ still, int B) {
@@ -2074,7 +2025,7 @@ __global__ void k_ens_odom_multi(const double* __restrict__ odom_chunk, const ui
   still[b] = mv ? 0 : 1;
 }
 
-// The mixed frame's save (kRestore = false, before prs_pc_step) and restore (after it) of every still network: its
+// The mixed tick's save (kRestore = false, before prs_pc_step) and restore (after it) of every still network: its
 // state slice of `words` W-words, and its pc_work slots (arg-max, total of total_bytes, err), to and from one snapshot per agent.
 // Blocks of other networks return at once.
 template <bool kRestore, typename W>
@@ -2110,21 +2061,11 @@ __global__ void k_ens_snapshot(W* __restrict__ state, W* __restrict__ snap, long
   }
 }
 
-__global__ void k_ens_odom(const double* __restrict__ odom_chunk, const int* __restrict__ ctr, double* __restrict__ odom,
-                           int B) {
-  const int b = blockIdx.x * blockDim.x + threadIdx.x;
-  if (b >= B) return;
-  const int t = *ctr;
-  odom[2 * b] = odom_chunk[2 * t];
-  odom[2 * b + 1] = odom_chunk[2 * t + 1];
-}
-
 __global__ void k_ens_advance(int* ctr) { ++*ctr; }
 
-// The odometry-only tick of a message-stream replay (prs_ens_events_run) in place of the decision: every agent's
-// "no image" record -- the arg-max, error bits and template count as the tick's update left them, template -1, as
-// k_vt_decide_append writes for an agent whose recording has no frame -- then the tick counter advances.  One block,
-// one thread per agent (strided past 1024).
+// A tick without an image in any recording, in place of the decision: every agent's "no image" record -- the arg-max,
+// error bits and template count as the tick's update left them, template -1, as k_vt_decide_append writes for an agent
+// whose recording has no image -- then the tick counter advances.  One block, one thread per agent (strided past 1024).
 __global__ void __launch_bounds__(1024)
     k_ens_no_image(const long long* __restrict__ argmax, const int* __restrict__ pc_err, const int* __restrict__ n_dev,
                    prs_frame_result* __restrict__ rec, int* __restrict__ ctr, int B) {
@@ -2158,61 +2099,106 @@ struct prs_ens_plan {
   const double* thr_dev;
   const double* energy_dev;
   long long* loc_dev;
-  int B, capacity;
-  long long lib_u4, fbytes, room;  // room: frames the libraries can still take (one template per agent and frame)
+  int B, R, capacity;
+  const int* rec_of;
+  long long lib_u4, fbytes, room;  // room: image ticks the libraries can still take (one template per agent and image)
   int im_cols, row_lo, row_step, col_lo, col_step;
   char* scratch;
   EnsScratch lay;
-  cudaGraphExec_t exec[2];
-  bool ready[2];
-  int warm[2];
+  // the tick's graphs: [v] with an image in some recording, [3 + v] without; v = 0 no recording moved, 1 every
+  // recording moved, 2 mixed
+  cudaGraphExec_t exec[6];
+  bool ready[6];
+  int warm[6];
   cudaStream_t side;
   cudaEvent_t ev_fork, ev_join;
-  // prs_ens_set_recordings (R = 0: not set): agent b replays recording rec_of[b]; the frame's three graphs are
-  // [0] no recording moved, [1] every recording has a frame and moved, [2] mixed
-  int R;
-  const int* rec_of;
-  char* mscratch;
-  EnsMultiScratch mlay;
-  cudaGraphExec_t mexec[3];
-  bool mready[3];
-  int mwarm[3];
-  // prs_ens_events_run's ticks: [v] with an image in some recording, [3 + v] odometry only, v as above
-  cudaGraphExec_t eexec[6];
-  bool eready[6];
-  int ewarm[6];
 };
 
-static int ens_enqueue(prs_ens_plan* e, bool moved, cudaStream_t st) {
+static size_t ens_net_bytes(const prs_pc_plan* pc) { return (size_t)pc->N * (pc->dtype == PRS_F32 ? 4 : 8); }
+
+static int ens_tick_enqueue(prs_ens_plan* e, int v, bool image, cudaStream_t st) {
   char* sc = e->scratch;
-  const EnsScratch& L = e->lay;
+  const EnsScratch& M = e->lay;
+  prs_pc_plan* pc = e->pc;
   long long* d_argmax = (long long*)e->pc_work;
   void* d_total = (char*)e->pc_work + 8 * (size_t)e->B;
   int* d_err = (int*)((char*)e->pc_work + 16 * (size_t)e->B);
-  int* d_ctr = (int*)(sc + L.misc);
+  int* d_ctr = (int*)(sc + M.misc);
   int* d_gmax = d_ctr + 1;
-  double* d_odom = (double*)(sc + L.odom);
-  unsigned long long* d_key = (unsigned long long*)(sc + L.key);
-  prs_frame_result* d_rec = (prs_frame_result*)(sc + L.rec);
-  const int B = e->B;
+  double* d_odom = (double*)(sc + M.odom);
+  unsigned long long* d_key = (unsigned long long*)(sc + M.key);
+  prs_frame_result* d_rec = (prs_frame_result*)(sc + M.rec);
+  const uint8_t* d_gate = (const uint8_t*)(sc + M.gate);
+  uint8_t* d_present = (uint8_t*)(sc + M.present);
+  uint8_t* d_still = (uint8_t*)(sc + M.still);
+  const int B = e->B, R = e->R;
+  const cudaStream_t side = image ? e->side : st;
   int rc;
-  if (moved) {  // fork: the pose-cell update does not depend on the frame until the decision
-    PRS_CUDA(cudaEventRecord(e->ev_fork, st));
-    PRS_CUDA(cudaStreamWaitEvent(e->side, e->ev_fork, 0));
-    k_ens_odom<<<(B + 255) / 256, 256, 0, e->side>>>((const double*)(sc + L.odom_chunk), d_ctr, d_odom, B);
+  if (v != 0) {
+    if (image) {  // fork: the pose-cell update does not depend on the images until the decision
+      PRS_CUDA(cudaEventRecord(e->ev_fork, st));
+      PRS_CUDA(cudaStreamWaitEvent(e->side, e->ev_fork, 0));
+    }
+    k_ens_odom_multi<<<(B + 255) / 256, 256, 0, side>>>((const double*)(sc + M.odom_chunk), d_gate, d_ctr, e->rec_of, R,
+                                                        d_odom, d_still, B);
     PRS_CUDA(cudaGetLastError());
-    rc = prs_pc_step(e->pc, e->pc_state, d_odom, e->gi, d_argmax, d_total, d_err, e->side);
+    const int es = pc->dtype == PRS_F32 ? 4 : 8;
+    const size_t net_bytes = ens_net_bytes(pc);
+    const bool wide = net_bytes % 16 == 0;
+    const long long words = (long long)(net_bytes / (wide ? 16 : 4));
+    const int per_net = (int)((words + 4095) / 4096);  // 256 threads x 16 words per block
+    auto snapshot = [&](bool restore) {
+      long long* ws = (long long*)(sc + M.wsnap);
+      long long* w = (long long*)e->pc_work;
+      const dim3 grid((unsigned)B * per_net);
+      if (wide) {
+        if (restore)
+          k_ens_snapshot<true, uint4><<<grid, 256, 0, side>>>((uint4*)e->pc_state, (uint4*)(sc + M.snap), words, per_net,
+                                                                 d_still, w, ws, B, es);
+        else
+          k_ens_snapshot<false, uint4><<<grid, 256, 0, side>>>((uint4*)e->pc_state, (uint4*)(sc + M.snap), words,
+                                                                  per_net, d_still, w, ws, B, es);
+      } else {
+        if (restore)
+          k_ens_snapshot<true, unsigned><<<grid, 256, 0, side>>>((unsigned*)e->pc_state, (unsigned*)(sc + M.snap), words,
+                                                                    per_net, d_still, w, ws, B, es);
+        else
+          k_ens_snapshot<false, unsigned><<<grid, 256, 0, side>>>((unsigned*)e->pc_state, (unsigned*)(sc + M.snap),
+                                                                     words, per_net, d_still, w, ws, B, es);
+      }
+      return cudaGetLastError();
+    };
+    if (v == 2) PRS_CUDA(snapshot(false));
+    rc = prs_pc_step(pc, e->pc_state, d_odom, e->gi, d_argmax, d_total, d_err, side);
     if (rc != PRS_OK) return rc;
-    PRS_CUDA(cudaEventRecord(e->ev_join, e->side));
+    if (v == 2) {
+      PRS_CUDA(snapshot(true));
+      if (int rc_ = prs_pc_active_invalidate(pc, side)) return rc_;  // the carried lists describe the undone update
+    }
+    if (image) PRS_CUDA(cudaEventRecord(e->ev_join, e->side));
   }
-  k_vt_frame_prepare<<<1, 1024, 0, st>>>((const uint8_t*)(sc + L.frames), e->im_cols, e->row_lo, e->row_step, e->col_lo,
-                                         e->col_step, (uint8_t*)(sc + L.tpl), (uint32_t*)(sc + L.planes), d_key, d_ctr,
-                                         e->fbytes, B);
+  if (!image) {
+    k_ens_no_image<<<1, B < 1024 ? (B + 31) / 32 * 32 : 1024, 0, st>>>(d_argmax, d_err, e->n_dev, d_rec, d_ctr, B);
+    PRS_CUDA(cudaGetLastError());
+    return PRS_OK;
+  }
+  k_vt_frame_prepare_multi<<<R, 1024, 0, st>>>((const uint8_t*)(sc + M.frames), M.chunk, e->fbytes, e->im_cols, e->row_lo,
+                                               e->row_step, e->col_lo, e->col_step, (uint8_t*)(sc + M.tpl),
+                                               (uint32_t*)(sc + M.planes), d_key, B, d_ctr, d_present,
+                                               (const int*)(sc + M.slots));
   long long blocks = (long long)B * ((e->capacity + 31) / 32);
   if (blocks > 148LL * 4) blocks = 148LL * 4;
-  k_vt_sweep_packed_ref_small<false><<<(int)blocks, kSmallThreads, 0, st>>>((const uint4*)e->libs, (const uint32_t*)(sc + L.planes),
-                                                                     d_key, e->n_dev, B, e->lib_u4, d_gmax);
-  if (moved) PRS_CUDA(cudaStreamWaitEvent(st, e->ev_join, 0));  // the decision reports the new arg-max
+  // With one recording a tick with an image has it for every agent: the per-agent recording and presence checks
+  // cannot fail, and they cost the latency-bound sweep a chain of dependent loads per item (6 % of the frame at B = 1024)
+  const bool one = R == 1;
+  if (one)
+    k_vt_sweep_packed_ref_small<false><<<(int)blocks, kSmallThreads, 0, st>>>(
+        (const uint4*)e->libs, (const uint32_t*)(sc + M.planes), d_key, e->n_dev, B, e->lib_u4, d_gmax);
+  else
+    k_vt_sweep_packed_ref_small<true><<<(int)blocks, kSmallThreads, 0, st>>>(
+        (const uint4*)e->libs, (const uint32_t*)(sc + M.planes), d_key, e->n_dev, B, e->lib_u4, d_gmax, e->rec_of,
+        d_present);
+  if (v != 0) PRS_CUDA(cudaStreamWaitEvent(st, e->ev_join, 0));  // the decision reports the new arg-max
   VtAgents ag;
   ag.B = B;
   ag.lib_u4 = e->lib_u4;
@@ -2221,11 +2207,14 @@ static int ens_enqueue(prs_ens_plan* e, bool moved, cudaStream_t st) {
   ag.loc_stride = e->capacity;
   ag.g_max = d_gmax;
   ag.ctr = d_ctr;
-  k_vt_decide_append<<<(B + 3) / 4, 128, 0, st>>>(d_key, (const uint8_t*)(sc + L.tpl), (uint4*)e->libs, 0, 0.0, d_argmax,
+  if (!one) {
+    ag.rec_of = e->rec_of;
+    ag.present = d_present;
+  }
+  k_vt_decide_append<<<(B + 3) / 4, 128, 0, st>>>(d_key, (const uint8_t*)(sc + M.tpl), (uint4*)e->libs, 0, 0.0, d_argmax,
                                                   d_err, d_rec, e->n_dev, 1, nullptr, ag);
   PRS_CUDA(cudaGetLastError());
   if (e->energy_dev) {
-    prs_pc_plan* pc = e->pc;
     if (int rc_ = prs_pc_active_invalidate(pc, st)) return rc_;  // as prs_pc_inject: the carried lists are stale
     if (pc->dtype == PRS_F32)
       k_frame_inject<float><<<(B + 127) / 128, 128, 0, st>>>((float*)e->pc_state, e->loc_dev, d_rec, d_argmax, d_err, d_rec,
@@ -2240,17 +2229,47 @@ static int ens_enqueue(prs_ens_plan* e, bool moved, cudaStream_t st) {
   return PRS_OK;
 }
 
-extern "C" size_t prs_ens_scratch_bytes(int B, int im_rows, int im_cols) {
-  if (B < 1 || im_rows < 1 || im_cols < 1) return 0;
-  return EnsScratch(B, (long long)im_rows * im_cols).bytes;
+// One tick: the first call of each kind runs eagerly (lazily initialised kernel attributes), the second captures the
+// graph, later ones replay it.
+static int ens_tick_launch(prs_ens_plan* e, int v, bool image, cudaStream_t st) {
+  const int i = image ? v : 3 + v;
+  if (e->ready[i]) {
+    PRS_CUDA(cudaGraphLaunch(e->exec[i], st));
+    return PRS_OK;
+  }
+  if (e->warm[i] < 1) {
+    ++e->warm[i];
+    return ens_tick_enqueue(e, v, image, st);
+  }
+  cudaGraph_t g = nullptr;
+  PRS_CUDA(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
+  int rc = ens_tick_enqueue(e, v, image, st);
+  cudaError_t err = cudaStreamEndCapture(st, &g);
+  if (rc != PRS_OK || err != cudaSuccess) {
+    if (g) cudaGraphDestroy(g);
+    if (rc == PRS_OK) prs_set_error("prs_ens_run: capture failed: %s", cudaGetErrorString(err));
+    return rc != PRS_OK ? rc : PRS_E_CUDA;
+  }
+  err = cudaGraphInstantiate(&e->exec[i], g, 0);
+  cudaGraphDestroy(g);
+  PRS_CUDA(err);
+  e->ready[i] = true;
+  PRS_CUDA(cudaGraphLaunch(e->exec[i], st));
+  return PRS_OK;
+}
+
+extern "C" size_t prs_ens_scratch_bytes(prs_pc_handle pc, int R, int im_rows, int im_cols) {
+  if (!pc || R < 1 || im_rows < 1 || im_cols < 1) return 0;
+  return EnsScratch(pc->B, R, (long long)im_rows * im_cols, ens_net_bytes(pc)).bytes;
 }
 
 extern "C" int prs_ens_create(prs_pc_handle pc, void* pc_state, const void* gi, void* pc_work, void* libs, int capacity,
                               int* n_dev, const double* threshold_dev, const double* energy_dev, long long* loc_dev,
-                              int mode, int im_rows, int im_cols, int row_lo, int row_hi, int row_step, int col_lo,
-                              int col_hi, int col_step, void* scratch, prs_ens_plan** out) {
-  PRS_REQUIRE(pc && pc_state && gi && pc_work && libs && n_dev && threshold_dev && loc_dev && scratch && out,
+                              int R, const int* rec_of_dev, int mode, int im_rows, int im_cols, int row_lo, int row_hi,
+                              int row_step, int col_lo, int col_hi, int col_step, void* scratch, prs_ens_plan** out) {
+  PRS_REQUIRE(pc && pc_state && gi && pc_work && libs && n_dev && threshold_dev && loc_dev && rec_of_dev && scratch && out,
               "prs_ens_create: null argument");
+  PRS_REQUIRE(R >= 1, "prs_ens_create: %d recordings", R);
   PRS_REQUIRE(mode == PRS_VT_MODE_REF, "prs_ens_create: only the reference mode (PRS_VT_MODE_REF) is supported, got %d",
               mode);
   PRS_REQUIRE(capacity >= 1 && capacity <= kSmallLibrary, "prs_ens_create: capacity %d outside [1, %d]", capacity,
@@ -2260,12 +2279,13 @@ extern "C" int prs_ens_create(prs_pc_handle pc, void* pc_state, const void* gi, 
   if (int rc = check_mask(im_rows, im_cols, row_lo, row_hi, row_step, col_lo, col_hi, col_step, 32, 32)) return rc;
   if (int rc = prs_pc_check_device(pc, "prs_ens_create")) return rc;
   const int B = pc->B;
+  const long long fbytes = (long long)im_rows * im_cols;
   prs_ens_plan* e = new (std::nothrow) prs_ens_plan{pc, pc_state, pc_work, libs, gi, n_dev, threshold_dev, energy_dev,
-                                                     loc_dev, B, capacity, (long long)(prs_vt_packed_bytes(capacity) / 16),
-                                                     (long long)im_rows * im_cols, 0, im_cols, row_lo, row_step, col_lo,
-                                                     col_step, (char*)scratch, EnsScratch(B, (long long)im_rows * im_cols),
-                                                     {nullptr, nullptr}, {false, false}, {0, 0}, nullptr, nullptr, nullptr,
-                                                     0, nullptr, nullptr, EnsMultiScratch(), {}, {}, {}, {}, {}, {}};
+                                                     loc_dev, B, R, capacity, rec_of_dev,
+                                                     (long long)(prs_vt_packed_bytes(capacity) / 16), fbytes, 0, im_cols,
+                                                     row_lo, row_step, col_lo, col_step, (char*)scratch,
+                                                     EnsScratch(B, R, fbytes, ens_net_bytes(pc)), {}, {}, {}, nullptr,
+                                                     nullptr, nullptr};
   PRS_REQUIRE(e, "prs_ens_create: out of host memory");
   int* misc = (int*)(e->scratch + e->lay.misc);
   int init[3] = {0, 0, 0};
@@ -2288,8 +2308,8 @@ extern "C" int prs_ens_create(prs_pc_handle pc, void* pc_state, const void* gi, 
   return PRS_OK;
 }
 
-// Room counts frames, not templates (a run may append one per frame); a session that feeds a plan in pieces recounts
-// it from the libraries as they are after the earlier runs.
+// Room counts image ticks, not templates (a run may append one per image tick); a session that feeds a plan in pieces
+// recounts it from the libraries as they are after the earlier runs.
 extern "C" int prs_ens_refresh_room(prs_ens_plan* e, void* stream) {
   PRS_REQUIRE(e && stream, "prs_ens_refresh_room: bad argument");
   const cudaStream_t st = (cudaStream_t)stream;
@@ -2306,12 +2326,8 @@ extern "C" int prs_ens_refresh_room(prs_ens_plan* e, void* stream) {
 
 extern "C" int prs_ens_destroy(prs_ens_plan* e) {
   if (e) {
-    for (int i = 0; i < 2; ++i)
-      if (e->ready[i]) cudaGraphExecDestroy(e->exec[i]);
-    for (int i = 0; i < 3; ++i)
-      if (e->mready[i]) cudaGraphExecDestroy(e->mexec[i]);
     for (int i = 0; i < 6; ++i)
-      if (e->eready[i]) cudaGraphExecDestroy(e->eexec[i]);
+      if (e->ready[i]) cudaGraphExecDestroy(e->exec[i]);
     if (e->side) cudaStreamDestroy(e->side);
     if (e->ev_fork) cudaEventDestroy(e->ev_fork);
     if (e->ev_join) cudaEventDestroy(e->ev_join);
@@ -2320,331 +2336,13 @@ extern "C" int prs_ens_destroy(prs_ens_plan* e) {
   return PRS_OK;
 }
 
-// One frame of the ensemble: the first call of each kind runs eagerly (lazily initialised kernel attributes), the
-// second captures the graph, later ones replay it.
-static int ens_launch(prs_ens_plan* e, int moved, cudaStream_t st) {
-  const int v = moved ? 1 : 0;
-  if (e->ready[v]) {
-    PRS_CUDA(cudaGraphLaunch(e->exec[v], st));
-    return PRS_OK;
-  }
-  if (e->warm[v] < 1) {
-    ++e->warm[v];
-    return ens_enqueue(e, moved != 0, st);
-  }
-  cudaGraph_t g = nullptr;
-  PRS_CUDA(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
-  int rc = ens_enqueue(e, moved != 0, st);
-  cudaError_t err = cudaStreamEndCapture(st, &g);
-  if (rc != PRS_OK || err != cudaSuccess) {
-    if (g) cudaGraphDestroy(g);
-    if (rc == PRS_OK) prs_set_error("prs_ens_replay_run: capture failed: %s", cudaGetErrorString(err));
-    return rc != PRS_OK ? rc : PRS_E_CUDA;
-  }
-  err = cudaGraphInstantiate(&e->exec[v], g, 0);
-  cudaGraphDestroy(g);
-  PRS_CUDA(err);
-  e->ready[v] = true;
-  PRS_CUDA(cudaGraphLaunch(e->exec[v], st));
-  return PRS_OK;
-}
-
-extern "C" int prs_ens_replay_run(prs_ens_plan* e, const uint8_t* frames, const double* odom, const uint8_t* moved, int T,
-                                  prs_frame_result* results, void* stream) {
-  PRS_REQUIRE(e && T >= 0 && (T == 0 || (frames && odom && moved && results)), "prs_ens_replay_run: bad argument");
-  PRS_REQUIRE(stream != nullptr, "prs_ens_replay_run: needs a non-default stream (the frames replay as CUDA graphs)");
-  PRS_REQUIRE(T <= e->room, "prs_ens_replay_run: %d frames do not fit the libraries (room for %lld more templates)", T,
-              e->room);
-  if (int rc = prs_pc_check_device(e->pc, "prs_ens_replay_run")) return rc;
-  cudaStream_t st = (cudaStream_t)stream;
-  char* sc = e->scratch;
-  const EnsScratch& L = e->lay;
-  const size_t rec_bytes = (size_t)e->B * sizeof(prs_frame_result);
-  int rc = PRS_OK;
-  for (int c0 = 0; c0 < T && rc == PRS_OK; c0 += kEnsChunk) {
-    const int n = T - c0 < kEnsChunk ? T - c0 : kEnsChunk;
-    PRS_CUDA(cudaMemcpyAsync(sc + L.frames, frames + (size_t)c0 * e->fbytes, (size_t)n * e->fbytes,
-                             cudaMemcpyHostToDevice, st));
-    PRS_CUDA(cudaMemcpyAsync(sc + L.odom_chunk, odom + 2 * (size_t)c0, (size_t)n * 2 * sizeof(double),
-                             cudaMemcpyHostToDevice, st));
-    PRS_CUDA(cudaMemsetAsync(sc + L.misc, 0, sizeof(int), st));  // the frame counter
-    int done = 0;
-    for (; done < n; ++done) {
-      rc = ens_launch(e, moved[c0 + done], st);
-      if (rc != PRS_OK) break;
-    }
-    if (done > 0)
-      PRS_CUDA(cudaMemcpyAsync(results + (size_t)c0 * e->B, sc + L.rec, (size_t)done * rec_bytes, cudaMemcpyDeviceToHost,
-                               st));
-    e->room -= done;
-  }
-  const cudaError_t err = cudaStreamSynchronize(st);
-  if (rc == PRS_OK && err != cudaSuccess) {
-    prs_set_error("prs_ens_replay_run: %s", cudaGetErrorString(err));
-    return PRS_E_CUDA;
-  }
-  return rc;
-}
-
-// ---------------------------------------------------------------------------------------------
-// Multi-recording ensemble replay: agent b replays recording rec_of[b] (prs_ens_set_recordings).  The frame graph is
-// the one above with a query per recording and a per-agent gate:
-//   side branch  k_ens_odom_multi (each network its recording's twist, (0, 0) where that recording is still or has
-//                ended) -> [mixed: k_ens_snapshot save] -> prs_pc_step -> [mixed: k_ens_snapshot restore ->
-//                prs_pc_active_invalidate]
-//   template     k_vt_frame_prepare_multi (one block per recording) -> k_vt_sweep_packed_ref_small<true>
-//   join         k_vt_decide_append / k_frame_inject with VtAgents::rec_of and ::present -> k_ens_advance
-// The restore runs before the join, so the decision and the injection of a still network see its state, arg-max and
-// error bits as they were: what the single-recording frame leaves when it skips the update.  A frame where no recording
-// moved runs no update; one where every recording has a frame and moved needs no snapshot.
-// events (message-stream ticks, prs_ens_events_run): the query reads its image through the chunk's slot table
-// (k_vt_frame_prepare_multi<true>).  A tick without an image in any recording (!image) is lean: the side branch's
-// nodes run on `st` itself, then k_ens_no_image writes the records and advances the counter -- no query, sweep,
-// decision or injection.
-static int ens_multi_enqueue(prs_ens_plan* e, int v, cudaStream_t st, bool events = false, bool image = true) {
-  char* sc = e->scratch;
-  char* ms = e->mscratch;
-  const EnsMultiScratch& M = e->mlay;
-  prs_pc_plan* pc = e->pc;
-  long long* d_argmax = (long long*)e->pc_work;
-  void* d_total = (char*)e->pc_work + 8 * (size_t)e->B;
-  int* d_err = (int*)((char*)e->pc_work + 16 * (size_t)e->B);
-  int* d_ctr = (int*)(sc + e->lay.misc);
-  int* d_gmax = d_ctr + 1;
-  double* d_odom = (double*)(ms + M.odom);
-  unsigned long long* d_key = (unsigned long long*)(ms + M.key);
-  prs_frame_result* d_rec = (prs_frame_result*)(ms + M.rec);
-  const uint8_t* d_gate = (const uint8_t*)(ms + M.gate);
-  uint8_t* d_present = (uint8_t*)(ms + M.present);
-  uint8_t* d_still = (uint8_t*)(ms + M.still);
-  const int B = e->B, R = e->R;
-  const cudaStream_t side = image ? e->side : st;
-  int rc;
-  if (v != 0) {
-    if (image) {
-      PRS_CUDA(cudaEventRecord(e->ev_fork, st));
-      PRS_CUDA(cudaStreamWaitEvent(e->side, e->ev_fork, 0));
-    }
-    k_ens_odom_multi<<<(B + 255) / 256, 256, 0, side>>>((const double*)(ms + M.odom_chunk), d_gate, d_ctr, e->rec_of, R,
-                                                        d_odom, d_still, B);
-    PRS_CUDA(cudaGetLastError());
-    const int es = pc->dtype == PRS_F32 ? 4 : 8;
-    const size_t net_bytes = (size_t)pc->N * es;
-    const bool wide = net_bytes % 16 == 0;
-    const long long words = (long long)(net_bytes / (wide ? 16 : 4));
-    const int per_net = (int)((words + 4095) / 4096);  // 256 threads x 16 words per block
-    auto snapshot = [&](bool restore) {
-      long long* ws = (long long*)(ms + M.wsnap);
-      long long* w = (long long*)e->pc_work;
-      const dim3 grid((unsigned)B * per_net);
-      if (wide) {
-        if (restore)
-          k_ens_snapshot<true, uint4><<<grid, 256, 0, side>>>((uint4*)e->pc_state, (uint4*)(ms + M.snap), words, per_net,
-                                                                 d_still, w, ws, B, es);
-        else
-          k_ens_snapshot<false, uint4><<<grid, 256, 0, side>>>((uint4*)e->pc_state, (uint4*)(ms + M.snap), words,
-                                                                  per_net, d_still, w, ws, B, es);
-      } else {
-        if (restore)
-          k_ens_snapshot<true, unsigned><<<grid, 256, 0, side>>>((unsigned*)e->pc_state, (unsigned*)(ms + M.snap), words,
-                                                                    per_net, d_still, w, ws, B, es);
-        else
-          k_ens_snapshot<false, unsigned><<<grid, 256, 0, side>>>((unsigned*)e->pc_state, (unsigned*)(ms + M.snap),
-                                                                     words, per_net, d_still, w, ws, B, es);
-      }
-      return cudaGetLastError();
-    };
-    if (v == 2) PRS_CUDA(snapshot(false));
-    rc = prs_pc_step(pc, e->pc_state, d_odom, e->gi, d_argmax, d_total, d_err, side);
-    if (rc != PRS_OK) return rc;
-    if (v == 2) {
-      PRS_CUDA(snapshot(true));
-      if (int rc_ = prs_pc_active_invalidate(pc, side)) return rc_;  // the carried lists describe the undone update
-    }
-    if (image) PRS_CUDA(cudaEventRecord(e->ev_join, e->side));
-  }
-  if (!image) {
-    k_ens_no_image<<<1, B < 1024 ? (B + 31) / 32 * 32 : 1024, 0, st>>>(d_argmax, d_err, e->n_dev, d_rec, d_ctr, B);
-    PRS_CUDA(cudaGetLastError());
-    return PRS_OK;
-  }
-  if (events)
-    k_vt_frame_prepare_multi<true><<<R, 1024, 0, st>>>((const uint8_t*)(ms + M.frames), M.chunk, e->fbytes, e->im_cols,
-                                                       e->row_lo, e->row_step, e->col_lo, e->col_step,
-                                                       (uint8_t*)(ms + M.tpl), (uint32_t*)(ms + M.planes), d_key, B, d_ctr,
-                                                       d_gate, d_present, (const int*)(ms + M.slots));
-  else
-    k_vt_frame_prepare_multi<false><<<R, 1024, 0, st>>>((const uint8_t*)(ms + M.frames), M.chunk, e->fbytes, e->im_cols,
-                                                        e->row_lo, e->row_step, e->col_lo, e->col_step,
-                                                        (uint8_t*)(ms + M.tpl), (uint32_t*)(ms + M.planes), d_key, B,
-                                                        d_ctr, d_gate, d_present);
-  long long blocks = (long long)B * ((e->capacity + 31) / 32);
-  if (blocks > 148LL * 4) blocks = 148LL * 4;
-  k_vt_sweep_packed_ref_small<true><<<(int)blocks, kSmallThreads, 0, st>>>(
-      (const uint4*)e->libs, (const uint32_t*)(ms + M.planes), d_key, e->n_dev, B, e->lib_u4, d_gmax, e->rec_of, d_present);
-  if (v != 0) PRS_CUDA(cudaStreamWaitEvent(st, e->ev_join, 0));
-  VtAgents ag;
-  ag.B = B;
-  ag.lib_u4 = e->lib_u4;
-  ag.threshold = e->thr_dev;
-  ag.loc = e->loc_dev;
-  ag.loc_stride = e->capacity;
-  ag.g_max = d_gmax;
-  ag.ctr = d_ctr;
-  ag.rec_of = e->rec_of;
-  ag.present = d_present;
-  k_vt_decide_append<<<(B + 3) / 4, 128, 0, st>>>(d_key, (const uint8_t*)(ms + M.tpl), (uint4*)e->libs, 0, 0.0, d_argmax,
-                                                  d_err, d_rec, e->n_dev, 1, nullptr, ag);
-  PRS_CUDA(cudaGetLastError());
-  if (e->energy_dev) {
-    if (int rc_ = prs_pc_active_invalidate(pc, st)) return rc_;
-    if (pc->dtype == PRS_F32)
-      k_frame_inject<float><<<(B + 127) / 128, 128, 0, st>>>((float*)e->pc_state, e->loc_dev, d_rec, d_argmax, d_err, d_rec,
-                                                             pc->X, pc->Y, pc->Th, 0.0f, e->energy_dev, ag);
-    else
-      k_frame_inject<double><<<(B + 127) / 128, 128, 0, st>>>((double*)e->pc_state, e->loc_dev, d_rec, d_argmax, d_err,
-                                                              d_rec, pc->X, pc->Y, pc->Th, 0.0, e->energy_dev, ag);
-    PRS_CUDA(cudaGetLastError());
-  }
-  k_ens_advance<<<1, 1, 0, st>>>(d_ctr);
-  PRS_CUDA(cudaGetLastError());
-  return PRS_OK;
-}
-
-// as ens_launch: eager first call, capture on the second, replay after.  kind 0: a frame of prs_ens_multi_replay_run
-// (graphs mexec[v]); 1 / 2: a tick of prs_ens_events_run with / without an image (eexec[v] / eexec[3 + v])
-static int ens_multi_launch(prs_ens_plan* e, int v, cudaStream_t st, int kind = 0) {
-  cudaGraphExec_t* exec = kind == 0 ? &e->mexec[v] : &e->eexec[kind == 1 ? v : 3 + v];
-  bool* ready = kind == 0 ? &e->mready[v] : &e->eready[kind == 1 ? v : 3 + v];
-  int* warm = kind == 0 ? &e->mwarm[v] : &e->ewarm[kind == 1 ? v : 3 + v];
-  const char* who = kind == 0 ? "prs_ens_multi_replay_run" : "prs_ens_events_run";
-  if (*ready) {
-    PRS_CUDA(cudaGraphLaunch(*exec, st));
-    return PRS_OK;
-  }
-  if (*warm < 1) {
-    ++*warm;
-    return ens_multi_enqueue(e, v, st, kind != 0, kind != 2);
-  }
-  cudaGraph_t g = nullptr;
-  PRS_CUDA(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
-  int rc = ens_multi_enqueue(e, v, st, kind != 0, kind != 2);
-  cudaError_t err = cudaStreamEndCapture(st, &g);
-  if (rc != PRS_OK || err != cudaSuccess) {
-    if (g) cudaGraphDestroy(g);
-    if (rc == PRS_OK) prs_set_error("%s: capture failed: %s", who, cudaGetErrorString(err));
-    return rc != PRS_OK ? rc : PRS_E_CUDA;
-  }
-  err = cudaGraphInstantiate(exec, g, 0);
-  cudaGraphDestroy(g);
-  PRS_CUDA(err);
-  *ready = true;
-  PRS_CUDA(cudaGraphLaunch(*exec, st));
-  return PRS_OK;
-}
-
-extern "C" size_t prs_ens_multi_scratch_bytes(const prs_ens_plan* e, int R) {
-  if (!e || R < 1) return 0;
-  return EnsMultiScratch(e->B, R, e->fbytes, (size_t)e->pc->N * (e->pc->dtype == PRS_F32 ? 4 : 8)).bytes;
-}
-
-extern "C" int prs_ens_set_recordings(prs_ens_plan* e, int R, const int* rec_of_dev, void* multi_scratch) {
-  PRS_REQUIRE(e && R >= 1 && rec_of_dev && multi_scratch, "prs_ens_set_recordings: bad argument");
-  for (int i = 0; i < 3; ++i) {
-    if (e->mready[i]) cudaGraphExecDestroy(e->mexec[i]);
-    e->mready[i] = false;
-    e->mwarm[i] = 0;
-  }
-  for (int i = 0; i < 6; ++i) {
-    if (e->eready[i]) cudaGraphExecDestroy(e->eexec[i]);
-    e->eready[i] = false;
-    e->ewarm[i] = 0;
-  }
-  e->R = R;
-  e->rec_of = rec_of_dev;
-  e->mscratch = (char*)multi_scratch;
-  e->mlay = EnsMultiScratch(e->B, R, e->fbytes, (size_t)e->pc->N * (e->pc->dtype == PRS_F32 ? 4 : 8));
-  return PRS_OK;
-}
-
-extern "C" int prs_ens_multi_replay_run(prs_ens_plan* e, const uint8_t* const* frames, const double* odom,
-                                        const uint8_t* moved, const int* lengths, int T_max, prs_frame_result* results,
-                                        void* stream) {
-  PRS_REQUIRE(e && T_max >= 0 && lengths && (T_max == 0 || (frames && odom && moved && results)),
-              "prs_ens_multi_replay_run: bad argument");
-  PRS_REQUIRE(e->R >= 1, "prs_ens_multi_replay_run: no recordings set (prs_ens_set_recordings)");
-  PRS_REQUIRE(stream != nullptr, "prs_ens_multi_replay_run: needs a non-default stream (the frames replay as CUDA graphs)");
-  const int R = e->R;
-  for (int r = 0; r < R; ++r)
-    PRS_REQUIRE(lengths[r] >= 0 && lengths[r] <= T_max && (lengths[r] == 0 || frames[r]),
-                "prs_ens_multi_replay_run: recording %d has length %d outside [0, %d] or no frames", r, lengths[r], T_max);
-  PRS_REQUIRE(T_max <= e->room,
-              "prs_ens_multi_replay_run: %d frames do not fit the libraries (room for %lld more templates)", T_max, e->room);
-  if (int rc = prs_pc_check_device(e->pc, "prs_ens_multi_replay_run")) return rc;
-  // gate[t][r]: bit 0 = recording r has frame t, bit 1 = and it moved
-  std::vector<uint8_t> gate((size_t)T_max * R);
-  std::vector<uint8_t> variant(T_max);
-  for (int t = 0; t < T_max; ++t) {
-    bool any = false, all = true;
-    for (int r = 0; r < R; ++r) {
-      const bool here = t < lengths[r], mv = here && moved[(size_t)t * R + r] != 0;
-      gate[(size_t)t * R + r] = (uint8_t)((here ? 1 : 0) | (mv ? 2 : 0));
-      any |= mv;
-      all &= mv;
-    }
-    variant[t] = (uint8_t)(!any ? 0 : all ? 1 : 2);
-  }
-  cudaStream_t st = (cudaStream_t)stream;
-  char* ms = e->mscratch;
-  const EnsMultiScratch& M = e->mlay;
-  const size_t rec_bytes = (size_t)e->B * sizeof(prs_frame_result);
-  int rc = PRS_OK;
-  for (int c0 = 0; c0 < T_max && rc == PRS_OK; c0 += M.chunk) {
-    const int n = T_max - c0 < M.chunk ? T_max - c0 : M.chunk;
-    for (int r = 0; r < R; ++r) {
-      const int nr = lengths[r] - c0 < n ? lengths[r] - c0 : n;
-      if (nr > 0)
-        PRS_CUDA(cudaMemcpyAsync(ms + M.frames + (size_t)r * M.chunk * e->fbytes, frames[r] + (size_t)c0 * e->fbytes,
-                                 (size_t)nr * e->fbytes, cudaMemcpyHostToDevice, st));
-    }
-    PRS_CUDA(cudaMemcpyAsync(ms + M.odom_chunk, odom + (size_t)c0 * R * 2, (size_t)n * R * 2 * sizeof(double),
-                             cudaMemcpyHostToDevice, st));
-    PRS_CUDA(cudaMemcpyAsync(ms + M.gate, gate.data() + (size_t)c0 * R, (size_t)n * R, cudaMemcpyHostToDevice, st));
-    PRS_CUDA(cudaMemsetAsync(e->scratch + e->lay.misc, 0, sizeof(int), st));  // the frame counter
-    int done = 0;
-    for (; done < n; ++done) {
-      rc = ens_multi_launch(e, variant[c0 + done], st);
-      if (rc != PRS_OK) break;
-    }
-    if (done > 0)
-      PRS_CUDA(cudaMemcpyAsync(results + (size_t)c0 * e->B, ms + M.rec, (size_t)done * rec_bytes, cudaMemcpyDeviceToHost,
-                               st));
-    e->room -= done;
-  }
-  const cudaError_t err = cudaStreamSynchronize(st);
-  if (rc == PRS_OK && err != cudaSuccess) {
-    prs_set_error("prs_ens_multi_replay_run: %s", cudaGetErrorString(err));
-    return PRS_E_CUDA;
-  }
-  return rc;
-}
-
-// ---------------------------------------------------------------------------------------------
-// Message-stream ensemble replay: the node's message loop (ros_simulate.replay_events) for every agent, one pose-cell
-// update per gated odometry message.  The caller compacts each recording's stream into ticks of (optional gated twist,
-// optional image), odometry before image; tick t of recording r has gate[t][r] bit 0 = image, bit 1 = moved.  A tick
-// is the multi-recording frame graph with two differences: the query of recording r is its image at slot
-// slots[t][r] of the chunk (images are contiguous per recording, not one per tick), and a tick with no image in any
-// recording runs the side branch alone, then k_ens_no_image.  Six graphs: {no update, all moved, mixed} x {image, none}.
-extern "C" int prs_ens_events_run(prs_ens_plan* e, const uint8_t* const* frames, const double* odom, const uint8_t* gate,
-                                  const int* n_images, int T, prs_frame_result* results, void* stream) {
-  PRS_REQUIRE(e && T >= 0 && n_images && (T == 0 || (frames && odom && gate && results)),
-              "prs_ens_events_run: bad argument");
-  PRS_REQUIRE(e->R >= 1, "prs_ens_events_run: no recordings set (prs_ens_set_recordings)");
-  PRS_REQUIRE(stream != nullptr, "prs_ens_events_run: needs a non-default stream (the ticks replay as CUDA graphs)");
+extern "C" int prs_ens_run(prs_ens_plan* e, const uint8_t* const* frames, const double* odom, const uint8_t* gate,
+                           const int* n_images, int T, prs_frame_result* results, void* stream) {
+  PRS_REQUIRE(e && T >= 0 && n_images && (T == 0 || (frames && odom && gate && results)), "prs_ens_run: bad argument");
+  PRS_REQUIRE(stream != nullptr, "prs_ens_run: needs a non-default stream (the ticks replay as CUDA graphs)");
   const int R = e->R;
   // slots[t][r]: recording r's image at tick t, counted from the first image of t's chunk; -1 = none
-  const EnsMultiScratch& M = e->mlay;
+  const EnsScratch& M = e->lay;
   std::vector<int> slots((size_t)T * R);
   std::vector<uint8_t> variant(T), has_image(T);
   std::vector<int> seen(R, 0), in_chunk(R, 0);
@@ -2667,14 +2365,14 @@ extern "C" int prs_ens_events_run(prs_ens_plan* e, const uint8_t* const* frames,
   }
   for (int r = 0; r < R; ++r)
     PRS_REQUIRE(n_images[r] == seen[r] && (seen[r] == 0 || frames[r]),
-                "prs_ens_events_run: recording %d has %d images in its gate, n_images says %d (or no frames)", r, seen[r],
+                "prs_ens_run: recording %d has %d images in its gate, n_images says %d (or no frames)", r, seen[r],
                 n_images[r]);
   PRS_REQUIRE(image_ticks <= e->room,
-              "prs_ens_events_run: %lld ticks with images do not fit the libraries (room for %lld more templates)",
+              "prs_ens_run: %lld ticks with images do not fit the libraries (room for %lld more templates)",
               image_ticks, e->room);
-  if (int rc = prs_pc_check_device(e->pc, "prs_ens_events_run")) return rc;
+  if (int rc = prs_pc_check_device(e->pc, "prs_ens_run")) return rc;
   cudaStream_t st = (cudaStream_t)stream;
-  char* ms = e->mscratch;
+  char* ms = e->scratch;
   const size_t rec_bytes = (size_t)e->B * sizeof(prs_frame_result);
   std::vector<long long> first(R, 0);  // each recording's first image of the chunk
   int rc = PRS_OK;
@@ -2695,10 +2393,10 @@ extern "C" int prs_ens_events_run(prs_ens_plan* e, const uint8_t* const* frames,
     PRS_CUDA(cudaMemcpyAsync(ms + M.gate, gate + (size_t)c0 * R, (size_t)n * R, cudaMemcpyHostToDevice, st));
     PRS_CUDA(cudaMemcpyAsync(ms + M.slots, slots.data() + (size_t)c0 * R, (size_t)n * R * sizeof(int),
                              cudaMemcpyHostToDevice, st));
-    PRS_CUDA(cudaMemsetAsync(e->scratch + e->lay.misc, 0, sizeof(int), st));  // the tick counter
+    PRS_CUDA(cudaMemsetAsync(ms + M.misc, 0, sizeof(int), st));  // the tick counter
     int done = 0;
     for (; done < n; ++done) {
-      rc = ens_multi_launch(e, variant[c0 + done], st, has_image[c0 + done] ? 1 : 2);
+      rc = ens_tick_launch(e, variant[c0 + done], has_image[c0 + done] != 0, st);
       if (rc != PRS_OK) break;
     }
     if (done > 0)
@@ -2708,7 +2406,7 @@ extern "C" int prs_ens_events_run(prs_ens_plan* e, const uint8_t* const* frames,
   }
   const cudaError_t err = cudaStreamSynchronize(st);
   if (rc == PRS_OK && err != cudaSuccess) {
-    prs_set_error("prs_ens_events_run: %s", cudaGetErrorString(err));
+    prs_set_error("prs_ens_run: %s", cudaGetErrorString(err));
     return PRS_E_CUDA;
   }
   return rc;

@@ -4,13 +4,14 @@ Tuning RatSLAM offline means replaying one recording under many settings -- the 
 the view-template -> pose-cell injection energy -- and comparing the runs.  ``replay_ensemble`` runs all of them at
 once: agent ``b`` is the ROS loop of ``ros_simulate.replay(native=True, match_threshold=..., inject_energy=...)`` with
 ``pcn.global_inhibition`` set to its own value, and it has its own pose-cell network, view-template library and
-experience map.  The frames and the odometry are shared, so a frame is one CUDA graph for the whole ensemble
-(``prs_ens_replay_run``, csrc/view_templates.cu): one pose-cell update of all B networks, one query, one sweep over
-every agent's library, then the per-agent create-or-match decision and injection.
+experience map.  Tuning on several recordings keeps the settings from fitting one route: with ``frames`` and ``odom``
+given as lists of R recordings, agent ``b`` replays recording ``recording[b]``.  ``replay_ensemble_events`` replays
+message streams instead, every odometry message its own pose-cell update, as the node does.
 
-Tuning on several recordings keeps the settings from fitting one route: with ``frames`` and ``odom`` given as lists of
-R recordings, agent ``b`` replays recording ``recording[b]`` (``prs_ens_multi_replay_run``), still in one graph per
-frame.
+Every form runs as ticks (``prs_ens_run``, csrc/view_templates.cu): a tick is an optional twist and an optional image
+per recording, and a frame is a tick with an image.  A tick is one CUDA graph for the whole ensemble: one pose-cell
+update of all B networks, one query per recording, one sweep over every agent's library, then the per-agent
+create-or-match decision and injection.
 
 ``EnsembleSession`` keeps the agents on the device between calls and feeds them recordings in pieces: bags streamed
 in chunks, recordings longer than 65535 frames, or a second run of a route continuing the maps of the first.
@@ -32,8 +33,8 @@ from . import experience_ensemble as xens
 from .experience_map import ExperienceMap
 from .kernels import PC_GLOBAL_INHIB
 from .posecell_network import PoseCellEnsemble, _as_np_dtype
-from .ros_simulate import (IM_SIZE, MATCH_THRESHOLD, POSE_SIZE, X_RANGE, X_STEP, Y_RANGE, Y_STEP, RatslamRos,
-                           key_scores)
+from .ros_simulate import (IM_SIZE, MATCH_THRESHOLD, ODOM_FREQ, POSE_SIZE, X_RANGE, X_STEP, Y_RANGE, Y_STEP,
+                           RatslamRos, key_scores)
 
 MAX_CAPACITY = 1 << 16          # templates per agent the frame's library sweep takes (kSmallLibrary)
 
@@ -124,8 +125,9 @@ def _recording_count(recording):
         return None
 
 
-def _multi_chunk(R, frame_bytes):
-    """Frames per recording in one device chunk (prs_ens_multi_scratch_bytes): 256 MiB over R recordings, in [1, 256]."""
+def _ens_chunk(R, frame_bytes):
+    """Ticks per recording in one device chunk (prs_ens_scratch_bytes): 256 MiB of images over R recordings, in
+    [1, 256]."""
     return int(min(max((256 << 20) // (R * frame_bytes), 1), 256))
 
 
@@ -225,6 +227,11 @@ def feed_inputs(frames, odom, n_recordings):
         fr.append(np.ascontiguousarray(f))
         od.append(o)
     return fr, od
+
+
+def _frame_ticks(frames, odom):
+    """Recordings of paired frames and twists as tick streams (``event_ticks``'s form): every tick has an image."""
+    return [(np.ascontiguousarray(f), o, xens.gate(o)[0], np.ones(len(f), np.bool_)) for f, o in zip(frames, odom)]
 
 
 def _is_event(x):
@@ -361,10 +368,8 @@ class EnsembleSession:
                                         dtype=torch.float64, device=dev) if injecting else None
         self._rec_dev = torch.from_numpy(rec_of[self._order].astype(np.int32)).to(dev)
         self._pc_work = torch.zeros(3 * B, dtype=torch.int64, device=dev)
-        self._scratch = torch.empty(int(L.prs_ens_scratch_bytes(B, IM_SIZE[0], IM_SIZE[1])), dtype=torch.uint8,
+        self._scratch = torch.empty(int(L.prs_ens_scratch_bytes(ens._h, R, IM_SIZE[0], IM_SIZE[1])), dtype=torch.uint8,
                                     device=dev)
-        self._mscratch = None
-        self._multi = R > 1          # the several-recordings machinery is attached (always for R > 1)
         self._stream = torch.cuda.Stream(device=dev)
         self.frames_fed = np.zeros(R, np.int64)
         self._n = np.zeros(B, np.int64)                       # templates per device row
@@ -393,17 +398,11 @@ class EnsembleSession:
         nat.check(L.prs_ens_create(
             e._h, e.state.data_ptr(), e._gi.data_ptr(), self._pc_work.data_ptr(), self._libs.data_ptr(), self.capacity,
             self._n_dev.data_ptr(), self._thr_dev.data_ptr(),
-            None if self._energy_dev is None else self._energy_dev.data_ptr(), self._loc.data_ptr(), nat.VT_MODE_REF,
-            IM_SIZE[0], IM_SIZE[1], Y_RANGE[0], Y_RANGE[1], Y_STEP, X_RANGE[0], X_RANGE[1], X_STEP,
-            self._scratch.data_ptr(), ctypes.byref(plan)), "prs_ens_create")
+            None if self._energy_dev is None else self._energy_dev.data_ptr(), self._loc.data_ptr(), self.R,
+            self._rec_dev.data_ptr(), nat.VT_MODE_REF, IM_SIZE[0], IM_SIZE[1], Y_RANGE[0], Y_RANGE[1], Y_STEP,
+            X_RANGE[0], X_RANGE[1], X_STEP, self._scratch.data_ptr(), ctypes.byref(plan)), "prs_ens_create")
         self._plan = plan
         self._room = self.capacity - int(self._n.max())
-        if self._multi:
-            if self._mscratch is None:
-                self._mscratch = torch.empty(int(L.prs_ens_multi_scratch_bytes(plan, self.R)), dtype=torch.uint8,
-                                             device=self._dev)
-            nat.check(L.prs_ens_set_recordings(plan, self.R, self._rec_dev.data_ptr(), self._mscratch.data_ptr()),
-                      "prs_ens_set_recordings")
 
     def _grow(self, cap):
         """Libraries of ``cap`` templates: a larger library is the old one with groups appended, so each agent's row is
@@ -432,131 +431,24 @@ class EnsembleSession:
         if self._closed:
             raise RuntimeError("EnsembleSession: the session is closed")
         fr, od = feed_inputs(frames, odom, self.R)
-        R, B = self.R, self.B
-        lengths = np.array([len(f) for f in fr], dtype=np.int64)
-        T = int(lengths.max())
-        moved = np.zeros((T, R), np.uint8)             # past a recording's end: not moved
-        tw = np.zeros((T, R, 2))
-        for r in range(R):
-            moved[:lengths[r], r], tw[:lengths[r], r] = xens.gate(od[r])
-        res = np.zeros((T, B), dtype=RatslamRos._RESULT_DTYPE)     # device rows
-        if self._linked:
-            n_exp = np.zeros((T, B), np.int32)
-            exp_id = np.zeros((T, B), np.int32)
-            em_xy = np.zeros((T, B, 2))
-        try:
-            with torch.cuda.device(self._dev):
-                s0 = 0
-                while s0 < T:
-                    cap, run = grow_capacity(self.capacity, int(self._n.max()), T - s0)
-                    if run == 0:
-                        d = int(np.argmax(self._n))
-                        raise ValueError("EnsembleSession: agent %d holds %d templates, the most the library sweep "
-                                         "takes, and frame %d of its recording remains"
-                                         % (self._order[d], self._n[d],
-                                            self.frames_fed[self._rec_of[self._order[d]]] + s0))
-                    if cap != self.capacity:
-                        self._grow(cap)
-                    if self._room < run:     # the plan counted earlier runs' frames, not their templates
-                        nat.check(nat.lib().prs_ens_refresh_room(self._plan, ctypes.c_void_p(self._stream.cuda_stream)),
-                                  "prs_ens_refresh_room")
-                        self._room = self.capacity - int(self._n.max())
-                    sub = slice(s0, s0 + run)
-                    self._replay(fr, tw[sub], moved[sub], lengths, s0, run, res[sub])
-                    self._room -= run
-                    self._n = res["n_templates"][s0 + run - 1].astype(np.int64)
-                    if self._linked:
-                        sub_len = np.clip(lengths - s0, 0, run)
-                        tpl = res["template_index"][sub]
-                        tag = np.empty((run, B), np.int32)
-                        tag[0] = self._prev_tpl
-                        tag[1:] = np.maximum(tpl[:-1], -1)
-                        mine = sub_len[self._rec_of[self._order]]        # per device row: its frames in this sub-run
-                        here = mine > 0
-                        self._prev_tpl[here] = tpl[mine[here] - 1, np.nonzero(here)[0]]
-                        self._maps(res[sub], tag, run, tw[sub], moved[sub], n_exp[sub], exp_id[sub], em_xy[sub])
-                    s0 += run
-        except BaseException:
-            self.close()
-            raise
-        self.frames_fed += lengths
-        inv = self._rows
-        res = res[:, inv]
-        length = lengths[self._rec_of]
-        past = np.arange(T)[None, :] >= length[:, None]  # [B, T]
-        argmax = _unravel(res["argmax"].T, self.pose_size)
-        argmax[past] = -1
-        score = key_scores(res["key"].T)
-        score[past] = -1
-        out = {"template": res["template_index"].T.astype(np.int64), "created": res["created"].T != 0,
-               "score": score, "argmax": argmax, "n_templates": self.n_templates, "length": length}
-        if self._map:
-            if self._linked:
-                out["n_exp"] = n_exp[:, inv].T.astype(np.int64)
-                out["exp_id"] = exp_id[:, inv].T.astype(np.int64)
-                out["em_xy"] = em_xy[:, inv].transpose(1, 0, 2)
-                for r in range(R):       # the recording's accumulators, for maps.experience_map(b)
-                    self._dead_reckoning(r, moved[:, r], tw[:, r], lengths[r])
-            else:
-                per = [self._dead_reckoning(r, moved[:, r], tw[:, r], lengths[r]) for r in range(R)]
-                out["n_exp"] = np.stack([per[r][0] for r in self._rec_of])
-                out["em_xy"] = np.stack([per[r][1] for r in self._rec_of])
-                out["exp_id"] = out["n_exp"] - 1
-            out["n_loop_closures"] = self.n_loop_closures
-            out["n_exp"][past] = -1
-            out["exp_id"][past] = -1
-            out["em_xy"][past] = np.nan
-        return out
-
-    def _replay(self, fr, tw, moved, lengths, s0, run, res):
-        """Frames [s0, s0 + run) of the feed through the plan; raises a pose-cell error as replay_ensemble does."""
-        L = nat.lib()
-        stream = ctypes.c_void_p(self._stream.cuda_stream)
-        if self.R == 1:
-            tw1, mv1 = np.ascontiguousarray(tw[:, 0]), np.ascontiguousarray(moved[:, 0])
-            nat.check(L.prs_ens_replay_run(self._plan, fr[0].ctypes.data + s0 * IM_SIZE[0] * IM_SIZE[1], tw1.ctypes.data,
-                                           mv1.ctypes.data, run, res.ctypes.data, stream), "prs_ens_replay_run")
-            bad = np.nonzero((((res["pc_err"] & ~nat.ERR_INJECT_LOC) != 0) & (mv1[:, None] != 0)).any(axis=1))[0]
-            if len(bad):
-                self._ens._raise_on_err(np.asarray(res["pc_err"][int(bad[0])] & ~nat.ERR_INJECT_LOC, dtype=np.int32))
-            return
-        sub_len = np.clip(lengths - s0, 0, run).astype(np.int32)
-        ptrs = (ctypes.c_void_p * self.R)(*[fr[r].ctypes.data + s0 * IM_SIZE[0] * IM_SIZE[1] if sub_len[r] else None
-                                            for r in range(self.R)])
-        tw, moved = np.ascontiguousarray(tw), np.ascontiguousarray(moved)
-        nat.check(L.prs_ens_multi_replay_run(self._plan, ptrs, tw.ctypes.data, moved.ctypes.data, sub_len.ctypes.data,
-                                             run, res.ctypes.data, stream), "prs_ens_multi_replay_run")
-        rc = res[:, self._rows]
-        bad = ((rc["pc_err"] & ~nat.ERR_INJECT_LOC) != 0) & (moved[:, self._rec_of] != 0)
-        if bad.any():
-            t, b = np.argwhere(bad)[0]                  # frame-major: the earliest frame, then the lowest agent
-            self._ens._raise_on_err(np.array([rc["pc_err"][t, b] & ~nat.ERR_INJECT_LOC], dtype=np.int32))
-
-    def _attach_multi(self):
-        """The several-recordings machinery for a session of one recording, at its first ``feed_events``; ``feed`` keeps
-        using the single-recording frames."""
-        L = nat.lib()
-        self._multi = True
-        self._mscratch = torch.empty(int(L.prs_ens_multi_scratch_bytes(self._plan, self.R)), dtype=torch.uint8,
-                                     device=self._dev)
-        nat.check(L.prs_ens_set_recordings(self._plan, self.R, self._rec_dev.data_ptr(), self._mscratch.data_ptr()),
-                  "prs_ens_set_recordings")
+        return self._feed_ticks(_frame_ticks(fr, od), "frame")
 
     def feed_events(self, events):
         """Replay the next messages of every recording the way the node's message loop does
         (``ros_simulate.replay_events``): one pose-cell update and one experience-map update per gated odometry message,
         one match per image.  ``events`` is a message stream (``rosbag_io.read_events``, or a piece of ``iter_events``)
         for R = 1 and a list of R streams otherwise, any of them empty; a piece may end anywhere, inside a run of
-        odometry too.  The streams are compacted into ticks (``event_ticks``) and replayed with
-        ``prs_ens_events_run``.  Returns per image: ``template``, ``created``, ``score``, ``argmax`` ``[B, i_max]``,
+        odometry too.  The streams are compacted into ticks (``event_ticks``).  Returns per image: ``template``, ``created``, ``score``, ``argmax`` ``[B, i_max]``,
         ``length [B]`` (the images of the agent's recording in this feed; -1 / False past it), ``n_templates [B]``, and
         with ``experience_map="device"`` ``n_exp``, ``exp_id``, ``em_xy`` at each image (-1 / NaN past the length) and
         ``n_loop_closures``.  ``feed`` and ``feed_events`` continue the same agents, libraries and maps."""
         if self._closed:
             raise RuntimeError("EnsembleSession: the session is closed")
-        return self._feed_ticks(event_streams(events, self.R))
+        return self._feed_ticks(event_streams(events, self.R), "image")
 
-    def _feed_ticks(self, streams):
+    def _feed_ticks(self, streams, unit="image"):
+        """The feed of R tick streams (``event_ticks``'s form) with the result of ``feed_events``: per image, ``unit``
+        ("frame" or "image") naming one in the error of a full library."""
         R, B = self.R, self.B
         n_ticks = np.array([len(st[2]) for st in streams], dtype=np.int64)
         n_img = np.array([len(st[0]) for st in streams], dtype=np.int64)
@@ -564,8 +456,9 @@ class EnsembleSession:
         moved = np.zeros((K, R), np.uint8)             # past a recording's ticks: no update, no image
         tw = np.zeros((K, R, 2))
         img = np.zeros((K, R), np.bool_)
-        for r, (_, od, _, im) in enumerate(streams):
-            moved[:n_ticks[r], r], tw[:n_ticks[r], r] = xens.gate(od)
+        for r, (_, od, mv, im) in enumerate(streams):
+            moved[:n_ticks[r], r] = mv
+            tw[:n_ticks[r], r] = od / float(ODOM_FREQ)                 # the twist given to update(), as xens.gate
             img[:n_ticks[r], r] = im
         gate = np.ascontiguousarray(img.astype(np.uint8) | (moved << 1))
         img_tick = img.any(axis=1)
@@ -578,8 +471,6 @@ class EnsembleSession:
         first = np.zeros(R, np.int64)                  # per recording: its first image of the sub-run
         try:
             with torch.cuda.device(self._dev):
-                if not self._multi:
-                    self._attach_multi()
                 k0 = 0
                 while k0 < K:
                     left = int(img_tick[k0:].sum())
@@ -587,8 +478,9 @@ class EnsembleSession:
                     if run == 0 and left:
                         d = int(np.argmax(self._n))
                         raise ValueError("EnsembleSession: agent %d holds %d templates, the most the library sweep "
-                                         "takes, and image %d of its recording remains"
-                                         % (self._order[d], self._n[d], self.frames_fed[rec_rows[d]] + first[rec_rows[d]]))
+                                         "takes, and %s %d of its recording remains"
+                                         % (self._order[d], self._n[d], unit,
+                                            self.frames_fed[rec_rows[d]] + first[rec_rows[d]]))
                     if cap != self.capacity:
                         self._grow(cap)
                     # ticks [k0, k1) hold `run` ticks with images; the last sub-run takes the trailing odometry
@@ -599,7 +491,7 @@ class EnsembleSession:
                         self._room = self.capacity - int(self._n.max())
                     sub = slice(k0, k1)
                     sub_img = img[sub].sum(axis=0)
-                    self._replay_events(streams, first, sub_img, tw[sub], moved[sub], gate[sub], res[sub])
+                    self._run(streams, first, sub_img, tw[sub], moved[sub], gate[sub], res[sub])
                     self._room -= int(img_tick[sub].sum())
                     self._n = res["n_templates"][k1 - 1].astype(np.int64)
                     if self._linked:
@@ -614,53 +506,60 @@ class EnsembleSession:
         self.frames_fed += n_img
         length = n_img[self._rec_of]
         i_max = int(n_img.max())
+        # built in device rows, where each recording's agents are one slice, and put in the caller's order at the end
         out = {"template": np.full((B, i_max), -1, np.int64), "created": np.zeros((B, i_max), np.bool_),
-               "score": np.full((B, i_max), -1, np.int64), "argmax": np.full((B, i_max, 3), -1, np.int64),
-               "n_templates": self.n_templates, "length": length}
+               "score": np.full((B, i_max), -1, np.int64), "argmax": np.full((B, i_max, 3), -1, np.int64)}
         if self._map:
             out["n_exp"] = np.full((B, i_max), -1, np.int64)
             out["exp_id"] = np.full((B, i_max), -1, np.int64)
             out["em_xy"] = np.full((B, i_max, 2), np.nan)
         for r in range(R):
+            d = slice(*np.searchsorted(rec_rows, [r, r + 1]))
             ticks = np.nonzero(img[:, r])[0]
-            agents = np.nonzero(self._rec_of == r)[0]
-            cols = self._rows[agents]
             m = len(ticks)
-            out["template"][agents, :m] = res["template_index"][ticks][:, cols].T
-            out["created"][agents, :m] = res["created"][ticks][:, cols].T != 0
-            out["score"][agents, :m] = key_scores(res["key"][ticks][:, cols].T)
-            out["argmax"][agents, :m] = _unravel(res["argmax"][ticks][:, cols].T, self.pose_size)
+            at = slice(0, m) if m == 0 or ticks[-1] == m - 1 else ticks    # a frame feed's images: the first m ticks
+            sel = res[at, d]
+            out["template"][d, :m] = sel["template_index"].T
+            out["created"][d, :m] = sel["created"].T != 0
+            out["score"][d, :m] = key_scores(sel["key"].T)
+            out["argmax"][d, :m] = _unravel(sel["argmax"].T, self.pose_size)
             if self._linked:
-                out["n_exp"][agents, :m] = n_exp[ticks][:, cols].T
-                out["exp_id"][agents, :m] = exp_id[ticks][:, cols].T
-                out["em_xy"][agents, :m] = em_xy[ticks][:, cols].transpose(1, 0, 2)
+                out["n_exp"][d, :m] = n_exp[at, d].T
+                out["exp_id"][d, :m] = exp_id[at, d].T
+                out["em_xy"][d, :m] = em_xy[at, d].transpose(1, 0, 2)
             if self._map:
                 n_r, xy_r = self._dead_reckoning(r, moved[:, r], tw[:, r], n_ticks[r])
                 if not self._linked:
-                    out["n_exp"][agents, :m] = n_r[ticks]
-                    out["exp_id"][agents, :m] = n_r[ticks] - 1
-                    out["em_xy"][agents, :m] = xy_r[ticks]
+                    out["n_exp"][d, :m] = n_r[ticks]
+                    out["exp_id"][d, :m] = n_r[ticks] - 1
+                    out["em_xy"][d, :m] = xy_r[ticks]
+        if not (self._order == np.arange(B)).all():
+            out = {k: v[self._rows] for k, v in out.items()}
+        out["n_templates"], out["length"] = self.n_templates, length
         if self._map:
             out["n_loop_closures"] = self.n_loop_closures
         return out
 
-    def _replay_events(self, streams, first, sub_img, tw, moved, gate, res):
-        """One sub-run of ticks through ``prs_ens_events_run``; raises a pose-cell error as ``replay_events`` does, for
-        the earliest tick and, within it, the lowest agent."""
+    def _run(self, streams, first, sub_img, tw, moved, gate, res):
+        """One sub-run of ticks through ``prs_ens_run``.  A pose-cell error raises what the native replay raises, for
+        the earliest tick: with one recording, with the bits of every agent at it (they share the odometry), else for
+        the lowest agent at it."""
         L = nat.lib()
         fb = IM_SIZE[0] * IM_SIZE[1]
         ptrs = (ctypes.c_void_p * self.R)(*[streams[r][0].ctypes.data + int(first[r]) * fb if sub_img[r] else None
                                             for r in range(self.R)])
         tw, n_images = np.ascontiguousarray(tw), np.ascontiguousarray(sub_img, dtype=np.int32)
-        nat.check(L.prs_ens_events_run(self._plan, ptrs, tw.ctypes.data, gate.ctypes.data, n_images.ctypes.data,
-                                       len(gate), res.ctypes.data, ctypes.c_void_p(self._stream.cuda_stream)),
-                  "prs_ens_events_run")
-        if not (((res["pc_err"] & ~nat.ERR_INJECT_LOC) != 0) & (moved[:, self._rec_of[self._order]] != 0)).any():
+        nat.check(L.prs_ens_run(self._plan, ptrs, tw.ctypes.data, gate.ctypes.data, n_images.ctypes.data, len(gate),
+                                res.ctypes.data, ctypes.c_void_p(self._stream.cuda_stream)), "prs_ens_run")
+        err = res["pc_err"] & ~nat.ERR_INJECT_LOC                            # device rows
+        bad = (err != 0) & (moved[:, self._rec_of[self._order]] != 0)
+        if not bad.any():
             return
-        rc = res[:, self._rows]
-        bad = ((rc["pc_err"] & ~nat.ERR_INJECT_LOC) != 0) & (moved[:, self._rec_of] != 0)
-        t, b = np.argwhere(bad)[0]
-        self._ens._raise_on_err(np.array([rc["pc_err"][t, b] & ~nat.ERR_INJECT_LOC], dtype=np.int32))
+        t = int(np.nonzero(bad.any(axis=1))[0][0])
+        if self.R == 1:
+            self._ens._raise_on_err(err[t].astype(np.int32))
+        d = self._rows[np.nonzero(bad[t, self._rows])[0][0]]
+        self._ens._raise_on_err(err[t, d:d + 1].astype(np.int32))
 
     def _event_tags(self, res, img):
         """``tag [K,B]`` of one sub-run of ticks (device rows): the template of the agent's most recent image before
@@ -802,14 +701,9 @@ def replay_ensemble(frames, odom, n_agents=None, match_threshold=MATCH_THRESHOLD
     if not (isinstance(experience_map, (bool, np.bool_))
             or (isinstance(experience_map, str) and experience_map == "device")):
         raise ValueError("experience_map must be False, True or 'device', got %r" % (experience_map,))
-    B, thr, gi, energies = agent_parameters(n_agents if n_agents is not None else _recording_count(recording),
-                                            match_threshold, global_inhibition, inject_energy)
-    if mode != "ref":
-        raise ValueError("replay_ensemble supports the reference matching mode only, got mode=%r" % (mode,))
     several = isinstance(frames, (list, tuple)) and (len(frames) == 0 or np.ndim(frames[0]) == 3)
     if several:
         R = len(frames)
-        rec_of = agent_recordings(recording, B, max(R, 1))
         if not isinstance(odom, (list, tuple)) or len(odom) != R or R == 0:
             raise ValueError("replay_ensemble: frames and odom must be lists of the same, non-zero number of "
                              "recordings, got %d and %s"
@@ -820,54 +714,27 @@ def replay_ensemble(frames, odom, n_agents=None, match_threshold=MATCH_THRESHOLD
             if f.dtype != np.uint8 or f.ndim != 3 or tuple(f.shape[1:]) != IM_SIZE or o.shape != (len(f), 2):
                 raise ValueError("replay_ensemble: recording %d: frames must be uint8 [T,%d,%d] and odom [T,2], got %s "
                                  "%r and %r" % (r, IM_SIZE[0], IM_SIZE[1], f.dtype, f.shape, o.shape))
-            fr.append(np.ascontiguousarray(f))
+            fr.append(f)
             od.append(o)
-        T = max(len(f) for f in fr)
     else:
-        rec_of = agent_recordings(recording, B, 1)
-        fr, od = [np.asarray(frames)], [np.asarray(odom, dtype=np.float64)]
-        T = len(fr[0])
-        if fr[0].dtype != np.uint8 or fr[0].ndim != 3 or tuple(fr[0].shape[1:]) != IM_SIZE or od[0].shape != (T, 2):
+        f, o = np.asarray(frames), np.asarray(odom, dtype=np.float64)
+        if f.dtype != np.uint8 or f.ndim != 3 or tuple(f.shape[1:]) != IM_SIZE or o.shape != (len(f), 2):
             raise ValueError("replay_ensemble: frames must be uint8 [T,%d,%d] and odom [T,2], got %s %r and %r"
-                             % (IM_SIZE[0], IM_SIZE[1], fr[0].dtype, fr[0].shape, od[0].shape))
-        R = 1
-    pose_size = tuple(int(s) for s in pose_size)
-    np_dtype = _as_np_dtype(dtype)
-    cap = capacity_for(T)
-    if cap > MAX_CAPACITY:
+                             % (IM_SIZE[0], IM_SIZE[1], f.dtype, f.shape, o.shape))
+        fr, od = [f], [o]
+    R = len(fr)
+    T = max(len(f) for f in fr)
+    if capacity_for(T) > MAX_CAPACITY:
         raise ValueError("replay_ensemble: %d frames need %d templates per agent; the library sweep takes at most %d"
-                         % (T, cap, MAX_CAPACITY))
-    lib_bytes = (cap // 32) * 34816
-    net_bytes = int(np.prod(pose_size)) * np.dtype(np_dtype).itemsize
-    if several:
-        frame_bytes = IM_SIZE[0] * IM_SIZE[1]
-        # per agent: library, locations, network, its snapshot and the records; plus one chunk of every recording's
-        # frames
-        need = B * (lib_bytes + cap * 8 + 2 * net_bytes + 64) + R * _multi_chunk(R, frame_bytes) * frame_bytes
-    else:
-        need = B * (lib_bytes + cap * 8 + net_bytes + 64)
-    if experience_map == "device" and experience_links:
-        need += xens.work_bytes(B, T, cap) + xens.record_bytes(B, T)
-    nat.require_cuda()
-    dev = torch.device("cuda", torch.cuda.current_device())
-    free, _ = torch.cuda.mem_get_info(dev)
-    if need > free:
-        raise ValueError("replay_ensemble: %d agents x %d templates need %.2f GB of device memory, %.2f GB are free"
-                         % (B, cap, need / 1e9, free / 1e9))
-
-    session = EnsembleSession(B, thr, gi, energies, pose_size, np_dtype, active_set,
-                              "device" if experience_map == "device" else False, experience_links, R, rec_of, cap)
-    try:
-        out = session.feed(fr if R > 1 else fr[0], od if R > 1 else od[0])
-        out["agents"] = session.agents
-        if experience_map == "device":
-            out["maps"] = session.maps
-    finally:
-        session.close()
+                         % (T, capacity_for(T), MAX_CAPACITY))
+    out, rec_of = _replay_once("replay_ensemble", _frame_ticks(fr, od), n_agents, recording, match_threshold,
+                               global_inhibition, inject_energy, pose_size, dtype, active_set,
+                               "device" if experience_map == "device" else False, experience_links, mode)
     if isinstance(experience_map, (bool, np.bool_)) and experience_map:
         moved, tw = np.zeros((T, R), np.uint8), np.zeros((T, R, 2))
         for r in range(R):
             moved[:len(fr[r]), r], tw[:len(fr[r]), r] = xens.gate(od[r])
+        pose_size = tuple(int(s) for s in pose_size)
         if several:
             out["n_exp"], out["em_xy"] = _experience_maps(out, moved, tw, pose_size, experience_links, rec_of)
             past = np.arange(T)[None, :] >= out["length"][:, None]
@@ -897,14 +764,24 @@ def replay_ensemble_events(events, n_agents=None, match_threshold=MATCH_THRESHOL
             or (isinstance(experience_map, str) and experience_map == "device")):
         raise ValueError("replay_ensemble_events: experience_map must be False or 'device' (the host maps need the "
                          "paired frames of replay_ensemble), got %r" % (experience_map,))
+    several = (isinstance(events, (list, tuple)) and len(events) > 0 and not _is_event(events[0]))
+    streams = [event_ticks(st) for st in events] if several else [event_ticks(events)]
+    return _replay_once("replay_ensemble_events", streams, n_agents, recording, match_threshold, global_inhibition,
+                        inject_energy, pose_size, dtype, active_set, experience_map, experience_links, mode)[0]
+
+
+def _replay_once(who, streams, n_agents, recording, match_threshold, global_inhibition, inject_energy, pose_size,
+                 dtype, active_set, experience_map, experience_links, mode):
+    """``replay_ensemble`` and ``replay_ensemble_events`` after their inputs are validated: the agents' parameters and
+    recordings are broadcast and validated and the device memory is checked before any other CUDA call, then one
+    ``EnsembleSession`` with libraries for every image is fed the R tick streams once.  Returns the feed's result with
+    ``agents`` (and ``maps`` for ``experience_map="device"``), and the agents' recordings."""
     B, thr, gi, energies = agent_parameters(n_agents if n_agents is not None else _recording_count(recording),
                                             match_threshold, global_inhibition, inject_energy)
     if mode != "ref":
-        raise ValueError("replay_ensemble_events supports the reference matching mode only, got mode=%r" % (mode,))
-    several = (isinstance(events, (list, tuple)) and len(events) > 0 and not _is_event(events[0]))
-    R = len(events) if several else 1
+        raise ValueError("%s supports the reference matching mode only, got mode=%r" % (who, mode))
+    R = len(streams)
     rec_of = agent_recordings(recording, B, R)
-    streams = [event_ticks(st) for st in events] if several else [event_ticks(events)]
     pose_size = tuple(int(s) for s in pose_size)
     np_dtype = _as_np_dtype(dtype)
     K = max(len(st[2]) for st in streams)
@@ -912,19 +789,21 @@ def replay_ensemble_events(events, n_agents=None, match_threshold=MATCH_THRESHOL
     for r, st in enumerate(streams):
         img[:len(st[3]), r] = st[3]
     cap = min(capacity_for(int(img.any(axis=1).sum())), MAX_CAPACITY)
-    lib_bytes = (cap // 32) * 34816
-    net_bytes = int(np.prod(pose_size)) * np.dtype(np_dtype).itemsize
-    # per agent: library, locations, network, its snapshot and the records; plus one chunk of every recording's images
+    # what the session allocates: per agent its library, template locations, network, the network's snapshot of a
+    # mixed tick (R > 1 only), a chunk of records and a few scalars; one chunk of every recording's images
     frame_bytes = IM_SIZE[0] * IM_SIZE[1]
-    need = B * (lib_bytes + cap * 8 + 2 * net_bytes + 64) + R * _multi_chunk(R, frame_bytes) * frame_bytes
+    chunk = _ens_chunk(R, frame_bytes)
+    net_bytes = int(np.prod(pose_size)) * np.dtype(np_dtype).itemsize
+    need = (B * ((cap // 32) * 34816 + cap * 8 + (2 if R > 1 else 1) * net_bytes + chunk * 32 + 128)
+            + R * chunk * frame_bytes)
     if experience_map == "device" and experience_links:
         need += xens.work_bytes(B, K, cap) + xens.record_bytes(B, K)
     nat.require_cuda()
     dev = torch.device("cuda", torch.cuda.current_device())
     free, _ = torch.cuda.mem_get_info(dev)
     if need > free:
-        raise ValueError("replay_ensemble_events: %d agents x %d templates need %.2f GB of device memory, %.2f GB are "
-                         "free" % (B, cap, need / 1e9, free / 1e9))
+        raise ValueError("%s: %d agents x %d templates need %.2f GB of device memory, %.2f GB are free"
+                         % (who, B, cap, need / 1e9, free / 1e9))
     session = EnsembleSession(B, thr, gi, energies, pose_size, np_dtype, active_set, experience_map, experience_links,
                               R, rec_of, cap)
     try:
@@ -934,7 +813,7 @@ def replay_ensemble_events(events, n_agents=None, match_threshold=MATCH_THRESHOL
             out["maps"] = session.maps
     finally:
         session.close()
-    return out
+    return out, rec_of
 
 
 def _experience_maps(out, moved, tw, pose_size, linked, rec_of=None):
