@@ -433,6 +433,22 @@ PRS_API int prs_ens_refresh_room(prs_ens_plan* plan, void* stream);
  * non-default stream).  PRS_E_INVALID when the libraries have no room for the ticks with an image. */
 PRS_API int prs_ens_run(prs_ens_plan* plan, const uint8_t* const* frames, const double* odom, const uint8_t* gate,
                 const int* n_images, int T, prs_frame_result* results, void* stream);
+/* Agent copies between a plan's rows (an ensemble session's reassignment of agents): move m makes row dst[m] an exact
+ * copy of row src[m] as it was before the call -- the state slice, the pc_work slots, n_dev, the library groups of its
+ * n_dev templates and the first n_dev entries of its location row.  Slots past n_dev are never read and an append
+ * writes its slot whole, so nothing past the copied templates is cleared.  A source that is itself a destination (a
+ * swap, a cycle) is gathered into the stage before any row is written; the others are read in place.  Work follows
+ * the live bytes: the kernels copy the source's live groups, not the capacity.  The thresholds, inhibitions and
+ * energies the plan reads are the caller's to rewrite.
+ *   dst, src     : host int32 [n_moves], rows in [0, B); the dst distinct, no src equal to its dst
+ *   n_templates  : host int32 [B], every row's template count as n_dev holds it (sizes the stage)
+ *   stage        : device, prs_ens_copy_stage_bytes(...) bytes for these moves (a pair table and the gathered rows)
+ * Asynchronous on `stream`, which also receives prs_pc_invalidate_active's reset; the next prs_ens_run on any stream
+ * must be ordered after it.  prs_ens_copy_stage_bytes returns 0 for invalid moves. */
+PRS_API size_t prs_ens_copy_stage_bytes(prs_ens_plan* plan, int n_moves, const int* dst, const int* src,
+                                const int* n_templates);
+PRS_API int prs_ens_copy_agents(prs_ens_plan* plan, int n_moves, const int* dst, const int* src, const int* n_templates,
+                        void* stage, size_t stage_bytes, void* stream);
 
 /* ------------------------------------------------------- ensemble experience maps */
 
@@ -492,6 +508,16 @@ PRS_API int prs_em_session_grow(int B, int E0, int N0, int E1, int N1, const voi
 PRS_API int prs_em_linked_resume_run(int B, int T, int E, int N, const long long* argmax, const int* tag, int R,
                              const double* tw, const uint8_t* moved, const int* rec_of, int X, int Y, int Th,
                              double delta_pc, void* work, int* n_exp, int* exp_id, double* em_xy, void* stream);
+/* The same agent copies for a session workspace (B, E, N): column dst[m] receives column src[m]'s experiences and links
+ * below its counts, all N rows of vt_head, rel and the counts (loop closures included).  Rows at or past the counts are
+ * never read, so the destination's are not cleared.  Overwritten sources are staged as in prs_ens_copy_agents.
+ *   n_rows : host int32 [B], max(experiences, links) of every column, at most E (sizes the stage)
+ *   stage  : device, prs_em_session_copy_stage_bytes(...) bytes for these moves
+ * Asynchronous on `stream`.  prs_em_session_copy_stage_bytes returns 0 for invalid moves. */
+PRS_API size_t prs_em_session_copy_stage_bytes(int B, int E, int N, int n_moves, const int* dst, const int* src,
+                                       const int* n_rows);
+PRS_API int prs_em_session_copy_agents(int B, int E, int N, void* work, int n_moves, const int* dst, const int* src,
+                               const int* n_rows, void* stage, size_t stage_bytes, void* stream);
 
 #ifdef __cplusplus
 }

@@ -101,6 +101,9 @@ _SIGNATURES["prs_ens_create"] = (c_int, [c_void_p, c_void_p, c_void_p, c_void_p,
 _SIGNATURES["prs_ens_destroy"] = (c_int, [c_void_p])
 _SIGNATURES["prs_ens_refresh_room"] = (c_int, [c_void_p, c_void_p])
 _SIGNATURES["prs_ens_run"] = (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p])
+_SIGNATURES["prs_ens_copy_stage_bytes"] = (c_size_t, [c_void_p, c_int, c_void_p, c_void_p, c_void_p])
+_SIGNATURES["prs_ens_copy_agents"] = (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t,
+                                              c_void_p])
 _SIGNATURES["prs_em_work_bytes"] = (c_size_t, [c_int, c_int, c_int])
 _SIGNATURES["prs_em_linked_run"] = (c_int, [c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int,
                                             c_int, c_double, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p])
@@ -110,6 +113,9 @@ _SIGNATURES["prs_em_linked_multi_run"] = (c_int, [c_int, c_int, c_int, c_void_p,
 _SIGNATURES["prs_em_session_bytes"] = (c_size_t, [c_int, c_int, c_int])
 _SIGNATURES["prs_em_session_init"] = (c_int, [c_int, c_int, c_int, c_void_p, c_void_p])
 _SIGNATURES["prs_em_session_grow"] = (c_int, [c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p])
+_SIGNATURES["prs_em_session_copy_stage_bytes"] = (c_size_t, [c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p])
+_SIGNATURES["prs_em_session_copy_agents"] = (c_int, [c_int, c_int, c_int, c_void_p, c_int, c_void_p, c_void_p, c_void_p,
+                                                     c_void_p, c_size_t, c_void_p])
 _SIGNATURES["prs_em_linked_resume_run"] = (c_int, [c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_int, c_void_p,
                                                    c_void_p, c_void_p, c_int, c_int, c_int, c_double, c_void_p, c_void_p,
                                                    c_void_p, c_void_p, c_void_p])

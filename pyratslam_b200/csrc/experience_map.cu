@@ -12,6 +12,7 @@
 // and the link headings, never a decision.
 #include <math.h>
 
+#include "agent_moves.cuh"
 #include "common.cuh"
 
 namespace {
@@ -291,5 +292,132 @@ extern "C" int prs_em_linked_resume_run(int B, int T, int E, int N, const long l
       B, T, N, argmax, tag, tw, moved, X, Y, Th, delta_pc, em_work(work, L), n_exp, exp_id, em_xy, R, rec_of, E,
       (int*)((char*)work + L.bytes));
   PRS_CUDA(cudaGetLastError());
+  return PRS_OK;
+}
+
+// ---------------------------------------------------------------------------------------------
+// Agent copies inside a session workspace (prs_em_session_copy_agents, EnsembleSession.reassign): column d receives
+// column s's experiences and links below its counts, all N rows of vt_head, rel and counts.  Rows at or past the counts
+// are never read -- every list (vt_head, exp_next, out_head, link_next) points below them and a new experience or link
+// writes its row whole -- so the destination's stale rows need no clearing.  The stage is a workspace of K columns with
+// `rows` rows, the most experiences or links any gathered column holds.
+namespace {
+
+// array a of a workspace: 0-6 the experience arrays, 7-12 the link arrays, 13 vt_head, 14 rel, 15 counts
+__device__ __forceinline__ char* em_array(const EmWork& w, int a, int& es) {
+  es = 8;
+  switch (a) {
+    case 0: return (char*)w.exp_x;
+    case 1: return (char*)w.exp_y;
+    case 2: return (char*)w.exp_th;
+    case 3: return (char*)w.exp_cell;
+    case 4: es = 4; return (char*)w.exp_tag;
+    case 5: es = 4; return (char*)w.exp_next;
+    case 6: es = 4; return (char*)w.out_head;
+    case 7: return (char*)w.link_d;
+    case 8: return (char*)w.link_heading;
+    case 9: return (char*)w.link_facing;
+    case 10: es = 4; return (char*)w.link_from;
+    case 11: es = 4; return (char*)w.link_to;
+    case 12: es = 4; return (char*)w.link_next;
+    case 13: es = 4; return (char*)w.vt_head;
+    case 14: return (char*)w.rel;
+    default: es = 4; return (char*)w.counts;
+  }
+}
+
+// Pair p copies column pairs[p] of `src` (src_cols columns) into column pairs[n_pairs + p] of `dst` (dst_cols
+// columns); thread (row j, pair p), pairs fastest, so a row's neighbouring destinations are written together.  Row j
+// runs over 7 x `rows` experience rows, 6 x `rows` link rows, N vt_head rows, 3 rel and 4 count rows; rows at or past
+// the source's counts return at once.  No pair's destination is another pair's source within one launch.
+__global__ void __launch_bounds__(256)
+    k_em_copy_cols(EmWork src, int src_cols, EmWork dst, int dst_cols, const int* __restrict__ pairs, int n_pairs,
+                   int rows, int N) {
+  const long long total = ((long long)13 * rows + N + 7) * n_pairs;
+  for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < total;
+       idx += (long long)gridDim.x * blockDim.x) {
+    const int p = (int)(idx % n_pairs);
+    long long j = idx / n_pairs;
+    const int s = pairs[p], d = pairs[n_pairs + p];
+    int a, i;
+    if (j < 13LL * rows) {
+      a = (int)(j / rows), i = (int)(j % rows);
+      if (i >= src.counts[(a < 7 ? 0 : 1) * (size_t)src_cols + s]) continue;
+    } else if ((j -= 13LL * rows) < N) {
+      a = 13, i = (int)j;
+    } else if ((j -= N) < 3) {
+      a = 14, i = (int)j;
+    } else {
+      a = 15, i = (int)j - 3;
+    }
+    int es;
+    const char* from = em_array(src, a, es);
+    char* to = em_array(dst, a, es);
+    const size_t si = (size_t)i * src_cols + s, di = (size_t)i * dst_cols + d;
+    if (es == 8)
+      ((long long*)to)[di] = ((const long long*)from)[si];
+    else
+      ((int*)to)[di] = ((const int*)from)[si];
+  }
+}
+
+}  // namespace
+
+static int em_copy_plan(const char* who, int B, int E, int N, int n_moves, const int* dst, const int* src,
+                        const int* n_rows, AgentMoves& mv, int& rows) {
+  PRS_REQUIRE(B >= 1 && E >= 0 && N >= 0 && (n_moves == 0 || n_rows), "%s: bad argument B=%d E=%d N=%d", who, B, E, N);
+  if (int rc = agent_moves(who, B, n_moves, dst, src, mv)) return rc;
+  for (int m = 0; m < n_moves; ++m)
+    PRS_REQUIRE(n_rows[src[m]] >= 0 && n_rows[src[m]] <= E, "%s: column %d uses %d rows, the workspace has %d", who,
+                src[m], n_rows[src[m]], E);
+  rows = 0;
+  for (int r : mv.stage_rows) rows = std::max(rows, n_rows[r]);
+  return PRS_OK;
+}
+
+static size_t em_copy_stage_offset(const AgentMoves& mv) {
+  return (mv.table().size() * sizeof(int) + 255) / 256 * 256;
+}
+
+extern "C" size_t prs_em_session_copy_stage_bytes(int B, int E, int N, int n_moves, const int* dst, const int* src,
+                                                  const int* n_rows) {
+  AgentMoves mv;
+  int rows = 0;
+  if (em_copy_plan("prs_em_session_copy_stage_bytes", B, E, N, n_moves, dst, src, n_rows, mv, rows)) return 0;
+  return em_copy_stage_offset(mv) + (mv.K() ? EmLayout(mv.K(), rows, N).bytes : 0);
+}
+
+extern "C" int prs_em_session_copy_agents(int B, int E, int N, void* work, int n_moves, const int* dst, const int* src,
+                                          const int* n_rows, void* stage, size_t stage_bytes, void* stream) {
+  AgentMoves mv;
+  int rows = 0;
+  if (int rc = em_copy_plan("prs_em_session_copy_agents", B, E, N, n_moves, dst, src, n_rows, mv, rows)) return rc;
+  if (n_moves == 0) return PRS_OK;
+  const std::vector<int> table = mv.table();
+  const int K = mv.K();
+  const size_t off = em_copy_stage_offset(mv);
+  const size_t need = off + (K ? EmLayout(K, rows, N).bytes : 0);
+  PRS_REQUIRE(work && stage && stage_bytes >= need, "prs_em_session_copy_agents: the stage has %zu bytes, the moves need %zu",
+              stage_bytes, need);
+  const cudaStream_t st = (cudaStream_t)stream;
+  char* p = (char*)stage;
+  PRS_CUDA(cudaMemcpyAsync(p, table.data(), table.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+  const EmWork w = em_work(work, EmLayout(B, E, N));
+  const EmWork sw = em_work(p + off, EmLayout(K, rows, N));
+  int direct_rows = 0;
+  for (size_t m = 0; m < mv.direct.size() / 2; ++m) direct_rows = std::max(direct_rows, n_rows[mv.direct[m]]);
+  auto launch = [&](const EmWork& from, int from_cols, const EmWork& to, int to_cols, const int* pairs, int n_pairs,
+                    int bound) {
+    if (n_pairs == 0) return cudaSuccess;
+    const long long total = ((long long)13 * bound + N + 7) * n_pairs;
+    const long long blocks = std::min((total + 255) / 256, 148LL * 16);
+    k_em_copy_cols<<<(unsigned)blocks, 256, 0, st>>>(from, from_cols, to, to_cols, pairs, n_pairs, bound, N);
+    return cudaGetLastError();
+  };
+  const int* d_table = (const int*)p;
+  const int n_direct = (int)mv.direct.size() / 2, n_staged = (int)mv.staged.size() / 2;
+  PRS_CUDA(launch(w, B, sw, K, d_table, K, rows));
+  PRS_CUDA(launch(w, B, w, B, d_table + 2 * K, n_direct, direct_rows));
+  PRS_CUDA(launch(sw, K, w, B, d_table + 2 * K + 2 * n_direct, n_staged, rows));
   return PRS_OK;
 }

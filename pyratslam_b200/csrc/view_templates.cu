@@ -37,6 +37,7 @@
 
 #include "common.cuh"
 #include "vt_pack.cuh"
+#include "agent_moves.cuh"
 
 namespace {
 
@@ -2410,4 +2411,139 @@ extern "C" int prs_ens_run(prs_ens_plan* e, const uint8_t* const* frames, const 
     return PRS_E_CUDA;
   }
   return rc;
+}
+
+// ---------------------------------------------------------------------------------------------
+// Agent copies inside a plan's buffers (prs_ens_copy_agents, EnsembleSession.reassign).  A row's live data: its state
+// slice, its pc_work slots, n_dev, the library groups of its n templates and the first n entries of its location row.
+// Slots past n are never read (the sweep masks lanes >= n) and an append writes its slot whole (vt_pack_row: all 32
+// plane rows and row sums of its lane), so the destination's stale tail needs no clearing.  The stage holds K rows with
+// room for the largest live count among them.
+struct EnsRows {
+  char* state;  // [rows][state bytes]
+  long long* argmax;
+  char* total;  // 8-byte slots; a float32 plan's totals are 4-byte elements of the region
+  int* err;
+  int* n;
+  char* lib;            // [rows][lib_bytes]
+  long long lib_bytes;
+  long long* loc;       // [rows][loc_stride]
+  long long loc_stride;
+};
+
+struct EnsCopyStage {
+  size_t table = 0, state = 0, argmax = 0, total = 0, err = 0, n = 0, lib = 0, loc = 0, bytes = 0;
+  int max_n = 0;
+  EnsCopyStage(int K, size_t table_ints, size_t net_bytes, int max_n_) : max_n(max_n_) {
+    auto up = [](size_t v) { return (v + 255) & ~(size_t)255; };
+    state = up(table_ints * sizeof(int));
+    argmax = state + up((size_t)K * net_bytes);
+    total = argmax + up((size_t)K * 8);
+    err = total + up((size_t)K * 8);
+    n = err + up((size_t)K * 4);
+    lib = n + up((size_t)K * 4);
+    loc = lib + up((size_t)K * prs_vt_packed_bytes(max_n));
+    bytes = loc + up((size_t)K * max_n * 8);
+  }
+  EnsRows rows(char* p) const {
+    return EnsRows{p + state, (long long*)(p + argmax), p + total, (int*)(p + err), (int*)(p + n), p + lib,
+                   (long long)prs_vt_packed_bytes(max_n), (long long*)(p + loc), max_n};
+  }
+};
+
+// Pair m copies row src_row[m] of `src` into row dst_row[m] of `dst`: blockIdx.y strides over the pairs, the blocks
+// along x share each region of a pair.  The live count is the source's n_dev, at most max_n (the stage's room).  No
+// pair's destination is another pair's source within one launch.
+template <typename W>
+__global__ void __launch_bounds__(256)
+    k_ens_copy_rows(EnsRows src, EnsRows dst, const int* __restrict__ pairs, int n_pairs, long long state_words,
+                    int total_bytes, int max_n) {
+  const long long i0 = (long long)blockIdx.x * blockDim.x + threadIdx.x, step = (long long)gridDim.x * blockDim.x;
+  for (int m = blockIdx.y; m < n_pairs; m += gridDim.y) {
+    const int s = pairs[m], d = pairs[n_pairs + m];
+    const int n = min(src.n[s], max_n);
+    const W* ss = (const W*)src.state + s * state_words;
+    W* ds = (W*)dst.state + d * state_words;
+    for (long long i = i0; i < state_words; i += step) ds[i] = ss[i];
+    const long long lib_u4 = (long long)((n + 31) >> 5) * kVtGroupU4;
+    const uint4* sl = (const uint4*)(src.lib + s * src.lib_bytes);
+    uint4* dl = (uint4*)(dst.lib + d * dst.lib_bytes);
+    for (long long i = i0; i < lib_u4; i += step) dl[i] = sl[i];
+    for (long long i = i0; i < n; i += step) dst.loc[d * dst.loc_stride + i] = src.loc[s * src.loc_stride + i];
+    if (blockIdx.x == 0 && threadIdx.x == 0) {
+      dst.argmax[d] = src.argmax[s];
+      if (total_bytes == 4)
+        ((int*)dst.total)[d] = ((const int*)src.total)[s];
+      else
+        ((long long*)dst.total)[d] = ((const long long*)src.total)[s];
+      dst.err[d] = src.err[s];
+      dst.n[d] = n;
+    }
+  }
+}
+
+static int ens_copy_plan(const char* who, prs_ens_plan* e, int n_moves, const int* dst, const int* src,
+                         const int* n_templates, AgentMoves& mv, int& max_n) {
+  PRS_REQUIRE(e && (n_moves == 0 || n_templates), "%s: bad argument", who);
+  if (int rc = agent_moves(who, e->B, n_moves, dst, src, mv)) return rc;
+  max_n = 0;
+  for (int m = 0; m < n_moves; ++m) {
+    const int n = n_templates[src[m]];
+    PRS_REQUIRE(n >= 0 && n <= e->capacity, "%s: row %d holds %d templates, the capacity is %d", who, src[m], n,
+                e->capacity);
+  }
+  for (int r : mv.stage_rows) max_n = std::max(max_n, n_templates[r]);
+  return PRS_OK;
+}
+
+extern "C" size_t prs_ens_copy_stage_bytes(prs_ens_plan* e, int n_moves, const int* dst, const int* src,
+                                           const int* n_templates) {
+  AgentMoves mv;
+  int max_n = 0;
+  if (ens_copy_plan("prs_ens_copy_stage_bytes", e, n_moves, dst, src, n_templates, mv, max_n)) return 0;
+  return EnsCopyStage(mv.K(), mv.table().size(), ens_net_bytes(e->pc), max_n).bytes;
+}
+
+extern "C" int prs_ens_copy_agents(prs_ens_plan* e, int n_moves, const int* dst, const int* src, const int* n_templates,
+                                   void* stage, size_t stage_bytes, void* stream) {
+  AgentMoves mv;
+  int max_n = 0;
+  if (int rc = ens_copy_plan("prs_ens_copy_agents", e, n_moves, dst, src, n_templates, mv, max_n)) return rc;
+  if (n_moves == 0) return PRS_OK;
+  const std::vector<int> table = mv.table();
+  const size_t net_bytes = ens_net_bytes(e->pc);
+  const EnsCopyStage L(mv.K(), table.size(), net_bytes, max_n);
+  PRS_REQUIRE(stage && stage_bytes >= L.bytes, "prs_ens_copy_agents: the stage has %zu bytes, the moves need %zu",
+              stage_bytes, L.bytes);
+  if (int rc = prs_pc_check_device(e->pc, "prs_ens_copy_agents")) return rc;
+  const cudaStream_t st = (cudaStream_t)stream;
+  char* p = (char*)stage;
+  PRS_CUDA(cudaMemcpyAsync(p, table.data(), table.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+  const int B = e->B;
+  const EnsRows plan{(char*)e->pc_state, (long long*)e->pc_work, (char*)e->pc_work + 8 * (size_t)B,
+                     (int*)((char*)e->pc_work + 16 * (size_t)B), e->n_dev, (char*)e->libs, e->lib_u4 * 16, e->loc_dev,
+                     e->capacity};
+  const EnsRows rows = L.rows(p);
+  const bool wide = net_bytes % 16 == 0;
+  const long long state_words = (long long)(net_bytes / (wide ? 16 : 4));
+  const int es = e->pc->dtype == PRS_F32 ? 4 : 8;
+  auto launch = [&](const EnsRows& from, const EnsRows& to, const int* pairs, int n_pairs, int bound) {
+    if (n_pairs == 0) return cudaSuccess;
+    // about 16 blocks per SM over all pairs, no more along x than a pair's largest region takes
+    const long long words = std::max((long long)((bound + 31) >> 5) * kVtGroupU4, state_words);
+    long long gx = (148LL * 16 + n_pairs - 1) / n_pairs;
+    gx = std::max(1LL, std::min(gx, (words + 1023) / 1024));
+    const dim3 grid((unsigned)gx, (unsigned)std::min(n_pairs, 65535));
+    if (wide)
+      k_ens_copy_rows<uint4><<<grid, 256, 0, st>>>(from, to, pairs, n_pairs, state_words, es, bound);
+    else
+      k_ens_copy_rows<unsigned><<<grid, 256, 0, st>>>(from, to, pairs, n_pairs, state_words, es, bound);
+    return cudaGetLastError();
+  };
+  const int* d_table = (const int*)p;
+  const int K = mv.K(), n_direct = (int)mv.direct.size() / 2, n_staged = (int)mv.staged.size() / 2;
+  PRS_CUDA(launch(plan, rows, d_table, K, max_n));
+  PRS_CUDA(launch(plan, plan, d_table + 2 * K, n_direct, e->capacity));
+  PRS_CUDA(launch(rows, plan, d_table + 2 * K + 2 * n_direct, n_staged, max_n));
+  return prs_pc_active_invalidate(e->pc, st);  // the carried lists describe the rows as they were
 }

@@ -39,6 +39,17 @@ from .ros_simulate import (IM_SIZE, MATCH_THRESHOLD, ODOM_FREQ, POSE_SIZE, X_RAN
 MAX_CAPACITY = 1 << 16          # templates per agent the frame's library sweep takes (kSmallLibrary)
 
 
+class _Keep:
+    """The value of an omitted ``EnsembleSession.reassign`` setting: each agent keeps its parent's.  (``None`` is a
+    setting: no injection.)"""
+
+    def __repr__(self):
+        return "KEEP"
+
+
+KEEP = _Keep()
+
+
 def _real(v):
     return isinstance(v, (numbers.Real, np.number)) and not isinstance(v, (bool, np.bool_))
 
@@ -88,6 +99,41 @@ def agent_parameters(n_agents=None, match_threshold=MATCH_THRESHOLD, global_inhi
                              "got %r" % (v,))
         energies.append(None if v is None else float(v))
     return B, np.array(thr, dtype=np.float64), np.array(gi, dtype=np.float64), energies
+
+
+def reassign_parameters(parents, rec_of, match_threshold, global_inhibition, inject_energy, new_threshold=KEEP,
+                        new_inhibition=KEEP, new_energy=KEEP):
+    """``EnsembleSession.reassign``'s arguments validated (no CUDA involved): ``parents`` against the agents'
+    recordings ``rec_of [B]``, and the children's settings -- each the parent's setting of the current
+    ``match_threshold``, ``global_inhibition`` and ``inject_energy`` (caller order), or the ``new_*`` value where it is
+    not ``KEEP``, broadcast and validated by ``agent_parameters``.  Returns ``(parents int64 [B], thresholds,
+    inhibitions, energies)``; ``ValueError`` for a wrong length, a parent that is not an integer in [0, B) or replays
+    another recording than its child, and refused settings."""
+    B = len(rec_of)
+    if isinstance(parents, (str, bytes)):
+        raise ValueError("parents must be a sequence of %d agent indices, got %r" % (B, parents))
+    try:
+        par = list(parents)
+    except TypeError:
+        raise ValueError("parents must be a sequence of %d agent indices, got %r" % (B, parents)) from None
+    if len(par) != B:
+        raise ValueError("parents has %d values for %d agents" % (len(par), B))
+    for p in par:
+        if (not isinstance(p, (numbers.Integral, np.integer)) or isinstance(p, (bool, np.bool_))
+                or not 0 <= int(p) < B):
+            raise ValueError("parents must be agent indices in [0, %d), got %r" % (B, p))
+    par = np.array(par, dtype=np.int64)
+    rec_of = np.asarray(rec_of)
+    cross = np.nonzero(rec_of[par] != rec_of)[0]
+    if len(cross):
+        b = int(cross[0])
+        raise ValueError("agent %d replays recording %d, its parent %d recording %d: an agent continues from its own "
+                         "recording's position" % (b, rec_of[b], par[b], rec_of[par[b]]))
+    pick = lambda new, own: own if new is KEEP else new                   # noqa: E731
+    _, thr, gi, energies = agent_parameters(B, pick(new_threshold, np.asarray(match_threshold)[par]),
+                                            pick(new_inhibition, np.asarray(global_inhibition)[par]),
+                                            pick(new_energy, [inject_energy[p] for p in par]))
+    return par, thr, gi, energies
 
 
 def capacity_for(T):
@@ -348,6 +394,7 @@ class EnsembleSession:
         nat.require_cuda()
         dev = torch.device("cuda", torch.cuda.current_device())
         self.B, self.R, self.pose_size, self.capacity = B, R, pose_size, cap
+        self._thr, self._gi, self._energies = thr, gi, list(energies)     # the settings in force, caller order
         self._dev, self._rec_of = dev, rec_of
         self._map = isinstance(experience_map, str)
         self._linked = self._map and bool(experience_links)
@@ -424,6 +471,98 @@ class EnsembleSession:
         nat.check(L.prs_em_session_grow(self.B, self._E, self._N, E, N, self._work.data_ptr(), work.data_ptr(),
                                         nat.stream_ptr()), "prs_em_session_grow")
         self._work, self._E, self._N = work, E, N
+
+    # ------------------------------------------------------------------ reassigning agents
+    def reassign(self, parents, match_threshold=KEEP, global_inhibition=KEEP, inject_energy=KEEP):
+        """Make agent b an exact copy of agent ``parents[b]`` as it was before the call, then give the agents new
+        settings; call it between feeds.  The next feed continues every agent from the current frame.
+
+        ``parents`` is a length-B sequence of agent indices in the caller's order; ``parents[b] == b`` leaves agent b
+        as it is, and any mapping is valid (many children of one parent, swaps, cycles).  A copy is everything a later
+        feed reads: the pose cells and their cached arg-max, the library, the template locations, the template of the
+        last image (the map tag of ``feed_events``), the linked map with its loop closures, and the parent's settings.
+        A setting given replaces the copied one for every agent; it is a scalar or a length-B sequence, broadcast and
+        validated as ``agent_parameters`` does, and ``inject_energy=None`` turns injection off.  ``KEEP`` (the
+        default) keeps the copied settings.  ``ValueError`` before any CUDA call for a wrong length, a non-integer or
+        out-of-range parent, a parent that replays another recording than its child, or refused settings;
+        ``RuntimeError`` on a closed session.  The copies run as kernels over the live bytes of the device rows; an
+        error there closes the session, as in ``feed``."""
+        if self._closed:
+            raise RuntimeError("EnsembleSession: the session is closed")
+        B = self.B
+        par, thr, gi, energies = reassign_parameters(parents, self._rec_of, self._thr, self._gi, self._energies,
+                                                     match_threshold, global_inhibition, inject_energy)
+        moves = np.nonzero(par != np.arange(B))[0]
+        try:
+            self._reassign(par, moves, thr, gi, energies)
+        except BaseException:
+            self.close()
+            raise
+
+    def _reassign(self, par, moves, thr, gi, energies):
+        L = nat.lib()
+        with torch.cuda.device(self._dev):
+            if len(moves):
+                dst = np.ascontiguousarray(self._rows[moves], dtype=np.int32)
+                src = np.ascontiguousarray(self._rows[par[moves]], dtype=np.int32)
+                self._copy_rows(L, dst, src)
+            self._thr, self._gi = thr, gi
+            self._thr_dev.copy_(torch.from_numpy(thr[self._order]))
+            self._ens.global_inhibition = gi[self._order]
+            was_injecting = self._energy_dev is not None
+            self._energies = energies
+            injecting = any(e is not None for e in energies)
+            e_rows = torch.tensor([-1.0 if energies[i] is None else energies[i] for i in self._order],
+                                  dtype=torch.float64)
+            if injecting and was_injecting:
+                self._energy_dev.copy_(e_rows)
+            self._stream.wait_stream(torch.cuda.current_stream(self._dev))
+            if injecting != was_injecting:
+                # the plan has an injection node exactly when some agent injects: made again, as _grow makes it
+                self._energy_dev = e_rows.to(self._dev) if injecting else None
+                torch.cuda.current_stream(self._dev).synchronize()
+                L.prs_ens_destroy(self._plan)
+                self._plan = None
+                self._create_plan()
+
+    def _copy_rows(self, L, dst, src):
+        """Device rows ``dst[m]`` <- ``src[m]`` in the plan's buffers and the map workspace, and the host's copies of
+        their counts and last templates."""
+        n = len(dst)
+        stream = nat.stream_ptr()
+        n_tpl = np.ascontiguousarray(self._n, dtype=np.int32)
+        args = (n, dst.ctypes.data, src.ctypes.data)
+        stage = torch.empty(int(L.prs_ens_copy_stage_bytes(self._plan, *args, n_tpl.ctypes.data)), dtype=torch.uint8,
+                            device=self._dev)
+        nat.check(L.prs_ens_copy_agents(self._plan, *args, n_tpl.ctypes.data, stage.data_ptr(), stage.numel(), stream),
+                  "prs_ens_copy_agents")
+        if self._linked:
+            n_rows = np.ascontiguousarray(self._counts[:2].max(axis=0), dtype=np.int32)
+            em_stage = torch.empty(int(L.prs_em_session_copy_stage_bytes(self.B, self._E, self._N, *args,
+                                                                         n_rows.ctypes.data)),
+                                   dtype=torch.uint8, device=self._dev)
+            nat.check(L.prs_em_session_copy_agents(self.B, self._E, self._N, self._work.data_ptr(), *args,
+                                                   n_rows.ctypes.data, em_stage.data_ptr(), em_stage.numel(), stream),
+                      "prs_em_session_copy_agents")
+            self._counts[:, dst] = self._counts[:, src]
+        self._n[dst] = self._n[src]
+        self._prev_tpl[dst] = self._prev_tpl[src]
+        self._ens._state_gen += 1
+
+    @property
+    def match_threshold(self):
+        """float64 [B]: every agent's match threshold in force, in the caller's order."""
+        return self._thr.copy()
+
+    @property
+    def global_inhibition(self):
+        """float64 [B]: every agent's global inhibition in force, in the caller's order."""
+        return self._gi.copy()
+
+    @property
+    def inject_energy(self):
+        """list of B energies (None = no injection) in force, in the caller's order."""
+        return list(self._energies)
 
     # ------------------------------------------------------------------ feeding
     def feed(self, frames, odom):
