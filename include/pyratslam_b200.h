@@ -98,19 +98,10 @@ PRS_API size_t prs_pc_state_bytes(prs_pc_handle h);
 #define PRS_PATH_CLUSTER 3
 #define PRS_PATH_PAIR 4 /* fused SMEM-resident kernel, one network per 2-CTA cluster (float32 and float64) */
 PRS_API int prs_pc_path(prs_pc_handle h);
-/* force the generic path (1) or let the plan choose (0); for tests and profiling */
-PRS_API int prs_pc_force_generic(prs_pc_handle h, int on);
 /* choose the kernel family explicitly (PRS_PATH_*, PRS_PATH_AUTO = the plan's own choice); PRS_E_INVALID if the
  * plan's shape / dtype is not supported by that family; for tests and profiling */
 PRS_API int prs_pc_set_path(prs_pc_handle h, int path);
-/* Per-plan options.  PRS_OPT_TILED_TMA: the tiled (large-grid) family runs its 7x7 + theta stages as ONE kernel fed by
- * TMA tensor copies from a padded, origin-aligned intermediate (value 1) or as two kernels (value 0, the default: the
- * fused kernel is parity-equal but measured slower on B200, see DESIGN.md). */
-#define PRS_OPT_TILED_TMA 0
-/* PRS_OPT_TILED_DOG: the tiled family runs the theta, y and x passes of the DoG as ONE kernel (shared-memory ring fed by
- * cp.async, no (E, I) intermediate in L2) instead of two; parity-equal, measured slower, off by default. */
-#define PRS_OPT_TILED_DOG 1
-/* PRS_OPT_ACTIVE_SET: sparsity-aware update (csrc/posecell_active.cu).  The attractor dynamics of
+/* Per-plan options.  PRS_OPT_ACTIVE_SET: sparsity-aware update (csrc/posecell_active.cu).  The attractor dynamics of
  * posecell_network.py:326-353 keep the activity in a compact packet (tens of non-zero cells out of thousands); with this
  * option an update does the reference's arithmetic only where the result can be non-zero and writes the state in place,
  * instead of the dense kernels whose cost does not depend on the state.  Exact for any state: a network whose non-zero

@@ -44,7 +44,6 @@ _SIGNATURES = {
     "prs_pc_destroy": (c_int, [c_void_p]),
     "prs_pc_state_bytes": (c_size_t, [c_void_p]),
     "prs_pc_path": (c_int, [c_void_p]),
-    "prs_pc_force_generic": (c_int, [c_void_p, c_int]),
     "prs_pc_set_path": (c_int, [c_void_p, c_int]),
     "prs_pc_set_option": (c_int, [c_void_p, c_int, c_int]),
     "prs_pc_invalidate_active": (c_int, [c_void_p, c_void_p]),

@@ -50,7 +50,7 @@ static void fill_tables(PcTables<T>& t, const prs_pc_config* c) {
 static void free_plan(prs_pc_plan* p) {
   void* ptrs[] = {p->cos_th, p->sin_th, p->s1,       nullptr,      p->s3,     nullptr,     p->shift, p->fsel,
                   p->ogi,    p->part_val, p->part_idx, p->inv_total, p->d_odom, p->d_argmax, p->d_err, p->d_total,
-                  p->tab_dev, p->d_xyze, p->done_ctr, p->apad, p->lg_tmap_dev};
+                  p->tab_dev, p->d_xyze, p->done_ctr};
   for (void* q : ptrs)
     if (q) cudaFree(q);
   if (p->sgraph) cudaGraphExecDestroy(p->sgraph);
@@ -158,8 +158,8 @@ extern "C" int prs_pc_create(const prs_pc_config* cfg, prs_pc_handle* out) {
   ALLOC(p->d_err, (size_t)p->B * sizeof(int));
   ALLOC(p->d_total, (size_t)p->B * es);
   ALLOC(p->d_xyze, (size_t)p->B * 4 * sizeof(int));
-  ALLOC(p->done_ctr, (size_t)p->B * 2 * sizeof(unsigned));
-  cudaMemset(p->done_ctr, 0, (size_t)p->B * 2 * sizeof(unsigned));
+  ALLOC(p->done_ctr, (size_t)p->B * sizeof(unsigned));
+  cudaMemset(p->done_ctr, 0, (size_t)p->B * sizeof(unsigned));
   ALLOC(p->tab_dev, sizeof(PcTables<float>));
   ALLOC(p->net_seq, (size_t)p->B * sizeof(unsigned));
   cudaMemset(p->net_seq, 0, (size_t)p->B * sizeof(unsigned));
@@ -174,7 +174,7 @@ extern "C" int prs_pc_create(const prs_pc_config* cfg, prs_pc_handle* out) {
   // 16.4 us (pair kernel) / 18.5 us (one CTA per network), a 50x50x10 one 12.6 us against 19 us (tiled).
   p->cluster_pref = p->cluster_ok && one_wave;
   // The multi-kernel paths need scratch of four state tensors; it is only allocated when such a path
-  // can be taken for this plan (prs_pc_force_generic / path_integration allocate it lazily otherwise).
+  // can be taken for this plan (prs_pc_set_path / path_integration allocate it lazily otherwise).
   if (!p->resident_ok && !p->pair_ok) {
     ALLOC(p->s1, 2 * sbytes);
     ALLOC(p->s3, 2 * sbytes);
@@ -222,7 +222,7 @@ static int ensure_scratch(prs_pc_handle h) {
 }
 
 extern "C" int prs_pc_path(prs_pc_handle h) {
-  if (!h || h->force_generic) return PRS_PATH_GENERIC;
+  if (!h) return PRS_PATH_GENERIC;
   if (h->forced_path >= 0) return h->forced_path;
   if (h->cluster_pref) return PRS_PATH_CLUSTER;
   // PRS_PC_PREFER (profiling): "resident" keeps round 1's one-CTA kernel as the automatic choice for float32
@@ -251,32 +251,24 @@ extern "C" int prs_pc_set_path(prs_pc_handle h, int path) {
     if (rc != PRS_OK) return rc;
   }
   h->forced_path = path;
-  h->force_generic = 0;
   drop_graphs(h);
   return PRS_OK;
 }
 
 extern "C" int prs_pc_set_option(prs_pc_handle h, int option, int value) {
   PRS_REQUIRE(h, "prs_pc_set_option: null handle");
-  PRS_REQUIRE(option == PRS_OPT_TILED_TMA || option == PRS_OPT_TILED_DOG || option == PRS_OPT_ACTIVE_SET,
-              "prs_pc_set_option: unknown option %d", option);
-  if (option == PRS_OPT_TILED_TMA)
-    h->opt_tiled_tma = value ? 1 : -1;
-  else if (option == PRS_OPT_TILED_DOG)
-    h->opt_tiled_dog = value ? 1 : -1;
-  else {
-    PRS_REQUIRE(value >= 0 && value <= 2, "prs_pc_set_option: PRS_OPT_ACTIVE_SET takes 0, 1 or 2, got %d", value);
-    if (value) {
-      if (int rc_ = prs_pc_check_device(h, "prs_pc_set_option")) return rc_;
-      int rc = prs_pc_active_prepare(h);
-      if (rc == PRS_OK && !h->resident_ok) rc = ensure_scratch(h);  // the dense fallback is then the generic path
-      if (rc != PRS_OK) return rc;
-      rc = prs_pc_active_invalidate(h, nullptr);
-      if (rc != PRS_OK) return rc;
-      PRS_CUDA(cudaStreamSynchronize(nullptr));
-    }
-    h->opt_active = value;
+  PRS_REQUIRE(option == PRS_OPT_ACTIVE_SET, "prs_pc_set_option: unknown option %d", option);
+  PRS_REQUIRE(value >= 0 && value <= 2, "prs_pc_set_option: PRS_OPT_ACTIVE_SET takes 0, 1 or 2, got %d", value);
+  if (value) {
+    if (int rc_ = prs_pc_check_device(h, "prs_pc_set_option")) return rc_;
+    int rc = prs_pc_active_prepare(h);
+    if (rc == PRS_OK && !h->resident_ok) rc = ensure_scratch(h);  // the dense fallback is then the generic path
+    if (rc != PRS_OK) return rc;
+    rc = prs_pc_active_invalidate(h, nullptr);
+    if (rc != PRS_OK) return rc;
+    PRS_CUDA(cudaStreamSynchronize(nullptr));
   }
+  h->opt_active = value;
   drop_graphs(h);
   return PRS_OK;
 }
@@ -284,17 +276,6 @@ extern "C" int prs_pc_set_option(prs_pc_handle h, int option, int value) {
 extern "C" int prs_pc_invalidate_active(prs_pc_handle h, void* stream) {
   PRS_REQUIRE(h, "prs_pc_invalidate_active: null handle");
   return prs_pc_active_invalidate(h, (cudaStream_t)stream);
-}
-
-extern "C" int prs_pc_force_generic(prs_pc_handle h, int on) {
-  PRS_REQUIRE(h, "prs_pc_force_generic: null handle");
-  if (on) {
-    int rc = ensure_scratch(h);
-    if (rc != PRS_OK) return rc;
-  }
-  h->force_generic = on ? 1 : 0;
-  drop_graphs(h);
-  return PRS_OK;
 }
 
 static void drop_graphs(prs_pc_handle h) {

@@ -64,18 +64,10 @@ struct prs_pc_plan {
   int nblk_plane;       // blocks per theta plane in the generic kernels
   int np_max;           // partial-result slots per network (covers the generic and the tiled kernels)
   int tiled_ok;         // the tiled large-grid kernels support this shape/dtype
-  // TMA path of the tiled kernels (posecell_tiled.cu, lg_prepare): padded A tensor [B*Th][XP][YP] and its tensor map
-  float* apad;
-  int XP, YP;
-  int lg_state;         // 0 = not prepared yet, 1 = ready, -1 = unavailable (small grid, legacy knob, no driver entry)
-  alignas(64) unsigned char lg_tmap[128];
-  int opt_tiled_dog;    // prs_pc_set_option(PRS_OPT_TILED_DOG), same convention
-  int opt_tiled_tma;    // prs_pc_set_option(PRS_OPT_TILED_TMA): 1 = on, -1 = off, 0 = the PRS_TILED_TMA environment variable
-  void* lg_tmap_dev;    // device copy of the tensor map (the kernel takes the descriptor from global memory)
   void* part_val;       // [B][Th*nblk_plane] partial sums, later partial maxima
   long long* part_idx;  // [B][Th*nblk_plane]
   void* inv_total;      // [B]
-  unsigned* done_ctr;   // [2*B] last-block-done counters of the tiled kernels (atomicInc wraps them back to 0)
+  unsigned* done_ctr;   // [B] last-block-done counters of k_tl_theta_fin (atomicInc wraps them back to 0)
   // staging for the *_host entry points
   double* d_odom;
   long long* d_argmax;
@@ -102,7 +94,6 @@ struct prs_pc_plan {
   double* d_odom2[2];
   int* d_xyze2[2];
   int pipe_slot, pipe_used[2];
-  int force_generic;
   int forced_path;      // -1 = automatic choice, else one of the PRS_PATH_* codes (prs_pc_set_path)
   int cluster_C;        // CTAs per network of the thread-block-cluster kernel, 0 if it does not apply to this plan
   int cluster_ok;       // = cluster_C >= 2

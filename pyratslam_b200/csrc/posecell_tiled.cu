@@ -12,16 +12,12 @@
 //                   rows arrive by LDS.128; * 1/total, clamp (:300)                            5.3 + 4 B / cell
 //   k_tl_theta_fin  shifted 7-tap theta pass (convolution.py:344-359), clamp (:314), block arg-max  8 B / cell
 //
-// Four launches per update: the decisions (k_plan's arithmetic) run inside k_tl_theta, and the grid-wide sum
-// and arg-max are finished by the last block of k_tl_yx / k_tl_theta_fin to retire (atomicInc counters that
-// wrap back to zero, partials added in a fixed order).  Any X, Y, Th >= 3 (edge tiles are masked, halos
-// wrap by modulo); chosen by the plan for float32 grids of at least 1024 cells per plane that the fused
-// SMEM-resident kernel does not cover.
-#include <cuda.h>
-#include <stdlib.h>
-
-#include <mutex>
-
+// Four launches per update: the decisions (k_plan's arithmetic) run inside k_tl_theta, the grid-wide sum of
+// k_tl_yx's tile sums is formed by one block of the 7x7 kernel, and the arg-max is finished by the last block of
+// k_tl_theta_fin to retire (an atomicInc counter that wraps back to zero; partials are added in a fixed order).
+// k_tl_2d_pair takes the place of k_tl_2d when there are enough plane pairs to fill the chip.  Any X, Y, Th >= 3
+// (edge tiles are masked, halos wrap by modulo); chosen by the plan for float32 grids of at least 1024 cells per
+// plane that the fused SMEM-resident kernel does not cover.
 #include "common.cuh"
 
 namespace {
@@ -169,21 +165,9 @@ constexpr int kInStride = kYXcols + 1;   // 39: odd, so that lanes walking down 
 constexpr int kMidStride = kYXy + 1;     // 33
 constexpr int kTyx = 288;                // 9 warps: 4 x 70 = 280 y-pass items, 8 x 32 = 256 x-pass items
 
-// PAD: the output goes to the PADDED, ORIGIN-ALIGNED tensor Apad[plane][X + 6][YP] that the fused 7x7 + theta kernel
-// below fetches with TMA.  (i) Every plane is stored already displaced by its integer origin (convolution.py:329-331:
-// the 7x7 stage reads cell (x + ox, y + oy), so cell (x, y) is stored at (x - ox, y - oy) mod (X, Y)): the tile a CTA of
-// that kernel needs then starts at ITS OWN tile origin for every plane -- a multiple of four floats, which the tensor
-// copy demands of the innermost coordinate (an unaligned start is an illegal instruction; measured with
-// bench_tools/tma_probe.cu).  (ii) The 3-cell periodic halo is materialised -- a cell within 3 of a border is stored at
-// its periodic images as well -- so one wrap-free box is always enough.  Data cell (x, y) lives at [x + 3][y + 3].
-// And the last block of a network to retire adds up the tile sums (fixed order): that kernel needs 1/total from its start.
-constexpr int kHP = 3;
-template <bool PAD>
 __global__ void __launch_bounds__(kTyx) k_tl_yx(const float2* __restrict__ EI, float* __restrict__ A,
                                                 const float* __restrict__ gi, int X, int Y, int Th, TlPairs tp,
-                                                float* __restrict__ part, int YP, float* __restrict__ total,
-                                                float* __restrict__ inv_total, unsigned* __restrict__ done_ctr,
-                                                const int* __restrict__ shift) {
+                                                float* __restrict__ part) {
   constexpr int kT = kTyx;
   __shared__ float2 s_in[kYXrows * kInStride];
   __shared__ unsigned s_cnt;
@@ -290,39 +274,12 @@ __global__ void __launch_bounds__(kTyx) k_tl_yx(const float2* __restrict__ EI, f
     }
     // rows of this segment inside the grid (0 when the column is outside): one compare per element masks the edges
     const int nv = gy < Y ? X - gx0 : 0;
-    if (PAD) {
-      float* Pp = A + (size_t)plane * (X + 2 * kHP) * YP;
-      // where this plane's cells go: displaced by the plane's origin (one wrap per thread / per row)
-      const int ox = modp(shift[2 * plane], X), oy = modp(shift[2 * plane + 1], Y);
-      int ys = gy - oy;
-      ys += ys < 0 ? Y : 0;
-      const int cy = ys + kHP;
-      const int cy2 = ys < kHP ? cy + Y : (ys >= Y - kHP ? cy - Y : -1);  // periodic image of the column, if in the halo
-      int xs = gx0 - ox;
-      xs += xs < 0 ? X : 0;
+    float* q = Ap + (unsigned)(gx0 * Y + gy);
 #pragma unroll
-      for (int jj = 0; jj < 8; ++jj) {
-        if (jj < nv) {
-          const int rx = xs + kHP;
-          const int rx2 = xs < kHP ? rx + X : (xs >= X - kHP ? rx - X : -1);
-          Pp[rx * YP + cy] = a[jj];
-          if (cy2 >= 0) Pp[rx * YP + cy2] = a[jj];
-          if (rx2 >= 0) {
-            Pp[rx2 * YP + cy] = a[jj];
-            if (cy2 >= 0) Pp[rx2 * YP + cy2] = a[jj];
-          }
-          psum += a[jj];
-        }
-        xs = xs + 1 == X ? 0 : xs + 1;
-      }
-    } else {
-      float* q = Ap + (unsigned)(gx0 * Y + gy);
-#pragma unroll
-      for (int jj = 0; jj < 8; ++jj) {
-        if (jj < nv) {
-          q[(unsigned)(jj * Y)] = a[jj];
-          psum += a[jj];
-        }
+    for (int jj = 0; jj < 8; ++jj) {
+      if (jj < nv) {
+        q[(unsigned)(jj * Y)] = a[jj];
+        psum += a[jj];
       }
     }
   }
@@ -339,33 +296,6 @@ __global__ void __launch_bounds__(kTyx) k_tl_yx(const float2* __restrict__ EI, f
     for (int w = 0; w < kT / 32; ++w) sum += s_red[w];
     const int ntiles = gridDim.x * gridDim.y, b = plane / Th, k = plane - b * Th;
     part[(size_t)b * Th * ntiles + (size_t)k * ntiles + blockIdx.y * gridDim.x + blockIdx.x] = sum;
-  }
-  if (PAD) {  // the last block of this network to retire forms the total (posecell_network.py:343-345)
-    const int np = Th * gridDim.x * gridDim.y, b = plane / Th;
-    int last = 0;
-    if (lane == 0) {
-      __threadfence();
-      last = (atomicInc(&done_ctr[b], (unsigned)(np - 1)) == (unsigned)(np - 1)) ? 1 : 0;
-    }
-    last = __shfl_sync(0xffffffffu, last, 0);
-    if (last) {
-      __threadfence();
-      const float* pp = part + (size_t)b * np;
-      float acc = 0.f;
-      for (int i0 = lane; i0 < np; i0 += 32 * 8) {  // eight independent L2 loads in flight per lane
-        float v[8];
-#pragma unroll
-        for (int u = 0; u < 8; ++u) v[u] = i0 + 32 * u < np ? __ldcg(pp + i0 + 32 * u) : 0.f;
-#pragma unroll
-        for (int u = 0; u < 8; ++u) acc += v[u];
-      }
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
-      if (lane == 0) {
-        total[b] = acc;
-        inv_total[b] = (acc != 0.f) ? 1.f / acc : 1.f;
-      }
-    }
   }
 }
 
@@ -397,182 +327,6 @@ __device__ __forceinline__ void block_tile_total(const float* __restrict__ part,
   }
 }
 
-
-// ------------------------------------------------------------------------------------------------
-// Fused separable DoG: theta + y + x passes, inhibition and partial sums in ONE kernel (k_tl_theta + k_tl_yx fused).
-//
-// The (E, I) intermediate of the two-kernel sequence is the largest tensor of the update -- 37.7 MB written and 49 MB
-// read back (with the tile halo) per 256x256x72 update, 38 % of all L2 traffic of a path that is bound by L2 bandwidth
-// (profiles/r2_large_grid_kernels.txt).  Here a CTA owns a 32x32 tile of (x, y), walks a chunk of theta planes and
-// keeps everything between the input state and A in shared memory:
-//   * every thread owns (up to) six of the tile's 38x38 halo positions for the whole walk.  It streams its positions of
-//     the next planes into a shared-memory ring of nine planes with 4-byte cp.async copies (periodic wrap: the source
-//     offsets are computed once), two planes ahead of the one being processed; as a thread only ever reads ring entries
-//     it wrote itself, no barrier is needed between the copies and the theta pass (cp.async.wait_group is enough).
-//   * theta pass: seven ring reads per position, symmetric fold, (E, I) pair into s_ei            (11 op / halo cell)
-//   * y pass (8 outputs per item, 152 items) and x pass (128 items) as in k_tl_yx, FFMA2 on (E, I)
-//   * A = max(aE E - aI I - gi, 0) to global memory; the CTA keeps ONE partial sum for all its planes.
-// Two block barriers per plane.  The first block of a network also evaluates the update's decisions (prs_plan_cell).
-// MEASURED (B200, round 2): slower than the two kernels it replaces -- 39 us against 31.5 us for 256x256x72 with six
-// chunks (fewer chunks are slower still), 1.155 ms against 1.065 ms for 2600 networks of 50x50x10 -- although it moves
-// less than half of their bytes: three short dependent phases per plane with 24 warps per SM are latency bound, where
-// k_tl_yx keeps 45 warps per SM on independent tiles.  Kept as an opt-in (PRS_OPT_TILED_DOG), not the default.
-constexpr int kDgT = 32;                    // tile edge
-constexpr int kDgH = kDgT + 6;              // 38 halo positions per edge
-constexpr int kDgPos = kDgH * kDgH;         // 1444
-constexpr int kDgNT = 256;
-constexpr int kDgPP = (kDgPos + kDgNT - 1) / kDgNT;  // 6 positions per thread
-constexpr int kDgAhead = 2;                 // planes in flight beyond the one being processed
-constexpr int kDgRing = 7 + kDgAhead;
-constexpr int kDgEiStride = kDgH + 1;       // 39
-constexpr int kDgMidStride = kDgT + 1;      // 33
-constexpr size_t kDgSmem = (size_t)kDgRing * kDgPos * 4 + (size_t)kDgH * kDgEiStride * 8 + (size_t)kDgH * kDgMidStride * 8 + 64;
-
-__global__ void __launch_bounds__(kDgNT, 3)
-    k_tl_dog(const float* __restrict__ P, float* __restrict__ A, const float* __restrict__ gi, int X, int Y, int Th,
-             int nchunks, int tiles_y, PcTables<float> tab, TlPairs tp, PlanArgs pa, float* __restrict__ part,
-             float* __restrict__ total, float* __restrict__ inv_total, unsigned* __restrict__ done_ctr) {
-  extern __shared__ __align__(16) unsigned char dg_smem[];
-  float* ring = reinterpret_cast<float*>(dg_smem);                                              // [kDgRing][kDgPos]
-  float2* s_ei = reinterpret_cast<float2*>(dg_smem + (size_t)kDgRing * kDgPos * 4);             // [38][39]
-  float2* s_mid = s_ei + kDgH * kDgEiStride;                                                    // [38][33]
-  float* s_red = reinterpret_cast<float*>(s_mid + kDgH * kDgMidStride);                         // [8]
-  const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-  const int tile = blockIdx.x, txi = tile / tiles_y, tyi = tile - txi * tiles_y;
-  const int x0 = txi * kDgT, y0 = tyi * kDgT;
-  const int chunk = blockIdx.y, b = blockIdx.z;
-  const int XY = X * Y;
-  if (tile == 0 && chunk == 0) {  // decisions of this update, needed by the kernels behind this one
-    for (int k = tid; k < Th; k += kDgNT)
-      prs_plan_cell(b, k, Th, pa.minXY, pa.odom, pa.cos_th, pa.sin_th, pa.vtrans_scale, pa.vrot_scale, pa.shift, pa.fsel,
-                    pa.ogi, pa.err);
-  }
-  const int k_begin = (int)((long long)chunk * Th / nchunks), k_end = (int)((long long)(chunk + 1) * Th / nchunks);
-  const int C = k_end - k_begin;
-  // my positions: source offset inside a plane (periodic wrap), and where the (E, I) pair goes
-  int goff[kDgPP], eoff[kDgPP];
-#pragma unroll
-  for (int i = 0; i < kDgPP; ++i) {
-    const int e = tid + i * kDgNT;
-    const int r = e / kDgH, c = e - r * kDgH;
-    goff[i] = e < kDgPos ? modp(x0 - 3 + r, X) * Y + modp(y0 - 3 + c, Y) : -1;
-    eoff[i] = r * kDgEiStride + c;
-  }
-  const float* Pb = P + (size_t)b * Th * XY;
-  const unsigned ring_a = (unsigned)__cvta_generic_to_shared(ring);
-  auto issue = [&](int j) {  // rel plane j <-> plane k_begin - 3 + j, into ring slot j % kDgRing
-    if (j < C + 6) {
-      const float* src = Pb + (size_t)modp(k_begin - 3 + j, Th) * XY;
-      const unsigned dst = ring_a + (unsigned)((j % kDgRing) * kDgPos + tid) * 4u;
-#pragma unroll
-      for (int i = 0; i < kDgPP; ++i)
-        if (goff[i] >= 0)
-          asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(dst + (unsigned)(i * kDgNT * 4)), "l"(src + goff[i])
-                       : "memory");
-    }
-    asm volatile("cp.async.commit_group;" ::: "memory");
-  };
-#pragma unroll 1
-  for (int j = 0; j < 6 + kDgAhead; ++j) issue(j);
-  const float e0 = pin(tab.ge[3]), e1 = pin(tab.ge[2]), e2 = pin(tab.ge[1]), e3 = pin(tab.ge[0]);
-  const float i0 = pin(tab.gi[3]), i1 = pin(tab.gi[2]), i2 = pin(tab.gi[1]), i3 = pin(tab.gi[0]);
-  const float g = gi[b];
-  float psum = 0.f;
-#pragma unroll 1
-  for (int kk = 0; kk < C; ++kk) {
-    issue(kk + 6 + kDgAhead);
-    asm volatile("cp.async.wait_group %0;" ::"n"(kDgAhead) : "memory");  // rel planes kk .. kk + 6 have landed
-    // ---- theta pass on my positions
-#pragma unroll
-    for (int i = 0; i < kDgPP; ++i) {
-      if (goff[i] >= 0) {
-        float w[7];
-#pragma unroll
-        for (int t = 0; t < 7; ++t) w[t] = ring[((kk + t) % kDgRing) * kDgPos + tid + i * kDgNT];
-        const float s1 = w[2] + w[4], s2 = w[1] + w[5], s3 = w[0] + w[6];
-        s_ei[eoff[i]] = make_float2(fmaf(e0, w[3], fmaf(e1, s1, fmaf(e2, s2, e3 * s3))),
-                                    fmaf(i0, w[3], fmaf(i1, s1, fmaf(i2, s2, i3 * s3))));
-      }
-    }
-    __syncthreads();
-    // ---- y pass: item = (halo row, segment of 8 outputs)
-    if (tid < 4 * kDgH) {
-      const int seg = tid / kDgH, r = tid - seg * kDgH;
-      const float2* sp = s_ei + r * kDgEiStride + seg * 8;
-      float2 in[14];
-#pragma unroll
-      for (int j = 0; j < 14; ++j) in[j] = sp[j];
-      float2* mp = s_mid + r * kDgMidStride + seg * 8;
-#pragma unroll
-      for (int jj = 0; jj < 8; ++jj) {
-        float2 acc = make_float2(0.f, 0.f);
-#pragma unroll
-        for (int t = 0; t < 7; ++t) acc = __ffma2_rn(in[jj + t], tp.ty[t], acc);
-        mp[jj] = acc;
-      }
-    }
-    __syncthreads();
-    // ---- x pass + inhibition: item = (segment of 8 rows, column); lanes along y
-    if (tid < 4 * kDgT) {
-      const int seg = wid, y = lane;
-      const float2* sp = s_mid + seg * 8 * kDgMidStride + y;
-      float2 in[14];
-#pragma unroll
-      for (int j = 0; j < 14; ++j) in[j] = sp[j * kDgMidStride];
-      const int gy = y0 + y, gx0 = x0 + seg * 8;
-      const int nv = gy < Y ? X - gx0 : 0;
-      float* q = A + ((size_t)b * Th + k_begin + kk) * XY + (unsigned)(gx0 * Y + gy);
-#pragma unroll
-      for (int jj = 0; jj < 8; ++jj) {
-        float2 acc = make_float2(0.f, 0.f);
-#pragma unroll
-        for (int t = 0; t < 7; ++t) acc = __ffma2_rn(in[jj + t], tp.tx[t], acc);
-        const float a = fmaxf((acc.x - acc.y) - g, 0.f);  // posecell_network.py:339-340: (a < gi) ? 0 : a - gi
-        if (jj < nv) {
-          q[(unsigned)(jj * Y)] = a;
-          psum += a;
-        }
-      }
-    }
-    // no barrier here: the next theta pass writes s_ei (last read before the barrier above); the next y pass writes
-    // s_mid only behind the next barrier, which every thread passes after its x pass
-  }
-  // one partial sum per CTA; the last CTA of the network to retire forms the total (posecell_network.py:343-345)
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) psum += __shfl_xor_sync(0xffffffffu, psum, o);
-  if (lane == 0) s_red[wid] = psum;
-  __syncthreads();
-  if (wid != 0) return;
-  const int np = gridDim.x * gridDim.y;
-  int last = 0;
-  if (lane == 0) {
-    float sum = 0.f;
-#pragma unroll
-    for (int w = 0; w < 4; ++w) sum += s_red[w];  // only the four x-pass warps hold a sum
-    part[(size_t)b * np + (size_t)chunk * gridDim.x + tile] = sum;
-    __threadfence();
-    last = (atomicInc(&done_ctr[b], (unsigned)(np - 1)) == (unsigned)(np - 1)) ? 1 : 0;
-  }
-  last = __shfl_sync(0xffffffffu, last, 0);
-  if (last) {
-    __threadfence();
-    const float* pp = part + (size_t)b * np;
-    float acc = 0.f;
-    for (int i0 = lane; i0 < np; i0 += 32 * 8) {
-      float v[8];
-#pragma unroll
-      for (int u = 0; u < 8; ++u) v[u] = i0 + 32 * u < np ? __ldcg(pp + i0 + 32 * u) : 0.f;
-#pragma unroll
-      for (int u = 0; u < 8; ++u) acc += v[u];
-    }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
-    if (lane == 0) {
-      total[b] = acc;
-      inv_total[b] = (acc != 0.f) ? 1.f / acc : 1.f;
-    }
-  }
-}
 
 // ------------------------------------------------------------------------------------------------
 constexpr int k2X = 64, k2Y = 32;          // outputs per tile
@@ -678,34 +432,28 @@ __global__ void __launch_bounds__(kT) k_tl_2d(const float* __restrict__ A, float
 // instruction issue: 49 FFMA per cell).  The two planes' tiles -- each displaced by its own origin -- are
 // interleaved as float2 in shared memory; the coefficient pairs (F_k0[a][q], F_k1[a][q]) come from the constant
 // bank as uniform-register operands of the FFMA2 (no registers, no shared-memory traffic).
-// A thread owns a patch of 2 rows x PW columns of outputs: 8 halo rows of PW + 6 float2 feed 98 * PW FFMA2.
-// The eight lanes of a quarter warp read windows that start PW float2 apart; 16-byte unit u of a row is
-// therefore stored at u ^ ((u >> 3) & M) (M = 3 for PW = 8, 1 for PW = 4), which spreads the eight units
-// {h, h + PW/2, ...} over all eight 16-byte bank groups: conflict-free LDS.128 (the unswizzled 2 x 4 patch
-// needed 7.75 wavefronts per LDS.128 and was bound by the shared-memory pipe).
-constexpr int k2pX = 64;  // output rows per tile
-template <int PW>
-struct Pair2D {
-  static constexpr int kY = 8 * PW;                     // output columns per tile
-  static constexpr int kXH = k2pX + 6, kYH = kY + 6;    // halo tile
-  static constexpr int kUnits = ((kYH + 1) / 2 + 7) / 8 * 8;  // 16-byte units per row, a multiple of 8
-  static constexpr int kStride = 2 * kUnits;            // float2 per halo row
-  static constexpr int kMask = PW == 8 ? 3 : 1;
-  static constexpr int kNH = (PW + 6) / 2;              // LDS.128 per window row
-  static constexpr int kNC = (kYH + 31) / 32;           // columns per lane in the fill
-  static constexpr int kMinBlocks = PW == 8 ? 3 : 4;
-  __device__ static __forceinline__ int swz(int u) { return u ^ ((u >> 3) & kMask); }
-};
+// A thread owns a patch of 2 rows x 4 columns of outputs: 8 halo rows of 10 float2 feed 392 FFMA2.
+// The eight lanes of a quarter warp read windows that start 4 float2 apart; 16-byte unit u of a row is
+// therefore stored at u ^ ((u >> 3) & 1), which spreads the eight units {h, h + 2, ...} over all eight
+// 16-byte bank groups: conflict-free LDS.128 (the unswizzled 2 x 4 patch needed 7.75 wavefronts per LDS.128
+// and was bound by the shared-memory pipe).
+constexpr int k2pX = 64;                                   // output rows per tile
+constexpr int k2pW = 4;                                    // output columns per thread
+constexpr int k2pY = 8 * k2pW;                             // output columns per tile
+constexpr int k2pXH = k2pX + 6, k2pYH = k2pY + 6;          // halo tile
+constexpr int k2pUnits = ((k2pYH + 1) / 2 + 7) / 8 * 8;    // 16-byte units per row, a multiple of 8
+constexpr int k2pStride = 2 * k2pUnits;                    // float2 per halo row
+constexpr int k2pNH = (k2pW + 6) / 2;                      // LDS.128 per window row
+constexpr int k2pNC = (k2pYH + 31) / 32;                   // columns per lane in the fill
+__device__ __forceinline__ int swz2p(int u) { return u ^ ((u >> 3) & 1); }
 
-template <int PW>
-__global__ void __launch_bounds__(kT, Pair2D<PW>::kMinBlocks)
+__global__ void __launch_bounds__(kT, 4)
     k_tl_2d_pair(const float* __restrict__ A, float* __restrict__ Bp, const int* __restrict__ shift,
                  const unsigned char* __restrict__ fsel, const float* __restrict__ part, int np,
                  float* __restrict__ total, float* __restrict__ inv_total, int X, int Y, int Th, int NPh, TlPairs tp) {
-  using C = Pair2D<PW>;
-  __shared__ __align__(16) float2 s_a[C::kXH * C::kStride];
+  __shared__ __align__(16) float2 s_a[k2pXH * k2pStride];
   const int XY = X * Y;
-  const int x0 = blockIdx.x * k2pX, y0 = blockIdx.y * C::kY;
+  const int x0 = blockIdx.x * k2pX, y0 = blockIdx.y * k2pY;
   const int b = blockIdx.z / NPh, kp = blockIdx.z - b * NPh;
   const int k0 = 2 * kp, k1 = (2 * kp + 1 < Th) ? 2 * kp + 1 : 2 * kp;
   const int pl0 = b * Th + k0, pl1 = b * Th + k1;
@@ -715,14 +463,14 @@ __global__ void __launch_bounds__(kT, Pair2D<PW>::kMinBlocks)
     // each plane's integer origin displaces the tile that is loaded (convolution.py:329-331); one warp per halo
     // row, lanes along y (columns lane, lane + 32, ...)
     constexpr int NW = kT / 32;
-    constexpr int NR = (C::kXH + NW - 1) / NW;
-    constexpr int NC = C::kNC;
-    const bool xnear = X >= C::kXH;
+    constexpr int NR = (k2pXH + NW - 1) / NW;
+    constexpr int NC = k2pNC;
+    const bool xnear = X >= k2pXH;
     int dcol[NC];  // where this lane's columns land in the swizzled row
 #pragma unroll
     for (int c = 0; c < NC; ++c) {
       const int col = lane + 32 * c;
-      dcol[c] = C::swz(col >> 1) * 2 + (col & 1);
+      dcol[c] = swz2p(col >> 1) * 2 + (col & 1);
     }
     float v[2][NR][NC];
 #pragma unroll
@@ -730,17 +478,17 @@ __global__ void __launch_bounds__(kT, Pair2D<PW>::kMinBlocks)
       const int pl = h == 0 ? pl0 : pl1;
       const float* src = A + (size_t)pl * XY;
       const int gx0 = modp(x0 + shift[2 * pl] - 3, X), gy0 = modp(y0 + shift[2 * pl + 1] - 3, Y);
-      if (gy0 + C::kYH <= Y && xnear) {  // no wrap along y (block-uniform): one row pointer, immediate column offsets
+      if (gy0 + k2pYH <= Y && xnear) {  // no wrap along y (block-uniform): one row pointer, immediate column offsets
 #pragma unroll
         for (int i = 0; i < NR; ++i) {
           const int r = wid + i * NW;
-          if (r < C::kXH) {
+          if (r < k2pXH) {
             int gx = gx0 + r;
             gx -= gx >= X ? X : 0;
             const float* q = src + (size_t)gx * Y + (gy0 + lane);
 #pragma unroll
             for (int c = 0; c < NC; ++c)
-              if (32 * c + 32 <= C::kYH || lane + 32 * c < C::kYH) v[h][i][c] = q[32 * c];
+              if (32 * c + 32 <= k2pYH || lane + 32 * c < k2pYH) v[h][i][c] = q[32 * c];
           }
         }
       } else {
@@ -753,13 +501,13 @@ __global__ void __launch_bounds__(kT, Pair2D<PW>::kMinBlocks)
 #pragma unroll
         for (int i = 0; i < NR; ++i) {
           const int r = wid + i * NW;
-          if (r < C::kXH) {
+          if (r < k2pXH) {
             int gx = gx0 + r;
             gx = xnear ? (gx >= X ? gx - X : gx) : gx % X;
             const int rb = gx * Y;
 #pragma unroll
             for (int c = 0; c < NC; ++c)
-              if (32 * c + 32 <= C::kYH || lane + 32 * c < C::kYH) v[h][i][c] = src[rb + gy[c]];
+              if (32 * c + 32 <= k2pYH || lane + 32 * c < k2pYH) v[h][i][c] = src[rb + gy[c]];
           }
         }
       }
@@ -767,51 +515,51 @@ __global__ void __launch_bounds__(kT, Pair2D<PW>::kMinBlocks)
 #pragma unroll
     for (int i = 0; i < NR; ++i) {
       const int r = wid + i * NW;
-      if (r < C::kXH) {
-        float2* d = s_a + r * C::kStride;
+      if (r < k2pXH) {
+        float2* d = s_a + r * k2pStride;
 #pragma unroll
         for (int c = 0; c < NC; ++c)
-          if (32 * c + 32 <= C::kYH || lane + 32 * c < C::kYH) d[dcol[c]] = make_float2(v[0][i][c], v[1][i][c]);
+          if (32 * c + 32 <= k2pYH || lane + 32 * c < k2pYH) d[dcol[c]] = make_float2(v[0][i][c], v[1][i][c]);
       }
     }
   }
   __syncthreads();
   const int xb = tid >> 3, yb = tid & 7;
-  const int x = 2 * xb, y = PW * yb;
+  const int x = 2 * xb, y = k2pW * yb;
   // the 16-byte units of this thread's window, as pointers into row x (rows add immediates)
-  const float4* rp[C::kNH];
+  const float4* rp[k2pNH];
 #pragma unroll
-  for (int h = 0; h < C::kNH; ++h)
-    rp[h] = reinterpret_cast<const float4*>(s_a + x * C::kStride) + C::swz((PW / 2) * yb + h);
-  float2 acc[2][PW];
+  for (int h = 0; h < k2pNH; ++h)
+    rp[h] = reinterpret_cast<const float4*>(s_a + x * k2pStride) + swz2p((k2pW / 2) * yb + h);
+  float2 acc[2][k2pW];
 #pragma unroll
   for (int d = 0; d < 2; ++d)
 #pragma unroll
-    for (int j = 0; j < PW; ++j) acc[d][j] = make_float2(0.f, 0.f);
+    for (int j = 0; j < k2pW; ++j) acc[d][j] = make_float2(0.f, 0.f);
 #pragma unroll
   for (int rr = 0; rr < 8; ++rr) {
-    float2 in[2 * C::kNH];
+    float2 in[2 * k2pNH];
 #pragma unroll
-    for (int h = 0; h < C::kNH; ++h) {
-      const float4 v = rp[h][rr * (C::kStride / 2)];
+    for (int h = 0; h < k2pNH; ++h) {
+      const float4 v = rp[h][rr * (k2pStride / 2)];
       in[2 * h] = make_float2(v.x, v.y);
       in[2 * h + 1] = make_float2(v.z, v.w);
     }
     if (rr <= 6) {
 #pragma unroll
-      for (int j = 0; j < PW; ++j)
+      for (int j = 0; j < k2pW; ++j)
 #pragma unroll
         for (int q = 0; q < 7; ++q) acc[0][j] = __ffma2_rn(in[j + q], tp.f2p[combo][rr][q], acc[0][j]);
     }
     if (rr >= 1) {
 #pragma unroll
-      for (int j = 0; j < PW; ++j)
+      for (int j = 0; j < k2pW; ++j)
 #pragma unroll
         for (int q = 0; q < 7; ++q) acc[1][j] = __ffma2_rn(in[j + q], tp.f2p[combo][rr - 1][q], acc[1][j]);
     }
   }
   const int gy = y0 + y;
-  const bool vec = (Y & 3) == 0 && gy + PW - 1 < Y;
+  const bool vec = (Y & 3) == 0 && gy + k2pW - 1 < Y;
 #pragma unroll
   for (int d = 0; d < 2; ++d) {
     const int gx = x0 + x + d;
@@ -819,21 +567,21 @@ __global__ void __launch_bounds__(kT, Pair2D<PW>::kMinBlocks)
 #pragma unroll
     for (int h = 0; h < 2; ++h) {
       if (h == 1 && k1 == k0) continue;  // odd Th: the last pair has one plane
-      float o[PW];
+      float o[k2pW];
 #pragma unroll
-      for (int j = 0; j < PW; ++j) o[j] = fmaxf(h == 0 ? acc[d][j].x : acc[d][j].y, 0.f);  // posecell_network.py:300 (1/total: see block_tile_total)
+      for (int j = 0; j < k2pW; ++j) o[j] = fmaxf(h == 0 ? acc[d][j].x : acc[d][j].y, 0.f);  // posecell_network.py:300 (1/total: see block_tile_total)
       float* dst = Bp + (size_t)(h == 0 ? pl0 : pl1) * XY + gx * Y + gy;
       if (vec) {
 #pragma unroll
-        for (int j = 0; j < PW; j += 4) reinterpret_cast<float4*>(dst)[j / 4] = make_float4(o[j], o[j + 1], o[j + 2], o[j + 3]);
+        for (int j = 0; j < k2pW; j += 4) reinterpret_cast<float4*>(dst)[j / 4] = make_float4(o[j], o[j + 1], o[j + 2], o[j + 3]);
       } else {
 #pragma unroll
-        for (int j = 0; j < PW; ++j)
+        for (int j = 0; j < k2pW; ++j)
           if (gy + j < Y) dst[j] = o[j];
       }
     }
   }
-  if (np > 0 && blockIdx.x == 0 && blockIdx.y == 0 && kp == 0)  // side job of one block per network (np == 0: k_tl_dog did it)
+  if (np > 0 && blockIdx.x == 0 && blockIdx.y == 0 && kp == 0)  // side job of one block per network
     block_tile_total(part + (size_t)b * np, np, total + b, inv_total + b, reinterpret_cast<float*>(s_a));
 }
 
@@ -962,252 +710,6 @@ __global__ void __launch_bounds__(kT, MINB) k_tl_theta_fin(const float* __restri
   }
 }
 
-
-// ------------------------------------------------------------------------------------------------
-// Fused 7x7 stage + shifted theta pass + arg-max for large grids (BASELINE config 3), fed by TMA.
-//
-// k_tl_2d_pair + k_tl_theta_fin stream the B tensor through L2 twice (18.9 MB written, 33 MB read back with the
-// theta halo) and are two dependent launches.  Here a CTA owns a 16x32 tile of (x, y) and walks a chunk of theta
-// planes; B never leaves shared memory:
-//   * seven warps work on seven consecutive planes at once.  Each warp fetches the 22x40 halo tile of ITS plane of
-//     the padded A tensor with one cp.async.bulk.tensor (3-D tensor map, box 40 x 22 x 1).  k_tl_yx<true> stored every
-//     plane displaced by its integer origin (convolution.py:329-331) and materialised the periodic wrap in the halo,
-//     so the box of every plane starts at the tile's own origin (aligned, wrap-free); two slots per warp, the copy of
-//     the warp's next plane is in flight while it computes (mbarrier complete_tx).
-//   * 7x7 correlate (posecell_network.py:273-274,300): a lane owns a 4x4 patch, ten window rows of three LDS.128
-//     (row stride 40 floats: the eight lanes of a quarter warp read eight consecutive 16-byte units, conflict-free)
-//     feed 784 FFMA; the clamped plane goes into a ring of 14 B planes in shared memory.
-//   * after each round of seven planes the CTA runs the theta pass (convolution.py:344-359) for the (up to) seven
-//     output planes whose +-3 neighbours are now in the ring, 1/total folded into the taps, clamp (:314), float4
-//     stores of whole 128-byte rows, running arg-max; the last block of a network to retire picks its arg-max.
-// A chunk of C output planes costs C + 6 planes of 7x7 work; two chunks of 36 for Th = 72 (overhead 1.17).
-constexpr int kSTX = 16, kSTY = 32;        // tile: x rows, y columns
-constexpr int kSBH = kSTX + 6;             // 22 box rows
-constexpr int kSBW = 40;                   // box columns: 38 used, a multiple of four floats
-constexpr int kSW = 7;                     // planes in flight per CTA, one warp each
-constexpr int kSNT = kSW * 32;
-constexpr int kSSlot = (kSBH * kSBW * 4 + 127) / 128 * 128;  // 3584 bytes
-constexpr int kSRing = 2 * kSW;            // B planes kept in shared memory
-constexpr size_t kSSmem = (size_t)kSW * 2 * kSSlot + (size_t)kSRing * kSTX * kSTY * 4 + kSW * 2 * 8 + 256;
-
-struct StArgs {
-  const float* Apad;
-  float* S;
-  const int* shift;
-  const unsigned char* fsel;
-  const int* ogi;
-  const float* inv_total;
-  float* part_val;
-  long long* part_idx;
-  unsigned* done_ctr;
-  long long* argmax;
-  int X, Y, Th, XP, YP, nchunks, tiles_y;
-};
-
-__device__ __forceinline__ unsigned st_smem(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
-
-__global__ void __launch_bounds__(kSNT, 2)
-    k_tl_shift_theta(const CUtensorMap* __restrict__ tmap_g, StArgs a, PcTables<float> tab) {
-  extern __shared__ __align__(128) unsigned char st_smem_raw[];
-  float* a_slots = reinterpret_cast<float*>(st_smem_raw);                                 // [kSW][2][kSSlot / 4]
-  float* b_ring = reinterpret_cast<float*>(st_smem_raw + (size_t)kSW * 2 * kSSlot);       // [kSRing][kSTX * kSTY]
-  unsigned long long* bars = reinterpret_cast<unsigned long long*>(st_smem_raw + (size_t)kSW * 2 * kSSlot +
-                                                                   (size_t)kSRing * kSTX * kSTY * 4);
-  float* s_v = reinterpret_cast<float*>(bars + kSW * 2);
-  long long* s_i = reinterpret_cast<long long*>(s_v + 8);  // 8-byte aligned: 14 barriers * 8 + 32
-  const int tid = threadIdx.x, lane = tid & 31;
-  const int wid = __shfl_sync(0xffffffffu, tid >> 5, 0);
-  const int X = a.X, Y = a.Y, Th = a.Th;
-  const int tile = blockIdx.x, tx = tile / a.tiles_y, ty = tile - tx * a.tiles_y;
-  const int x0 = tx * kSTX, y0 = ty * kSTY;
-  const int chunk = blockIdx.y, b = blockIdx.z;
-  const int k_begin = (int)((long long)chunk * Th / a.nchunks), k_end = (int)((long long)(chunk + 1) * Th / a.nchunks);
-  const int NB = k_end - k_begin + 6;              // B planes this chunk needs: rel j <-> plane k_begin - 3 + j
-  const int rounds = (NB + kSW - 1) / kSW;
-  const unsigned bar0 = st_smem(bars + wid * 2);
-  float* my_slots = a_slots + (size_t)wid * 2 * (kSSlot / 4);
-  if (lane == 0) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar0));
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar0 + 8));
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-  }
-  __syncwarp();
-  unsigned phase = 0;    // bit s: parity of the next completion of slot s's barrier
-
-  // fetch the halo tile of rel plane j into slot s: one tensor copy; the plane was stored displaced by its origin, so
-  // the box starts at the tile's own origin (padded coordinates: data cell (x, y) at [x + 3][y + 3], halo 3)
-  auto fetch = [&](int j, int s) {
-    if (j >= NB) return;
-    const int pl = b * Th + modp(k_begin - 3 + j, Th);
-    if (lane == 0) {
-      const unsigned bar = bar0 + 8 * s;
-      asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(kSBH * kSBW * 4) : "memory");
-      asm volatile(
-          "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];" ::"r"(
-              st_smem(my_slots + (size_t)s * (kSSlot / 4))),
-          "l"(tmap_g), "r"(y0), "r"(x0), "r"(pl), "r"(bar)
-          : "memory");
-    }
-  };
-  fetch(wid, 0);
-  fetch(kSW + wid, 1);
-
-  const float* f1 = tab.f1d[a.ogi[b]];
-  const float inv = a.inv_total[b];  // 1/total of the normalisation (posecell_network.py:344-345), folded into the taps
-  float fc[7];
-#pragma unroll
-  for (int t = 0; t < 7; ++t) fc[t] = f1[t] * inv;
-  float bestv = -1.f;
-  long long besti = 0x7fffffffffffffffLL;
-  const int li = lane >> 3, lj = lane & 7;  // patch rows 4 li .. 4 li + 3, columns 4 lj .. 4 lj + 3
-  const bool vec = (Y & 3) == 0;
-
-  for (int r = 0; r < rounds; ++r) {
-    const int j = r * kSW + wid;
-    const int s = r & 1;
-    float acc[4][4];
-#pragma unroll
-    for (int d = 0; d < 4; ++d)
-#pragma unroll
-      for (int c = 0; c < 4; ++c) acc[d][c] = 0.f;
-    if (j < NB) {
-      {
-        const unsigned bar = bar0 + 8 * s, parity = (phase >> s) & 1u;
-        phase ^= 1u << s;
-        asm volatile(
-            "{\n"
-            ".reg .pred p;\n"
-            "WAIT_%=:\n"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-            "@!p bra WAIT_%=;\n"
-            "}\n" ::"r"(bar),
-            "r"(parity)
-            : "memory");
-      }
-      const int pl = b * Th + modp(k_begin - 3 + j, Th);
-      float F[49];
-      {
-        const float* f = tab.f2d[a.fsel[pl]];
-#pragma unroll
-        for (int i = 0; i < 49; ++i) F[i] = f[i];
-      }
-      const float* sp = my_slots + (size_t)s * (kSSlot / 4) + (4 * li) * kSBW + 4 * lj;
-#pragma unroll
-      for (int rr = 0; rr < 10; ++rr) {
-        const float4* rp = reinterpret_cast<const float4*>(sp + rr * kSBW);
-        const float4 v0 = rp[0], v1 = rp[1], v2 = rp[2];
-        const float in[12] = {v0.x, v0.y, v0.z, v0.w, v1.x, v1.y, v1.z, v1.w, v2.x, v2.y, v2.z, v2.w};
-#pragma unroll
-        for (int d = 0; d < 4; ++d) {
-          const int ta = rr - d;  // tap row of output row 4 li + d
-          if (ta >= 0 && ta <= 6) {
-#pragma unroll
-            for (int c = 0; c < 4; ++c)
-#pragma unroll
-              for (int q = 0; q < 7; ++q) acc[d][c] = fmaf(in[c + q], F[ta * 7 + q], acc[d][c]);
-          }
-        }
-      }
-      __syncwarp();            // every lane has read its window: the slot may be refilled
-      fetch(j + 2 * kSW, s);   // the warp's plane of the round after next
-    }
-    __syncthreads();  // the theta pass of the previous round has finished reading the ring slots written now
-    if (j < NB) {
-      float* bp = b_ring + (size_t)(j % kSRing) * (kSTX * kSTY) + (4 * li) * kSTY + 4 * lj;
-#pragma unroll
-      for (int d = 0; d < 4; ++d)  // posecell_network.py:300 (1/total is applied by the taps of the theta pass)
-        *reinterpret_cast<float4*>(bp + d * kSTY) =
-            make_float4(fmaxf(acc[d][0], 0.f), fmaxf(acc[d][1], 0.f), fmaxf(acc[d][2], 0.f), fmaxf(acc[d][3], 0.f));
-    }
-    __syncthreads();
-    // theta pass: output rel planes whose neighbours j - 3 .. j + 3 are all in the ring now
-    const int hi_avail = (r * kSW + kSW - 1 < NB - 1 ? r * kSW + kSW - 1 : NB - 1) - 3;
-    const int o_lo = r == 0 ? 3 : r * kSW - 3;
-    const int n_out = hi_avail - o_lo + 1;
-    for (int it = tid; it < 128 * n_out; it += kSNT) {
-      const int q = it & 127, jo = o_lo + (it >> 7);
-      float4 o = make_float4(0.f, 0.f, 0.f, 0.f);
-#pragma unroll
-      for (int t = 0; t < 7; ++t) {
-        const float4 v = *reinterpret_cast<const float4*>(b_ring + (size_t)((jo + t - 3) % kSRing) * (kSTX * kSTY) + q * 4);
-        o.x = fmaf(fc[t], v.x, o.x);
-        o.y = fmaf(fc[t], v.y, o.y);
-        o.z = fmaf(fc[t], v.z, o.z);
-        o.w = fmaf(fc[t], v.w, o.w);
-      }
-      const int gx = x0 + (q >> 3), gy = y0 + (q & 7) * 4;
-      const int k = k_begin + jo - 3;
-      if (gx < X && gy < Y) {
-        const float c[4] = {fmaxf(o.x, 0.f), fmaxf(o.y, 0.f), fmaxf(o.z, 0.f), fmaxf(o.w, 0.f)};  // posecell_network.py:314
-        float* dst = a.S + ((size_t)b * Th + k) * ((size_t)X * Y) + (size_t)gx * Y + gy;
-        if (vec && gy + 3 < Y) {
-          *reinterpret_cast<float4*>(dst) = make_float4(c[0], c[1], c[2], c[3]);
-        } else {
-#pragma unroll
-          for (int u = 0; u < 4; ++u)
-            if (gy + u < Y) dst[u] = c[u];
-        }
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-          if (gy + u < Y) {
-            const long long flat = ((long long)gx * Y + gy + u) * Th + k;  // numpy.argmax order: [x][y][th]
-            if (c[u] > bestv || (c[u] == bestv && flat < besti)) bestv = c[u], besti = flat;
-          }
-        }
-      }
-    }
-  }
-  // block arg-max, then the network's in the last block to retire (as k_tl_theta_fin)
-  auto warp_best = [&](float& bv, long long& bi) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-      const float v2 = __shfl_xor_sync(0xffffffffu, bv, o);
-      const long long i2 = __shfl_xor_sync(0xffffffffu, bi, o);
-      if (v2 > bv || (v2 == bv && i2 < bi)) bv = v2, bi = i2;
-    }
-  };
-  warp_best(bestv, besti);
-  if (lane == 0) s_v[wid] = bestv, s_i[wid] = besti;
-  __syncthreads();
-  if (wid != 0) return;
-  float bv = lane < kSW ? s_v[lane] : -1.f;
-  long long bi = lane < kSW ? s_i[lane] : 0x7fffffffffffffffLL;
-  warp_best(bv, bi);
-  const int nslots = gridDim.x * gridDim.y;
-  int last = 0;
-  if (lane == 0) {
-    const size_t slot = (size_t)b * nslots + (size_t)blockIdx.y * gridDim.x + blockIdx.x;
-    a.part_val[slot] = bv;
-    a.part_idx[slot] = bi;
-    __threadfence();
-    last = (atomicInc(&a.done_ctr[b], (unsigned)(nslots - 1)) == (unsigned)(nslots - 1)) ? 1 : 0;
-  }
-  last = __shfl_sync(0xffffffffu, last, 0);
-  if (last) {
-    __threadfence();
-    const float* pv = a.part_val + (size_t)b * nslots;
-    const long long* pi = a.part_idx + (size_t)b * nslots;
-    bv = -1.f;
-    bi = 0x7fffffffffffffffLL;
-    for (int i0 = lane; i0 < nslots; i0 += 32 * 8) {
-      float v[8];
-      long long ix[8];
-#pragma unroll
-      for (int u = 0; u < 8; ++u) {
-        const int i = i0 + 32 * u;
-        v[u] = i < nslots ? __ldcg(pv + i) : -1.f;
-        ix[u] = i < nslots ? __ldcg(pi + i) : 0x7fffffffffffffffLL;
-      }
-#pragma unroll
-      for (int u = 0; u < 8; ++u)
-        if (v[u] > bv || (v[u] == bv && ix[u] < bi)) bv = v[u], bi = ix[u];
-    }
-    warp_best(bv, bi);
-    if (lane == 0) a.argmax[b] = bi;
-  }
-}
-
 }  // namespace
 
 int prs_pc_tiled_supported(const prs_pc_plan* p) {
@@ -1216,197 +718,53 @@ int prs_pc_tiled_supported(const prs_pc_plan* p) {
   return (p->X * p->Y >= 1024) ? 1 : 0;
 }
 
-// The TMA path (k_tl_theta -> k_tl_yx<true> -> k_tl_shift_theta: three launches, the B tensor never leaves shared
-// memory, 306 MB of L2 traffic per 256x256x72 update against 344 MB).  Parity-green, but measured SLOWER than the
-// four-kernel sequence on B200 (76 us against 60 us per update, profiles/r2_large_grid_kernels.txt): its 7x7 stage is
-// scalar FFMA (17.7 M warp instructions against 13.4 M for k_tl_2d_pair + k_tl_theta_fin, whose plane-pair interleave
-// gives FFMA2 but needs a SIMT fill), and the displaced, halo-replicating stores cost k_tl_yx 9 us.  It is therefore
-// opt-in: prs_pc_set_option(h, PRS_OPT_TILED_TMA, 1) or PRS_TILED_TMA=1.  Needs the padded A tensor and its 3-D tensor
-// map, made on first use (a driver without cuTensorMapEncodeTiled keeps the four-kernel sequence).
-static int lg_prepare(prs_pc_plan* p) {
-  if (p->lg_state != 0) return p->lg_state;
-  static std::mutex mu;
-  std::lock_guard<std::mutex> lk(mu);
-  if (p->lg_state != 0) return p->lg_state;
-  p->lg_state = -1;
-  if (p->X < 64 || p->Y < 64 || p->Th < 8) return -1;
-  typedef CUresult (*encode_fn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-  void* fn = nullptr;
-  cudaDriverEntryPointQueryResult qres;
-  if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) != cudaSuccess ||
-      qres != cudaDriverEntryPointSuccess || fn == nullptr) {
-    (void)cudaGetLastError();
-    return -1;
-  }
-  p->XP = p->X + 2 * kHP;
-  p->YP = (p->Y + 2 * kHP + 2 + 3) / 4 * 4;  // + 2: the 40-column box overhangs the 38 columns a tile uses
-  const size_t bytes = (size_t)p->B * p->Th * p->XP * p->YP * sizeof(float);
-  if (cudaMalloc((void**)&p->apad, bytes) != cudaSuccess) {
-    (void)cudaGetLastError();
-    p->apad = nullptr;
-    return -1;
-  }
-  cudaMemset(p->apad, 0, bytes);  // the columns beyond Y + 6 are never written; keep them finite
-  static_assert(sizeof(CUtensorMap) <= sizeof(p->lg_tmap), "tensor map slot");
-  const cuuint64_t dims[3] = {(cuuint64_t)p->YP, (cuuint64_t)p->XP, (cuuint64_t)p->B * p->Th};
-  const cuuint64_t strides[2] = {(cuuint64_t)p->YP * 4, (cuuint64_t)p->YP * p->XP * 4};
-  const cuuint32_t box[3] = {kSBW, kSBH, 1};
-  const cuuint32_t estr[3] = {1, 1, 1};
-  const CUresult r = ((encode_fn)fn)(reinterpret_cast<CUtensorMap*>(p->lg_tmap), CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, p->apad,
-                                     dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-                                     CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    cudaFree(p->apad);
-    p->apad = nullptr;
-    return -1;
-  }
-  // the kernel reads the descriptor from global memory (written once, here, before any launch that uses it)
-  if (cudaMalloc(&p->lg_tmap_dev, 128) != cudaSuccess ||
-      cudaMemcpy(p->lg_tmap_dev, p->lg_tmap, 128, cudaMemcpyHostToDevice) != cudaSuccess ||
-      cudaFuncSetAttribute(k_tl_shift_theta, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSSmem) != cudaSuccess) {
-    (void)cudaGetLastError();
-    cudaFree(p->apad);
-    p->apad = nullptr;
-    return -1;
-  }
-  p->lg_state = 1;
-  return 1;
-}
-
 int prs_pc_tiled_step(prs_pc_plan* p, float* state, const double* odom, const float* gi, long long* argmax, float* total,
                       int* err, cudaStream_t st) {
   const int X = p->X, Y = p->Y, Th = p->Th, B = p->B, XY = X * Y;
   float2* EI = (float2*)p->s1;  // s1|s2 are contiguous: 2*B*N floats
   float* A = (float*)p->s3;
   float* Bp = (float*)p->s4;
-  static const bool tma_env = [] {
-    const char* e = getenv("PRS_TILED_TMA");
-    return e && atoi(e) != 0;
-  }();
-  const bool tma_path = (p->opt_tiled_tma > 0 || (p->opt_tiled_tma == 0 && tma_env)) && lg_prepare(p) == 1;
   const int nchunk = (Th + kTK - 1) / kTK;
   const PlanArgs pa{odom, p->cos_th, p->sin_th, p->vtrans_scale, p->vrot_scale, p->shift, p->fsel, p->ogi, err,
                     X < Y ? X : Y};
-  // The fused theta + y + x kernel (k_tl_dog) is parity-equal but measured slower than k_tl_theta + k_tl_yx (256x256x72:
-  // 39 us against 31.5 us; 2600 x 50x50x10: 1.155 ms against 1.065 ms per update): opt-in through
-  // prs_pc_set_option(h, PRS_OPT_TILED_DOG, 1) or PRS_TILED_DOG=1
-  static const int dog_env = [] {
-    const char* e = getenv("PRS_TILED_DOG");
-    return e ? atoi(e) : 0;
-  }();
-  const bool dog = (p->opt_tiled_dog > 0 || (p->opt_tiled_dog == 0 && dog_env != 0)) && !tma_path;
-  int np_2d = 0;  // partial sums the 7x7 kernel's side job still has to add up (0: k_tl_dog formed the total itself)
-  if (dog) {
-    static std::mutex mu;
-    static bool configured[64] = {};
-    {
-      std::lock_guard<std::mutex> lk(mu);
-      if (p->device >= 0 && p->device < 64 && !configured[p->device]) {
-        PRS_CUDA(cudaFuncSetAttribute(k_tl_dog, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kDgSmem));
-        configured[p->device] = true;
-      }
-    }
-    const int tiles_x = (X + kDgT - 1) / kDgT, tiles_y = (Y + kDgT - 1) / kDgT;
-    const long long tiles = (long long)tiles_x * tiles_y * B;
-    // chunks of theta: a chunk of C planes loads and theta-filters C + 6, so as few chunks as fill the chip
-    static const int force_chunks = [] {
-      const char* e = getenv("PRS_DOG_CHUNKS");
-      return e ? atoi(e) : 0;
-    }();
-    int nch = (int)((2 * 148 + tiles - 1) / tiles);
-    if (nch > Th / 12) nch = Th / 12;
-    if (force_chunks > 0) nch = force_chunks < Th ? force_chunks : Th;
-    if (nch < 1) nch = 1;
-    k_tl_dog<<<dim3((unsigned)(tiles_x * tiles_y), nch, B), kDgNT, kDgSmem, st>>>(
-        state, A, gi, X, Y, Th, nch, tiles_y, p->tf, p->tl, pa, (float*)p->part_val, total, (float*)p->inv_total, p->done_ctr);
+  const int V = (XY % 2 == 0) ? 2 : 1;
+  const int nline = (XY / V + kT - 1) / kT;
+  if (Th >= 36 && Th % 12 == 0) {  // longer chunks re-read fewer planes: (12 + 6) / 12 loads per cell
+    const dim3 g(nline, B, Th / 12);
+    if (V == 2)
+      k_tl_theta<2, 12><<<g, kT, 0, st>>>(state, EI, XY, Th, p->tf, pa);
+    else
+      k_tl_theta<1, 12><<<g, kT, 0, st>>>(state, EI, XY, Th, p->tf, pa);
   } else {
-    const int V = (XY % 2 == 0) ? 2 : 1;
-    const int nline = (XY / V + kT - 1) / kT;
-    if (Th >= 36 && Th % 12 == 0) {  // longer chunks re-read fewer planes: (12 + 6) / 12 loads per cell
-      const dim3 g(nline, B, Th / 12);
-      if (V == 2)
-        k_tl_theta<2, 12><<<g, kT, 0, st>>>(state, EI, XY, Th, p->tf, pa);
-      else
-        k_tl_theta<1, 12><<<g, kT, 0, st>>>(state, EI, XY, Th, p->tf, pa);
-    } else {
-      const dim3 g(nline, B, nchunk);
-      if (V == 2)
-        k_tl_theta<2, kTK><<<g, kT, 0, st>>>(state, EI, XY, Th, p->tf, pa);
-      else
-        k_tl_theta<1, kTK><<<g, kT, 0, st>>>(state, EI, XY, Th, p->tf, pa);
-    }
+    const dim3 g(nline, B, nchunk);
+    if (V == 2)
+      k_tl_theta<2, kTK><<<g, kT, 0, st>>>(state, EI, XY, Th, p->tf, pa);
+    else
+      k_tl_theta<1, kTK><<<g, kT, 0, st>>>(state, EI, XY, Th, p->tf, pa);
   }
   const dim3 g2((X + kYXx - 1) / kYXx, (Y + kYXy - 1) / kYXy, B * Th);
-  if (tma_path) {
-    k_tl_yx<true><<<g2, kTyx, 0, st>>>(EI, p->apad, gi, X, Y, Th, p->tl, (float*)p->part_val, p->YP, total,
-                                        (float*)p->inv_total, p->done_ctr, p->shift);
-    StArgs sa;
-    sa.Apad = p->apad, sa.S = state, sa.shift = p->shift, sa.fsel = p->fsel, sa.ogi = p->ogi;
-    sa.inv_total = (const float*)p->inv_total, sa.part_val = (float*)p->part_val, sa.part_idx = p->part_idx;
-    sa.done_ctr = p->done_ctr + B, sa.argmax = argmax;
-    sa.X = X, sa.Y = Y, sa.Th = Th, sa.XP = p->XP, sa.YP = p->YP;
-    const int tiles_x = (X + kSTX - 1) / kSTX;
-    sa.tiles_y = (Y + kSTY - 1) / kSTY;
-    const long long tiles = (long long)tiles_x * sa.tiles_y * B;
-    // chunks of theta: every chunk recomputes six planes of 7x7 work, so as few as fill the chip (two CTAs per SM)
-    static const int force_chunks = [] {
-      const char* e = getenv("PRS_TILED_CHUNKS");
-      return e ? atoi(e) : 0;
-    }();
-    int nch = (int)((2 * 148 + tiles / 2) / tiles);
-    if (force_chunks > 0) nch = force_chunks;
-    if (nch < 1) nch = 1;
-    if (nch > Th / 8) nch = Th / 8 > 0 ? Th / 8 : 1;
-    sa.nchunks = nch;
-    k_tl_shift_theta<<<dim3((unsigned)(tiles_x * sa.tiles_y), nch, B), kSNT, kSSmem, st>>>(
-        reinterpret_cast<const CUtensorMap*>(p->lg_tmap_dev), sa, p->tf);
-    PRS_CUDA(cudaGetLastError());
-    return PRS_OK;
-  }
-  if (!dog) {
-    k_tl_yx<false><<<g2, kTyx, 0, st>>>(EI, A, gi, X, Y, Th, p->tl, (float*)p->part_val, 0, nullptr, nullptr, nullptr, nullptr);
-    np_2d = Th * (int)(g2.x * g2.y);
-  }
-  const int np = np_2d;
+  k_tl_yx<<<g2, kTyx, 0, st>>>(EI, A, gi, X, Y, Th, p->tl, (float*)p->part_val);
+  const int np = Th * (int)(g2.x * g2.y);
   const int NPh = (Th + 1) / 2;
-  // PRS_TILED_PW (tuning knob): columns per thread patch in the plane-pair kernel, 4 (default) or 8
-  static const int pw = [] {
-    const char* e = getenv("PRS_TILED_PW");
-    return (e && atoi(e) == 8) ? 8 : 4;
-  }();
-  const int tileY = 8 * pw;
-  const dim3 g3p((X + k2pX - 1) / k2pX, (Y + tileY - 1) / tileY, B * NPh);
+  const dim3 g3p((X + k2pX - 1) / k2pX, (Y + k2pY - 1) / k2pY, B * NPh);
   if ((long long)g3p.x * g3p.y * g3p.z >= 2 * 148) {  // enough plane pairs to fill the chip: packed FFMA2 variant
-    if (pw == 8)
-      k_tl_2d_pair<8><<<g3p, kT, 0, st>>>(A, Bp, p->shift, p->fsel, (const float*)p->part_val, np, total, (float*)p->inv_total, X, Y, Th, NPh, p->tl);
-    else
-      k_tl_2d_pair<4><<<g3p, kT, 0, st>>>(A, Bp, p->shift, p->fsel, (const float*)p->part_val, np, total, (float*)p->inv_total, X, Y, Th, NPh, p->tl);
+    k_tl_2d_pair<<<g3p, kT, 0, st>>>(A, Bp, p->shift, p->fsel, (const float*)p->part_val, np, total, (float*)p->inv_total, X, Y, Th, NPh, p->tl);
   } else {
     const dim3 g3((X + k2X - 1) / k2X, (Y + k2Y - 1) / k2Y, B * Th);
     k_tl_2d<<<g3, kT, 0, st>>>(A, Bp, p->shift, p->fsel, (const float*)p->part_val, np, total, (float*)p->inv_total, X, Y, Th, p->tf);
   }
-  {
-    // PRS_TILED_FIN (tuning knob): cells x planes per thread, 0 = 2 x 8, 1 (default) = 4 x 8, 2 = 2 x 12
-    static const int fin = [] {
-      const char* e = getenv("PRS_TILED_FIN");
-      return e ? atoi(e) : 1;
-    }();
+  // cells x planes per thread of the shifted theta pass: 4 x 8 where X*Y allows, else 2 x 12, else 1 x 8
 #define PRS_FIN(V_, TK_, MB_)                                                                                      \
   k_tl_theta_fin<V_, TK_, MB_><<<dim3((XY / V_ + kT - 1) / kT, B, (Th + TK_ - 1) / TK_), kT, 0, st>>>(              \
-      Bp, state, p->ogi, (const float*)p->inv_total, XY, Th, p->tf, (float*)p->part_val, p->part_idx,              \
-      p->done_ctr + B, argmax)
-    if (XY % 4 == 0 && fin == 1)
-      PRS_FIN(4, 8, 4);
-    else if (XY % 2 == 0 && fin != 0)
-      PRS_FIN(2, 12, 5);
-    else if (XY % 2 == 0)
-      PRS_FIN(2, 8, 1);
-    else
-      PRS_FIN(1, 8, 1);
+      Bp, state, p->ogi, (const float*)p->inv_total, XY, Th, p->tf, (float*)p->part_val, p->part_idx, p->done_ctr, \
+      argmax)
+  if (XY % 4 == 0)
+    PRS_FIN(4, 8, 4);
+  else if (XY % 2 == 0)
+    PRS_FIN(2, 12, 5);
+  else
+    PRS_FIN(1, 8, 1);
 #undef PRS_FIN
-  }
   PRS_CUDA(cudaGetLastError());
   return PRS_OK;
 }

@@ -162,24 +162,19 @@ class PoseCellEnsemble:
             raise ValueError(nat.lib().prs_last_error().decode())
 
     def set_option(self, name, value):
-        """Per-plan options of the kernels: ``"tiled_tma"`` -- the large-grid family's TMA-fed fused 7x7 + theta kernel,
-        ``"tiled_dog"`` -- its fused theta + y + x kernel (both parity-equal, measured slower, off by default; DESIGN.md);
-        ``"active_set"`` -- 0 / 1 / 2: the sparsity-aware update of csrc/posecell_active.cu (off / the state is scanned for its
-        non-zero cells every update / the list of non-zero cells is carried from update to update), same results, a cost
-        that follows the size of the activity packet instead of the grid."""
-        code = {"tiled_tma": 0, "tiled_dog": 1, "active_set": 2}[name]
-        v = int(value) if name == "active_set" else (1 if value else 0)
+        """The per-plan option of the kernels, ``"active_set"`` -- 0 / 1 / 2: the sparsity-aware update of
+        csrc/posecell_active.cu (off / the state is scanned for its non-zero cells every update / the list of non-zero
+        cells is carried from update to update), same results, a cost that follows the size of the activity packet
+        instead of the grid."""
+        code = {"active_set": 2}[name]
         with torch.cuda.device(self.device):
-            nat.check(nat.lib().prs_pc_set_option(self._h, code, v), "prs_pc_set_option")
+            nat.check(nat.lib().prs_pc_set_option(self._h, code, int(value)), "prs_pc_set_option")
 
     def invalidate_active(self):
         """``active_set=2`` keeps the list of non-zero cells from one update to the next; whoever writes ``state`` other
         than through this class (a torch operation on the tensor) calls this afterwards."""
         with torch.cuda.device(self.device):
             nat.check(nat.lib().prs_pc_invalidate_active(self._h, nat.stream_ptr()), "prs_pc_invalidate_active")
-
-    def force_generic(self, on=True):
-        nat.check(nat.lib().prs_pc_force_generic(self._h, 1 if on else 0), "prs_pc_force_generic")
 
     # ------------------------------------------------------------------ state access
     @property
