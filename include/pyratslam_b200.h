@@ -215,14 +215,6 @@ PRS_API int prs_vt_pack_u8(const uint8_t* src, long long n, void* packed, long l
 PRS_API int prs_vt_unpack_u8(const void* packed, long long index, uint8_t* dst, void* stream);
 PRS_API int prs_vt_sweep_packed_u8(const void* packed, long long n, const uint8_t* query, int mode, long long base_index,
                            unsigned long long* key_out, uint32_t* scores, void* scratch, void* stream);
-/* Tuning knobs of the sweeps, for profiling (defaults are the measured best): knob 0 = ring depth of the packed
- * reference-mode sweep (slots of 2 KiB per warp fed by TMA bulk copies; 0 = the register-prefetch kernel, else 2, 4
- * or 8; 34 = four slots and the warps of a CTA kept in lock step by a barrier per ring item, 44 = the same with one
- * 640-thread CTA per SM), knob 1 = CTAs per SM that sweep's grid is sized for, knob 2 = ring depth of the float32 sweep (0 = the register
- * kernel; 1..4 = templates in flight per warp, one template per warp; 11..13 = the column-pair kernel -- two columns per
- * lane, two templates per warp -- with 1..3 template pairs in flight per warp), knob 3 = CTAs per SM of that sweep, knob 4 = the
- * circular-mode sweep keeps the warps of a CTA in lock step (1, default) or not (0). */
-PRS_API int prs_vt_tune(int knob, int value);
 /* Any template shape rows x cols (row-major library) and any max_offset (view_templates.py:14): the
  * reference's windowed match for configurations other than its 32x32 default.  Correctness path. */
 PRS_API int prs_vt_sweep_any_u8(const uint8_t* lib, long long n, const uint8_t* query, int rows, int cols, int max_offset,

@@ -76,7 +76,6 @@ _SIGNATURES = {
                                     c_void_p]),
     "prs_vt_sweep_any_f32": (c_int, [c_void_p, c_longlong, c_void_p, c_int, c_int, c_int, c_longlong, c_void_p, c_void_p,
                                      c_void_p]),
-    "prs_vt_tune": (c_int, [c_int, c_int]),
     "prs_vt_match_host_u8": (c_int, [c_void_p, c_longlong, c_void_p, c_int, c_longlong, c_void_p, c_void_p, c_void_p]),
 }
 

@@ -31,7 +31,6 @@
 #include <string.h>
 
 #include <algorithm>
-#include <atomic>
 #include <mutex>
 #include <vector>
 
@@ -257,15 +256,6 @@ int sweep_grid(long long units_per_warp_total) {
 
 }  // namespace
 
-// Tuning knobs of the sweeps (prs_vt_tune): [0] ring depth of the packed reference-mode sweep (0 = the
-// register-prefetch kernel; 2, 4, 8 = slots per warp; 34 = 4 slots with the CTA's warps in lock step, 44 = the same
-// with one 640-thread CTA per SM), [1] CTAs per SM its grid is sized for, [2] ring depth of the float32 reference-mode
-// sweep (0 = the register kernel, 1..4 = one template per warp, 11..13 = the column-pair kernel with depth - 10 slots),
-// [3] CTAs per SM of that ring sweep.
-static std::atomic<int> g_vt_knob[4] = {{34}, {5}, {13}, {2}};  // measured best on B200 (bench_tools/vt_tune.py)
-static int launch_f32_ring(int depth, int ctas_per_sm, const float* lib, long long n, const float* query,
-                           long long base_index, unsigned long long* key_out, float* scores, cudaStream_t st);
-
 // the boolean mask of view_templates.py:48-57 must select exactly n_rows x n_cols pixels inside the frame
 static int check_mask(int im_rows, int im_cols, int row_lo, int row_hi, int row_step, int col_lo, int col_hi, int col_step,
                       int n_rows, int n_cols) {
@@ -304,25 +294,6 @@ extern "C" int prs_vt_sweep_u8(const uint8_t* lib, long long n, const uint8_t* q
     k_vt_sweep_u8<PRS_VT_MODE_REF><<<grid, kVtThreads, 0, st>>>(lib, n, query, base_index, key_out, scores);
   else
     k_vt_sweep_u8<PRS_VT_MODE_CIRCULAR><<<grid, kVtThreads, 0, st>>>(lib, n, query, base_index, key_out, scores);
-  PRS_CUDA(cudaGetLastError());
-  return PRS_OK;
-}
-
-extern "C" int prs_vt_sweep_f32(const float* lib, long long n, const float* query, int mode, long long base_index,
-                                unsigned long long* key_out, float* scores, void* stream) {
-  PRS_REQUIRE(query && key_out && n >= 0 && (lib || n == 0), "prs_vt_sweep_f32: bad argument");
-  PRS_REQUIRE(mode == PRS_VT_MODE_REF || mode == PRS_VT_MODE_CIRCULAR, "prs_vt_sweep_f32: unknown mode %d", mode);
-  PRS_REQUIRE(base_index >= 0 && base_index + n <= 0xffffffffLL, "prs_vt_sweep_f32: template index does not fit 32 bits");
-  cudaStream_t st = (cudaStream_t)stream;
-  PRS_CUDA(cudaMemsetAsync(key_out, 0xff, sizeof(unsigned long long), st));
-  if (n == 0) return PRS_OK;
-  int grid = sweep_grid(n);
-  if (mode == PRS_VT_MODE_REF && g_vt_knob[2] != 0)
-    return launch_f32_ring(g_vt_knob[2], g_vt_knob[3], lib, n, query, base_index, key_out, scores, st);
-  if (mode == PRS_VT_MODE_REF)
-    k_vt_sweep_f32<PRS_VT_MODE_REF><<<grid, kVtThreads, 0, st>>>(lib, n, query, base_index, key_out, scores);
-  else
-    k_vt_sweep_f32<PRS_VT_MODE_CIRCULAR><<<grid, kVtThreads, 0, st>>>(lib, n, query, base_index, key_out, scores);
   PRS_CUDA(cudaGetLastError());
   return PRS_OK;
 }
@@ -497,90 +468,19 @@ __device__ __forceinline__ void ref_row(const uint4& lo, const uint4& hi, uint32
   for (int s = s_lo; s <= s_hi; ++s) cnt[T - s + 7] += lt_row(lo, hi, s);
 }
 
-template <int T>
-struct RefRows {
-  __device__ __forceinline__ static void run(const uint4* gp, uint4 lo, uint4 hi, uint32_t (&cnt)[15]) {
-    if constexpr (T <= 30) {
-      uint4 nlo = lo, nhi = hi;
-      if constexpr (T < 30) {  // the next row is in flight while this one is compared
-        nlo = ld_stream_u4(gp + ((T + 1) * 2 + 0) * 32);
-        nhi = ld_stream_u4(gp + ((T + 1) * 2 + 1) * 32);
-      }
-      ref_row<T>(lo, hi, cnt);
-      RefRows<T + 1>::run(gp, nlo, nhi, cnt);
-    }
-  }
-};
-
 constexpr int kPkThreads = 128;
 
-// Reference mode (15 windowed row offsets, view_templates.py:16-28) over the packed library.
-__global__ void __launch_bounds__(kPkThreads)  // 96 registers (15 interleaved compare chains); capping them spills
-    k_vt_sweep_packed_ref(const uint4* __restrict__ packed, long long n, long long base_index,
-                          unsigned long long* __restrict__ key_out, uint32_t* __restrict__ scores,
-                          const int* __restrict__ n_dev) {
-  if (n_dev != nullptr) n = *n_dev;  // graph replays: the library size lives on the device
-  const int lane = threadIdx.x & 31;
-  const long long n_groups = (n + 31) >> 5;
-  const long long warp0 = ((long long)blockIdx.x * kPkThreads + threadIdx.x) >> 5;
-  const long long n_warps = ((long long)gridDim.x * kPkThreads) >> 5;
-  unsigned long long best = ~0ull;
-  for (long long g = warp0; g < n_groups; g += n_warps) {
-    const uint4* gp = packed + g * kGroupU4 + lane;
-    uint32_t cnt[15];
-#pragma unroll
-    for (int i = 0; i < 15; ++i) cnt[i] = 0;
-    RefRows<1>::run(gp, ld_stream_u4(gp + (1 * 2 + 0) * 32), ld_stream_u4(gp + (1 * 2 + 1) * 32), cnt);
-    // window sums of the stored rows: A(o) = sum_{r=8+o}^{23+o} R[r]
-    uint32_t R[32];
-#pragma unroll
-    for (int w4 = 0; w4 < 4; ++w4) {
-      const uint4 v = ld_stream_u4(gp + 32 * 2 * 32 + w4 * 32);
-      const uint32_t ww[4] = {v.x, v.y, v.z, v.w};
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        R[(w4 * 4 + j) * 2] = ww[j] & 0xffffu;
-        R[(w4 * 4 + j) * 2 + 1] = ww[j] >> 16;
-      }
-    }
-    uint32_t A = 0;
-#pragma unroll
-    for (int r = 1; r <= 16; ++r) A += R[r];
-    const uint32_t bq = c_vtq[256];
-    uint32_t m = 0xffffffffu;
-#pragma unroll
-    for (int o = -7; o <= 7; ++o) {
-      const uint32_t sc = A + 256u * cnt[o + 7] - bq;
-      m = min(m, sc);
-      if (o < 7) A = A - R[8 + o] + R[24 + o];
-    }
-    const long long ti = g * 32 + lane;
-    if (ti < n) {
-      const unsigned long long key = ((unsigned long long)m << 32) | (unsigned long long)(base_index + ti);
-      best = key < best ? key : best;
-      if (scores != nullptr) scores[ti] = m;
-    }
-  }
-  __shared__ unsigned long long sm[kPkThreads / 32];
-  best = warp_min_u64(best);
-  if (lane == 0) sm[threadIdx.x >> 5] = best;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    unsigned long long k = sm[0];
-#pragma unroll
-    for (int i = 1; i < kPkThreads / 32; ++i) k = sm[i] < k ? sm[i] : k;
-    if (k != ~0ull) atomicMin(key_out, k);
-  }
-}
-
-// ---- the same sweep fed by warp-private rings of TMA bulk copies -----------------------------------------
-// The register-prefetch kernel above keeps ONE row (1 KB per warp) in flight: 20 warps x 1 KB x 148 SMs = 3 MB,
-// less than half of what Little's law asks for at 6.5 TB/s x ~1 us.  Here every warp owns a ring of D slots of
-// 2 KB (two stored rows of its 32 templates) with one mbarrier each; one elected lane refills a slot with one
-// cp.async.bulk as soon as the warp has consumed it, so 2 D KB per warp are always in flight and the loads cost
-// no registers and no LSU issue slots beyond two LDS.128 per row.  A group is 16 ring items: rows 1..30 in
-// pairs (rows 0 and 31 are never read in reference mode) and the row-sum block; 16 / D fills per slot and
-// group is even, so the mbarrier parity of an item is a compile-time constant.
+// ---- reference mode (15 windowed row offsets, view_templates.py:16-28), fed by warp-private rings of TMA bulk copies
+// A warp that prefetches one row in registers keeps 1 KB in flight: 20 warps x 1 KB x 148 SMs = 3 MB, less than half
+// of what Little's law asks for at 6.5 TB/s x ~1 us.  Here every warp owns a ring of kRingSlots slots of 2 KB (two
+// stored rows of its 32 templates) with one mbarrier each; one elected lane refills a slot with one cp.async.bulk as
+// soon as the warp has consumed it, so 2 kRingSlots KB per warp are always in flight and the loads cost no registers
+// and no LSU issue slots beyond two LDS.128 per row.  A group is 16 ring items: rows 1..30 in pairs (rows 0 and 31
+// are never read in reference mode) and the row-sum block; 16 / kRingSlots fills per slot and group is even, so the
+// mbarrier parity of an item is a compile-time constant.  Four slots and five CTAs per SM are the fastest of the
+// depths and grid sizes measured (profiles/r1_vt_ring_tuning.txt).
+constexpr int kRingSlots = 4;
+constexpr int kRingCtasPerSm = 5;
 __device__ __forceinline__ uint32_t vt_smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void vt_mbar_init(uint32_t bar, int count) {
   asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
@@ -629,28 +529,28 @@ constexpr int kItemBytes = 2048;
 constexpr int kItemsPerGroup = 16;
 __host__ __device__ constexpr int pk_item_off(int j) { return (j < 15 ? 2 * j + 1 : 32) * 1024; }
 
-template <int D, int S>
+template <int S>
 struct RingPrologue {
   __device__ __forceinline__ static void run(uint32_t ring, uint32_t bars, const char* gb) {
-    if constexpr (S < D) {
+    if constexpr (S < kRingSlots) {
       vt_ring_fill<pk_item_off(S), kItemBytes>(ring + S * kItemBytes, gb, bars + S * 8);
-      RingPrologue<D, S + 1>::run(ring, bars, gb);
+      RingPrologue<S + 1>::run(ring, bars, gb);
     }
   }
 };
 
-template <int D, int J, bool LOCK>
+template <int J>
 struct RingItems {
   // ring / bars: shared addresses of this warp's slots and barriers; gb / nb: this group and the warp's next one.
-  // LOCK: the warps of the CTA meet at a barrier after every item, so that all of them execute the same stretch of
-  // the (48 KB, straight-line) code at the same time; `active` is false for a warp that has run out of groups.
+  // The warps of the CTA meet at a barrier after every item, so that all of them execute the same stretch of the
+  // (48 KB, straight-line) code at the same time; `active` is false for a warp that has run out of groups.
   __device__ __forceinline__ static void run(uint32_t ring, uint32_t bars, const char* gb, const char* nb, int lane,
                                              bool active, uint32_t (&cnt)[15], uint4 (&rs)[4]) {
     if constexpr (J < kItemsPerGroup) {
-      constexpr int slot = J % D;
-      if (!LOCK || active) {
+      constexpr int slot = J % kRingSlots;
+      if (active) {
         const uint32_t sl = ring + slot * kItemBytes + lane * 16;
-        vt_mbar_wait(bars + slot * 8, (J / D) & 1);
+        vt_mbar_wait(bars + slot * 8, (J / kRingSlots) & 1);
         const uint4 lo0 = lds_u4(sl), hi0 = lds_u4(sl + 512), lo1 = lds_u4(sl + 1024), hi1 = lds_u4(sl + 1536);
         if constexpr (J < 15) {
           ref_row<2 * J + 1>(lo0, hi0, cnt);
@@ -658,51 +558,52 @@ struct RingItems {
         } else {
           rs[0] = lo0, rs[1] = hi0, rs[2] = lo1, rs[3] = hi1;
         }
-        // the slot's contents are in registers (the compares above consumed them): refill it with item J + D
+        // the slot's contents are in registers (the compares above consumed them): refill it with item J + kRingSlots
         __syncwarp();
         if (vt_elect_one()) {
-          if constexpr (J + D < kItemsPerGroup)
-            vt_ring_fill<pk_item_off(J + D), kItemBytes>(ring + slot * kItemBytes, gb, bars + slot * 8);
+          if constexpr (J + kRingSlots < kItemsPerGroup)
+            vt_ring_fill<pk_item_off(J + kRingSlots), kItemBytes>(ring + slot * kItemBytes, gb, bars + slot * 8);
           else if (nb != nullptr)
-            vt_ring_fill<pk_item_off((J + D) % kItemsPerGroup), kItemBytes>(ring + slot * kItemBytes, nb, bars + slot * 8);
+            vt_ring_fill<pk_item_off((J + kRingSlots) % kItemsPerGroup), kItemBytes>(ring + slot * kItemBytes, nb,
+                                                                                    bars + slot * 8);
         }
       }
-      if constexpr (LOCK) __syncthreads();
-      RingItems<D, J + 1, LOCK>::run(ring, bars, gb, nb, lane, active, cnt, rs);
+      __syncthreads();
+      RingItems<J + 1>::run(ring, bars, gb, nb, lane, active, cnt, rs);
     }
   }
 };
 
-template <int D, int NT, bool LOCK>
-__global__ void __launch_bounds__(NT, NT == 128 ? 5 : 1)  // 96 registers: the query planes stay constant-bank operands
+__global__ void __launch_bounds__(kPkThreads, kRingCtasPerSm)  // 96 registers: the query planes stay constant-bank operands
     k_vt_sweep_packed_ref_ring(const uint4* __restrict__ packed, long long n, long long base_index,
                                unsigned long long* __restrict__ key_out, uint32_t* __restrict__ scores,
                                const int* __restrict__ n_dev) {
-  static_assert(kItemsPerGroup % D == 0 && (kItemsPerGroup / D) % 2 == 0, "the parity of an item must not depend on the group");
+  static_assert(kItemsPerGroup % kRingSlots == 0 && (kItemsPerGroup / kRingSlots) % 2 == 0,
+                "the parity of an item must not depend on the group");
   extern __shared__ __align__(128) unsigned char vt_ring_smem[];
   if (n_dev != nullptr) n = *n_dev;
   const int lane = threadIdx.x & 31;
   const int wid = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);  // warp-uniform, and known to be
   const long long n_groups = (n + 31) >> 5;
-  const long long warp0 = (long long)blockIdx.x * (NT / 32) + wid;
-  const long long n_warps = (long long)gridDim.x * (NT / 32);
-  const uint32_t ring = vt_smem_u32(vt_ring_smem) + wid * D * kItemBytes;
-  const uint32_t bars = vt_smem_u32(vt_ring_smem) + (NT / 32) * D * kItemBytes + wid * D * 8;
+  const long long warp0 = (long long)blockIdx.x * (kPkThreads / 32) + wid;
+  const long long n_warps = (long long)gridDim.x * (kPkThreads / 32);
+  const uint32_t ring = vt_smem_u32(vt_ring_smem) + wid * kRingSlots * kItemBytes;
+  const uint32_t bars = vt_smem_u32(vt_ring_smem) + (kPkThreads / 32) * kRingSlots * kItemBytes + wid * kRingSlots * 8;
   constexpr long long kGroupBytes = (long long)kGroupU4 * 16;
   if (vt_elect_one()) {
 #pragma unroll
-    for (int s = 0; s < D; ++s) vt_mbar_init(bars + s * 8, 1);
+    for (int s = 0; s < kRingSlots; ++s) vt_mbar_init(bars + s * 8, 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     if (warp0 < n_groups) {
       const char* gb = reinterpret_cast<const char*>(packed) + warp0 * kGroupBytes;
-      RingPrologue<D, 0>::run(ring, bars, gb);
+      RingPrologue<0>::run(ring, bars, gb);
     }
   }
   __syncwarp();
   unsigned long long best = ~0ull;
-  // LOCK: every warp of the CTA makes as many rounds as its first warp (the one with the lowest group index)
-  for (long long g = warp0; (LOCK ? g - wid : g) < n_groups; g += n_warps) {
+  // every warp of the CTA makes as many rounds as its first warp (the one with the lowest group index)
+  for (long long g = warp0; g - wid < n_groups; g += n_warps) {
     const bool active = g < n_groups;
     const char* gb = reinterpret_cast<const char*>(packed) + g * kGroupBytes;
     const char* nb = (g + n_warps < n_groups) ? gb + n_warps * kGroupBytes : nullptr;
@@ -710,7 +611,7 @@ __global__ void __launch_bounds__(NT, NT == 128 ? 5 : 1)  // 96 registers: the q
 #pragma unroll
     for (int i = 0; i < 15; ++i) cnt[i] = 0;
     uint4 rs[4] = {};
-    RingItems<D, 0, LOCK>::run(ring, bars, gb, nb, lane, active, cnt, rs);
+    RingItems<0>::run(ring, bars, gb, nb, lane, active, cnt, rs);
     uint32_t R[32];
 #pragma unroll
     for (int w4 = 0; w4 < 4; ++w4) {
@@ -739,111 +640,31 @@ __global__ void __launch_bounds__(NT, NT == 128 ? 5 : 1)  // 96 registers: the q
       if (scores != nullptr) scores[ti] = m;
     }
   }
-  __shared__ unsigned long long sm[NT / 32];
+  __shared__ unsigned long long sm[kPkThreads / 32];
   best = warp_min_u64(best);
   if (lane == 0) sm[wid] = best;
   __syncthreads();
   if (threadIdx.x == 0) {
     unsigned long long k = sm[0];
 #pragma unroll
-    for (int i = 1; i < NT / 32; ++i) k = sm[i] < k ? sm[i] : k;
+    for (int i = 1; i < kPkThreads / 32; ++i) k = sm[i] < k ? sm[i] : k;
     if (k != ~0ull) atomicMin(key_out, k);
   }
 }
 
-// ---- float32 library, reference mode, fed the same way ----------------------------------------------------
-// k_vt_sweep_f32 loads a template's 30 rows into registers and only then starts to compare: a warp has nothing
-// in flight while it computes.  Here a warp owns a ring of D templates (rows 1..30 = 3840 contiguous bytes each,
-// one bulk copy), so D templates per warp are always on their way while one is being compared out of shared
-// memory.  Same arithmetic in the same order as k_vt_sweep_f32: the scores are bit-identical.
-constexpr int kF32ItemBytes = 30 * 32 * 4;
-constexpr int kF32RingThreads = 128;
-
-template <int D>
-__global__ void __launch_bounds__(kF32RingThreads)
-    k_vt_sweep_f32_ring(const float* __restrict__ lib, long long n, const float* __restrict__ query, long long base_index,
-                        unsigned long long* __restrict__ key_out, float* __restrict__ scores) {
-  using S = VtShape<PRS_VT_MODE_REF>;
-  extern __shared__ __align__(128) unsigned char vt_ring_smem[];
-  const int lane = threadIdx.x & 31;
-  const int wid = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);
-  const long long warp0 = (long long)blockIdx.x * (kF32RingThreads / 32) + wid;
-  const long long n_warps = (long long)gridDim.x * (kF32RingThreads / 32);
-  const uint32_t ring = vt_smem_u32(vt_ring_smem) + wid * D * kF32ItemBytes;
-  const uint32_t bars = vt_smem_u32(vt_ring_smem) + (kF32RingThreads / 32) * D * kF32ItemBytes + wid * D * 8;
-  const char* base = reinterpret_cast<const char*>(lib) + 128;  // row 1 of template 0
-  if (vt_elect_one()) {
-#pragma unroll
-    for (int s = 0; s < D; ++s) vt_mbar_init(bars + s * 8, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-#pragma unroll
-    for (int s = 0; s < D; ++s)
-      if (warp0 + s * n_warps < n)
-        vt_ring_fill<0, kF32ItemBytes>(ring + s * kF32ItemBytes, base + (warp0 + s * n_warps) * 4096, bars + s * 8);
-  }
-  __syncwarp();
-  float q[S::NS];
-#pragma unroll
-  for (int s = 0; s < S::NS; ++s) q[s] = query[(S::S0 + s) * 32 + lane];
-  unsigned long long best = ~0ull;
-  int slot = 0;
-  uint32_t parity = 0;
-  for (long long ti = warp0; ti < n; ti += n_warps) {
-    const uint32_t sl = ring + slot * kF32ItemBytes;
-    vt_mbar_wait(bars + slot * 8, parity);
-    float a[S::T1 - S::T0];
-#pragma unroll
-    for (int t = 0; t < S::T1 - S::T0; ++t)
-      asm volatile("ld.shared.f32 %0, [%1];" : "=f"(a[t]) : "r"(sl + t * 128 + lane * 4));
-    __syncwarp();
-    if (vt_elect_one()) {
-      const long long nt = ti + D * n_warps;
-      if (nt < n) vt_ring_fill<0, kF32ItemBytes>(sl, base + nt * 4096, bars + slot * 8);
-    }
-    if (++slot == D) {
-      slot = 0;
-      parity ^= 1u;
-    }
-    float acc[S::NACC];
-#pragma unroll
-    for (int i = 0; i < S::NACC; ++i) acc[i] = 0.f;
-#pragma unroll
-    for (int t = S::T0; t < S::T1; ++t) {
-#pragma unroll
-      for (int s = 0; s < S::NS; ++s) {
-        if (S::valid(t, S::S0 + s)) acc[S::off(t, S::S0 + s)] += fabsf(a[t - S::T0] - q[s]);
-      }
-    }
-    int obase = 0;
-    Butterfly<S::NACC, 16, float>::run(acc, lane, obase);
-    float m = (obase < S::NOFF) ? acc[0] : INFINITY;
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) m = fminf(m, __shfl_xor_sync(0xffffffffu, m, o));
-    unsigned long long key = ((unsigned long long)__float_as_uint(m) << 32) | (unsigned long long)(base_index + ti);
-    best = key < best ? key : best;
-    if (scores != nullptr && lane == 0) scores[ti] = m;
-  }
-  __shared__ unsigned long long sm[kF32RingThreads / 32];
-  best = warp_min_u64(best);
-  if (lane == 0) sm[wid] = best;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    unsigned long long k = sm[0];
-#pragma unroll
-    for (int i = 1; i < kF32RingThreads / 32; ++i) k = sm[i] < k ? sm[i] : k;
-    if (k != ~0ull) atomicMin(key_out, k);
-  }
-}
-
-// ---- float32, two columns per lane -------------------------------------------------------------------------
-// The ring kernel above is bound by instruction issue (ncu: 85 % of the issue slots, 2 instructions per
-// element-difference).  Here a lane owns two adjacent columns, so that the subtraction is one packed add.f32x2 for
+// ---- float32 library, reference mode: two columns per lane, fed by warp-private rings ------------------------
+// One template per warp with lane == column (k_vt_sweep_f32) is bound by instruction issue: two instructions per
+// element-difference.  Here a lane owns two adjacent columns, so that the subtraction is one packed add.f32x2 for
 // two differences (3 instructions per two) and a template needs only half a warp: a warp works on templates
-// 2i and 2i+1 at once, a ring slot holds both (two bulk copies on one barrier).  The slot is refilled after it has
-// been compared (the other D - 1 slots are in flight meanwhile).  The sums are formed in another order than in
-// k_vt_sweep_f32: scores agree to rounding (exactly, for integer-valued profiles), not bit for bit.
-template <int D>
+// 2i and 2i+1 at once.  Every warp owns a ring of kF32PairSlots slots, a slot holds both templates' rows 1..30 (two
+// bulk copies on one barrier) and is refilled after it has been compared, while the other slots are in flight.
+// Three slots and two CTAs per SM are the fastest of the depths and grid sizes measured
+// (profiles/r1_vt_ring_tuning.txt).  The sums are formed in another order than in k_vt_sweep_f32: scores agree to
+// rounding (exactly, for integer-valued profiles), not bit for bit.
+constexpr int kF32ItemBytes = 30 * 32 * 4;  // rows 1..30 of one template
+constexpr int kF32RingThreads = 128;
+constexpr int kF32PairSlots = 3;
+constexpr int kF32PairCtasPerSm = 2;
 __global__ void __launch_bounds__(kF32RingThreads)
     k_vt_sweep_f32_pair(const float* __restrict__ lib, long long n, const float* __restrict__ query, long long base_index,
                         unsigned long long* __restrict__ key_out, float* __restrict__ scores) {
@@ -855,8 +676,9 @@ __global__ void __launch_bounds__(kF32RingThreads)
   const long long warp0 = (long long)blockIdx.x * (kF32RingThreads / 32) + wid;
   const long long n_warps = (long long)gridDim.x * (kF32RingThreads / 32);
   constexpr int kSlot = 2 * kF32ItemBytes;
-  const uint32_t ring = vt_smem_u32(vt_ring_smem) + wid * D * kSlot;
-  const uint32_t bars = vt_smem_u32(vt_ring_smem) + (kF32RingThreads / 32) * D * kSlot + wid * D * 8;
+  const uint32_t ring = vt_smem_u32(vt_ring_smem) + wid * kF32PairSlots * kSlot;
+  const uint32_t bars =
+      vt_smem_u32(vt_ring_smem) + (kF32RingThreads / 32) * kF32PairSlots * kSlot + wid * kF32PairSlots * 8;
   const char* base = reinterpret_cast<const char*>(lib) + 128;  // row 1 of template 0
   auto fill = [&](uint32_t slot_addr, long long pi, uint32_t bar) {  // one elected lane
     const char* src = base + pi * 8192;
@@ -876,11 +698,11 @@ __global__ void __launch_bounds__(kF32RingThreads)
   };
   if (vt_elect_one()) {
 #pragma unroll
-    for (int s = 0; s < D; ++s) vt_mbar_init(bars + s * 8, 1);
+    for (int s = 0; s < kF32PairSlots; ++s) vt_mbar_init(bars + s * 8, 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
 #pragma unroll
-    for (int s = 0; s < D; ++s)
+    for (int s = 0; s < kF32PairSlots; ++s)
       if (warp0 + s * n_warps < n_pairs) fill(ring + s * kSlot, warp0 + s * n_warps, bars + s * 8);
   }
   __syncwarp();
@@ -912,13 +734,13 @@ __global__ void __launch_bounds__(kF32RingThreads)
         }
       }
     }
-    // every lane's loads have been consumed by the sums above: refill the slot with the pair D rounds ahead
+    // every lane's loads have been consumed by the sums above: refill the slot with the pair kF32PairSlots rounds ahead
     __syncwarp();
     if (vt_elect_one()) {
-      const long long np = pi + D * n_warps;
+      const long long np = pi + kF32PairSlots * n_warps;
       if (np < n_pairs) fill(sl, np, bars + slot * 8);
     }
-    if (++slot == D) {
+    if (++slot == kF32PairSlots) {
       slot = 0;
       parity ^= 1u;
     }
@@ -952,25 +774,21 @@ __global__ void __launch_bounds__(kF32RingThreads)
 // pair (i, s) always adds into register (i - s) mod 32, and the rotation re-labels the registers for the next
 // block.  32 register MOVs per block replace 256 shared-memory read-modify-writes.
 // eight stored rows (t0 .. t0+7, held in registers) against every query row; query row outermost so that only
-// its eight plane words are live as (uniform-register) operands at a time
-#ifndef PRS_VT_CIRC_SYNC_MASK
-#define PRS_VT_CIRC_SYNC_MASK 3
-#endif
-// LOCK: the warps of the CTA meet at a barrier after every four query rows (32 row pairs), so that they fetch the
-// same stretch of the unrolled code together; `active` is false for a warp that has run out of groups.
-template <bool LOCK>
+// its eight plane words are live as (uniform-register) operands at a time.
+// The warps of the CTA meet at a barrier after every four query rows (32 row pairs), so that they fetch the same
+// stretch of the unrolled code together; `active` is false for a warp that has run out of groups.
+constexpr int kCircSyncMask = 3;
 __device__ __forceinline__ void circ_block(const uint4 (&lo)[8], const uint4 (&hi)[8], uint32_t (&cnt)[32], bool active) {
 #pragma unroll
   for (int s = 0; s < 32; ++s) {
-    if (!LOCK || active) {
+    if (active) {
 #pragma unroll
       for (int i = 0; i < 8; ++i) cnt[(i - s) & 31] += lt_row(lo[i], hi[i], s);
     }
-    if (LOCK && (s & PRS_VT_CIRC_SYNC_MASK) == PRS_VT_CIRC_SYNC_MASK) __syncthreads();
+    if ((s & kCircSyncMask) == kCircSyncMask) __syncthreads();
   }
 }
 
-template <bool LOCK>
 __global__ void __launch_bounds__(kPkThreads, 4)
     k_vt_sweep_packed_circ(const uint4* __restrict__ packed, long long n, long long base_index,
                            unsigned long long* __restrict__ key_out, uint32_t* __restrict__ scores,
@@ -981,8 +799,8 @@ __global__ void __launch_bounds__(kPkThreads, 4)
   const long long warp0 = ((long long)blockIdx.x * kPkThreads + threadIdx.x) >> 5;
   const long long n_warps = ((long long)gridDim.x * kPkThreads) >> 5;
   unsigned long long best = ~0ull;
-  // LOCK: every warp of the CTA makes as many rounds as its first warp; one without a group only keeps the barriers
-  for (long long g = warp0; (LOCK ? g - wid : g) < n_groups; g += n_warps) {
+  // every warp of the CTA makes as many rounds as its first warp; one without a group only keeps the barriers
+  for (long long g = warp0; g - wid < n_groups; g += n_warps) {
     const bool active = g < n_groups;
     const uint4* gp = packed + (active ? g : 0) * kGroupU4 + lane;
     uint32_t cnt[32];
@@ -997,7 +815,7 @@ __global__ void __launch_bounds__(kPkThreads, 4)
         lo[i] = ld_stream_u4(gp + ((8 * c + i) * 2 + 0) * 32);
         hi[i] = ld_stream_u4(gp + ((8 * c + i) * 2 + 1) * 32);
       }
-      circ_block<LOCK>(lo, hi, cnt, active);
+      circ_block(lo, hi, cnt, active);
       uint32_t rot[32];
 #pragma unroll
       for (int r = 0; r < 32; ++r) rot[r] = cnt[(r + 8) & 31];
@@ -1035,78 +853,25 @@ __global__ void __launch_bounds__(kPkThreads, 4)
   }
 }
 
-static int g_vt_circ_lock = 1;  // knob 4: warps of a CTA in lock step in the circular sweep
-
-extern "C" int prs_vt_tune(int knob, int value) {
-  PRS_REQUIRE(knob >= 0 && knob <= 4, "prs_vt_tune: unknown knob %d", knob);
-  if (knob == 4) {
-    g_vt_circ_lock = value != 0;
-    return PRS_OK;
-  }
-  if (knob == 0) PRS_REQUIRE(value == 0 || value == 2 || value == 4 || value == 8 || value == 34 || value == 44,
-                             "prs_vt_tune: ring depth must be 0, 2, 4 or 8, or 34 / 44 for the lock-step variants");
-  if (knob == 2)
-    PRS_REQUIRE((value >= 0 && value <= 4) || (value >= 11 && value <= 13),
-                "prs_vt_tune: float32 ring depth must be in 0..4, or 11..13 for the column-pair kernel");
-  if (knob == 1 || knob == 3) PRS_REQUIRE(value >= 1 && value <= 32, "prs_vt_tune: CTAs per SM must be in 1..32");
-  g_vt_knob[knob] = value;
-  return PRS_OK;
-}
-
-template <int D>
-static int launch_f32_ring_d(int blocks, const float* lib, long long n, const float* query, long long base_index,
-                             unsigned long long* key_out, float* scores, cudaStream_t st) {
-  constexpr int smem = (kF32RingThreads / 32) * D * (kF32ItemBytes + 8);
-  if (smem > 48 * 1024)
-    PRS_CUDA(cudaFuncSetAttribute(k_vt_sweep_f32_ring<D>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-  k_vt_sweep_f32_ring<D><<<blocks, kF32RingThreads, smem, st>>>(lib, n, query, base_index, key_out, scores);
-  PRS_CUDA(cudaGetLastError());
-  return PRS_OK;
-}
-
-template <int D>
-static int launch_f32_pair_d(int blocks, const float* lib, long long n, const float* query, long long base_index,
-                             unsigned long long* key_out, float* scores, cudaStream_t st) {
-  constexpr int smem = (kF32RingThreads / 32) * D * (2 * kF32ItemBytes + 8);
-  if (smem > 48 * 1024)
-    PRS_CUDA(cudaFuncSetAttribute(k_vt_sweep_f32_pair<D>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-  k_vt_sweep_f32_pair<D><<<blocks, kF32RingThreads, smem, st>>>(lib, n, query, base_index, key_out, scores);
-  PRS_CUDA(cudaGetLastError());
-  return PRS_OK;
-}
-
-static int launch_f32_ring(int depth, int ctas_per_sm, const float* lib, long long n, const float* query,
-                           long long base_index, unsigned long long* key_out, float* scores, cudaStream_t st) {
-  if (depth >= 11) {  // two columns per lane, two templates per warp; ring depth = depth - 10
+extern "C" int prs_vt_sweep_f32(const float* lib, long long n, const float* query, int mode, long long base_index,
+                                unsigned long long* key_out, float* scores, void* stream) {
+  PRS_REQUIRE(query && key_out && n >= 0 && (lib || n == 0), "prs_vt_sweep_f32: bad argument");
+  PRS_REQUIRE(mode == PRS_VT_MODE_REF || mode == PRS_VT_MODE_CIRCULAR, "prs_vt_sweep_f32: unknown mode %d", mode);
+  PRS_REQUIRE(base_index >= 0 && base_index + n <= 0xffffffffLL, "prs_vt_sweep_f32: template index does not fit 32 bits");
+  cudaStream_t st = (cudaStream_t)stream;
+  PRS_CUDA(cudaMemsetAsync(key_out, 0xff, sizeof(unsigned long long), st));
+  if (n == 0) return PRS_OK;
+  if (mode == PRS_VT_MODE_REF) {
+    constexpr int smem = (kF32RingThreads / 32) * kF32PairSlots * (2 * kF32ItemBytes + 8);  // 92 KB: above the default
+    PRS_CUDA(cudaFuncSetAttribute(k_vt_sweep_f32_pair, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     const long long pairs = (n + 1) / 2;
     long long blocks = (pairs + (kF32RingThreads / 32) - 1) / (kF32RingThreads / 32);
-    if (blocks > 148LL * ctas_per_sm) blocks = 148LL * ctas_per_sm;
-    switch (depth - 10) {
-      case 1: return launch_f32_pair_d<1>((int)blocks, lib, n, query, base_index, key_out, scores, st);
-      case 2: return launch_f32_pair_d<2>((int)blocks, lib, n, query, base_index, key_out, scores, st);
-      default: return launch_f32_pair_d<3>((int)blocks, lib, n, query, base_index, key_out, scores, st);
-    }
+    if (blocks > 148LL * kF32PairCtasPerSm) blocks = 148LL * kF32PairCtasPerSm;
+    k_vt_sweep_f32_pair<<<(int)blocks, kF32RingThreads, smem, st>>>(lib, n, query, base_index, key_out, scores);
+  } else {
+    k_vt_sweep_f32<PRS_VT_MODE_CIRCULAR><<<sweep_grid(n), kVtThreads, 0, st>>>(lib, n, query, base_index, key_out, scores);
   }
-  long long blocks = (n + (kF32RingThreads / 32) - 1) / (kF32RingThreads / 32);
-  if (blocks > 148LL * ctas_per_sm) blocks = 148LL * ctas_per_sm;
-  switch (depth) {
-    case 1: return launch_f32_ring_d<1>((int)blocks, lib, n, query, base_index, key_out, scores, st);
-    case 2: return launch_f32_ring_d<2>((int)blocks, lib, n, query, base_index, key_out, scores, st);
-    case 3: return launch_f32_ring_d<3>((int)blocks, lib, n, query, base_index, key_out, scores, st);
-    default: return launch_f32_ring_d<4>((int)blocks, lib, n, query, base_index, key_out, scores, st);
-  }
-}
-
-template <int D, int NT, bool LOCK>
-static int launch_ref_ring(long long groups, int ctas_per_sm, const uint4* packed, long long n, long long base_index,
-                           unsigned long long* key_out, uint32_t* scores, const int* n_dev, cudaStream_t st) {
-  constexpr int smem = (NT / 32) * D * (kItemBytes + 8);
-  if (smem > 48 * 1024)  // per device; cheap enough to repeat
-    PRS_CUDA(cudaFuncSetAttribute(k_vt_sweep_packed_ref_ring<D, NT, LOCK>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-  long long blocks = (groups + (NT / 32) - 1) / (NT / 32);
-  if (blocks > 148LL * ctas_per_sm) blocks = 148LL * ctas_per_sm;
-  if (blocks < 1) blocks = 1;
-  k_vt_sweep_packed_ref_ring<D, NT, LOCK><<<(int)blocks, NT, smem, st>>>(packed, n, base_index, key_out, scores, n_dev);
+  PRS_CUDA(cudaGetLastError());
   return PRS_OK;
 }
 
@@ -1117,28 +882,13 @@ static int launch_packed_sweep(const uint4* packed, long long n, long long n_gri
   long long blocks = (groups + (kPkThreads / 32) - 1) / (kPkThreads / 32);
   if (blocks < 1) blocks = 1;
   if (mode == PRS_VT_MODE_REF) {
-    const int depth = g_vt_knob[0];
-    const long long cap = 148LL * (depth ? (int)g_vt_knob[1] : 16);
-    if (blocks > cap) blocks = cap;
-    int rc = PRS_OK;
-    const int cps = g_vt_knob[1];
-    switch (depth) {
-      case 2: rc = launch_ref_ring<2, 128, false>(groups, cps, packed, n, base_index, key_out, scores, n_dev, st); break;
-      case 4: rc = launch_ref_ring<4, 128, false>(groups, cps, packed, n, base_index, key_out, scores, n_dev, st); break;
-      case 8: rc = launch_ref_ring<8, 128, false>(groups, cps, packed, n, base_index, key_out, scores, n_dev, st); break;
-      // lock-step variants: the warps of a CTA meet at a barrier after every ring item
-      case 34: rc = launch_ref_ring<4, 128, true>(groups, cps, packed, n, base_index, key_out, scores, n_dev, st); break;
-      case 44: rc = launch_ref_ring<4, 640, true>(groups, 1, packed, n, base_index, key_out, scores, n_dev, st); break;
-      default:
-        k_vt_sweep_packed_ref<<<(int)blocks, kPkThreads, 0, st>>>(packed, n, base_index, key_out, scores, n_dev);
-    }
-    if (rc != PRS_OK) return rc;
+    constexpr int smem = (kPkThreads / 32) * kRingSlots * (kItemBytes + 8);
+    static_assert(smem <= 48 * 1024, "the rings fit the default limit of dynamic shared memory");
+    if (blocks > 148LL * kRingCtasPerSm) blocks = 148LL * kRingCtasPerSm;
+    k_vt_sweep_packed_ref_ring<<<(int)blocks, kPkThreads, smem, st>>>(packed, n, base_index, key_out, scores, n_dev);
   } else {
     if (blocks > 148LL * 16) blocks = 148LL * 16;
-    if (g_vt_circ_lock)
-      k_vt_sweep_packed_circ<true><<<(int)blocks, kPkThreads, 0, st>>>(packed, n, base_index, key_out, scores, n_dev);
-    else
-      k_vt_sweep_packed_circ<false><<<(int)blocks, kPkThreads, 0, st>>>(packed, n, base_index, key_out, scores, n_dev);
+    k_vt_sweep_packed_circ<<<(int)blocks, kPkThreads, 0, st>>>(packed, n, base_index, key_out, scores, n_dev);
   }
   PRS_CUDA(cudaGetLastError());
   return PRS_OK;

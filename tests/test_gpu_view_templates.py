@@ -123,7 +123,7 @@ def _sweep_packed(lib, q, mode, want_scores=True):
 
 
 @pytest.mark.parametrize("mode", ["ref", "circular"])
-@pytest.mark.parametrize("n", [0, 1, 2, 31, 32, 33, 64, 1001])
+@pytest.mark.parametrize("n", [0, 1, 2, 31, 32, 33, 64, 1001, 2077])
 def test_packed_library_matches_oracle(mode, n):
     rng = np.random.default_rng(200 + n)
     lib = rng.integers(0, 256, (n, 32, 32), dtype=np.uint8)
@@ -179,6 +179,15 @@ def test_float32_library(mode):
     ref = ovt.library_scores(libr.astype(np.float64), qr.astype(np.float64), mode=mode)
     assert key & 0xFFFFFFFF == int(np.argmin(ref)) == 123
     assert np.abs(sc - ref).max() <= 1e-5 * ref.max()
+    # ragged library sizes: the key is the oracle's arg-min and the smallest of the returned scores
+    for n in (1, 31, 33, 2077):
+        libn = rng.uniform(0, 255, (n, 32, 32)).astype(np.float32)
+        qn = rng.uniform(0, 255, (32, 32)).astype(np.float32)
+        key, sc = _sweep(torch.from_numpy(libn).cuda(), torch.from_numpy(qn).cuda(), 0 if mode == "ref" else 1)
+        ref = ovt.library_scores(libn.astype(np.float64), qn.astype(np.float64), mode=mode)
+        assert np.abs(sc - ref).max() <= 1e-4 * ref.max(), n
+        assert key & 0xFFFFFFFF == int(np.argmin(ref)), n
+        assert np.array([key >> 32], dtype=np.uint32).view(np.float32)[0] == sc.min(), n
 
 
 def test_extract_matches_mask():
@@ -316,55 +325,59 @@ def test_replay_from_rosbag(golden, tmp_path, compression):
         assert np.array_equal(a[k], b[k]), k
 
 
-def test_sweep_variants_agree():
-    """Every kernel variant behind prs_vt_tune (register-prefetch kernels, ring depths, grid sizes) and the small-library
-    kernel of the frame chain produce the same key and the same per-template scores, on ragged library sizes."""
+def test_big_library_sweeps_back_to_back():
+    """Six queries enqueued back to back, without a synchronisation, each with its own key and score buffers, against
+    libraries big enough that every warp of the uint8 ring sweep refills its ring across groups (more than 94 720
+    templates) and the float32 pair sweep wraps its three-slot ring (more than 7 104).  The bit-sliced sweeps equal
+    the byte-wise kernel bit for bit; the float32 sweep of integer-valued profiles (exact sums) equals
+    prs_vt_sweep_any_f32."""
     from pyratslam_b200 import _native as nat
     L = nat.lib()
-    rng = np.random.default_rng(11)
-    key = torch.zeros(1, dtype=torch.int64, device="cuda")
-    scratch = torch.zeros(4096, dtype=torch.uint8, device="cuda")
-    try:
-        for n in (1, 31, 33, 2077):
-            lib = torch.from_numpy(rng.integers(0, 256, (n, 32, 32), dtype=np.uint8)).cuda()
-            q = torch.from_numpy(rng.integers(0, 256, (32, 32), dtype=np.uint8)).cuda()
-            packed = torch.zeros(int(L.prs_vt_packed_bytes(n)), dtype=torch.uint8, device="cuda")
-            nat.check(L.prs_vt_pack_u8(lib.data_ptr(), n, packed.data_ptr(), 0, nat.stream_ptr()))
-            want = ovt.library_scores(lib.cpu().numpy(), q.cpu().numpy()).astype(np.int64)
-            for depth, ctas in ((0, 1), (2, 1), (2, 5), (4, 5), (8, 3), (34, 5), (34, 2), (44, 1)):
-                nat.check(L.prs_vt_tune(0, depth))
-                nat.check(L.prs_vt_tune(1, ctas))
-                sc = torch.zeros(n, dtype=torch.int32, device="cuda")
-                nat.check(L.prs_vt_sweep_packed_u8(packed.data_ptr(), n, q.data_ptr(), 0, 0, key.data_ptr(), sc.data_ptr(),
-                                                   scratch.data_ptr(), nat.stream_ptr()))
-                assert sc.cpu().numpy().astype(np.int64).tolist() == want.tolist(), (n, depth, ctas)
-                k = int(key.item()) & (2 ** 64 - 1)
-                assert (k >> 32, k & 0xFFFFFFFF) == (int(want.min()), int(np.argmin(want))), (n, depth, ctas)
-            libf = lib.to(torch.float32) + torch.from_numpy(rng.uniform(0, 1, (n, 32, 32)).astype(np.float32)).cuda()
-            qf = q.to(torch.float32)
-            ref = None
-            for depth, ctas in ((0, 1), (1, 8), (2, 3), (3, 2), (4, 1), (11, 6), (12, 3), (13, 2)):
-                nat.check(L.prs_vt_tune(2, depth))
-                nat.check(L.prs_vt_tune(3, ctas))
-                sc = torch.zeros(n, dtype=torch.float32, device="cuda")
-                nat.check(L.prs_vt_sweep_f32(libf.data_ptr(), n, qf.data_ptr(), 0, 0, key.data_ptr(), sc.data_ptr(),
-                                             nat.stream_ptr()))
-                got = (int(key.item()) & (2 ** 64 - 1), sc.cpu().numpy())
-                if ref is None:
-                    ref = got
-                    exact = ovt.library_scores(libf.cpu().numpy().astype(np.float64), qf.cpu().numpy().astype(np.float64))
-                    assert np.abs(got[1] - exact).max() <= 1e-4 * exact.max()
-                elif depth < 10:   # same arithmetic in the same order: bit-identical
-                    assert got[0] == ref[0] and np.array_equal(got[1], ref[1]), (n, depth, ctas)
-                else:              # column-pair kernel: another summation order, same arg-min
-                    assert got[0] & 0xFFFFFFFF == ref[0] & 0xFFFFFFFF, (n, depth, ctas)
-                    assert np.abs(got[1] - ref[1]).max() <= 1e-5 * ref[1].max(), (n, depth, ctas)
-                    assert np.abs(got[1] - exact).max() <= 1e-4 * exact.max()
-        with pytest.raises(ValueError):
-            nat.check(L.prs_vt_tune(0, 3))
-    finally:   # the measured defaults (csrc/view_templates.cu)
-        for knob, val in enumerate((34, 5, 13, 2)):
-            L.prs_vt_tune(knob, val)
+    st = nat.stream_ptr()
+    g = torch.Generator(device="cuda").manual_seed(12)
+    n = (1 << 17) + 77
+    lib = torch.randint(0, 256, (n, 32, 32), dtype=torch.uint8, device="cuda", generator=g)
+    packed = torch.zeros(int(L.prs_vt_packed_bytes(n)), dtype=torch.uint8, device="cuda")
+    nat.check(L.prs_vt_pack_u8(lib.data_ptr(), n, packed.data_ptr(), 0, st))
+    nf = (1 << 17) + 5
+    libf = torch.randint(0, 256, (nf, 32, 32), dtype=torch.float32, device="cuda", generator=g)
+
+    def rand_u8():
+        return torch.randint(0, 256, (32, 32), dtype=torch.uint8, device="cuda", generator=g)
+    # (kind, mode, query, index of the planted template or None)
+    sweeps = [("u8", 0, (lib[n - 3].to(torch.int16) - 2).clamp(0, 255).to(torch.uint8), n - 3),
+              ("u8", 0, rand_u8(), None),
+              ("u8", 1, torch.roll(lib[70000], 5, 0), 70000),
+              ("u8", 1, rand_u8(), None),
+              ("f32", 0, torch.roll(libf[nf - 1], 3, 0), nf - 1),
+              ("f32", 0, rand_u8().to(torch.float32), None)]
+    keys = torch.zeros(len(sweeps), dtype=torch.int64, device="cuda")
+    scores, scratch = [], [torch.zeros(4096, dtype=torch.uint8, device="cuda") for _ in sweeps]
+    for i, (kind, mode, q, _) in enumerate(sweeps):
+        if kind == "u8":
+            scores.append(torch.zeros(n, dtype=torch.int32, device="cuda"))
+            nat.check(L.prs_vt_sweep_packed_u8(packed.data_ptr(), n, q.data_ptr(), mode, 0, keys[i:].data_ptr(),
+                                               scores[i].data_ptr(), scratch[i].data_ptr(), st))
+        else:
+            scores.append(torch.zeros(nf, dtype=torch.float32, device="cuda"))
+            nat.check(L.prs_vt_sweep_f32(libf.data_ptr(), nf, q.data_ptr(), mode, 0, keys[i:].data_ptr(),
+                                         scores[i].data_ptr(), st))
+    torch.cuda.synchronize()
+    for i, (kind, mode, q, planted) in enumerate(sweeps):
+        want_key = torch.zeros(1, dtype=torch.int64, device="cuda")
+        if kind == "u8":
+            want = torch.zeros(n, dtype=torch.int32, device="cuda")
+            nat.check(L.prs_vt_sweep_u8(lib.data_ptr(), n, q.data_ptr(), mode, 0, want_key.data_ptr(), want.data_ptr(),
+                                        st))
+        else:
+            want = torch.zeros(nf, dtype=torch.float32, device="cuda")
+            nat.check(L.prs_vt_sweep_any_f32(libf.data_ptr(), nf, q.data_ptr(), 32, 32, 8, 0, want_key.data_ptr(),
+                                             want.data_ptr(), st))
+        torch.cuda.synchronize()
+        assert int(keys[i]) == int(want_key[0]), i
+        assert torch.equal(scores[i].view(torch.int32), want.view(torch.int32)), i
+        if planted is not None:
+            assert int(keys[i]) & 0xFFFFFFFF == planted, i
 
 
 def test_native_replay_matches_frame_by_frame():
