@@ -416,6 +416,26 @@ PRS_API int prs_ens_refresh_room(prs_ens_plan* plan, void* stream);
  * non-default stream).  PRS_E_INVALID when the libraries have no room for the ticks with an image. */
 PRS_API int prs_ens_run(prs_ens_plan* plan, const uint8_t* const* frames, const double* odom, const uint8_t* gate,
                 const int* n_images, int T, prs_frame_result* results, void* stream);
+/* Ticks of one device chunk (the image slots of the scratch; at most 256). */
+PRS_API int prs_ens_chunk(prs_ens_plan* plan);
+/* Pose-cell activity capture: at every tick, each agent whose recording has an image gets an entry computed from the
+ * state its match is made with -- after the tick's update (and a mixed tick's restore), before its injection: the
+ * count of cells with (double)value > threshold and the first max_cells of them in C order [x][y][th], each an int32
+ * flat index x*Y*Th + y*Th + th and its value in the state's dtype.  Agents without an image at the tick get count -1.
+ * The capture is one node of the image ticks' graphs (on the update's branch, or before the decision on a tick without
+ * update); a plan without it has no such node.  Setting it drops the captured graphs, as prs_frame_set_inject does.
+ *   threshold : finite; max_cells in [0, X*Y*Th] (0: counts only)
+ *   buffer    : device, prs_ens_activity_bytes(plan, max_cells) bytes, owned by the caller; NULL turns the capture off
+ * With the capture on a run takes at most prs_ens_chunk(plan) ticks.  After a run, prs_ens_activity_pack packs the
+ * kept cells of its ticks into one device prefix ([tick][agent] row-major, min(count, max_cells) cells per entry),
+ * copies the counts to counts (host int32 [T][B]) and the number of packed cells to *total, and synchronises
+ * `stream`; prs_ens_activity_copy then copies the first n packed cells to idx (host int32 [n]) and val (host, n values
+ * of the state's dtype) and synchronises.  Host memory and bus traffic scale with the cells kept, not with max_cells.
+ * prs_ens_activity_bytes returns 0 for a max_cells outside the range. */
+PRS_API size_t prs_ens_activity_bytes(prs_ens_plan* plan, int max_cells);
+PRS_API int prs_ens_set_activity(prs_ens_plan* plan, double threshold, int max_cells, void* buffer);
+PRS_API int prs_ens_activity_pack(prs_ens_plan* plan, int* counts, long long* total, void* stream);
+PRS_API int prs_ens_activity_copy(prs_ens_plan* plan, long long n, int* idx, void* val, void* stream);
 /* Agent copies between a plan's rows (an ensemble session's reassignment of agents): move m makes row dst[m] an exact
  * copy of row src[m] as it was before the call -- the state slice, the pc_work slots, n_dev, the library groups of its
  * n_dev templates and the first n_dev entries of its location row.  Slots past n_dev are never read and an append

@@ -99,6 +99,11 @@ _SIGNATURES["prs_ens_create"] = (c_int, [c_void_p, c_void_p, c_void_p, c_void_p,
 _SIGNATURES["prs_ens_destroy"] = (c_int, [c_void_p])
 _SIGNATURES["prs_ens_refresh_room"] = (c_int, [c_void_p, c_void_p])
 _SIGNATURES["prs_ens_run"] = (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p])
+_SIGNATURES["prs_ens_chunk"] = (c_int, [c_void_p])
+_SIGNATURES["prs_ens_activity_bytes"] = (c_size_t, [c_void_p, c_int])
+_SIGNATURES["prs_ens_set_activity"] = (c_int, [c_void_p, c_double, c_int, c_void_p])
+_SIGNATURES["prs_ens_activity_pack"] = (c_int, [c_void_p, c_void_p, c_void_p, c_void_p])
+_SIGNATURES["prs_ens_activity_copy"] = (c_int, [c_void_p, c_longlong, c_void_p, c_void_p, c_void_p])
 _SIGNATURES["prs_ens_copy_stage_bytes"] = (c_size_t, [c_void_p, c_int, c_void_p, c_void_p, c_void_p])
 _SIGNATURES["prs_ens_copy_agents"] = (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t,
                                               c_void_p])

@@ -31,6 +31,7 @@
 #include <string.h>
 
 #include <algorithm>
+#include <cmath>
 #include <mutex>
 #include <vector>
 
@@ -1715,7 +1716,7 @@ extern "C" int prs_replay_run(prs_frame_plan* const* plans, int n_plans, const u
 // tick is ONE graph for the whole ensemble:
 //   side branch  k_ens_odom_multi (each network its recording's twist, (0, 0) where that recording did not move or has
 //                ended) -> [mixed: k_ens_snapshot save] -> prs_pc_step -> [mixed: k_ens_snapshot restore ->
-//                prs_pc_active_invalidate]
+//                prs_pc_active_invalidate] -> [activity: k_ens_activity]
 //   template     k_vt_frame_prepare_multi (one block per recording) -> k_vt_sweep_packed_ref_small<true> over every
 //                agent's library (grid-stride over (agent, group))
 //   join         k_vt_decide_append, one warp per agent -> [k_frame_inject, one thread per agent] -> k_ens_advance (the
@@ -1725,6 +1726,8 @@ extern "C" int prs_replay_run(prs_frame_plan* const* plans, int n_plans, const u
 // every recording moved needs no snapshot, so with R = 1 no tick is mixed.  A tick without an image in any recording
 // is lean: the side branch's nodes run on the tick's stream itself, then k_ens_no_image writes the records and advances
 // the counter -- no query, sweep, decision or injection.  Six graphs: {no update, all moved, mixed} x {image, none}.
+// With the activity capture on (prs_ens_set_activity), an image tick without update runs k_ens_activity on the main
+// stream before the decision; a lean tick captures nothing.
 // Images, odometry, gates and image slots go to the device a chunk of ticks at a time, the records [chunk][B] come
 // back a chunk at a time.
 constexpr int kEnsChunk = 256;
@@ -1842,6 +1845,159 @@ __global__ void k_ens_init(const int* __restrict__ n_dev, int B, int* __restrict
   }
 }
 
+// ---------------------------------------------------------------------------------------------
+// Pose-cell activity capture (prs_ens_set_activity, DESIGN.md 4.15): at every tick with an image, each agent's cells
+// above a threshold in the state its match is made with -- after the tick's update (and a mixed tick's restore),
+// before its injection -- as the viewers draw them (cells > 0.002).  An entry is the count of such cells and the first
+// K of them in the reference's C order [x][y][th]: an int32 flat index x*Y*Th + y*Th + th and the state's value.
+// Entries live in slots [chunk][B][K] indexed by the tick counter; after a run, k_ens_activity_scan and
+// k_ens_activity_gather pack the kept cells of the run's ticks into one prefix, so what crosses the bus scales with the
+// captured cells, not with B * K * ticks.
+constexpr int kActThreads = 512;
+
+// Buffer of the capture (prs_ens_activity_bytes), every part 256-byte aligned: counts int32 [chunk][B] (-1 = no image),
+// slots int32 idx [chunk][B][K] and T val [chunk][B][K], the packed offsets int64 [chunk * B + 1] (the last one is the
+// total) and the packed idx and val [chunk * B * K].
+struct EnsActivity {
+  size_t counts = 0, idx = 0, val = 0, off = 0, pidx = 0, pval = 0, bytes = 0;
+  EnsActivity() = default;
+  EnsActivity(int B, int chunk, int K, int es) {
+    auto up = [](size_t v) { return (v + 255) & ~(size_t)255; };
+    const size_t rows = (size_t)chunk * B, cells = rows * K;
+    counts = 0;
+    idx = counts + up(rows * sizeof(int));
+    val = idx + up(cells * sizeof(int));
+    off = val + up(cells * es);
+    pidx = off + up((rows + 1) * sizeof(long long));
+    pval = pidx + up(cells * sizeof(int));
+    bytes = pval + up(cells * es);
+  }
+};
+
+// Block-wide exclusive scan of one int per thread (blockDim a multiple of 32, at most 1024); `total` gets the sum.
+__device__ __forceinline__ int act_block_scan(int v, int* total) {
+  __shared__ int warp_sum[32];
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5, nw = blockDim.x >> 5;
+  int x = v;
+#pragma unroll
+  for (int d = 1; d < 32; d <<= 1) {
+    const int y = __shfl_up_sync(0xffffffffu, x, d);
+    if (lane >= d) x += y;
+  }
+  __syncthreads();  // warp_sum of an earlier call has been read
+  if (lane == 31) warp_sum[w] = x;
+  __syncthreads();
+  if (w == 0) {
+    int s = lane < nw ? warp_sum[lane] : 0;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+      const int y = __shfl_up_sync(0xffffffffu, s, d);
+      if (lane >= d) s += y;
+    }
+    if (lane < nw) warp_sum[lane] = s;  // inclusive sums of the warps
+  }
+  __syncthreads();
+  *total = warp_sum[nw - 1];
+  return x - v + (w > 0 ? warp_sum[w - 1] : 0);
+}
+
+// One CTA per network.  The state is theta-major [B][Th][X][Y], so line p = x*Y + y of plane th sits at th*X*Y + p and a
+// thread owns lines p0 + threadIdx.x of consecutive rounds p0: its loads are coalesced across the block, and C order is
+// line-major (flat = p*Th + th), so a block scan of the per-line counts in each round gives every cell its C-order rank
+// -- deterministic, no sort.  A second, cached read of the (few) lines with kept cells writes them.  An agent whose
+// recording has no image at the tick gets count -1 (bit 0 of the tick's gate, as k_ens_odom_multi reads bit 1).
+template <typename T>
+__global__ void __launch_bounds__(kActThreads, 2)
+    k_ens_activity(const T* __restrict__ state, int P, int Th, double thr, int K, const uint8_t* __restrict__ gate,
+                   const int* __restrict__ ctr, const int* __restrict__ rec_of, int R, int B, int* __restrict__ counts,
+                   int* __restrict__ idx, T* __restrict__ val) {
+  const int b = blockIdx.x, c = *ctr;
+  const size_t row = (size_t)c * B + b;
+  if (!(gate[(size_t)c * R + rec_of[b]] & 1)) {
+    if (threadIdx.x == 0) counts[row] = -1;
+    return;
+  }
+  const T* s = state + (size_t)b * P * Th;
+  int* out_idx = idx + row * K;
+  T* out_val = val + row * K;
+  int base = 0;  // cells of the earlier rounds
+  for (int p0 = 0; p0 < P; p0 += blockDim.x) {
+    const int p = p0 + threadIdx.x;
+    int n = 0;
+    if (p < P) {
+#pragma unroll 6
+      for (int th = 0; th < Th; ++th) n += (double)s[(size_t)th * P + p] > thr ? 1 : 0;  // independent loads in flight
+    }
+    int total;
+    int o = base + act_block_scan(n, &total);
+    if (n > 0 && o < K) {
+      for (int th = 0; th < Th && o < K; ++th) {
+        const T v = s[(size_t)th * P + p];
+        if ((double)v > thr) {
+          out_idx[o] = p * Th + th;
+          out_val[o] = v;
+          ++o;
+        }
+      }
+    }
+    base += total;
+  }
+  if (threadIdx.x == 0) counts[row] = base;
+}
+
+// After a run of n = ticks * B entries: entries of agents without an image at the tick (the lean ticks' rows are never
+// written) become -1, and off[i] = sum of min(count, K) over the entries before i, off[n] the total.  One block: each
+// thread a contiguous segment, a block scan of the segment sums (in 64 bits).
+constexpr int kActScanThreads = 512;
+__global__ void __launch_bounds__(kActScanThreads)
+    k_ens_activity_scan(int* __restrict__ counts, const uint8_t* __restrict__ gate, const int* __restrict__ rec_of, int R,
+                        int B, long long n, int K, long long* __restrict__ off) {
+  __shared__ long long part[kActScanThreads];
+  const long long per = (n + kActScanThreads - 1) / kActScanThreads;
+  const long long i0 = threadIdx.x * per < n ? threadIdx.x * per : n, i1 = i0 + per < n ? i0 + per : n;
+  long long t = i0 / B;
+  int b = (int)(i0 - t * B);
+  long long sum = 0;
+  for (long long i = i0; i < i1; ++i) {
+    int cnt = counts[i];
+    if (!(gate[t * R + rec_of[b]] & 1)) counts[i] = cnt = -1;
+    sum += cnt < 0 ? 0 : cnt < K ? cnt : K;
+    if (++b == B) b = 0, ++t;
+  }
+  part[threadIdx.x] = sum;
+  __syncthreads();
+  for (int d = 1; d < kActScanThreads; d <<= 1) {
+    const long long y = (int)threadIdx.x >= d ? part[threadIdx.x - d] : 0;
+    __syncthreads();
+    part[threadIdx.x] += y;
+    __syncthreads();
+  }
+  long long o = part[threadIdx.x] - sum;
+  for (long long i = i0; i < i1; ++i) {
+    off[i] = o;
+    const int cnt = counts[i];
+    o += cnt < 0 ? 0 : cnt < K ? cnt : K;
+  }
+  if (threadIdx.x == kActScanThreads - 1) off[n] = part[threadIdx.x];
+}
+
+// One warp per entry: its min(count, K) kept cells to the packed prefix at off[i].
+template <typename T>
+__global__ void k_ens_activity_gather(const int* __restrict__ counts, const long long* __restrict__ off,
+                                      const int* __restrict__ idx, const T* __restrict__ val, long long n, int K,
+                                      int* __restrict__ pidx, T* __restrict__ pval) {
+  const long long i = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (i >= n) return;
+  const int cnt = counts[i];
+  const int k = cnt < 0 ? 0 : cnt < K ? cnt : K;
+  const long long o = off[i];
+  for (int j = lane; j < k; j += 32) {
+    pidx[o + j] = idx[i * K + j];
+    pval[o + j] = val[i * K + j];
+  }
+}
+
 struct prs_ens_plan {
   prs_pc_handle pc;
   void *pc_state, *pc_work, *libs;
@@ -1863,6 +2019,11 @@ struct prs_ens_plan {
   int warm[6];
   cudaStream_t side;
   cudaEvent_t ev_fork, ev_join;
+  // prs_ens_set_activity: the capture buffer (null = no capture node), its threshold and cells per entry, and the
+  // ticks of the last run, which prs_ens_activity_pack packs
+  char* act = nullptr;
+  double act_thr = 0.0;
+  int act_k = 0, act_ticks = 0;
 };
 
 static size_t ens_net_bytes(const prs_pc_plan* pc) { return (size_t)pc->N * (pc->dtype == PRS_F32 ? 4 : 8); }
@@ -1884,6 +2045,21 @@ static int ens_tick_enqueue(prs_ens_plan* e, int v, bool image, cudaStream_t st)
   uint8_t* d_still = (uint8_t*)(sc + M.still);
   const int B = e->B, R = e->R;
   const cudaStream_t side = image ? e->side : st;
+  // the activity capture (image ticks only): the state the tick's match is made with, before its injection
+  auto activity = [&](cudaStream_t s) {
+    const EnsActivity A(B, M.chunk, e->act_k, pc->dtype == PRS_F32 ? 4 : 8);
+    const int P = pc->X * pc->Y;
+    const int threads = P >= kActThreads ? kActThreads : (P + 31) / 32 * 32;
+    if (pc->dtype == PRS_F32)
+      k_ens_activity<float><<<B, threads, 0, s>>>((const float*)e->pc_state, P, pc->Th, e->act_thr, e->act_k, d_gate,
+                                                  d_ctr, e->rec_of, R, B, (int*)(e->act + A.counts),
+                                                  (int*)(e->act + A.idx), (float*)(e->act + A.val));
+    else
+      k_ens_activity<double><<<B, threads, 0, s>>>((const double*)e->pc_state, P, pc->Th, e->act_thr, e->act_k, d_gate,
+                                                   d_ctr, e->rec_of, R, B, (int*)(e->act + A.counts),
+                                                   (int*)(e->act + A.idx), (double*)(e->act + A.val));
+    return cudaGetLastError();
+  };
   int rc;
   if (v != 0) {
     if (image) {  // fork: the pose-cell update does not depend on the images until the decision
@@ -1926,6 +2102,8 @@ static int ens_tick_enqueue(prs_ens_plan* e, int v, bool image, cudaStream_t st)
       PRS_CUDA(snapshot(true));
       if (int rc_ = prs_pc_active_invalidate(pc, side)) return rc_;  // the carried lists describe the undone update
     }
+    // on the side branch, beside the sweep: only reads the state, so the active-set lists stay valid
+    if (image && e->act) PRS_CUDA(activity(side));
     if (image) PRS_CUDA(cudaEventRecord(e->ev_join, e->side));
   }
   if (!image) {
@@ -1950,6 +2128,7 @@ static int ens_tick_enqueue(prs_ens_plan* e, int v, bool image, cudaStream_t st)
         (const uint4*)e->libs, (const uint32_t*)(sc + M.planes), d_key, e->n_dev, B, e->lib_u4, d_gmax, e->rec_of,
         d_present);
   if (v != 0) PRS_CUDA(cudaStreamWaitEvent(st, e->ev_join, 0));  // the decision reports the new arg-max
+  if (v == 0 && e->act) PRS_CUDA(activity(st));                 // no update: the state as the last tick left it
   VtAgents ag;
   ag.B = B;
   ag.lib_u4 = e->lib_u4;
@@ -2094,6 +2273,8 @@ extern "C" int prs_ens_run(prs_ens_plan* e, const uint8_t* const* frames, const 
   const int R = e->R;
   // slots[t][r]: recording r's image at tick t, counted from the first image of t's chunk; -1 = none
   const EnsScratch& M = e->lay;
+  PRS_REQUIRE(!e->act || T <= M.chunk, "prs_ens_run: with the activity capture on, a run takes at most %d ticks, got %d",
+              M.chunk, T);
   std::vector<int> slots((size_t)T * R);
   std::vector<uint8_t> variant(T), has_image(T);
   std::vector<int> seen(R, 0), in_chunk(R, 0);
@@ -2127,6 +2308,7 @@ extern "C" int prs_ens_run(prs_ens_plan* e, const uint8_t* const* frames, const 
   const size_t rec_bytes = (size_t)e->B * sizeof(prs_frame_result);
   std::vector<long long> first(R, 0);  // each recording's first image of the chunk
   int rc = PRS_OK;
+  e->act_ticks = 0;
   for (int c0 = 0; c0 < T && rc == PRS_OK; c0 += M.chunk) {
     const int n = T - c0 < M.chunk ? T - c0 : M.chunk;
     long long img_ticks = 0;
@@ -2154,6 +2336,7 @@ extern "C" int prs_ens_run(prs_ens_plan* e, const uint8_t* const* frames, const 
       PRS_CUDA(cudaMemcpyAsync(results + (size_t)c0 * e->B, ms + M.rec, (size_t)done * rec_bytes, cudaMemcpyDeviceToHost,
                                st));
     e->room -= img_ticks;
+    e->act_ticks = done;
   }
   const cudaError_t err = cudaStreamSynchronize(st);
   if (rc == PRS_OK && err != cudaSuccess) {
@@ -2161,6 +2344,79 @@ extern "C" int prs_ens_run(prs_ens_plan* e, const uint8_t* const* frames, const 
     return PRS_E_CUDA;
   }
   return rc;
+}
+
+extern "C" int prs_ens_chunk(prs_ens_plan* e) { return e ? e->lay.chunk : 0; }
+
+extern "C" size_t prs_ens_activity_bytes(prs_ens_plan* e, int max_cells) {
+  if (!e || max_cells < 0 || max_cells > e->pc->N) return 0;
+  return EnsActivity(e->B, e->lay.chunk, max_cells, e->pc->dtype == PRS_F32 ? 4 : 8).bytes;
+}
+
+// Turning the capture on or off, or changing its threshold or cells per entry, adds or changes a node of the image
+// ticks: the captured graphs go, as in prs_frame_set_inject.
+extern "C" int prs_ens_set_activity(prs_ens_plan* e, double threshold, int max_cells, void* buffer) {
+  PRS_REQUIRE(e, "prs_ens_set_activity: null plan");
+  if (buffer != nullptr) {
+    PRS_REQUIRE(std::isfinite(threshold), "prs_ens_set_activity: the threshold must be finite, got %g", threshold);
+    PRS_REQUIRE(max_cells >= 0 && max_cells <= e->pc->N,
+                "prs_ens_set_activity: max_cells %d outside [0, %lld]", max_cells, (long long)e->pc->N);
+  }
+  for (int i = 0; i < 6; ++i) {
+    if (e->ready[i]) cudaGraphExecDestroy(e->exec[i]);
+    e->ready[i] = false;
+    e->warm[i] = 0;
+  }
+  e->act = (char*)buffer;
+  e->act_thr = buffer ? threshold : 0.0;
+  e->act_k = buffer ? max_cells : 0;
+  e->act_ticks = 0;
+  return PRS_OK;
+}
+
+extern "C" int prs_ens_activity_pack(prs_ens_plan* e, int* counts, long long* total, void* stream) {
+  PRS_REQUIRE(e && e->act && counts && total && stream, "prs_ens_activity_pack: bad argument (or no capture)");
+  const cudaStream_t st = (cudaStream_t)stream;
+  const int es = e->pc->dtype == PRS_F32 ? 4 : 8;
+  const EnsActivity A(e->B, e->lay.chunk, e->act_k, es);
+  const long long n = (long long)e->act_ticks * e->B;
+  char* a = e->act;
+  *total = 0;
+  if (n == 0) return PRS_OK;
+  k_ens_activity_scan<<<1, kActScanThreads, 0, st>>>((int*)(a + A.counts), (const uint8_t*)(e->scratch + e->lay.gate), e->rec_of,
+                                          e->R, e->B, n, e->act_k, (long long*)(a + A.off));
+  PRS_CUDA(cudaGetLastError());
+  if (e->act_k > 0) {
+    const unsigned grid = (unsigned)((n * 32 + 255) / 256);
+    if (es == 4)
+      k_ens_activity_gather<float><<<grid, 256, 0, st>>>((const int*)(a + A.counts), (const long long*)(a + A.off),
+                                                         (const int*)(a + A.idx), (const float*)(a + A.val), n, e->act_k,
+                                                         (int*)(a + A.pidx), (float*)(a + A.pval));
+    else
+      k_ens_activity_gather<double><<<grid, 256, 0, st>>>((const int*)(a + A.counts), (const long long*)(a + A.off),
+                                                          (const int*)(a + A.idx), (const double*)(a + A.val), n,
+                                                          e->act_k, (int*)(a + A.pidx), (double*)(a + A.pval));
+    PRS_CUDA(cudaGetLastError());
+  }
+  PRS_CUDA(cudaMemcpyAsync(counts, a + A.counts, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, st));
+  PRS_CUDA(cudaMemcpyAsync(total, a + A.off + (size_t)n * sizeof(long long), sizeof(long long), cudaMemcpyDeviceToHost,
+                           st));
+  PRS_CUDA(cudaStreamSynchronize(st));
+  return PRS_OK;
+}
+
+extern "C" int prs_ens_activity_copy(prs_ens_plan* e, long long n, int* idx, void* val, void* stream) {
+  PRS_REQUIRE(e && e->act && n >= 0 && (n == 0 || (idx && val)) && stream, "prs_ens_activity_copy: bad argument");
+  PRS_REQUIRE(n <= (long long)e->act_ticks * e->B * e->act_k, "prs_ens_activity_copy: %lld cells, the run kept at most %lld",
+              n, (long long)e->act_ticks * e->B * e->act_k);
+  if (n == 0) return PRS_OK;
+  const cudaStream_t st = (cudaStream_t)stream;
+  const int es = e->pc->dtype == PRS_F32 ? 4 : 8;
+  const EnsActivity A(e->B, e->lay.chunk, e->act_k, es);
+  PRS_CUDA(cudaMemcpyAsync(idx, e->act + A.pidx, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, st));
+  PRS_CUDA(cudaMemcpyAsync(val, e->act + A.pval, (size_t)n * es, cudaMemcpyDeviceToHost, st));
+  PRS_CUDA(cudaStreamSynchronize(st));
+  return PRS_OK;
 }
 
 // ---------------------------------------------------------------------------------------------

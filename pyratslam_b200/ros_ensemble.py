@@ -136,6 +136,32 @@ def reassign_parameters(parents, rec_of, match_threshold, global_inhibition, inj
     return par, thr, gi, energies
 
 
+def activity_parameters(activity_threshold=None, max_active_cells=128, pose_size=POSE_SIZE):
+    """The pose-cell activity capture's settings validated (no CUDA involved): ``activity_threshold`` None (no capture)
+    or a finite real number, ``max_active_cells`` an integer in [0, X*Y*Th] (0: counts only).  Returns ``(threshold
+    float or None, max_cells int)``; ``ValueError`` otherwise."""
+    if activity_threshold is not None and (not _real(activity_threshold)
+                                           or not math.isfinite(float(activity_threshold))):
+        raise ValueError("activity_threshold must be None or a finite number, got %r" % (activity_threshold,))
+    n = int(np.prod([int(s) for s in pose_size]))
+    if (not isinstance(max_active_cells, (numbers.Integral, np.integer)) or isinstance(max_active_cells, (bool, np.bool_))
+            or not 0 <= int(max_active_cells) <= n):
+        raise ValueError("max_active_cells must be an integer in [0, %d], got %r" % (n, max_active_cells))
+    return (None if activity_threshold is None else float(activity_threshold)), int(max_active_cells)
+
+
+def activity_entry(result, b, i):
+    """Agent b's activity at image i of a result with the capture on: ``(index int64 [k,3], value float64 [k])``, the
+    captured cells (x, y, th) in C order and their values, as ``PoseCellNetwork.active_cells`` returns them.  k is
+    ``min(activity_count[b, i], max_active_cells)``, 0 past the agent's length."""
+    n = result["activity_count"].shape[1]
+    if not 0 <= b < result["activity_count"].shape[0] or not 0 <= i < n:
+        raise IndexError("activity_entry: (%r, %r) outside the result's [%d, %d]"
+                         % (b, i, result["activity_count"].shape[0], n))
+    lo, hi = result["activity_ptr"][b * n + i], result["activity_ptr"][b * n + i + 1]
+    return result["activity_cell"][lo:hi], result["activity_value"][lo:hi]
+
+
 def capacity_for(T):
     """Templates per agent for a T-frame replay: one frame appends at most one template, whole groups of 32."""
     return (int(T) + 1 + 31) // 32 * 32
@@ -365,11 +391,19 @@ class EnsembleSession:
     ``replay_ensemble`` returns on the concatenation of its recording's feeds.  The libraries grow when a feed could
     overfill them (``grow_capacity``), so a session replays any number of frames while no agent holds more than 65536
     templates.  A pose-cell error raises what ``replay_ensemble`` raises and closes the session; a closed session's
-    ``feed`` raises ``RuntimeError``."""
+    ``feed`` raises ``RuntimeError``.
+
+    ``activity_threshold`` (None: off) captures every agent's pose-cell activity at each image on the device: the
+    cells above the threshold in the state the match was made with (after the image's update, before its injection),
+    the first ``max_active_cells`` of them in C order, and their true count.  The result then also holds
+    ``activity_count [B, i_max]`` (-1 past the length), ``activity_ptr [B * i_max + 1]`` (row pointers over the (agent,
+    image) pairs, row-major), ``activity_cell int64 [n, 3]`` and ``activity_value float64 [n]``; ``activity_entry``
+    returns one entry.  Concatenating agent b's entries over the feeds gives the one-call activity."""
 
     def __init__(self, n_agents=None, match_threshold=MATCH_THRESHOLD, global_inhibition=PC_GLOBAL_INHIB,
                  inject_energy=None, pose_size=POSE_SIZE, dtype=np.float32, active_set=0, experience_map=False,
-                 experience_links=False, n_recordings=1, recording=0, capacity=None):
+                 experience_links=False, n_recordings=1, recording=0, capacity=None, activity_threshold=None,
+                 max_active_cells=128):
         self._plan, self._ens, self._work = None, None, None
         self._closed = True
         if isinstance(experience_map, (bool, np.bool_)) and experience_map:
@@ -390,10 +424,14 @@ class EnsembleSession:
             raise ValueError("capacity must be an integer in [1, %d], got %r" % (MAX_CAPACITY, capacity))
         cap = (int(cap) + 31) // 32 * 32
         pose_size = tuple(int(s) for s in pose_size)
+        act_thr, act_k = activity_parameters(activity_threshold, max_active_cells, pose_size)
         np_dtype = _as_np_dtype(dtype)
         nat.require_cuda()
         dev = torch.device("cuda", torch.cuda.current_device())
         self.B, self.R, self.pose_size, self.capacity = B, R, pose_size, cap
+        self._act_thr, self._act_k, self._act_buf = act_thr, act_k, None    # the capture's settings and buffer
+        self._cells = None
+        self._np_dtype = np_dtype
         self._thr, self._gi, self._energies = thr, gi, list(energies)     # the settings in force, caller order
         self._dev, self._rec_of = dev, rec_of
         self._map = isinstance(experience_map, str)
@@ -450,6 +488,15 @@ class EnsembleSession:
             X_RANGE[0], X_RANGE[1], X_STEP, self._scratch.data_ptr(), ctypes.byref(plan)), "prs_ens_create")
         self._plan = plan
         self._room = self.capacity - int(self._n.max())
+        self._chunk = int(L.prs_ens_chunk(plan))
+        if self._act_thr is not None:
+            # every plan of the session captures (a growth or an injection change makes the plan again); the buffer
+            # depends on B, the chunk and the dtype only, so it is made once
+            if self._act_buf is None:
+                self._act_buf = torch.empty(int(L.prs_ens_activity_bytes(plan, self._act_k)), dtype=torch.uint8,
+                                            device=self._dev)
+            nat.check(L.prs_ens_set_activity(plan, self._act_thr, self._act_k, self._act_buf.data_ptr()),
+                      "prs_ens_set_activity")
 
     def _grow(self, cap):
         """Libraries of ``cap`` templates: a larger library is the old one with groups appended, so each agent's row is
@@ -580,7 +627,9 @@ class EnsembleSession:
         odometry too.  The streams are compacted into ticks (``event_ticks``).  Returns per image: ``template``, ``created``, ``score``, ``argmax`` ``[B, i_max]``,
         ``length [B]`` (the images of the agent's recording in this feed; -1 / False past it), ``n_templates [B]``, and
         with ``experience_map="device"`` ``n_exp``, ``exp_id``, ``em_xy`` at each image (-1 / NaN past the length) and
-        ``n_loop_closures``.  ``feed`` and ``feed_events`` continue the same agents, libraries and maps."""
+        ``n_loop_closures``.  ``feed`` and ``feed_events`` continue the same agents, libraries and maps.  With the
+        activity capture on, its entries are per image too: the state each image's match was made with; odometry-only
+        ticks capture nothing (there is no per-update capture of message streams)."""
         if self._closed:
             raise RuntimeError("EnsembleSession: the session is closed")
         return self._feed_ticks(event_streams(events, self.R), "image")
@@ -608,6 +657,8 @@ class EnsembleSession:
             exp_id = np.zeros((K, B), np.int32)
             em_xy = np.zeros((K, B, 2))
         first = np.zeros(R, np.int64)                  # per recording: its first image of the sub-run
+        if self._act_thr is not None:                  # per tick and device row the count, and the packed cells
+            act_counts, act_cells = np.full((K, B), -1, np.int32), []
         try:
             with torch.cuda.device(self._dev):
                 k0 = 0
@@ -630,7 +681,8 @@ class EnsembleSession:
                         self._room = self.capacity - int(self._n.max())
                     sub = slice(k0, k1)
                     sub_img = img[sub].sum(axis=0)
-                    self._run(streams, first, sub_img, tw[sub], moved[sub], gate[sub], res[sub])
+                    self._run(streams, first, sub_img, tw[sub], moved[sub], gate[sub], res[sub],
+                              None if self._act_thr is None else (act_counts[sub], act_cells))
                     self._room -= int(img_tick[sub].sum())
                     self._n = res["n_templates"][k1 - 1].astype(np.int64)
                     if self._linked:
@@ -677,19 +729,66 @@ class EnsembleSession:
         out["n_templates"], out["length"] = self.n_templates, length
         if self._map:
             out["n_loop_closures"] = self.n_loop_closures
+        if self._act_thr is not None:
+            out.update(self._activity(act_counts, act_cells, img, i_max))
         return out
 
-    def _run(self, streams, first, sub_img, tw, moved, gate, res):
-        """One sub-run of ticks through ``prs_ens_run``.  A pose-cell error raises what the native replay raises, for
-        the earliest tick: with one recording, with the bits of every agent at it (they share the odometry), else for
-        the lowest agent at it."""
+    def _activity(self, counts, cells, img, i_max):
+        """The activity keys of one feed in the caller's order, from ``counts [K,B]`` (per tick and device row) and
+        the packed cells of its runs (tick-major, then device row), selected per recording as the records are."""
+        B, k_max = self.B, self._act_k
+        kept = np.clip(counts, 0, k_max).astype(np.int64)
+        start = (np.cumsum(kept.ravel()) - kept.ravel()).reshape(kept.shape)     # first packed cell of each entry
+        idx = np.concatenate([c[0] for c in cells] + [np.zeros(0, np.int32)])
+        val = np.concatenate([c[1] for c in cells] + [np.zeros(0, self._np_dtype)])
+        count = np.full((B, i_max), -1, np.int64)
+        src = np.zeros((B, i_max), np.int64)
+        for r in range(self.R):
+            ticks = np.nonzero(img[:, r])[0]
+            agents = np.nonzero(self._rec_of == r)[0]
+            d = self._rows[agents]
+            count[agents, :len(ticks)] = counts[ticks][:, d].T
+            src[agents, :len(ticks)] = start[ticks][:, d].T
+        n = np.clip(count, 0, k_max).ravel()
+        ptr = np.zeros(B * i_max + 1, np.int64)
+        np.cumsum(n, out=ptr[1:])
+        g = np.repeat(src.ravel() - ptr[:-1], n) + np.arange(ptr[-1])
+        if self._cells is None:         # flat C-order index -> (x, y, th): one row gather per cell instead of divisions
+            self._cells = _unravel(np.arange(int(np.prod(self.pose_size))), self.pose_size)
+        return {"activity_count": count, "activity_ptr": ptr, "activity_cell": self._cells[idx[g]],
+                "activity_value": val[g].astype(np.float64)}
+
+    def _run(self, streams, first, sub_img, tw, moved, gate, res, act=None):
+        """One sub-run of ticks through ``prs_ens_run``; with the activity capture, ``act`` = (counts [T,B], list of
+        packed cells) receives it, one device chunk of ticks per run.  A pose-cell error raises what the native replay
+        raises, for the earliest tick: with one recording, with the bits of every agent at it (they share the
+        odometry), else for the lowest agent at it."""
         L = nat.lib()
         fb = IM_SIZE[0] * IM_SIZE[1]
-        ptrs = (ctypes.c_void_p * self.R)(*[streams[r][0].ctypes.data + int(first[r]) * fb if sub_img[r] else None
-                                            for r in range(self.R)])
-        tw, n_images = np.ascontiguousarray(tw), np.ascontiguousarray(sub_img, dtype=np.int32)
-        nat.check(L.prs_ens_run(self._plan, ptrs, tw.ctypes.data, gate.ctypes.data, n_images.ctypes.data, len(gate),
-                                res.ctypes.data, ctypes.c_void_p(self._stream.cuda_stream)), "prs_ens_run")
+        stream = ctypes.c_void_p(self._stream.cuda_stream)
+        T = len(gate)
+        step = max(T if act is None else self._chunk, 1)         # the capture packs the ticks of one chunk per run
+        at = np.array(first, dtype=np.int64)
+        for a in range(0, T, step):
+            z = min(a + step, T)
+            n_img = sub_img if step == T else (gate[a:z] & 1).sum(axis=0).astype(np.int64)
+            ptrs = (ctypes.c_void_p * self.R)(*[streams[r][0].ctypes.data + int(at[r]) * fb if n_img[r] else None
+                                                for r in range(self.R)])
+            tw_p, n_images = np.ascontiguousarray(tw[a:z]), np.ascontiguousarray(n_img, dtype=np.int32)
+            gate_p = np.ascontiguousarray(gate[a:z])
+            nat.check(L.prs_ens_run(self._plan, ptrs, tw_p.ctypes.data, gate_p.ctypes.data, n_images.ctypes.data,
+                                    z - a, res[a:z].ctypes.data, stream), "prs_ens_run")
+            if act is not None:
+                counts = np.empty((z - a, self.B), np.int32)
+                total = ctypes.c_longlong(0)
+                nat.check(L.prs_ens_activity_pack(self._plan, counts.ctypes.data, ctypes.byref(total), stream),
+                          "prs_ens_activity_pack")
+                idx, val = np.empty(total.value, np.int32), np.empty(total.value, self._np_dtype)
+                nat.check(L.prs_ens_activity_copy(self._plan, total.value, idx.ctypes.data, val.ctypes.data, stream),
+                          "prs_ens_activity_copy")
+                act[0][a:z] = counts
+                act[1].append((idx, val))
+            at += n_img
         err = res["pc_err"] & ~nat.ERR_INJECT_LOC                            # device rows
         bad = (err != 0) & (moved[:, self._rec_of[self._order]] != 0)
         if not bad.any():
@@ -809,7 +908,7 @@ class EnsembleSession:
 
 def replay_ensemble(frames, odom, n_agents=None, match_threshold=MATCH_THRESHOLD, global_inhibition=PC_GLOBAL_INHIB,
                     inject_energy=None, pose_size=POSE_SIZE, dtype=np.float32, active_set=0, experience_map=False,
-                    experience_links=False, mode="ref", recording=0):
+                    experience_links=False, mode="ref", recording=0, activity_threshold=None, max_active_cells=128):
     """Replay ``frames[T,256,256]`` (uint8) and ``odom[T,2]`` = (linear.x, angular.z) through B agents.
 
     ``match_threshold``, ``global_inhibition`` and ``inject_energy`` (None = no injection, else a finite energy >= 0)
@@ -834,6 +933,15 @@ def replay_ensemble(frames, odom, n_agents=None, match_threshold=MATCH_THRESHOLD
     ``argmax`` are -1, ``created`` False, ``n_exp`` and ``exp_id`` -1 and ``em_xy`` NaN.  A pose-cell error raises what
     the native replay of that recording raises, for the earliest frame and, within it, the lowest agent.  With single
     arrays ``recording`` can only be 0.
+
+    ``activity_threshold`` (None: off, else a finite number) captures every agent's pose-cell activity at each frame
+    on the device, from the state the frame's match was made with -- after its update, before its injection, the state
+    ``argmax`` describes: the cells with a value above the threshold (compared in double, 0.002 is what the viewers
+    draw) in C order [x][y][th], at most ``max_active_cells`` of them (an integer in [0, X*Y*Th], 0 for counts only;
+    the first ones, as ``PoseCellNetwork.active_cells(max_cells=...)`` keeps), and their true count.  The result then
+    holds ``activity_count [B, T]`` (-1 past the agent's length), ``activity_ptr [B * T + 1]`` (row pointers over the
+    (agent, frame) pairs, row-major), ``activity_cell int64 [n, 3]`` and ``activity_value float64 [n]``;
+    ``activity_entry(out, b, t)`` returns one entry as ``(index, value)``.  Off by default; off, nothing changes.
 
     This is one ``EnsembleSession`` fed once, with libraries reserved for every frame up front; a session fed in
     pieces replays recordings that do not fit in host memory, or longer than 65535 frames."""
@@ -868,7 +976,8 @@ def replay_ensemble(frames, odom, n_agents=None, match_threshold=MATCH_THRESHOLD
                          % (T, capacity_for(T), MAX_CAPACITY))
     out, rec_of = _replay_once("replay_ensemble", _frame_ticks(fr, od), n_agents, recording, match_threshold,
                                global_inhibition, inject_energy, pose_size, dtype, active_set,
-                               "device" if experience_map == "device" else False, experience_links, mode)
+                               "device" if experience_map == "device" else False, experience_links, mode,
+                               activity_threshold, max_active_cells)
     if isinstance(experience_map, (bool, np.bool_)) and experience_map:
         moved, tw = np.zeros((T, R), np.uint8), np.zeros((T, R, 2))
         for r in range(R):
@@ -888,7 +997,8 @@ def replay_ensemble(frames, odom, n_agents=None, match_threshold=MATCH_THRESHOLD
 
 def replay_ensemble_events(events, n_agents=None, match_threshold=MATCH_THRESHOLD, global_inhibition=PC_GLOBAL_INHIB,
                            inject_energy=None, pose_size=POSE_SIZE, dtype=np.float32, active_set=0, experience_map=False,
-                           experience_links=False, mode="ref", recording=0):
+                           experience_links=False, mode="ref", recording=0, activity_threshold=None,
+                           max_active_cells=128):
     """``replay_ensemble`` over message streams (``rosbag_io.read_events``) instead of paired frames and twists: agent b
     is the node's message loop, ``ros_simulate.replay_events(events, match_threshold=..., inject_energy=...,
     experience_links=...)`` with ``pcn.global_inhibition`` set to its own value, so every gated odometry message is its
@@ -898,7 +1008,9 @@ def replay_ensemble_events(events, n_agents=None, match_threshold=MATCH_THRESHOL
     ``EnsembleSession.feed_events`` returns -- per image ``template``, ``created``, ``score``, ``argmax``
     ``[B, i_max]`` and ``length [B]``, the maps' ``n_exp``, ``exp_id``, ``em_xy`` and ``n_loop_closures`` -- plus
     ``agents`` and, with ``experience_map="device"``, ``maps``.  On a stream in which odometry and images alternate it equals
-    ``replay_ensemble`` on ``rosbag_io.events_to_arrays(events)[:2]``.  This is one ``EnsembleSession`` fed once."""
+    ``replay_ensemble`` on ``rosbag_io.events_to_arrays(events)[:2]``.  The activity capture (``activity_threshold``,
+    ``max_active_cells``) is ``replay_ensemble``'s, per image: odometry-only ticks capture nothing (there is no
+    per-update capture of message streams).  This is one ``EnsembleSession`` fed once."""
     if not (isinstance(experience_map, (bool, np.bool_)) and not experience_map
             or (isinstance(experience_map, str) and experience_map == "device")):
         raise ValueError("replay_ensemble_events: experience_map must be False or 'device' (the host maps need the "
@@ -906,11 +1018,12 @@ def replay_ensemble_events(events, n_agents=None, match_threshold=MATCH_THRESHOL
     several = (isinstance(events, (list, tuple)) and len(events) > 0 and not _is_event(events[0]))
     streams = [event_ticks(st) for st in events] if several else [event_ticks(events)]
     return _replay_once("replay_ensemble_events", streams, n_agents, recording, match_threshold, global_inhibition,
-                        inject_energy, pose_size, dtype, active_set, experience_map, experience_links, mode)[0]
+                        inject_energy, pose_size, dtype, active_set, experience_map, experience_links, mode,
+                        activity_threshold, max_active_cells)[0]
 
 
 def _replay_once(who, streams, n_agents, recording, match_threshold, global_inhibition, inject_energy, pose_size,
-                 dtype, active_set, experience_map, experience_links, mode):
+                 dtype, active_set, experience_map, experience_links, mode, activity_threshold=None, max_active_cells=128):
     """``replay_ensemble`` and ``replay_ensemble_events`` after their inputs are validated: the agents' parameters and
     recordings are broadcast and validated and the device memory is checked before any other CUDA call, then one
     ``EnsembleSession`` with libraries for every image is fed the R tick streams once.  Returns the feed's result with
@@ -922,6 +1035,7 @@ def _replay_once(who, streams, n_agents, recording, match_threshold, global_inhi
     R = len(streams)
     rec_of = agent_recordings(recording, B, R)
     pose_size = tuple(int(s) for s in pose_size)
+    act_thr, act_k = activity_parameters(activity_threshold, max_active_cells, pose_size)
     np_dtype = _as_np_dtype(dtype)
     K = max(len(st[2]) for st in streams)
     img = np.zeros((K, R), np.bool_)
@@ -937,6 +1051,9 @@ def _replay_once(who, streams, n_agents, recording, match_threshold, global_inhi
             + R * chunk * frame_bytes)
     if experience_map == "device" and experience_links:
         need += xens.work_bytes(B, K, cap) + xens.record_bytes(B, K)
+    if act_thr is not None:     # the capture's counts, slots and packed cells of one chunk (prs_ens_activity_bytes)
+        rows = chunk * B
+        need += rows * 4 + 2 * rows * act_k * (4 + np.dtype(np_dtype).itemsize) + (rows + 1) * 8 + 6 * 256
     nat.require_cuda()
     dev = torch.device("cuda", torch.cuda.current_device())
     free, _ = torch.cuda.mem_get_info(dev)
@@ -944,7 +1061,7 @@ def _replay_once(who, streams, n_agents, recording, match_threshold, global_inhi
         raise ValueError("%s: %d agents x %d templates need %.2f GB of device memory, %.2f GB are free"
                          % (who, B, cap, need / 1e9, free / 1e9))
     session = EnsembleSession(B, thr, gi, energies, pose_size, np_dtype, active_set, experience_map, experience_links,
-                              R, rec_of, cap)
+                              R, rec_of, cap, act_thr, act_k)
     try:
         out = session._feed_ticks(streams)
         out["agents"] = session.agents
@@ -990,7 +1107,19 @@ def _chunk_arg(text):
     return n
 
 
-def _replay_chunked(bags, chunk, image_topic, odom_topic, recording, **kw):
+def _activity_stats(out, acc):
+    """``--activity-threshold``: one result's active-cell counts added to ``acc`` = per agent (sum, images, max)."""
+    if acc is None:
+        return
+    c = out["activity_count"]
+    live = c >= 0
+    acc[0] += np.where(live, c, 0).sum(axis=1)
+    acc[1] += live.sum(axis=1)
+    if c.shape[1]:
+        np.maximum(acc[2], c.max(axis=1), out=acc[2])
+
+
+def _replay_chunked(bags, chunk, image_topic, odom_topic, recording, acc=None, **kw):
     """The bags fed through one ``EnsembleSession`` ``chunk`` frames per bag at a time: per agent the templates, the
     frames created on, its bag's frame count and final arg-max (None for an empty bag), and the session's maps."""
     from . import rosbag_io as rb
@@ -1009,6 +1138,7 @@ def _replay_chunked(bags, chunk, image_topic, odom_topic, recording, **kw):
             od = [p[1] if p is not None else np.zeros((0, 2)) for p in pieces]
             out = s.feed(fr if R > 1 else fr[0], od if R > 1 else od[0])
             created += out["created"].sum(axis=1)
+            _activity_stats(out, acc)
             for b in range(B):
                 if out["length"][b]:
                     last[b] = tuple(int(c) for c in out["argmax"][b, out["length"][b] - 1])
@@ -1017,7 +1147,7 @@ def _replay_chunked(bags, chunk, image_topic, odom_topic, recording, **kw):
         s.close()
 
 
-def _replay_all_messages(bags, chunk, image_topic, odom_topic, recording, **kw):
+def _replay_all_messages(bags, chunk, image_topic, odom_topic, recording, acc=None, **kw):
     """``--all-messages``: the bags' message streams fed through one ``EnsembleSession`` with ``feed_events``, ``chunk``
     images per bag at a time (each bag whole without it): per agent the templates, the images created on, its bag's
     image count and final arg-max, and the experience and loop-closure counts of its map."""
@@ -1040,6 +1170,7 @@ def _replay_all_messages(bags, chunk, image_topic, odom_topic, recording, **kw):
             ev = [p if p is not None else [] for p in pieces]
             out = s.feed_events(ev if R > 1 else ev[0])
             created += out["created"].sum(axis=1)
+            _activity_stats(out, acc)
             for b in range(B):
                 if out["length"][b]:
                     last[b] = tuple(int(c) for c in out["argmax"][b, out["length"][b] - 1])
@@ -1069,6 +1200,10 @@ def main(argv=None):
                     help="replay every odometry message as its own pose-cell update, as the node's message loop does "
                          "(ros_simulate), instead of pairing each image with the last twist before it; also prints "
                          "every agent's experience count")
+    ap.add_argument("--activity-threshold", type=float, metavar="T",
+                    help="capture every agent's pose cells above T at each image on the device (0.002 is what the "
+                         "viewers draw) and print each agent's mean and max active-cell count; only the counts come "
+                         "back from the device")
     a = ap.parse_args(argv)
     from . import rosbag_io as rb
     thr = _list(a.match_threshold, float)
@@ -1081,14 +1216,20 @@ def main(argv=None):
               global_inhibition=[c[1] for _, c in agents], inject_energy=[c[2] for _, c in agents],
               experience_map="device" if a.experience_links or a.all_messages else False,
               experience_links=a.experience_links)
+    acc, extra = None, {}
+    if a.activity_threshold is not None:
+        kw.update(activity_threshold=a.activity_threshold, max_active_cells=0)
+        acc = [np.zeros(len(agents), np.int64), np.zeros(len(agents), np.int64), np.full(len(agents), -1, np.int64)]
+        extra = {"acc": acc}
     n_exp = None
     if a.all_messages:
         n_templates, created, fed, last, n_exp, loops = _replay_all_messages(a.bag, a.chunk, a.image_topic,
-                                                                             a.odom_topic, [r for r, _ in agents], **kw)
+                                                                             a.odom_topic, [r for r, _ in agents], **kw,
+                                                                             **extra)
         frames = [int(fed[r if several else 0]) for r, _ in agents]
     elif a.chunk is not None:
         n_templates, created, fed, last, maps = _replay_chunked(a.bag, a.chunk, a.image_topic, a.odom_topic,
-                                                                [r for r, _ in agents], **kw)
+                                                                [r for r, _ in agents], **kw, **extra)
         frames = [int(fed[r if several else 0]) for r, _ in agents]
         loops = maps.n_loop_closures if maps is not None else None
     else:
@@ -1099,6 +1240,7 @@ def main(argv=None):
         else:
             out = replay_ensemble(recs[0][0], recs[0][1], **kw)
         n_templates, maps, loops = out["n_templates"], out.get("maps"), out.get("n_loop_closures")
+        _activity_stats(out, acc)
         frames = [len(recs[r][0]) for r, _ in agents]
         created = [int(out["created"][b].sum()) for b in range(len(agents))]
         last = [tuple(int(c) for c in out["argmax"][b, T - 1]) if T else None for b, T in enumerate(frames)]
@@ -1114,6 +1256,8 @@ def main(argv=None):
                 line += "  loop closures %d" % loops[b]
         elif a.experience_links:
             line += "  experiences %d  loop closures %d" % (maps.n_experiences[b], loops[b])
+        if acc is not None:
+            line += "  active cells mean %.1f max %d" % (acc[0][b] / max(int(acc[1][b]), 1), max(int(acc[2][b]), 0))
         print(line)
 
 
