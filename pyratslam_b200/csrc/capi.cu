@@ -225,15 +225,10 @@ extern "C" int prs_pc_path(prs_pc_handle h) {
   if (!h) return PRS_PATH_GENERIC;
   if (h->forced_path >= 0) return h->forced_path;
   if (h->cluster_pref) return PRS_PATH_CLUSTER;
-  // PRS_PC_PREFER (profiling): "resident" keeps round 1's one-CTA kernel as the automatic choice for float32
-  static const bool prefer_resident = [] {
-    const char* e = getenv("PRS_PC_PREFER");
-    return e && strcmp(e, "resident") == 0;
-  }();
   // Fused kernels.  float64: the pair kernel is the only fused one.  float32: two CTAs per network finish a wave in
   // 16.4 us against 18.5 us while every CTA has an SM of its own (B <= #SM / 2); beyond that the one-CTA kernel
   // wins (0.344 ms against 0.463 ms for 4096 networks, profiles/r2_path_compare.txt).
-  if (h->pair_ok && !(prefer_resident && h->resident_ok) && (!h->resident_ok || h->B <= 74)) return PRS_PATH_PAIR;
+  if (h->pair_ok && (!h->resident_ok || h->B <= 74)) return PRS_PATH_PAIR;
   return h->resident_ok ? PRS_PATH_RESIDENT : (h->tiled_ok ? PRS_PATH_TILED : PRS_PATH_GENERIC);
 }
 
@@ -395,7 +390,7 @@ static int step_dispatch(prs_pc_handle h, void* state, const double* odom, int T
     if (path == PRS_PATH_CLUSTER)
       rc = prs_pc_cluster_step(h, (float*)state, odom + (size_t)t * h->B * 2, (const float*)gi,
                                argmax + (size_t)t * h->B, (float*)total + (size_t)t * h->B, err, err_store && T == 1, st);
-    else if (path == 2)
+    else if (path == PRS_PATH_TILED)
       rc = prs_pc_tiled_step(h, (float*)state, odom + (size_t)t * h->B * 2, (const float*)gi, argmax + (size_t)t * h->B,
                              (float*)total + (size_t)t * h->B, err, st);
     else
@@ -457,11 +452,7 @@ extern "C" int prs_pc_step(prs_pc_handle h, void* state, const double* odom, con
       h->sgraph = nullptr;
     }
     cudaGraph_t g = nullptr;
-    static const bool no_cond = [] {  // PRS_ACTIVE_NO_COND (tuning knob): the fall-back's launches unconditionally
-      const char* e = getenv("PRS_ACTIVE_NO_COND");
-      return e && atoi(e) != 0;
-    }();
-    if (h->opt_active && !no_cond) {
+    if (h->opt_active) {
       if (capture_active_graph(h, state, gi, argmax, total, err, &g) == PRS_OK &&
           cudaGraphInstantiate(&h->sgraph, g, 0) != cudaSuccess) {
         (void)cudaGetLastError();

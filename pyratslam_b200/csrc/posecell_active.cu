@@ -33,8 +33,6 @@
 // input: k_pc_scan then returns at once for that network and an update no longer reads the state at all.  Every
 // library call that writes the state invalidates the lists; a caller that writes it by other means must call
 // prs_pc_invalidate_active.
-#include <stdlib.h>
-
 #include "common.cuh"
 
 namespace {
@@ -235,29 +233,9 @@ struct ActArgs {
 };
 
 constexpr int kActMaxT = 256;
-// Optional in-kernel phase timing (profiling builds only: -DPRS_ACTIVE_TIMING): thread 0 of CTA 0 accumulates the cycles
-// between consecutive stamps into g_act_cycles[i].
-#ifdef PRS_ACTIVE_TIMING
-__device__ unsigned long long g_act_cycles[32];
-#define ACT_STAMP(i)                                        \
-  do {                                                      \
-    if (blockIdx.x == 0 && threadIdx.x == 0) {              \
-      const long long now_ = clock64();                     \
-      g_act_cycles[i] += (unsigned long long)(now_ - stamp_); \
-      stamp_ = now_;                                        \
-    }                                                       \
-  } while (0)
-#else
-#define ACT_STAMP(i) \
-  do {               \
-  } while (0)
-#endif
-#ifndef PRS_ACTIVE_CH
-#define PRS_ACTIVE_CH 12
-#endif
-#ifndef PRS_ACTIVE_CH2
-#define PRS_ACTIVE_CH2 8
-#endif
+// outputs per register window of the WIDE kernels in float32 (half as many in float64): 1-D passes, 7x7 stage
+constexpr int kActCh = 12;
+constexpr int kActCh2 = 8;
 
 // l / n for 0 <= l < 2^21, n > 0, inv = 1.0f / n: (l + 0.5) / n is never within float rounding of an integer there
 __device__ __forceinline__ int fdiv(int l, float inv) { return __float2int_rz((__int2float_rn(l) + 0.5f) * inv); }
@@ -270,8 +248,8 @@ template <typename T, int MAXD, bool WIDE>
 __global__ void __launch_bounds__(kActMaxT, 4) k_pc_active(const __grid_constant__ ActArgs<T> a) {
   // Outputs per register window.  A work item costs ~100 instructions before its first FMA (window positions, predicated
   // loads, line decode), so a window covers the whole line of a typical packet (11 outputs) where the registers allow it.
-  constexpr int CH = !WIDE ? 4 : (sizeof(T) == 4 ? PRS_ACTIVE_CH : PRS_ACTIVE_CH / 2);      // 1-D passes
-  constexpr int CH2 = !WIDE ? 4 : (sizeof(T) == 4 ? PRS_ACTIVE_CH2 : PRS_ACTIVE_CH2 / 2);   // 7x7 stage (accumulators + two windows)
+  constexpr int CH = !WIDE ? 4 : (sizeof(T) == 4 ? kActCh : kActCh / 2);      // 1-D passes
+  constexpr int CH2 = !WIDE ? 4 : (sizeof(T) == 4 ? kActCh2 : kActCh2 / 2);   // 7x7 stage (accumulators + two windows)
   constexpr int MW = MAXD / 32;
   using Set = AxisSet<MAXD>;
   extern __shared__ __align__(16) unsigned char arena_raw[];
@@ -294,9 +272,6 @@ __global__ void __launch_bounds__(kActMaxT, 4) k_pc_active(const __grid_constant
   __shared__ T s_total;
 
   const int tid = threadIdx.x, nt = blockDim.x, lane = tid & 31, wid = tid >> 5, nw = nt >> 5;
-#ifdef PRS_ACTIVE_TIMING
-  long long stamp_ = clock64();
-#endif
   if (a.wl_cnt != nullptr && (int)blockIdx.x >= *a.wl_cnt) return;
   const int b = a.wl != nullptr ? a.wl[blockIdx.x] : (int)blockIdx.x;
   const int X = a.X, Y = a.Y, Th = a.Th, XY = X * Y;
@@ -322,7 +297,6 @@ __global__ void __launch_bounds__(kActMaxT, 4) k_pc_active(const __grid_constant
   for (int i = tid; i < 98; i += nt) (&s_F[0][0])[i] = a.tab.f2d[i / 49][i % 49];
   if (tid == 0) s_newcnt = 0;
   __syncthreads();
-  ACT_STAMP(0);
 
   auto go_dense = [&]() {
     if (tid == 0) {
@@ -363,12 +337,10 @@ __global__ void __launch_bounds__(kActMaxT, 4) k_pc_active(const __grid_constant
       atomicOr(&s_mS[2][k >> 5], 1u << (k & 31));
     }
     __syncthreads();
-    ACT_STAMP(1);
     derive_mask(X, s_mG[0], [&](int c) { return dilated(s_mS[0], c, X); });
     derive_mask(Y, s_mG[1], [&](int c) { return dilated(s_mS[1], c, Y); });
     derive_mask(Th, s_mG[2], [&](int c) { return dilated(s_mS[2], c, Th); });
     __syncthreads();
-    ACT_STAMP(2);
 #pragma unroll 1
     for (int q = wid; q < 6; q += nw) {
       const int ax = q % 3, n = ax == 0 ? X : (ax == 1 ? Y : Th);
@@ -376,7 +348,6 @@ __global__ void __launch_bounds__(kActMaxT, 4) k_pc_active(const __grid_constant
       if (lane == 0) s_n[q] = c;
     }
     __syncthreads();
-    ACT_STAMP(3);
     const int nSx = s_n[0], nSy = s_n[1], nSk = s_n[2], nGx = s_n[3], nGy = s_n[4], nGk = s_n[5];
 #pragma unroll 1
     for (int ax = 0; ax < 3; ++ax)
@@ -393,7 +364,6 @@ __global__ void __launch_bounds__(kActMaxT, 4) k_pc_active(const __grid_constant
 #pragma unroll 1
     for (int c = tid; c < (int)nXc; c += nt) Xc[c] = T(0);
     __syncthreads();
-    ACT_STAMP(4);
 #pragma unroll 1
     for (int e = tid; e < n_act; e += nt) {
       const int f = lidx[e];
@@ -401,7 +371,6 @@ __global__ void __launch_bounds__(kActMaxT, 4) k_pc_active(const __grid_constant
       Xc[(s_set[0].pos[x] * nSy + s_set[1].pos[y]) * nSk + s_set[2].pos[k]] = st[f];
     }
     __syncthreads();
-    ACT_STAMP(5);
     // ---- theta pass (k_dog_theta), one thread per (i, j) line: P1[i][j][g] pairs (R1)
     Pr<T>* P1 = reinterpret_cast<Pr<T>*>(R1);
     const int chK = (nGk + CH - 1) / CH, chY = (nGy + CH - 1) / CH, chX = (nGx + CH - 1) / CH;
@@ -421,7 +390,6 @@ __global__ void __launch_bounds__(kActMaxT, 4) k_pc_active(const __grid_constant
           });
     }
     __syncthreads();
-    ACT_STAMP(6);
     // ---- y pass (k_dog_y), one thread per (i, g) line: P2[i][gy][g] pairs (R0)
     Pr<T>* P2 = reinterpret_cast<Pr<T>*>(R0);
 #pragma unroll 1
@@ -440,7 +408,6 @@ __global__ void __launch_bounds__(kActMaxT, 4) k_pc_active(const __grid_constant
           });
     }
     __syncthreads();
-    ACT_STAMP(7);
     // ---- x pass, inhibition (posecell_network.py:339-340), sum (:343) (k_dog_x_inhib), one thread per (gy, g) line:
     //      A[gx][gy][g] (R1); the axes' occupancy of the result
     T* A = R1;
@@ -479,7 +446,6 @@ __global__ void __launch_bounds__(kActMaxT, 4) k_pc_active(const __grid_constant
     for (int o = 16; o > 0; o >>= 1) psum += __shfl_down_sync(0xffffffffu, psum, o);
     if (lane == 0) s_red[wid] = psum;
     __syncthreads();
-    ACT_STAMP(8);
     if (tid == 0) {
       T s = T(0);
 #pragma unroll 1
@@ -491,7 +457,6 @@ __global__ void __launch_bounds__(kActMaxT, 4) k_pc_active(const __grid_constant
     derive_mask(Y, s_mD[1], [&](int c) { return dilated(s_mA[1], c, Y); });
     derive_mask(Th, s_mD[2], [&](int c) { return dilated(s_mA[2], c, Th); });
     __syncthreads();
-    ACT_STAMP(9);
     tot = s_total;
     alive = tot != T(0);
     if (alive) {
@@ -504,7 +469,6 @@ __global__ void __launch_bounds__(kActMaxT, 4) k_pc_active(const __grid_constant
         if (lane == 0) s_n[6 + q] = c;
       }
       __syncthreads();
-      ACT_STAMP(10);
       const int nSAx = s_n[6], nSAy = s_n[7], nSAk = s_n[8], nDAx = s_n[9], nDAy = s_n[10];
       nDK = s_n[11];
 #pragma unroll 1
@@ -524,7 +488,6 @@ __global__ void __launch_bounds__(kActMaxT, 4) k_pc_active(const __grid_constant
 #pragma unroll 1
       for (int g = tid; g < nSAy; g += nt) s_a2g[1][g] = Gy->pos[SAy->list[g]];
       __syncthreads();
-      ACT_STAMP(11);
       // where the result of the 7x7 stage can be non-zero: cell x of plane k reads rows x + ox_k - 3 .. + 3
       // (convolution.py:329-331), i.e. x + ox_k must be in DA_x for one of the active planes
       derive_mask(X, s_mB[0], [&](int c) {
@@ -548,14 +511,12 @@ __global__ void __launch_bounds__(kActMaxT, 4) k_pc_active(const __grid_constant
         return in;
       });
       __syncthreads();
-      ACT_STAMP(12);
 #pragma unroll 1
       for (int q = wid; q < 2; q += nw) {
         const int c = set_from_mask(s_mB[q], q == 0 ? X : Y, &s_set[8 + q], lane);
         if (lane == 0) s_n[12 + q] = c;
       }
       __syncthreads();
-      ACT_STAMP(13);
       nBX = s_n[12], nBY = s_n[13];
       if ((long long)nDAx * nDAy * nSAk > cap0) {
         overflow();
@@ -624,7 +585,6 @@ __global__ void __launch_bounds__(kActMaxT, 4) k_pc_active(const __grid_constant
         }
       }
       __syncthreads();
-      ACT_STAMP(14);
       // ---- theta stage (k_theta_final), clamp (:314), arg-max candidates, one thread per (x, y) line, written straight into the state
       T ft[7];
 #pragma unroll
@@ -672,13 +632,11 @@ __global__ void __launch_bounds__(kActMaxT, 4) k_pc_active(const __grid_constant
     if (v2 > best_v || (v2 == best_v && i2 < best_i)) best_v = v2, best_i = i2;
   }
   __syncthreads();
-  ACT_STAMP(15);
   if (lane == 0) s_red[wid] = best_v, s_redi[wid] = best_i;
   if (!zeroed)  // a network that died in this update (nothing survived the inhibition): its old cells go to zero
 #pragma unroll 1
     for (int e = tid; e < n_act; e += nt) st[lidx[e]] = T(0);
   __syncthreads();
-  ACT_STAMP(16);
   if (tid == 0) {
     T v = s_red[0];
     int i = s_redi[0];
@@ -692,7 +650,6 @@ __global__ void __launch_bounds__(kActMaxT, 4) k_pc_active(const __grid_constant
     a.al_cnt[b] = keep ? s_newcnt : 0;
     a.al_valid[b] = keep ? 1 : 0;
   }
-  ACT_STAMP(17);
 }
 
 template <typename T>
@@ -762,18 +719,6 @@ int active_launch(prs_pc_plan* p, T* state, const double* odom, const T* gi, lon
 
 }  // namespace
 
-#ifdef PRS_ACTIVE_TIMING
-extern "C" __attribute__((visibility("default"))) int prs_debug_active_cycles(unsigned long long* out32, int reset) {
-  PRS_CUDA(cudaDeviceSynchronize());
-  PRS_CUDA(cudaMemcpyFromSymbol(out32, g_act_cycles, 32 * sizeof(unsigned long long)));
-  if (reset) {
-    unsigned long long z[32] = {};
-    PRS_CUDA(cudaMemcpyToSymbol(g_act_cycles, z, sizeof(z)));
-  }
-  return PRS_OK;
-}
-#endif
-
 int prs_pc_active_supported(const prs_pc_plan* p) {
   return p->X <= kMaxDim && p->Y <= kMaxDim && p->Th <= kMaxDim && p->X >= 3 && p->Y >= 3 && p->Th >= 3;
 }
@@ -787,14 +732,8 @@ int prs_pc_active_prepare(prs_pc_plan* p) {
   const bool few = p->B <= 16 || (maxd0 > 64 && p->B <= 2 * 148);  // big CTAs only where a network can need the room
   // (measured, 4096 networks of 21x21x36: first tier of 20 KB 0.158 ms per update; of 12 KB 0.192 ms: too many networks
   // run twice; of 48 KB 0.20 ms: too few in flight)
-  int threads = few ? 256 : 128, arena = few ? 160 * 1024 : 72 * 1024, arena1 = few ? 0 : 20 * 1024, cap = few ? 8192 : 512;
-  if (const char* e = getenv("PRS_ACTIVE_THREADS")) threads = atoi(e);
-  if (const char* e = getenv("PRS_ACTIVE_ARENA_KB")) arena = atoi(e) * 1024;
-  if (const char* e = getenv("PRS_ACTIVE_ARENA1_KB")) arena1 = atoi(e) * 1024;  // 0: one tier
-  if (const char* e = getenv("PRS_ACTIVE_CAP")) cap = atoi(e);
-  PRS_REQUIRE(threads >= 32 && threads <= kActMaxT && threads % 32 == 0, "PRS_ACTIVE_THREADS must be in [32, %d]", kActMaxT);
-  PRS_REQUIRE(arena >= 4096 && arena <= 200 * 1024 && cap >= 16, "PRS_ACTIVE_ARENA_KB / PRS_ACTIVE_CAP out of range");
-  PRS_REQUIRE(arena1 == 0 || (arena1 >= 4096 && arena1 < arena), "PRS_ACTIVE_ARENA1_KB must be 0 or in [4, arena)");
+  const int threads = few ? 256 : 128, arena = few ? 160 * 1024 : 72 * 1024, arena1 = few ? 0 : 20 * 1024;
+  const int cap = few ? 8192 : 512;
   p->act_threads = threads, p->act_arena = arena, p->act_arena1 = arena1, p->al_cap = cap;
   PRS_CUDA(cudaFuncSetAttribute(k_pc_active<float, 64, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
   PRS_CUDA(cudaFuncSetAttribute(k_pc_active<double, 64, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));

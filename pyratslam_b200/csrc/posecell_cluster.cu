@@ -22,7 +22,6 @@
 // Shapes are run-time values (strided item loops, ragged segments are masked); P is a template parameter so that
 // the theta windows live in registers.
 #include <cooperative_groups.h>
-#include <stdlib.h>
 
 #include <mutex>
 
@@ -559,20 +558,14 @@ int fits_dispatch(const prs_pc_plan* p, int C, int P) {
 // co-schedules about 12 clusters of 9, 16 of 6, 24 of 4 (cudaOccupancyMaxActiveClusters), and a second wave doubles the
 // time (profiles/r2_b_sweep.txt).  So: the largest C whose clusters all fit at once for this B; an even P (the packed
 // two-plane 7x7 stage) is preferred over a slightly larger C with an odd P.  *one_wave tells whether the chosen C runs
-// the B networks in a single wave.  PRS_CLUSTER_MAX lowers the limit (tuning knob).  Returns C, or 0 if the path does
-// not apply to this plan.
+// the B networks in a single wave.  Returns C, or 0 if the path does not apply to this plan.
 int prs_pc_cluster_choose(const prs_pc_plan* p, int* one_wave) {
   if (one_wave) *one_wave = 0;
   if (p->dtype != PRS_F32) return 0;
   if (p->X < 7 || p->Y < 7) return 0;  // a halo of 3 must be a single periodic image
   if ((long long)p->X * p->Y >= 65536) return 0;  // FastDiv range
-  static const int cmax = [] {
-    const char* e = getenv("PRS_CLUSTER_MAX");
-    const int v = e ? atoi(e) : 16;
-    return v < 2 ? 2 : (v > 16 ? 16 : v);
-  }();
   int cand[16], nact[16], nc = 0;
-  for (int C = cmax; C >= 2; --C) {
+  for (int C = 16; C >= 2; --C) {
     if (p->Th % C != 0) continue;
     const int P = p->Th / C;
     if (P > 9) break;

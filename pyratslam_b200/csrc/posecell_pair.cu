@@ -32,7 +32,6 @@
 //   -- cluster barrier: the peer has read my B2; CTA 1's arg-max candidate has reached CTA 0 --
 // The grid is persistent: as many clusters as are co-resident (2 CTAs per SM in float32) stride over the networks.
 #include <cooperative_groups.h>
-#include <stdlib.h>
 
 #include <mutex>
 
@@ -114,22 +113,6 @@ __device__ __forceinline__ void pair_plan_plane(int k, const double* __restrict_
   if (e && err_b != nullptr) atomicOr(err_b, e);
 }
 
-#ifdef PRS_PAIR_TIMING
-__device__ unsigned long long g_pair_cycles[12];
-#define PAIR_STAMP(i)                                               \
-  do {                                                              \
-    if (blockIdx.x == 0 && threadIdx.x == 0) {                      \
-      const long long now_ = clock64();                             \
-      if (stamp_) g_pair_cycles[(i)] += now_ - stamp_;              \
-      stamp_ = now_;                                                \
-    }                                                               \
-  } while (0)
-#else
-#define PAIR_STAMP(i) \
-  do {                \
-  } while (0)
-#endif
-
 template <int X, int Y, int T, int NT, typename R>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NT, sizeof(R) == 4 ? 2 : 1)
     k_pc_pair(R* state, const double* __restrict__ odom, int n_steps, const R* __restrict__ gi,
@@ -190,9 +173,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NT, sizeof(R) == 4 ?
   if (tid == 0) *s_best_flat = 0x7fffffff;
   cluster.sync();  // both CTAs of the cluster are running (DSMEM may be touched) and the set-up is visible
   int slot = 0;
-#ifdef PRS_PAIR_TIMING
-  long long stamp_ = 0;
-#endif
 
   for (int b = cid; b < B; b += ncl) {
     R* gst = state + (size_t)b * (XY * T);
@@ -200,7 +180,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NT, sizeof(R) == 4 ?
     for (int step = 0; step < n_steps; ++step) {
       const int* plan = s_plan + slot * L::kPlanInts;
       const int4* plan4 = reinterpret_cast<const int4*>(plan);
-      PAIR_STAMP(0);
 
       // ---- 1. theta pass of the separable DoG: global -> (E, I) pairs of my H planes.  The state is read with
       //      ld.global.cg: on later steps half of it was written by the peer CTA (another SM's L1 would be stale).
@@ -240,7 +219,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NT, sizeof(R) == 4 ?
         }
       }
       __syncthreads();
-      PAIR_STAMP(1);
 
       // ---- 2. y pass, in place on each (plane, x) line
       {
@@ -267,7 +245,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NT, sizeof(R) == 4 ?
         }
       }
       __syncthreads();
-      PAIR_STAMP(2);
 
       // ---- 3. x pass + global inhibition (posecell_network.py:339-340) + sum (:343): a thread takes the same y
       //      column of BOTH planes of a pair; the column it READS is y + oy of the plane (the y part of the origin)
@@ -310,7 +287,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NT, sizeof(R) == 4 ?
       for (int o = 16; o > 0; o >>= 1) psum += __shfl_xor_sync(0xffffffffu, psum, o);
       if (lane == 0) s_wsum[wid] = psum;
       __syncthreads();  // every (E, I) pair has been consumed: the bytes become A2 / B2
-      PAIR_STAMP(3);
       if (tid < NQ * Y) {
         R2* dst = A2 + q3 * PS + y3;  // row r of the halo layout is grid row r - 3
 #pragma unroll
@@ -330,7 +306,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NT, sizeof(R) == 4 ?
         }
       }
       __syncthreads();  // publishes A2
-      PAIR_STAMP(4);
 
       // ---- 4. 7x7 periodic correlate of both planes of a pair at once (posecell_network.py:273-274,300);
       //      meanwhile two otherwise idle warps prepare the plan of the next update.
@@ -375,7 +350,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NT, sizeof(R) == 4 ?
           o[j] = mk2(max0(acc[j].x), max0(acc[j].y));
       }
       cluster.sync();  // B2 and the partial sums of both halves are complete and visible to both CTAs
-      PAIR_STAMP(5);
 
       // ---- 5. theta pass (convolution.py:344-359), clamp (:314), -> global, maximum.
       //      V(j) = (plane LC+j, plane LC-j) for any j: pin[j] inside the window, the halves swapped for j < 0, the
@@ -483,7 +457,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NT, sizeof(R) == 4 ?
       }
       if (lane == 0) s_wmax[wid] = wm;
       __syncthreads();
-      PAIR_STAMP(6);
       unsigned long long gm = lane < NW ? s_wmax[lane] : 0ull;
 #pragma unroll
       for (int o = 16; o > 0; o >>= 1) {
@@ -498,7 +471,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NT, sizeof(R) == 4 ?
       }
       cluster.sync();  // the peer has read my B2 (stage 1 of the next update may overwrite it); candidates exchanged;
                        // the state in global memory is consistent for the next update
-      PAIR_STAMP(7);
       if (tid == 0) {
         if (rank == 0) {
           const unsigned long long pv = *s_peer_val;
@@ -521,48 +493,48 @@ struct PairState {
   int clusters[64] = {};
 };
 
+// Once per device and kernel (S belongs to one kernel): allow the kernel its dynamic shared memory, and find how many
+// of its 2-CTA clusters fit on the device at once (half the SMs if the occupancy query fails).  The count, capped at
+// B, goes to *ncl.
+template <typename K>
+int pair_clusters(PairState& S, K kern, int nt, size_t smem, int dev, int B, int* ncl) {
+  PRS_REQUIRE(dev >= 0 && dev < 64, "pair path: device index %d out of range", dev);
+  std::lock_guard<std::mutex> lk(S.mu);
+  if (!S.configured[dev]) {
+    PRS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(2 * 148, 1, 1);
+    cfg.blockDim = dim3(nt, 1, 1);
+    cfg.dynamicSmemBytes = smem;
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeClusterDimension;
+    at[0].val.clusterDim.x = 2;
+    at[0].val.clusterDim.y = 1;
+    at[0].val.clusterDim.z = 1;
+    cfg.attrs = at;
+    cfg.numAttrs = 1;
+    int n = 0;
+    if (cudaOccupancyMaxActiveClusters(&n, kern, &cfg) != cudaSuccess || n < 1) {
+      (void)cudaGetLastError();
+      int nsm = 0;
+      PRS_CUDA(cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev));
+      n = nsm / 2 > 0 ? nsm / 2 : 1;
+    }
+    S.clusters[dev] = n;
+    S.configured[dev] = true;
+  }
+  *ncl = B < S.clusters[dev] ? B : S.clusters[dev];
+  return PRS_OK;
+}
+
 template <int X, int Y, int T, int NT, typename R>
 int pair_launch(prs_pc_plan* p, R* state, const double* odom, int n_steps, const R* gi, long long* argmax, R* total,
                 int* err, const PcTables<R>& tab, cudaStream_t st) {
   using L = PairLayout<X, Y, T, R>;
   auto kern = k_pc_pair<X, Y, T, NT, R>;
   static PairState S;
-  const int dev = p->device;
-  PRS_REQUIRE(dev >= 0 && dev < 64, "pair path: device index %d out of range", dev);
-  {
-    std::lock_guard<std::mutex> lk(S.mu);
-    if (!S.configured[dev]) {
-      PRS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L::kBytes));
-      cudaLaunchConfig_t cfg = {};
-      cfg.gridDim = dim3(2 * 148, 1, 1);
-      cfg.blockDim = dim3(NT, 1, 1);
-      cfg.dynamicSmemBytes = L::kBytes;
-      cudaLaunchAttribute at[1];
-      at[0].id = cudaLaunchAttributeClusterDimension;
-      at[0].val.clusterDim.x = 2;
-      at[0].val.clusterDim.y = 1;
-      at[0].val.clusterDim.z = 1;
-      cfg.attrs = at;
-      cfg.numAttrs = 1;
-      int n = 0;
-      cudaError_t e = cudaOccupancyMaxActiveClusters(&n, kern, &cfg);
-      if (e != cudaSuccess || n < 1) {
-        (void)cudaGetLastError();
-        int nsm = 0;
-        PRS_CUDA(cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev));
-        n = nsm / 2 > 0 ? nsm / 2 : 1;
-      }
-      S.clusters[dev] = n;
-      S.configured[dev] = true;
-    }
-  }
-  static int cap = [] {  // PRS_PAIR_CLUSTERS: cap of co-resident clusters (profiling knob)
-    const char* e = getenv("PRS_PAIR_CLUSTERS");
-    return e ? atoi(e) : 0;
-  }();
-  int ncl = S.clusters[dev];
-  if (cap > 0 && cap < ncl) ncl = cap;
-  if (p->B < ncl) ncl = p->B;
+  int ncl = 0;
+  if (int rc_ = pair_clusters(S, kern, NT, L::kBytes, p->device, p->B, &ncl)) return rc_;
   kern<<<2 * ncl, NT, L::kBytes, st>>>(state, odom, n_steps, gi, argmax, total, err, p->cos_th, p->sin_th,
                                        p->vtrans_scale, p->vrot_scale, p->B, tab);
   PRS_CUDA(cudaGetLastError());
@@ -974,36 +946,8 @@ int pair_seg_launch(prs_pc_plan* p, float* state, const double* odom, int n_step
   using L = SegLayout<X, Y, T>;
   auto kern = k_pc_pair_seg<X, Y, T, NT>;
   static PairState S;
-  const int dev = p->device;
-  PRS_REQUIRE(dev >= 0 && dev < 64, "pair path: device index %d out of range", dev);
-  {
-    std::lock_guard<std::mutex> lk(S.mu);
-    if (!S.configured[dev]) {
-      PRS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L::kBytes));
-      int nsm = 0;
-      PRS_CUDA(cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev));
-      cudaLaunchConfig_t cfg = {};
-      cfg.gridDim = dim3(2 * 148, 1, 1);
-      cfg.blockDim = dim3(NT, 1, 1);
-      cfg.dynamicSmemBytes = L::kBytes;
-      cudaLaunchAttribute at[1];
-      at[0].id = cudaLaunchAttributeClusterDimension;
-      at[0].val.clusterDim.x = 2;
-      at[0].val.clusterDim.y = 1;
-      at[0].val.clusterDim.z = 1;
-      cfg.attrs = at;
-      cfg.numAttrs = 1;
-      int n = 0;
-      if (cudaOccupancyMaxActiveClusters(&n, kern, &cfg) != cudaSuccess || n < 1) {
-        (void)cudaGetLastError();
-        n = nsm / 2 > 0 ? nsm / 2 : 1;
-      }
-      S.clusters[dev] = n;
-      S.configured[dev] = true;
-    }
-  }
-  int ncl = S.clusters[dev];
-  if (p->B < ncl) ncl = p->B;
+  int ncl = 0;
+  if (int rc_ = pair_clusters(S, kern, NT, L::kBytes, p->device, p->B, &ncl)) return rc_;
   kern<<<2 * ncl, NT, L::kBytes, st>>>(state, odom, n_steps, gi, argmax, total, err, p->cos_th, p->sin_th, p->vtrans_scale,
                                        p->vrot_scale, p->B, p->tf);
   PRS_CUDA(cudaGetLastError());
@@ -1011,18 +955,6 @@ int pair_seg_launch(prs_pc_plan* p, float* state, const double* odom, int n_step
 }
 
 }  // namespace
-
-#ifdef PRS_PAIR_TIMING
-extern "C" __attribute__((visibility("default"))) int prs_debug_pair_cycles(unsigned long long* out12, int reset) {
-  PRS_CUDA(cudaDeviceSynchronize());
-  PRS_CUDA(cudaMemcpyFromSymbol(out12, g_pair_cycles, 12 * sizeof(unsigned long long)));
-  if (reset) {
-    unsigned long long z[12] = {};
-    PRS_CUDA(cudaMemcpyToSymbol(g_pair_cycles, z, sizeof(z)));
-  }
-  return PRS_OK;
-}
-#endif
 
 // The kernel applies ONE x origin per mirror pair: around(vt * cos) must be the same for both planes, which holds
 // when the host's cosine table is bitwise even about MID and about plane 0 (numpy's cos is).
@@ -1046,17 +978,9 @@ int prs_pc_pair_step(prs_pc_plan* p, void* state, const double* odom, int T, con
                                                 err, p->td, st);
   }
   if (p->X == 50 && p->Y == 50 && p->Th == 10 && p->dtype == PRS_F32) {
-    // PRS_PAIRSEG_NT (tuning knob): CTA size of the segmented kernel; measured for 2600 networks: 0.855 ms (256
-    // threads, 178 registers), 0.791 ms (384), 0.768 ms (512, 120 registers) -- one CTA per SM, so more warps win
-    static const int nt = [] {
-      const char* e = getenv("PRS_PAIRSEG_NT");
-      return e ? atoi(e) : 512;
-    }();
-    if (nt == 512)
-      return pair_seg_launch<50, 50, 10, 512>(p, (float*)state, odom, T, (const float*)gi, argmax, (float*)total, err, st);
-    if (nt == 384)
-      return pair_seg_launch<50, 50, 10, 384>(p, (float*)state, odom, T, (const float*)gi, argmax, (float*)total, err, st);
-    return pair_seg_launch<50, 50, 10, 256>(p, (float*)state, odom, T, (const float*)gi, argmax, (float*)total, err, st);
+    // 512 threads: measured for 2600 networks, 0.855 ms (256 threads, 178 registers), 0.791 ms (384), 0.768 ms (512,
+    // 120 registers) -- one CTA per SM, so more warps win
+    return pair_seg_launch<50, 50, 10, 512>(p, (float*)state, odom, T, (const float*)gi, argmax, (float*)total, err, st);
   }
   prs_set_error("pair path not available for this plan");
   return PRS_E_INVALID;

@@ -16,7 +16,6 @@
 // seen every peer's query s, i.e. after every peer has finished reading query s-1, so two parities are enough.
 // A bounded spin (default 10 s of %globaltimer) turns a missing peer into an error instead of a hung GPU.
 #include <new>
-#include <stdlib.h>
 #include <string.h>
 #include <time.h>
 
@@ -381,13 +380,9 @@ extern "C" int prs_vt_shard_query(prs_xchg* x, int dtype, void* lib, long long n
                                       (unsigned long long)(uintptr_t)scratch, (unsigned long long)decide, thr_bits,
                                       (unsigned long long)n_total, (unsigned long long)owner,
                                       (unsigned long long)(uintptr_t)result_pinned, (unsigned long long)x->device};
-  static const bool no_graph = [] {  // PRS_SHARD_NO_GRAPH (tuning knob): always enqueue the chain eagerly
-    const char* e = getenv("PRS_SHARD_NO_GRAPH");
-    return e && atoi(e) != 0;
-  }();
   const bool same_as_graph = x->gexec != nullptr && memcmp(key, x->gkey, sizeof(key)) == 0;
   // a decision that may APPEND changes n_local / n_total for the next call: such chains never repeat, stay eager
-  const bool repeatable = !no_graph && !(decide && owner);
+  const bool repeatable = !(decide && owner);
   if (!same_as_graph) {
     if (repeatable && memcmp(key, x->glast, sizeof(key)) == 0)
       ++x->gsame;
