@@ -189,6 +189,14 @@ __device__ __forceinline__ int prs_modp_dev(int v, int n) {
   int r = v % n;
   return r < 0 ? r + n : r;
 }
+// Global inhibition (posecell_network.py:339-340) is two masked writes, `pc[pc < gi] = 0` then `pc[pc >= gi] -= gi`.
+// A cell below gi is zeroed by the first and, when 0 >= gi, lowered by gi again by the second: it ends at max(-gi, 0),
+// not at 0.  Every other cell ends at a - gi.  For gi >= 0 this is max(a - gi, 0); for gi < 0 it is not.  The floor is
+// +0 for gi = -0 and gi = +0 alike, as numpy's 0.0 - (-0.0).
+template <typename T>
+__device__ __forceinline__ T inhib_floor(T gi) {
+  return gi < T(0) ? -gi : T(0);
+}
 // Decisions of one path-integration step for (network b, plane k): bit-for-bit the float64 arithmetic numpy
 // does on the host (posecell_network.py:252-267,249,304); explicit _rn intrinsics keep the compiler from
 // contracting mul+sub into an FMA.

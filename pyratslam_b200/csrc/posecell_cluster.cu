@@ -11,7 +11,7 @@
 //   load     P + 6 state planes (own planes + 3 periodic neighbours each side) global -> SMEM
 //   1 theta  separable DoG along theta                                   s_in  -> s_ei  (E, I) pairs, y halo
 //   2 y      7-tap pass, packed FFMA2 on (E, I)                          s_ei  -> s_mid, x halo
-//   3 x      7-tap pass, A = max(aE*E - aI*I - gi, 0), CTA partial sum; stored moved by the plane's integer
+//   3 x      7-tap pass, A = aE*E - aI*I inhibited (inhib_floor), CTA partial sum; stored moved by the plane's integer
 //            origin (convolution.py:320-340) with periodic halos         s_mid -> s_a
 //   4 7x7    wrap-free correlate with the plane's LUT filter, clamp      s_a   -> s_b
 //   -- cluster barrier: partial sums and s_b become visible to the other CTAs --
@@ -244,7 +244,7 @@ __global__ void __launch_bounds__(kNT, 1) k_pc_cluster(ClArgs a, PcTables<float>
   //         the plane's integer origin, with 3 periodic halo rows and columns, so that stage 4 never wraps
   {
     float psum = 0.f;
-    const float g = a.gi[b];
+    const float g = a.gi[b], g_lo = inhib_floor(g);
     const FastDiv dS = a.dNsx;
     for (int it = tid; it < P * L.nsx * Y; it += kNT) {
       const int t2 = dY.div(it), y = it - t2 * Y;
@@ -272,7 +272,8 @@ __global__ void __launch_bounds__(kNT, 1) k_pc_cluster(ClArgs a, PcTables<float>
 #pragma unroll
         for (int t = 0; t < 7; ++t) acc = __ffma2_rn(in[jj + t], tp.tx[t], acc);
         if (seg * 8 + jj < X) {
-          const float v = fmaxf((acc.x - acc.y) - g, 0.f);
+          const float d = (acc.x - acc.y) - g;
+          const float v = d < 0.f ? g_lo : d;  // (a < gi) ? max(-gi, 0) : a - gi, see inhib_floor
           psum += v;
           const int xoffb = xd < 3 ? Xb : (xd >= X - 3 ? -Xb : 0);
           st_shared_f32(sa, v);

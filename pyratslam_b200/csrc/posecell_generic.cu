@@ -6,7 +6,7 @@
 //   k_plan         odometry -> integer origins, LUT filter choice, theta origin   (:252-267,249,304)
 //   k_dog_theta    E,I = ge*P, gi*P along theta   \  the 7x7x7 DoG correlate of :336 (convolution.py
 //   k_dog_y        E,I along y                     > :228-246) as separable E - I: kernel_3d ==
-//   k_dog_x_inhib  A = max(aE*E - aI*I - gi, 0)   /  aE ge(x)ge(x)ge - aI gi(x)gi(x)gi; inhibition :339-340,
+//   k_dog_x_inhib  A = aE*E - aI*I, inhibited     /  aE ge(x)ge(x)ge - aI gi(x)gi(x)gi; inhibition :339-340,
 //                  + per-block partial sums                                        sum for :343
 //   k_sum_final    total, 1/total                                                  (:343-345)
 //   k_shift2d      per-plane shifted 7x7 correlate, * 1/total, clamp               (:273-274,300; convolution.py:320-340)
@@ -135,8 +135,8 @@ __global__ void __launch_bounds__(kThreads)
         i = fma_t(tab.gix[t], Ii[plane + (size_t)xx * Y + y], i);
       }
       a = e - i;
-      T g = gi[bz];
-      a = (a < g) ? T(0) : a - g;  // posecell_network.py:339-340
+      const T g = gi[bz];
+      a = (a < g) ? inhib_floor(g) : a - g;  // posecell_network.py:339-340
       A[plane + p] = a;
     }
     T s = block_sum(a, sm);

@@ -23,7 +23,7 @@
 //   1 theta pass   thread = (x,y) line: H + 6 planes from global memory (the 3-plane halos of the window are simply
 //                  read as well: 24 of 36 planes per CTA, the overlap comes from L2) -> (E, I) pairs      11 op / cell
 //   2 y pass       thread = (plane, x) line, in place, FFMA2 on (E, I)                                    7 FFMA2 / cell
-//   3 x pass       thread = (pair, y) column of both planes, A = max(aE*E - aI*I - gi, 0), partial sum;
+//   3 x pass       thread = (pair, y) column of both planes, A = aE*E - aI*I inhibited (inhib_floor), partial sum;
 //                  written with 3 periodic halo rows as the float2 pair tensor A2                          7 FFMA2 / cell
 //   4 7x7 stage    thread = (pair, x) row, FFMA2 over the pair, result row stored at x - ox                24.5 FFMA2 / cell
 //   -- cluster barrier: B2 and the partial sums are visible to the peer --
@@ -176,7 +176,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NT, sizeof(R) == 4 ?
 
   for (int b = cid; b < B; b += ncl) {
     R* gst = state + (size_t)b * (XY * T);
-    const R g_inh = gi[b];
+    const R g_inh = gi[b], g_lo = inhib_floor(g_inh);
     for (int step = 0; step < n_steps; ++step) {
       const int* plan = s_plan + slot * L::kPlanInts;
       const int4* plan4 = reinterpret_cast<const int4*>(plan);
@@ -271,7 +271,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NT, sizeof(R) == 4 ?
             R2 acc = mk2(-g_inh, (R)0);  // the inhibition rides in the accumulator
 #pragma unroll
             for (int t = 0; t < 7; ++t) acc = fma2(in[(x + t + X - 3) % X], cf[t], acc);
-            const R a = max0(acc.x - acc.y);  // == (a < gi) ? 0 : a - gi (posecell_network.py:339-340)
+            const R d = acc.x - acc.y;
+            const R a = d < (R)0 ? g_lo : d;  // (a < gi) ? max(-gi, 0) : a - gi (posecell_network.py:339-340)
             if (h == 0)
               keep[x].x = a;
             else
@@ -637,7 +638,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NT, 1)
 
   for (int b = cid; b < B; b += ncl) {
     float* gst = state + (size_t)b * (XY * T);
-    const float g_inh = gi[b];
+    const float g_inh = gi[b], g_lo = inhib_floor(g_inh);
     for (int step = 0; step < n_steps; ++step) {
       // ---- 0. the decisions of this update (posecell_network.py:252-267,249,304), float64 as numpy computes them
       if (tid < T)
@@ -740,7 +741,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NT, 1)
               float2 acc = make_float2(-g_inh, 0.f);
 #pragma unroll
               for (int t = 0; t < 7; ++t) acc = __ffma2_rn(in[j + t], cf[t], acc);
-              const float a = fmaxf(acc.x - acc.y, 0.f);  // posecell_network.py:339-340
+              const float d = acc.x - acc.y;
+              const float a = d < 0.f ? g_lo : d;  // posecell_network.py:339-340, see inhib_floor
               if (h == 0)
                 keep[j].x = a;
               else

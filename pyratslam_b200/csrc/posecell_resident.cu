@@ -285,7 +285,7 @@ __global__ void __launch_bounds__(NT, 1)
   for (int wi = blockIdx.x; wi < nW; wi += gridDim.x) {
     const int b = net(wi);
     float* gst = state + (size_t)b * N;
-    const float g_inh = gi[b];
+    const float g_inh = gi[b], g_lo = inhib_floor(g_inh);
     for (int step = 0; step < n_steps; ++step) {
       const int* plan = s_plan + slot * L::kPlanInts;
       const int4* plan4 = reinterpret_cast<const int4*>(plan);
@@ -415,12 +415,13 @@ __global__ void __launch_bounds__(NT, 1)
               float2 acc = make_float2(-g_inh, 0.f);  // the inhibition rides in the accumulator: one FADD less per cell
 #pragma unroll
               for (int t = 0; t < 7; ++t) acc = ffma2(in[(x + t + X - 3) % X], cf[t], acc);
-              const float a = fmaxf(acc.x - acc.y, 0.f);  // == (a < gi) ? 0 : a - gi (posecell_network.py:339-340)
+              const float a = fmaxf(acc.x - acc.y, 0.f);  // (a < gi) ? 0 : a - gi; gi < 0: see below the loop
 #else
               float2 acc = make_float2(0.f, 0.f);
 #pragma unroll
               for (int t = 0; t < 7; ++t) acc = ffma2(in[(x + t + X - 3) % X], cf[t], acc);
-              const float a = fmaxf((acc.x - acc.y) - g_inh, 0.f);  // == (a < gi) ? 0 : a - gi, one FMNMX
+              const float d = (acc.x - acc.y) - g_inh;
+              const float a = d < 0.f ? g_lo : d;  // (a < gi) ? max(-gi, 0) : a - gi (inhib_floor)
 #endif
               if (h == 0)
                 keep[x].x = a;
@@ -433,6 +434,16 @@ __global__ void __launch_bounds__(NT, 1)
           }
         }
 #if PRS_RESIDENT_S3FOLD
+        // gi < 0 only (a uniform branch): the cells the max above clamped end at -gi, not at 0 (inhib_floor).  A cell with
+        // d == 0 exactly sits on the threshold within the rounding of the folded sum and goes with the cells below it.
+        // For gi >= 0 the clamp is the whole inhibition, one FMNMX per cell.
+        if (g_lo != 0.f) {
+#pragma unroll
+          for (int x = 0; x < X; ++x) {
+            keep[x].x = keep[x].x == 0.f ? g_lo : keep[x].x;
+            keep[x].y = keep[x].y == 0.f ? g_lo : keep[x].y;
+          }
+        }
         float2 ps2 = keep[0];  // both planes of the pair at once (add.f32x2)
 #pragma unroll
         for (int x = 1; x < X; ++x) ps2 = __fadd2_rn(ps2, keep[x]);

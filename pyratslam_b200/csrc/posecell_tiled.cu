@@ -261,7 +261,7 @@ __global__ void __launch_bounds__(kTyx) k_tl_yx(const float2* __restrict__ EI, f
     float2 in[14];
 #pragma unroll
     for (int j = 0; j < 14; ++j) in[j] = sp[j * kMidStride];
-    const float g = gi[plane / Th];
+    const float g = gi[plane / Th], g_lo = inhib_floor(g);
     const int gy = y0 + y, gx0 = x0 + seg * 8;
     float* Ap = A + (size_t)plane * XY;
     float a[8];
@@ -270,7 +270,8 @@ __global__ void __launch_bounds__(kTyx) k_tl_yx(const float2* __restrict__ EI, f
       float2 acc = make_float2(0.f, 0.f);
 #pragma unroll
       for (int t = 0; t < 7; ++t) acc = __ffma2_rn(in[jj + t], tp.tx[t], acc);
-      a[jj] = fmaxf((acc.x - acc.y) - g, 0.f);  // posecell_network.py:339-340: (a < gi) ? 0 : a - gi
+      const float d = (acc.x - acc.y) - g;
+      a[jj] = d < 0.f ? g_lo : d;  // posecell_network.py:339-340: (a < gi) ? max(-gi, 0) : a - gi
     }
     // rows of this segment inside the grid (0 when the column is outside): one compare per element masks the edges
     const int nv = gy < Y ? X - gx0 : 0;

@@ -81,6 +81,18 @@ def test_builders_match_reference_fixtures(golden):
     # beyond |og| = 4 every tap is negative: the clamp at og = +-8 in the kernel cannot change a result
     for og in range(5, nat.OG_RANGE + 1):
         assert (tab[nat.OG_RANGE + og] < 0).all() and (tab[nat.OG_RANGE - og] < 0).all()
+    # ... up to |og| = 64, the largest theta origin the kernels accept (PRS_ERR_THETA beyond): og 9..64 run with the
+    # og = 8 filter, and an all-negative filter followed by the clamp at zero zeroes the state whichever it is
+    wide = K.theta_filter_table(64)
+    for og in range(5, 65):
+        for f in (wide[64 + og], wide[64 - og], K.diff_gaussian_offset_1d(origin=float(og)),
+                  K.diff_gaussian_offset_1d(origin=float(-og))):
+            assert (f < 0).all(), og
+    # |og| = 3, 4 are the asymmetric filters with two or one positive taps at the edge
+    for og, npos in ((3, 2), (4, 1)):
+        for s in (1, -1):
+            f = tab[nat.OG_RANGE + s * og]
+            assert int((f > 0).sum()) == npos and (f[-npos:] > 0 if s > 0 else f[:npos] > 0).all(), (s * og, f)
 
 
 def test_separable_factorisation_reproduces_kernel_3d(golden):
