@@ -452,6 +452,27 @@ PRS_API size_t prs_ens_copy_stage_bytes(prs_ens_plan* plan, int n_moves, const i
                                 const int* n_templates);
 PRS_API int prs_ens_copy_agents(prs_ens_plan* plan, int n_moves, const int* dst, const int* src, const int* n_templates,
                         void* stage, size_t stage_bytes, void* stream);
+/* The same rows carried between two plans, which may live on different devices (a session's agents reassigned across
+ * devices).  prs_ens_export_agents gathers rows[k] into stage row k (a row may be listed more than once); the stage then
+ * depends on no plan: a header records K = n, the largest live template count, the network bytes, the dtype and the
+ * pose-cell shape.  Copy it whole to the importing plan's device (prs_stage_copy), then prs_ens_import_agents writes
+ * stage row k into row rows[k] (distinct) of its plan -- exactly what prs_ens_copy_agents writes -- and resets the
+ * active-set lists as prs_ens_copy_agents does.  Import reads the header (it synchronises `stream` once) and refuses,
+ * with PRS_E_INVALID, a stage of another row count, pose-cell shape or dtype, or with more live templates than its
+ * capacity.  Import writes its pair table into the stage, so a stage is imported once.
+ *   rows        : host int32 [n], rows in [0, B)
+ *   n_templates : host int32 [B], every row's template count as n_dev holds it (sizes the stage)
+ *   stage       : device, prs_ens_export_stage_bytes(...) bytes (0 for invalid rows or n = 0)
+ * Asynchronous on `stream`; the next prs_ens_run on any stream must be ordered after the import. */
+PRS_API size_t prs_ens_export_stage_bytes(prs_ens_plan* plan, int n, const int* rows, const int* n_templates);
+PRS_API int prs_ens_export_agents(prs_ens_plan* plan, int n, const int* rows, const int* n_templates, void* stage,
+                          size_t stage_bytes, void* stream);
+PRS_API int prs_ens_import_agents(prs_ens_plan* plan, int n, const int* rows, const void* stage, size_t stage_bytes,
+                          void* stream);
+/* bytes from src on device src_device to dst on device dst_device, asynchronous on `stream`: cudaMemcpyPeerAsync between
+ * two devices (peer access need not be enabled), cudaMemcpyAsync on one.  The stages of prs_ens_export_agents and
+ * prs_em_session_export_agents cross devices this way. */
+PRS_API int prs_stage_copy(void* dst, int dst_device, const void* src, int src_device, size_t bytes, void* stream);
 
 /* ------------------------------------------------------- ensemble experience maps */
 
@@ -521,6 +542,21 @@ PRS_API size_t prs_em_session_copy_stage_bytes(int B, int E, int N, int n_moves,
                                        const int* n_rows);
 PRS_API int prs_em_session_copy_agents(int B, int E, int N, void* work, int n_moves, const int* dst, const int* src,
                                const int* n_rows, void* stage, size_t stage_bytes, void* stream);
+/* The same columns carried between two workspaces, as prs_ens_export_agents carries plan rows: export gathers columns
+ * cols[k] (repeats allowed) of a (B, E, N) workspace into a stage whose header records K = n, `rows` (the largest
+ * max(experiences, links) among them) and the workspace's N; import writes stage column k into column cols[k]
+ * (distinct) of a (B', E', N') workspace -- the experiences and links below the counts, the stage's N vt_head rows, rel
+ * and the counts -- and sets vt_head rows [N, N') of those columns to -1, since the column's own are stale.  Import
+ * synchronises `stream` once to read the header and refuses, with PRS_E_INVALID, another column count, rows > E' or
+ * N > N'.  A stage is imported once.
+ *   n_rows : host int32 [B], max(experiences, links) of every column, at most E (sizes the stage)
+ *   stage  : device, prs_em_session_export_stage_bytes(...) bytes (0 for invalid columns or n = 0)
+ * Asynchronous on `stream`. */
+PRS_API size_t prs_em_session_export_stage_bytes(int B, int E, int N, int n, const int* cols, const int* n_rows);
+PRS_API int prs_em_session_export_agents(int B, int E, int N, const void* work, int n, const int* cols, const int* n_rows,
+                                 void* stage, size_t stage_bytes, void* stream);
+PRS_API int prs_em_session_import_agents(int B, int E, int N, void* work, int n, const int* cols, const void* stage,
+                                 size_t stage_bytes, void* stream);
 
 #ifdef __cplusplus
 }

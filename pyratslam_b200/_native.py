@@ -107,6 +107,10 @@ _SIGNATURES["prs_ens_activity_copy"] = (c_int, [c_void_p, c_longlong, c_void_p, 
 _SIGNATURES["prs_ens_copy_stage_bytes"] = (c_size_t, [c_void_p, c_int, c_void_p, c_void_p, c_void_p])
 _SIGNATURES["prs_ens_copy_agents"] = (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t,
                                               c_void_p])
+_SIGNATURES["prs_ens_export_stage_bytes"] = (c_size_t, [c_void_p, c_int, c_void_p, c_void_p])
+_SIGNATURES["prs_ens_export_agents"] = (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p])
+_SIGNATURES["prs_ens_import_agents"] = (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_size_t, c_void_p])
+_SIGNATURES["prs_stage_copy"] = (c_int, [c_void_p, c_int, c_void_p, c_int, c_size_t, c_void_p])
 _SIGNATURES["prs_em_work_bytes"] = (c_size_t, [c_int, c_int, c_int])
 _SIGNATURES["prs_em_linked_run"] = (c_int, [c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int,
                                             c_int, c_double, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p])
@@ -119,6 +123,11 @@ _SIGNATURES["prs_em_session_grow"] = (c_int, [c_int, c_int, c_int, c_int, c_int,
 _SIGNATURES["prs_em_session_copy_stage_bytes"] = (c_size_t, [c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p])
 _SIGNATURES["prs_em_session_copy_agents"] = (c_int, [c_int, c_int, c_int, c_void_p, c_int, c_void_p, c_void_p, c_void_p,
                                                      c_void_p, c_size_t, c_void_p])
+_SIGNATURES["prs_em_session_export_stage_bytes"] = (c_size_t, [c_int, c_int, c_int, c_int, c_void_p, c_void_p])
+_SIGNATURES["prs_em_session_export_agents"] = (c_int, [c_int, c_int, c_int, c_void_p, c_int, c_void_p, c_void_p,
+                                                       c_void_p, c_size_t, c_void_p])
+_SIGNATURES["prs_em_session_import_agents"] = (c_int, [c_int, c_int, c_int, c_void_p, c_int, c_void_p, c_void_p,
+                                                       c_size_t, c_void_p])
 _SIGNATURES["prs_em_linked_resume_run"] = (c_int, [c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_int, c_void_p,
                                                    c_void_p, c_void_p, c_int, c_int, c_int, c_double, c_void_p, c_void_p,
                                                    c_void_p, c_void_p, c_void_p])

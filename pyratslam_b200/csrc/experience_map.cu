@@ -11,6 +11,7 @@
 // Only cos, sin, atan2 and hypot may differ from glibc's by an ulp or two: they reach the positions, the link lengths
 // and the link headings, never a decision.
 #include <math.h>
+#include <string.h>
 
 #include "agent_moves.cuh"
 #include "common.cuh"
@@ -419,5 +420,125 @@ extern "C" int prs_em_session_copy_agents(int B, int E, int N, void* work, int n
   PRS_CUDA(launch(w, B, sw, K, d_table, K, rows));
   PRS_CUDA(launch(w, B, w, B, d_table + 2 * K, n_direct, direct_rows));
   PRS_CUDA(launch(sw, K, w, B, d_table + 2 * K + 2 * n_direct, n_staged, rows));
+  return PRS_OK;
+}
+
+// ---------------------------------------------------------------------------------------------
+// Columns carried between workspaces (prs_em_session_export_agents / prs_em_session_import_agents: a session's agents
+// reassigned across devices).  The stage is a header, the export's and the import's pair tables, then a workspace of K
+// columns with `rows` experience and link rows and the exporting workspace's N vt_head rows.  The header describes the
+// columns, so the stage depends on no workspace.
+namespace {
+
+constexpr int kEmStageMagic = 0x50524d45;  // "EMRP"
+constexpr int kEmHeaderInts = 8;
+struct EmStageHeader {
+  int magic, K, rows, N;
+  long long bytes;
+};
+
+size_t em_transfer_offset(int K) { return ((kEmHeaderInts + 4 * (size_t)K) * sizeof(int) + 255) / 256 * 256; }
+
+// vt_head rows [n0, N) of the listed columns set to -1: a column that received fewer template heads than its workspace
+// holds keeps none of its own.
+__global__ void __launch_bounds__(256) k_em_clear_heads(int* vt_head, int B, int n0, int N, const int* cols, int n_cols) {
+  const long long total = (long long)(N - n0) * n_cols;
+  for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < total;
+       idx += (long long)gridDim.x * blockDim.x) {
+    const int c = (int)(idx % n_cols);
+    const long long i = n0 + idx / n_cols;
+    vt_head[i * B + cols[c]] = -1;
+  }
+}
+
+}  // namespace
+
+static int em_export_check(const char* who, int B, int E, int N, int n, const int* cols, const int* n_rows, int& rows) {
+  PRS_REQUIRE(B >= 1 && E >= 0 && N >= 0 && n >= 0 && (n == 0 || (cols && n_rows)), "%s: bad argument B=%d E=%d N=%d",
+              who, B, E, N);
+  rows = 0;
+  for (int k = 0; k < n; ++k) {
+    PRS_REQUIRE(cols[k] >= 0 && cols[k] < B, "%s: column %d outside [0, %d)", who, cols[k], B);
+    PRS_REQUIRE(n_rows[cols[k]] >= 0 && n_rows[cols[k]] <= E, "%s: column %d uses %d rows, the workspace has %d", who,
+                cols[k], n_rows[cols[k]], E);
+    rows = std::max(rows, n_rows[cols[k]]);
+  }
+  return PRS_OK;
+}
+
+extern "C" size_t prs_em_session_export_stage_bytes(int B, int E, int N, int n, const int* cols, const int* n_rows) {
+  int rows = 0;
+  if (em_export_check("prs_em_session_export_stage_bytes", B, E, N, n, cols, n_rows, rows) || n == 0) return 0;
+  return em_transfer_offset(n) + EmLayout(n, rows, N).bytes;
+}
+
+extern "C" int prs_em_session_export_agents(int B, int E, int N, const void* work, int n, const int* cols,
+                                            const int* n_rows, void* stage, size_t stage_bytes, void* stream) {
+  int rows = 0;
+  if (int rc = em_export_check("prs_em_session_export_agents", B, E, N, n, cols, n_rows, rows)) return rc;
+  if (n == 0) return PRS_OK;
+  const size_t off = em_transfer_offset(n), need = off + EmLayout(n, rows, N).bytes;
+  PRS_REQUIRE(work && stage && stage_bytes >= need,
+              "prs_em_session_export_agents: the stage has %zu bytes, the columns need %zu", stage_bytes, need);
+  std::vector<int> table(kEmHeaderInts + 2 * (size_t)n, 0);
+  const EmStageHeader h{kEmStageMagic, n, rows, N, (long long)need};
+  memcpy(table.data(), &h, sizeof(h));
+  for (int k = 0; k < n; ++k) {  // workspace column cols[k] -> stage column k (a column may be exported more than once)
+    table[kEmHeaderInts + k] = cols[k];
+    table[kEmHeaderInts + n + k] = k;
+  }
+  const cudaStream_t st = (cudaStream_t)stream;
+  char* p = (char*)stage;
+  PRS_CUDA(cudaMemcpyAsync(p, table.data(), table.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+  const long long total = ((long long)13 * rows + N + 7) * n;
+  const long long blocks = std::min((total + 255) / 256, 148LL * 16);
+  k_em_copy_cols<<<(unsigned)blocks, 256, 0, st>>>(em_work((void*)work, EmLayout(B, E, N)), B,
+                                                   em_work(p + off, EmLayout(n, rows, N)), n,
+                                                   (const int*)p + kEmHeaderInts, n, rows, N);
+  PRS_CUDA(cudaGetLastError());
+  return PRS_OK;
+}
+
+extern "C" int prs_em_session_import_agents(int B, int E, int N, void* work, int n, const int* cols, const void* stage,
+                                            size_t stage_bytes, void* stream) {
+  PRS_REQUIRE(B >= 1 && E >= 0 && N >= 0 && n >= 0 && (n == 0 || (cols && work && stage)),
+              "prs_em_session_import_agents: bad argument B=%d E=%d N=%d", B, E, N);
+  if (n == 0) return PRS_OK;
+  std::vector<int> seen(B, 0);
+  for (int k = 0; k < n; ++k) {
+    PRS_REQUIRE(cols[k] >= 0 && cols[k] < B && !seen[cols[k]],
+                "prs_em_session_import_agents: column %d outside [0, %d) or imported twice", cols[k], B);
+    seen[cols[k]] = 1;
+  }
+  const cudaStream_t st = (cudaStream_t)stream;
+  EmStageHeader h;
+  PRS_REQUIRE(stage_bytes >= sizeof(h), "prs_em_session_import_agents: the stage has %zu bytes", stage_bytes);
+  PRS_CUDA(cudaMemcpyAsync(&h, stage, sizeof(h), cudaMemcpyDeviceToHost, st));
+  PRS_CUDA(cudaStreamSynchronize(st));
+  PRS_REQUIRE(h.magic == kEmStageMagic && h.K == n && (size_t)h.bytes <= stage_bytes,
+              "prs_em_session_import_agents: the stage does not hold %d exported columns", n);
+  PRS_REQUIRE(h.rows >= 0 && h.rows <= E && h.N >= 0 && h.N <= N,
+              "prs_em_session_import_agents: the stage holds %d rows and %d template heads, the workspace %d and %d",
+              h.rows, h.N, E, N);
+  std::vector<int> pairs(2 * (size_t)n);
+  for (int k = 0; k < n; ++k) {  // stage column k -> workspace column cols[k]
+    pairs[k] = k;
+    pairs[n + k] = cols[k];
+  }
+  char* p = (char*)stage;
+  int* d_pairs = (int*)p + kEmHeaderInts + 2 * n;
+  PRS_CUDA(cudaMemcpyAsync(d_pairs, pairs.data(), pairs.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+  const EmWork w = em_work(work, EmLayout(B, E, N));
+  const long long total = ((long long)13 * h.rows + h.N + 7) * n;
+  const long long blocks = std::min((total + 255) / 256, 148LL * 16);
+  k_em_copy_cols<<<(unsigned)blocks, 256, 0, st>>>(em_work(p + em_transfer_offset(n), EmLayout(n, h.rows, h.N)), n, w,
+                                                   B, d_pairs, n, h.rows, h.N);
+  PRS_CUDA(cudaGetLastError());
+  if (N > h.N) {
+    const long long cells = (long long)(N - h.N) * n;
+    k_em_clear_heads<<<(unsigned)std::min((cells + 255) / 256, 148LL * 16), 256, 0, st>>>(w.vt_head, B, h.N, N,
+                                                                                        d_pairs + n, n);
+    PRS_CUDA(cudaGetLastError());
+  }
   return PRS_OK;
 }

@@ -2510,6 +2510,34 @@ extern "C" size_t prs_ens_copy_stage_bytes(prs_ens_plan* e, int n_moves, const i
   return EnsCopyStage(mv.K(), mv.table().size(), ens_net_bytes(e->pc), max_n).bytes;
 }
 
+// The plan's own rows as a copy source or destination.
+static EnsRows ens_plan_rows(const prs_ens_plan* e) {
+  const int B = e->B;
+  return EnsRows{(char*)e->pc_state, (long long*)e->pc_work, (char*)e->pc_work + 8 * (size_t)B,
+                 (int*)((char*)e->pc_work + 16 * (size_t)B), e->n_dev, (char*)e->libs, e->lib_u4 * 16, e->loc_dev,
+                 e->capacity};
+}
+
+// One k_ens_copy_rows launch over n_pairs pairs whose live counts are at most `bound`.
+static cudaError_t ens_copy_launch(const prs_ens_plan* e, const EnsRows& from, const EnsRows& to, const int* pairs,
+                                   int n_pairs, int bound, cudaStream_t st) {
+  if (n_pairs == 0) return cudaSuccess;
+  const size_t net_bytes = ens_net_bytes(e->pc);
+  const bool wide = net_bytes % 16 == 0;
+  const long long state_words = (long long)(net_bytes / (wide ? 16 : 4));
+  const int es = e->pc->dtype == PRS_F32 ? 4 : 8;
+  // about 16 blocks per SM over all pairs, no more along x than a pair's largest region takes
+  const long long words = std::max((long long)((bound + 31) >> 5) * kVtGroupU4, state_words);
+  long long gx = (148LL * 16 + n_pairs - 1) / n_pairs;
+  gx = std::max(1LL, std::min(gx, (words + 1023) / 1024));
+  const dim3 grid((unsigned)gx, (unsigned)std::min(n_pairs, 65535));
+  if (wide)
+    k_ens_copy_rows<uint4><<<grid, 256, 0, st>>>(from, to, pairs, n_pairs, state_words, es, bound);
+  else
+    k_ens_copy_rows<unsigned><<<grid, 256, 0, st>>>(from, to, pairs, n_pairs, state_words, es, bound);
+  return cudaGetLastError();
+}
+
 extern "C" int prs_ens_copy_agents(prs_ens_plan* e, int n_moves, const int* dst, const int* src, const int* n_templates,
                                    void* stage, size_t stage_bytes, void* stream) {
   AgentMoves mv;
@@ -2517,39 +2545,133 @@ extern "C" int prs_ens_copy_agents(prs_ens_plan* e, int n_moves, const int* dst,
   if (int rc = ens_copy_plan("prs_ens_copy_agents", e, n_moves, dst, src, n_templates, mv, max_n)) return rc;
   if (n_moves == 0) return PRS_OK;
   const std::vector<int> table = mv.table();
-  const size_t net_bytes = ens_net_bytes(e->pc);
-  const EnsCopyStage L(mv.K(), table.size(), net_bytes, max_n);
+  const EnsCopyStage L(mv.K(), table.size(), ens_net_bytes(e->pc), max_n);
   PRS_REQUIRE(stage && stage_bytes >= L.bytes, "prs_ens_copy_agents: the stage has %zu bytes, the moves need %zu",
               stage_bytes, L.bytes);
   if (int rc = prs_pc_check_device(e->pc, "prs_ens_copy_agents")) return rc;
   const cudaStream_t st = (cudaStream_t)stream;
   char* p = (char*)stage;
   PRS_CUDA(cudaMemcpyAsync(p, table.data(), table.size() * sizeof(int), cudaMemcpyHostToDevice, st));
-  const int B = e->B;
-  const EnsRows plan{(char*)e->pc_state, (long long*)e->pc_work, (char*)e->pc_work + 8 * (size_t)B,
-                     (int*)((char*)e->pc_work + 16 * (size_t)B), e->n_dev, (char*)e->libs, e->lib_u4 * 16, e->loc_dev,
-                     e->capacity};
-  const EnsRows rows = L.rows(p);
-  const bool wide = net_bytes % 16 == 0;
-  const long long state_words = (long long)(net_bytes / (wide ? 16 : 4));
-  const int es = e->pc->dtype == PRS_F32 ? 4 : 8;
-  auto launch = [&](const EnsRows& from, const EnsRows& to, const int* pairs, int n_pairs, int bound) {
-    if (n_pairs == 0) return cudaSuccess;
-    // about 16 blocks per SM over all pairs, no more along x than a pair's largest region takes
-    const long long words = std::max((long long)((bound + 31) >> 5) * kVtGroupU4, state_words);
-    long long gx = (148LL * 16 + n_pairs - 1) / n_pairs;
-    gx = std::max(1LL, std::min(gx, (words + 1023) / 1024));
-    const dim3 grid((unsigned)gx, (unsigned)std::min(n_pairs, 65535));
-    if (wide)
-      k_ens_copy_rows<uint4><<<grid, 256, 0, st>>>(from, to, pairs, n_pairs, state_words, es, bound);
-    else
-      k_ens_copy_rows<unsigned><<<grid, 256, 0, st>>>(from, to, pairs, n_pairs, state_words, es, bound);
-    return cudaGetLastError();
-  };
+  const EnsRows plan = ens_plan_rows(e), rows = L.rows(p);
   const int* d_table = (const int*)p;
   const int K = mv.K(), n_direct = (int)mv.direct.size() / 2, n_staged = (int)mv.staged.size() / 2;
-  PRS_CUDA(launch(plan, rows, d_table, K, max_n));
-  PRS_CUDA(launch(plan, plan, d_table + 2 * K, n_direct, e->capacity));
-  PRS_CUDA(launch(rows, plan, d_table + 2 * K + 2 * n_direct, n_staged, max_n));
+  PRS_CUDA(ens_copy_launch(e, plan, rows, d_table, K, max_n, st));
+  PRS_CUDA(ens_copy_launch(e, plan, plan, d_table + 2 * K, n_direct, e->capacity, st));
+  PRS_CUDA(ens_copy_launch(e, rows, plan, d_table + 2 * K + 2 * n_direct, n_staged, max_n, st));
   return prs_pc_active_invalidate(e->pc, st);  // the carried lists describe the rows as they were
+}
+
+// ---------------------------------------------------------------------------------------------
+// Agents carried between plans (prs_ens_export_agents / prs_ens_import_agents: a session's agents reassigned across
+// devices).  The stage is EnsCopyStage's layout for K rows, its table region holding a header that describes the rows
+// -- so it depends on no plan -- then the export's and the import's pair tables.
+namespace {
+constexpr int kEnsStageMagic = 0x50525345;  // "ESRP"
+constexpr int kStageHeaderInts = 16;
+struct EnsStageHeader {
+  int magic, K, max_n, dtype, X, Y, Th, pad;
+  long long net_bytes, bytes;
+};
+static_assert(sizeof(EnsStageHeader) <= kStageHeaderInts * sizeof(int), "stage header");
+EnsCopyStage ens_transfer_stage(int K, size_t net_bytes, int max_n) {
+  return EnsCopyStage(K, kStageHeaderInts + 4 * (size_t)K, net_bytes, max_n);
+}
+}  // namespace
+
+static int ens_export_check(const char* who, prs_ens_plan* e, int n, const int* rows, const int* n_templates,
+                            int& max_n) {
+  PRS_REQUIRE(e && n >= 0 && (n == 0 || (rows && n_templates)), "%s: bad argument", who);
+  max_n = 0;
+  for (int k = 0; k < n; ++k) {
+    PRS_REQUIRE(rows[k] >= 0 && rows[k] < e->B, "%s: row %d outside [0, %d)", who, rows[k], e->B);
+    const int c = n_templates[rows[k]];
+    PRS_REQUIRE(c >= 0 && c <= e->capacity, "%s: row %d holds %d templates, the capacity is %d", who, rows[k], c,
+                e->capacity);
+    max_n = std::max(max_n, c);
+  }
+  return PRS_OK;
+}
+
+extern "C" size_t prs_ens_export_stage_bytes(prs_ens_plan* e, int n, const int* rows, const int* n_templates) {
+  int max_n = 0;
+  if (ens_export_check("prs_ens_export_stage_bytes", e, n, rows, n_templates, max_n) || n == 0) return 0;
+  return ens_transfer_stage(n, ens_net_bytes(e->pc), max_n).bytes;
+}
+
+extern "C" int prs_ens_export_agents(prs_ens_plan* e, int n, const int* rows, const int* n_templates, void* stage,
+                                     size_t stage_bytes, void* stream) {
+  int max_n = 0;
+  if (int rc = ens_export_check("prs_ens_export_agents", e, n, rows, n_templates, max_n)) return rc;
+  if (n == 0) return PRS_OK;
+  const size_t net_bytes = ens_net_bytes(e->pc);
+  const EnsCopyStage L = ens_transfer_stage(n, net_bytes, max_n);
+  PRS_REQUIRE(stage && stage_bytes >= L.bytes, "prs_ens_export_agents: the stage has %zu bytes, the rows need %zu",
+              stage_bytes, L.bytes);
+  if (int rc = prs_pc_check_device(e->pc, "prs_ens_export_agents")) return rc;
+  std::vector<int> table(kStageHeaderInts + 2 * (size_t)n, 0);
+  const EnsStageHeader h{kEnsStageMagic, n, max_n, e->pc->dtype, e->pc->X, e->pc->Y, e->pc->Th, 0,
+                         (long long)net_bytes, (long long)L.bytes};
+  memcpy(table.data(), &h, sizeof(h));
+  for (int k = 0; k < n; ++k) {  // plan row rows[k] -> stage row k (a row may be exported more than once)
+    table[kStageHeaderInts + k] = rows[k];
+    table[kStageHeaderInts + n + k] = k;
+  }
+  const cudaStream_t st = (cudaStream_t)stream;
+  char* p = (char*)stage;
+  PRS_CUDA(cudaMemcpyAsync(p, table.data(), table.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+  PRS_CUDA(ens_copy_launch(e, ens_plan_rows(e), L.rows(p), (const int*)p + kStageHeaderInts, n, max_n, st));
+  return PRS_OK;
+}
+
+extern "C" int prs_ens_import_agents(prs_ens_plan* e, int n, const int* rows, const void* stage, size_t stage_bytes,
+                                     void* stream) {
+  PRS_REQUIRE(e && n >= 0 && (n == 0 || (rows && stage)), "prs_ens_import_agents: bad argument");
+  if (n == 0) return PRS_OK;
+  std::vector<int> seen(e->B, 0);
+  for (int k = 0; k < n; ++k) {
+    PRS_REQUIRE(rows[k] >= 0 && rows[k] < e->B && !seen[rows[k]],
+                "prs_ens_import_agents: row %d outside [0, %d) or imported twice", rows[k], e->B);
+    seen[rows[k]] = 1;
+  }
+  if (int rc = prs_pc_check_device(e->pc, "prs_ens_import_agents")) return rc;
+  const cudaStream_t st = (cudaStream_t)stream;
+  EnsStageHeader h;
+  PRS_REQUIRE(stage_bytes >= sizeof(h), "prs_ens_import_agents: the stage has %zu bytes", stage_bytes);
+  PRS_CUDA(cudaMemcpyAsync(&h, stage, sizeof(h), cudaMemcpyDeviceToHost, st));
+  PRS_CUDA(cudaStreamSynchronize(st));
+  const size_t net_bytes = ens_net_bytes(e->pc);
+  PRS_REQUIRE(h.magic == kEnsStageMagic && h.K == n && (size_t)h.bytes <= stage_bytes,
+              "prs_ens_import_agents: the stage does not hold %d exported rows", n);
+  PRS_REQUIRE(h.dtype == e->pc->dtype && h.X == e->pc->X && h.Y == e->pc->Y && h.Th == e->pc->Th &&
+                  (size_t)h.net_bytes == net_bytes,
+              "prs_ens_import_agents: the stage holds %d x %d x %d networks of dtype %d, the plan %d x %d x %d of dtype %d",
+              h.X, h.Y, h.Th, h.dtype, e->pc->X, e->pc->Y, e->pc->Th, e->pc->dtype);
+  PRS_REQUIRE(h.max_n >= 0 && h.max_n <= e->capacity,
+              "prs_ens_import_agents: a staged row holds %d templates, the capacity is %d", h.max_n, e->capacity);
+  const EnsCopyStage L = ens_transfer_stage(n, net_bytes, h.max_n);
+  std::vector<int> pairs(2 * (size_t)n);
+  for (int k = 0; k < n; ++k) {  // stage row k -> plan row rows[k]
+    pairs[k] = k;
+    pairs[n + k] = rows[k];
+  }
+  char* p = (char*)stage;
+  int* d_pairs = (int*)p + kStageHeaderInts + 2 * n;
+  PRS_CUDA(cudaMemcpyAsync(d_pairs, pairs.data(), pairs.size() * sizeof(int), cudaMemcpyHostToDevice, st));
+  PRS_CUDA(ens_copy_launch(e, L.rows(p), ens_plan_rows(e), d_pairs, n, h.max_n, st));
+  // an imported row may hold more templates than any row had: the sweep's group bound and the room follow it
+  k_ens_init<<<1, 256, 0, st>>>(e->n_dev, e->B, (int*)(e->scratch + e->lay.misc));
+  PRS_CUDA(cudaGetLastError());
+  e->room = std::min(e->room, (long long)e->capacity - h.max_n);
+  return prs_pc_active_invalidate(e->pc, st);  // the carried lists describe the rows as they were
+}
+
+extern "C" int prs_stage_copy(void* dst, int dst_device, const void* src, int src_device, size_t bytes, void* stream) {
+  PRS_REQUIRE((bytes == 0 || (dst && src)) && dst_device >= 0 && src_device >= 0, "prs_stage_copy: bad argument");
+  if (bytes == 0) return PRS_OK;
+  const cudaStream_t st = (cudaStream_t)stream;
+  if (dst_device == src_device)
+    PRS_CUDA(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, st));
+  else
+    PRS_CUDA(cudaMemcpyPeerAsync(dst, dst_device, src, src_device, bytes, st));
+  return PRS_OK;
 }

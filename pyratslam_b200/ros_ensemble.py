@@ -16,6 +16,8 @@ create-or-match decision and injection.
 ``EnsembleSession`` keeps the agents on the device between calls and feeds them recordings in pieces: bags streamed
 in chunks, recordings longer than 65535 frames, or a second run of a route continuing the maps of the first.
 
+``ShardedEnsembleSession`` splits the agents over several GPUs (``devices=`` of the replays, ``--devices``).
+
     python -m pyratslam_b200.ros_ensemble BAG [BAG ...] --match-threshold 30000,45000,60000 --global-inhibition 0.1,0.2
 """
 from __future__ import annotations
@@ -24,6 +26,7 @@ import ctypes
 import itertools
 import math
 import numbers
+import threading
 
 import numpy as np
 import torch
@@ -374,6 +377,38 @@ def event_streams(events, n_recordings):
     return [event_ticks(s) for s in events]
 
 
+def _session_arguments(n_agents, match_threshold, global_inhibition, inject_energy, pose_size, dtype, experience_map,
+                       n_recordings, recording, capacity, activity_threshold, max_active_cells):
+    """``EnsembleSession``'s arguments validated and broadcast (no CUDA involved): ``(B, R, thresholds, inhibitions,
+    energies, rec_of, capacity, pose_size, activity threshold, max cells, numpy dtype)``; ``ValueError`` otherwise."""
+    if isinstance(experience_map, (bool, np.bool_)) and experience_map:
+        raise ValueError("EnsembleSession: experience_map=True replays the maps on the host from whole recordings; "
+                         "a session builds them on the device (experience_map='device')")
+    if not (isinstance(experience_map, (bool, np.bool_))
+            or (isinstance(experience_map, str) and experience_map == "device")):
+        raise ValueError("experience_map must be False or 'device', got %r" % (experience_map,))
+    if (not isinstance(n_recordings, (numbers.Integral, np.integer)) or isinstance(n_recordings, (bool, np.bool_))
+            or n_recordings < 1):
+        raise ValueError("n_recordings must be an integer >= 1, got %r" % (n_recordings,))
+    R = int(n_recordings)
+    B, thr, gi, energies = agent_parameters(n_agents if n_agents is not None else _recording_count(recording),
+                                            match_threshold, global_inhibition, inject_energy)
+    rec_of = agent_recordings(recording, B, R)
+    cap = 32 if capacity is None else capacity
+    if not _real(cap) or not 1 <= cap <= MAX_CAPACITY or cap != int(cap):
+        raise ValueError("capacity must be an integer in [1, %d], got %r" % (MAX_CAPACITY, capacity))
+    cap = (int(cap) + 31) // 32 * 32
+    pose_size = tuple(int(s) for s in pose_size)
+    act_thr, act_k = activity_parameters(activity_threshold, max_active_cells, pose_size)
+    np_dtype = _as_np_dtype(dtype)
+    return B, R, thr, gi, energies, rec_of, cap, pose_size, act_thr, act_k, np_dtype
+
+
+def _full_library(agent, n, unit, frame):
+    return ValueError("EnsembleSession: agent %d holds %d templates, the most the library sweep takes, and %s %d of its "
+                      "recording remains" % (agent, n, unit, frame))
+
+
 class EnsembleSession:
     """B RatSLAM agents that stay on the device between calls: ``feed`` replays the next frames of every recording.
 
@@ -406,26 +441,12 @@ class EnsembleSession:
                  max_active_cells=128):
         self._plan, self._ens, self._work = None, None, None
         self._closed = True
-        if isinstance(experience_map, (bool, np.bool_)) and experience_map:
-            raise ValueError("EnsembleSession: experience_map=True replays the maps on the host from whole recordings; "
-                             "a session builds them on the device (experience_map='device')")
-        if not (isinstance(experience_map, (bool, np.bool_))
-                or (isinstance(experience_map, str) and experience_map == "device")):
-            raise ValueError("experience_map must be False or 'device', got %r" % (experience_map,))
-        if (not isinstance(n_recordings, (numbers.Integral, np.integer)) or isinstance(n_recordings, (bool, np.bool_))
-                or n_recordings < 1):
-            raise ValueError("n_recordings must be an integer >= 1, got %r" % (n_recordings,))
-        R = int(n_recordings)
-        B, thr, gi, energies = agent_parameters(n_agents if n_agents is not None else _recording_count(recording),
-                                                match_threshold, global_inhibition, inject_energy)
-        rec_of = agent_recordings(recording, B, R)
-        cap = 32 if capacity is None else capacity
-        if not _real(cap) or not 1 <= cap <= MAX_CAPACITY or cap != int(cap):
-            raise ValueError("capacity must be an integer in [1, %d], got %r" % (MAX_CAPACITY, capacity))
-        cap = (int(cap) + 31) // 32 * 32
-        pose_size = tuple(int(s) for s in pose_size)
-        act_thr, act_k = activity_parameters(activity_threshold, max_active_cells, pose_size)
-        np_dtype = _as_np_dtype(dtype)
+        # the error a feed raised, where it names a tick and an agent: (tick of the feed, agent, and for a full library
+        # the (templates, unit, frame) of its message)
+        self._fault = None
+        B, R, thr, gi, energies, rec_of, cap, pose_size, act_thr, act_k, np_dtype = _session_arguments(
+            n_agents, match_threshold, global_inhibition, inject_energy, pose_size, dtype, experience_map, n_recordings,
+            recording, capacity, activity_threshold, max_active_cells)
         nat.require_cuda()
         dev = torch.device("cuda", torch.cuda.current_device())
         self.B, self.R, self.pose_size, self.capacity = B, R, pose_size, cap
@@ -596,6 +617,62 @@ class EnsembleSession:
         self._prev_tpl[dst] = self._prev_tpl[src]
         self._ens._state_gen += 1
 
+    # ------------------------------------------------------------------ agents carried to another session
+    def _export_agents(self, agents):
+        """Stages of agents ``agents`` (caller order, repeats allowed) as they are now, on the session's device:
+        ``(plan stage, map stage or None, host state)`` for ``_import_agents`` of another session (prs_ens_export_agents,
+        prs_em_session_export_agents).  Asynchronous on the current stream."""
+        L = nat.lib()
+        rows = np.ascontiguousarray(self._rows[agents], dtype=np.int32)
+        n, stream = len(rows), nat.stream_ptr()
+        n_tpl = np.ascontiguousarray(self._n, dtype=np.int32)
+        stage = torch.empty(int(L.prs_ens_export_stage_bytes(self._plan, n, rows.ctypes.data, n_tpl.ctypes.data)),
+                            dtype=torch.uint8, device=self._dev)
+        nat.check(L.prs_ens_export_agents(self._plan, n, rows.ctypes.data, n_tpl.ctypes.data, stage.data_ptr(),
+                                          stage.numel(), stream), "prs_ens_export_agents")
+        em_stage = None
+        if self._linked:
+            n_rows = np.ascontiguousarray(self._counts[:2].max(axis=0), dtype=np.int32)
+            em_stage = torch.empty(int(L.prs_em_session_export_stage_bytes(self.B, self._E, self._N, n, rows.ctypes.data,
+                                                                           n_rows.ctypes.data)),
+                                   dtype=torch.uint8, device=self._dev)
+            nat.check(L.prs_em_session_export_agents(self.B, self._E, self._N, self._work.data_ptr(), n,
+                                                     rows.ctypes.data, n_rows.ctypes.data, em_stage.data_ptr(),
+                                                     em_stage.numel(), stream), "prs_em_session_export_agents")
+        host = {"n": self._n[rows].copy(), "prev_tpl": self._prev_tpl[rows].copy(),
+                "counts": self._counts[:, rows].copy(), "N": self._N if self._linked else 0}
+        return stage, em_stage, host
+
+    def _fit_agents(self, host):
+        """Grow the libraries and the map workspace to take the exported agents ``host`` describes."""
+        need = max(int(host["n"].max()), int(host["N"]))
+        cap, _ = grow_capacity(self.capacity, need, 0)
+        if cap != self.capacity:
+            self._grow(cap)
+        if self._linked:
+            E = _grow_rows(self._E, int(host["counts"][:2].max()))
+            N = self.capacity if self._N < host["N"] else self._N
+            if E != self._E or N != self._N:
+                self._grow_maps(E, N)
+
+    def _import_agents(self, agents, stage, em_stage, host):
+        """Agents ``agents`` (caller order, distinct) become the exported ones, from stages on this session's device
+        (prs_ens_import_agents, prs_em_session_import_agents); ``_fit_agents`` ran before.  On the current stream."""
+        L = nat.lib()
+        rows = np.ascontiguousarray(self._rows[agents], dtype=np.int32)
+        n, stream = len(rows), nat.stream_ptr()
+        nat.check(L.prs_ens_import_agents(self._plan, n, rows.ctypes.data, stage.data_ptr(), stage.numel(), stream),
+                  "prs_ens_import_agents")
+        if self._linked:
+            nat.check(L.prs_em_session_import_agents(self.B, self._E, self._N, self._work.data_ptr(), n,
+                                                     rows.ctypes.data, em_stage.data_ptr(), em_stage.numel(), stream),
+                      "prs_em_session_import_agents")
+            self._counts[:, rows] = host["counts"]
+        self._n[rows] = host["n"]
+        self._prev_tpl[rows] = host["prev_tpl"]
+        self._ens._state_gen += 1
+        self._stream.wait_stream(torch.cuda.current_stream(self._dev))
+
     @property
     def match_threshold(self):
         """float64 [B]: every agent's match threshold in force, in the caller's order."""
@@ -667,10 +744,9 @@ class EnsembleSession:
                     cap, run = grow_capacity(self.capacity, int(self._n.max()), left)
                     if run == 0 and left:
                         d = int(np.argmax(self._n))
-                        raise ValueError("EnsembleSession: agent %d holds %d templates, the most the library sweep "
-                                         "takes, and %s %d of its recording remains"
-                                         % (self._order[d], self._n[d], unit,
-                                            self.frames_fed[rec_rows[d]] + first[rec_rows[d]]))
+                        frame = int(self.frames_fed[rec_rows[d]] + first[rec_rows[d]])
+                        self._fault = (k0, int(self._order[d]), (int(self._n[d]), unit, frame))
+                        raise _full_library(self._order[d], self._n[d], unit, frame)
                     if cap != self.capacity:
                         self._grow(cap)
                     # ticks [k0, k1) hold `run` ticks with images; the last sub-run takes the trailing odometry
@@ -682,7 +758,7 @@ class EnsembleSession:
                     sub = slice(k0, k1)
                     sub_img = img[sub].sum(axis=0)
                     self._run(streams, first, sub_img, tw[sub], moved[sub], gate[sub], res[sub],
-                              None if self._act_thr is None else (act_counts[sub], act_cells))
+                              None if self._act_thr is None else (act_counts[sub], act_cells), k0)
                     self._room -= int(img_tick[sub].sum())
                     self._n = res["n_templates"][k1 - 1].astype(np.int64)
                     if self._linked:
@@ -758,7 +834,7 @@ class EnsembleSession:
         return {"activity_count": count, "activity_ptr": ptr, "activity_cell": self._cells[idx[g]],
                 "activity_value": val[g].astype(np.float64)}
 
-    def _run(self, streams, first, sub_img, tw, moved, gate, res, act=None):
+    def _run(self, streams, first, sub_img, tw, moved, gate, res, act=None, k0=0):
         """One sub-run of ticks through ``prs_ens_run``; with the activity capture, ``act`` = (counts [T,B], list of
         packed cells) receives it, one device chunk of ticks per run.  A pose-cell error raises what the native replay
         raises, for the earliest tick: with one recording, with the bits of every agent at it (they share the
@@ -794,6 +870,7 @@ class EnsembleSession:
         if not bad.any():
             return
         t = int(np.nonzero(bad.any(axis=1))[0][0])
+        self._fault = (k0 + t, int(self._order[np.nonzero(bad[t])[0]].min()), None)    # the feed's tick k0 + t
         if self.R == 1:
             self._ens._raise_on_err(err[t].astype(np.int32))
         d = self._rows[np.nonzero(bad[t, self._rows])[0][0]]
@@ -906,9 +983,445 @@ class EnsembleSession:
             pass
 
 
+def _device_list(devices):
+    """``devices`` validated as a non-empty sequence of CUDA device indices (no CUDA involved): a list of ints."""
+    if isinstance(devices, (str, bytes)) or not hasattr(devices, "__iter__"):
+        raise ValueError("devices must be a non-empty sequence of CUDA device indices, got %r" % (devices,))
+    devs = list(devices)
+    if not devs:
+        raise ValueError("devices must be a non-empty sequence of CUDA device indices, got %r" % (devices,))
+    for d in devs:
+        if not isinstance(d, (numbers.Integral, np.integer)) or isinstance(d, (bool, np.bool_)) or int(d) < 0:
+            raise ValueError("devices must be CUDA device indices, got %r" % (d,))
+    return [int(d) for d in devs]
+
+
+def _check_devices(devs):
+    """``ValueError`` for a device index this process cannot see (after ``nat.require_cuda``)."""
+    n = torch.cuda.device_count()
+    for d in devs:
+        if d >= n:
+            raise ValueError("devices: cuda:%d does not exist, %d device(s) are visible" % (d, n))
+
+
+def shard_agents(rec_of, devices):
+    """Split B agents over ``devices`` (no CUDA involved beyond the range check): ``rec_of`` is each agent's recording
+    in the caller's order, ``devices`` a non-empty sequence of CUDA device indices, repeats allowed (two shards on one
+    device).  The agents sorted by recording (stable) -- the device-row order of ``EnsembleSession`` -- are cut into
+    ``len(devices)`` contiguous pieces whose sizes differ by at most one, so a shard holds few recordings and one
+    recording may span two shards.  Returns per shard ``(agents, recordings)``: its agents' caller-order indices in that
+    order (int64) and the global recordings it holds, increasing (int64); shard-local recording i is
+    ``recordings[i]``.
+
+    The split balances agent counts only.  An agent's cost grows with its recording's length and its library's size,
+    so shards of long recordings or large libraries take longer, and a feed lasts as long as its slowest shard.
+
+    ``ValueError`` for an empty ``devices``, an entry that is not an integer (bools included), more shards than agents
+    and, once CUDA is up, a device index outside ``torch.cuda.device_count()``."""
+    devs = _device_list(devices)
+    rec_of = np.asarray(rec_of, dtype=np.int64)
+    if len(devs) > len(rec_of):
+        raise ValueError("devices: %d shards for %d agents; a shard holds at least one agent" % (len(devs), len(rec_of)))
+    nat.require_cuda()
+    _check_devices(devs)
+    return _split(rec_of, len(devs))
+
+
+def _split(rec_of, n):
+    """``shard_agents``'s pieces of ``rec_of`` for n shards (pure)."""
+    order = np.argsort(rec_of, kind="stable")
+    return [(a, np.unique(rec_of[a])) for a in np.array_split(order, n)]
+
+
+def _shard_index(shards, B):
+    """Per agent: its shard and its index within the shard."""
+    shard_of, local_of = np.empty(B, np.int64), np.empty(B, np.int64)
+    for i, (a, _) in enumerate(shards):
+        shard_of[a], local_of[a] = i, np.arange(len(a))
+    return shard_of, local_of
+
+
+def plan_agent_moves(parents, shards):
+    """``ShardedEnsembleSession.reassign``'s moves (no CUDA involved): ``parents`` int [B] (validated) over the
+    ``shards`` of ``shard_agents``.  Returns ``(local, cross)``: ``local[s] = (dst, src)``, shard s's in-shard moves as
+    local agent indices, and ``cross``, one ``(s, t, src, dst)`` per pair of shards with moves from s to t, the parents'
+    local indices in s and the children's in t, children in increasing caller order.  Applied in three steps -- export
+    every cross parent from the state before the call, run each shard's in-shard copies, import -- every child ends as
+    its parent was before the call."""
+    par = np.asarray(parents, dtype=np.int64)
+    B = len(par)
+    shard_of, local_of = _shard_index(shards, B)
+    moved = np.nonzero(par != np.arange(B))[0]
+    src_shard, dst_shard = shard_of[par[moved]], shard_of[moved]
+    local = []
+    for s in range(len(shards)):
+        m = moved[(src_shard == s) & (dst_shard == s)]
+        local.append((local_of[m], local_of[par[m]]))
+    cross = []
+    for s in range(len(shards)):
+        for t in range(len(shards)):
+            m = moved[(src_shard == s) & (dst_shard == t)] if s != t else moved[:0]
+            if len(m):
+                cross.append((s, t, local_of[par[m]], local_of[m]))
+    return local, cross
+
+
+class ShardedAgents:
+    """``EnsembleAgents`` of a sharded session: every accessor goes to the agent's shard and its index there."""
+
+    def __init__(self, parts, shard_of, local_of, n_templates, shape):
+        self._parts, self._shard_of, self._local_of = parts, shard_of, local_of
+        self.n_templates = n_templates
+        self.shape = shape
+
+    def __len__(self):
+        return len(self.n_templates)
+
+    def _at(self, b):
+        b = int(b)
+        return self._parts[self._shard_of[b]], int(self._local_of[b])
+
+    @property
+    def path(self):
+        """The pose-cell kernel family of each shard (``PoseCellEnsemble.path``)."""
+        return [p.path for p in self._parts]
+
+    @property
+    def state(self):
+        """The device tensor ``[B, Th, X, Y]`` of every agent's pose cells, for one shard only."""
+        if len(self._parts) > 1:
+            raise RuntimeError("ShardedAgents.state: the pose cells live on %d shards; read each agent's with "
+                               "posecells(b)" % len(self._parts))
+        st = self._parts[0].state
+        return st[torch.from_numpy(self._local_of).to(st.device)]
+
+    def templates(self, b):
+        p, j = self._at(b)
+        return p.templates(j)
+
+    def locations(self, b):
+        p, j = self._at(b)
+        return p.locations(j)
+
+    def posecells(self, b):
+        p, j = self._at(b)
+        return p.posecells(j)
+
+
+class ShardedMaps:
+    """``EnsembleExperienceMaps`` of a sharded session: per-agent arrays in the caller's order, every accessor going to
+    the agent's shard."""
+
+    def __init__(self, parts, shards, shard_of, local_of):
+        self._parts, self._shard_of, self._local_of = parts, shard_of, local_of
+        B = len(shard_of)
+        for k in ("n_experiences", "n_links", "current", "n_loop_closures"):
+            v = np.zeros(B, np.int64)
+            for (a, _), p in zip(shards, parts):
+                v[a] = getattr(p, k)
+            setattr(self, k, v)
+        self.pose_size = parts[0].pose_size
+
+    def __len__(self):
+        return len(self.n_experiences)
+
+    def _at(self, b):
+        b = int(b)
+        return self._parts[self._shard_of[b]], int(self._local_of[b])
+
+    def experiences(self, b):
+        p, j = self._at(b)
+        return p.experiences(j)
+
+    def links(self, b):
+        p, j = self._at(b)
+        return p.links(j)
+
+    def experience_map(self, b):
+        p, j = self._at(b)
+        return p.experience_map(j)
+
+
+_FILL = {"template": -1, "created": False, "score": -1, "argmax": -1, "n_exp": -1, "exp_id": -1, "em_xy": np.nan,
+         "activity_count": -1}
+
+
+class ShardedEnsembleSession:
+    """``EnsembleSession`` with its agents split over several CUDA devices: ``devices`` (a sequence of device indices,
+    repeats allowed) comes first, the other arguments, the methods and the results are ``EnsembleSession``'s.
+
+    ``shard_agents`` cuts the agents, sorted by recording, into one contiguous piece per entry of ``devices``; each
+    piece is a plain ``EnsembleSession`` on its device, holding its agents' settings and the recordings they replay.
+    A feed runs every shard's ticks in its own host thread (the native runs release the GIL, so the devices overlap)
+    and joins them before it returns; the results are merged into the caller's agent order and equal one device's key
+    by key, the per-image arrays padded as one device pads them.  An error in any shard closes every shard and raises
+    what one device raises, for the earliest tick and, within it, the lowest agent.
+
+    ``reassign`` takes parents anywhere: a child whose parent lives on another shard receives it through a stage
+    exported from the parent's device before any shard changes, copied across with one peer copy and imported after
+    the shards' own copies (``plan_agent_moves``)."""
+
+    def __init__(self, devices, n_agents=None, match_threshold=MATCH_THRESHOLD, global_inhibition=PC_GLOBAL_INHIB,
+                 inject_energy=None, pose_size=POSE_SIZE, dtype=np.float32, active_set=0, experience_map=False,
+                 experience_links=False, n_recordings=1, recording=0, capacity=None, activity_threshold=None,
+                 max_active_cells=128):
+        self._shards, self._closed = [], True
+        devs = _device_list(devices)
+        B, R, thr, gi, energies, rec_of, cap, pose_size, act_thr, act_k, np_dtype = _session_arguments(
+            n_agents, match_threshold, global_inhibition, inject_energy, pose_size, dtype, experience_map, n_recordings,
+            recording, capacity, activity_threshold, max_active_cells)
+        if len(devs) > B:
+            raise ValueError("devices: %d shards for %d agents; a shard holds at least one agent" % (len(devs), B))
+        nat.require_cuda()
+        _check_devices(devs)
+        self.B, self.R, self.pose_size = B, R, pose_size
+        self._devs, self._rec_of = devs, rec_of
+        self._thr, self._gi, self._energies = thr, gi, list(energies)
+        self._map = isinstance(experience_map, str)
+        self._linked = self._map and bool(experience_links)
+        self._act = act_thr is not None
+        self._split = _split(rec_of, len(devs))
+        self._shard_of, self._local_of = _shard_index(self._split, B)
+        self.frames_fed = np.zeros(R, np.int64)
+        try:
+            for d, (a, recs) in zip(devs, self._split):
+                with torch.cuda.device(d):
+                    self._shards.append(EnsembleSession(
+                        len(a), thr[a], gi[a], [energies[i] for i in a], pose_size, np_dtype, active_set,
+                        experience_map, experience_links, len(recs), np.searchsorted(recs, rec_of[a]), cap, act_thr,
+                        act_k))
+        except BaseException:
+            self.close()
+            raise
+        self._closed = False
+
+    # ------------------------------------------------------------------ running on every shard
+    def _each(self, fn):
+        """``fn(i, shard)`` for every shard in its own thread under its device; the threads are joined before it
+        returns.  Returns the results; if any shard raised, closes every shard and raises (``_first_error``)."""
+        n = len(self._shards)
+        results, errors = [None] * n, [None] * n
+
+        def work(i):
+            try:
+                with torch.cuda.device(self._devs[i]):
+                    results[i] = fn(i, self._shards[i])
+            except BaseException as e:                  # noqa: B902 -- re-raised on the calling thread
+                errors[i] = e
+
+        threads = [threading.Thread(target=work, args=(i,)) for i in range(n)]
+        for t in threads:
+            t.start()
+        for t in threads:
+            t.join()
+        if any(e is not None for e in errors):
+            self.close()
+            raise self._first_error(errors)
+        return results
+
+    def _first_error(self, errors):
+        """The error one device raises: the faults that name a tick and an agent (pose-cell errors, a full library) go
+        by (tick, caller agent); a full library's text names the caller's agent."""
+        named = [(sh._fault[0], int(self._split[i][0][sh._fault[1]]), i) for i, sh in enumerate(self._shards)
+                 if errors[i] is not None and sh._fault is not None]
+        if not named:
+            return next(e for e in errors if e is not None)
+        _, b, i = min(named)
+        detail = self._shards[i]._fault[2]
+        return errors[i] if detail is None else _full_library(b, *detail)
+
+    def _check_open(self):
+        if self._closed:
+            raise RuntimeError("EnsembleSession: the session is closed")
+
+    # ------------------------------------------------------------------ feeding
+    def feed(self, frames, odom):
+        """``EnsembleSession.feed`` over every shard."""
+        self._check_open()
+        fr, od = feed_inputs(frames, odom, self.R)
+        return self._feed_ticks(_frame_ticks(fr, od), "frame")
+
+    def feed_events(self, events):
+        """``EnsembleSession.feed_events`` over every shard."""
+        self._check_open()
+        return self._feed_ticks(event_streams(events, self.R), "image")
+
+    def _feed_ticks(self, streams, unit="image"):
+        for sh in self._shards:
+            sh._fault = None
+        parts = self._each(lambda i, sh: sh._feed_ticks([streams[r] for r in self._split[i][1]], unit))
+        n_img = np.array([len(st[0]) for st in streams], dtype=np.int64)
+        self.frames_fed += n_img
+        return self._merge(parts, int(n_img.max()))
+
+    def _merge(self, parts, i_max):
+        """The shards' results in the caller's order: per-image arrays [B, i_max] padded as one device pads them,
+        per-agent arrays scattered, and the activity capture's CSR rebuilt over the merged agents."""
+        B = self.B
+        out = {}
+        for k, v in parts[0].items():
+            if k.startswith("activity_") and k != "activity_count":
+                continue
+            if k in _FILL:
+                out[k] = np.full((B, i_max) + v.shape[2:], _FILL[k], v.dtype)
+                for (a, _), p in zip(self._split, parts):
+                    out[k][a, :p[k].shape[1]] = p[k]
+            else:
+                out[k] = np.zeros(B, v.dtype)
+                for (a, _), p in zip(self._split, parts):
+                    out[k][a] = p[k]
+        if self._act:
+            # agent b's entries are one slice of its shard's packed cells (its row of the shard's [B_s, i_s] entries)
+            slices = [None] * B
+            for (a, _), p in zip(self._split, parts):
+                i_s = p["activity_count"].shape[1]
+                ptr = p["activity_ptr"]
+                for j, b in enumerate(a):
+                    slices[b] = (p, ptr[j * i_s], ptr[(j + 1) * i_s])
+            n = np.clip(out["activity_count"], 0, None)
+            kept = np.minimum(n, self._shards[0]._act_k).ravel()
+            ptr = np.zeros(B * i_max + 1, np.int64)
+            np.cumsum(kept, out=ptr[1:])
+            out["activity_ptr"] = ptr
+            out["activity_cell"] = np.concatenate([p["activity_cell"][lo:hi] for p, lo, hi in slices]
+                                                  + [np.zeros((0, 3), np.int64)])
+            out["activity_value"] = np.concatenate([p["activity_value"][lo:hi] for p, lo, hi in slices]
+                                                   + [np.zeros(0)])
+        return out
+
+    # ------------------------------------------------------------------ reassigning agents
+    def reassign(self, parents, match_threshold=KEEP, global_inhibition=KEEP, inject_energy=KEEP):
+        """``EnsembleSession.reassign`` with parents on any shard; ``ValueError`` before any CUDA call for what one
+        device refuses.  Every setting is resolved per agent first (KEEP: the parent's, wherever it lives).  Then
+        (``plan_agent_moves``): 1. every parent of a child on another shard is exported from the state as it was
+        before the call; 2. each shard runs its own copies and takes its settings; 3. each destination grows to fit
+        its incoming parents, receives the stages (one peer copy, ordered after the export with an event) and imports
+        them.  An error closes every shard."""
+        self._check_open()
+        par, thr, gi, energies = reassign_parameters(parents, self._rec_of, self._thr, self._gi, self._energies,
+                                                     match_threshold, global_inhibition, inject_energy)
+        try:
+            self._reassign(par, thr, gi, energies)
+        except BaseException:
+            self.close()
+            raise
+
+    def _reassign(self, par, thr, gi, energies):
+        local, cross = plan_agent_moves(par, self._split)
+        staged = []
+        for s, t, src, dst in cross:                   # 1. every cross parent as it is before the call
+            with torch.cuda.device(self._devs[s]):
+                stage, em_stage, host = self._shards[s]._export_agents(src)
+                done = torch.cuda.Event()
+                done.record(torch.cuda.current_stream())
+            staged.append((s, t, dst, stage, em_stage, host, done))
+
+        for i, sh in enumerate(self._shards):          # 2. each shard's own copies and settings
+            a = self._split[i][0]
+            p = np.arange(len(a))
+            p[local[i][0]] = local[i][1]
+            with torch.cuda.device(self._devs[i]):
+                sh._reassign(p, local[i][0], thr[a], gi[a], [energies[b] for b in a])
+        for s, t, dst, stage, em_stage, host, done in staged:     # 3. grow, copy across, import
+            sh, d = self._shards[t], self._devs[t]
+            with torch.cuda.device(d):
+                sh._fit_agents(host)
+                cur = torch.cuda.current_stream()
+                cur.wait_event(done)
+                there = [self._to_device(x, d, self._devs[s], cur) for x in (stage, em_stage)]
+                sh._import_agents(dst, there[0], there[1], host)
+        for d in sorted(set(self._devs)):
+            torch.cuda.synchronize(d)
+        self._thr, self._gi, self._energies = thr, gi, list(energies)
+
+    @staticmethod
+    def _to_device(stage, dst_dev, src_dev, stream):
+        """The stage on ``dst_dev``: one prs_stage_copy (a peer copy between devices) on ``stream``."""
+        if stage is None:
+            return None
+        out = torch.empty_like(stage, device=torch.device("cuda", dst_dev))
+        nat.check(nat.lib().prs_stage_copy(out.data_ptr(), dst_dev, stage.data_ptr(), src_dev, stage.numel(),
+                                           ctypes.c_void_p(stream.cuda_stream)), "prs_stage_copy")
+        return out
+
+    # ------------------------------------------------------------------ what the agents hold
+    def _gather(self, name):
+        self._require_shards()
+        v = np.zeros(self.B, np.int64)
+        for (a, _), sh in zip(self._split, self._shards):
+            v[a] = getattr(sh, name)
+        return v
+
+    def _require_shards(self):
+        if len(self._shards) != len(self._devs):
+            raise RuntimeError("EnsembleSession: the session is closed")
+
+    @property
+    def match_threshold(self):
+        """float64 [B]: every agent's match threshold in force, in the caller's order."""
+        return self._thr.copy()
+
+    @property
+    def global_inhibition(self):
+        """float64 [B]: every agent's global inhibition in force, in the caller's order."""
+        return self._gi.copy()
+
+    @property
+    def inject_energy(self):
+        """list of B energies (None = no injection) in force, in the caller's order."""
+        return list(self._energies)
+
+    @property
+    def n_templates(self):
+        """int64 [B]: templates in each agent's library."""
+        return self._gather("n_templates")
+
+    @property
+    def n_experiences(self):
+        """int64 [B]: experiences in each agent's map so far (0 without ``experience_map``)."""
+        return self._gather("n_experiences")
+
+    @property
+    def n_loop_closures(self):
+        """int64 [B]: loop closures of each agent's linked map (0 without one)."""
+        return self._gather("n_loop_closures")
+
+    @property
+    def agents(self):
+        """``ShardedAgents``, in the caller's agent order (the libraries as they are now)."""
+        self._require_shards()
+        if any(sh._ens is None for sh in self._shards):
+            raise RuntimeError("EnsembleSession: the session is closed")
+        return ShardedAgents([sh.agents for sh in self._shards], self._shard_of, self._local_of, self.n_templates,
+                             self.pose_size)
+
+    @property
+    def maps(self):
+        """``ShardedMaps`` of the linked device maps, in the caller's agent order; None without them."""
+        self._require_shards()
+        parts = [sh.maps for sh in self._shards]
+        if any(p is None for p in parts):
+            return None
+        return ShardedMaps(parts, self._split, self._shard_of, self._local_of)
+
+    def close(self):
+        """Close every shard; a closed session's ``feed`` raises ``RuntimeError``.  What ``agents`` and ``maps``
+        returned before stays readable."""
+        for sh in self._shards:
+            sh.close()
+        self._closed = True
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
 def replay_ensemble(frames, odom, n_agents=None, match_threshold=MATCH_THRESHOLD, global_inhibition=PC_GLOBAL_INHIB,
                     inject_energy=None, pose_size=POSE_SIZE, dtype=np.float32, active_set=0, experience_map=False,
-                    experience_links=False, mode="ref", recording=0, activity_threshold=None, max_active_cells=128):
+                    experience_links=False, mode="ref", recording=0, activity_threshold=None, max_active_cells=128,
+                    devices=None):
     """Replay ``frames[T,256,256]`` (uint8) and ``odom[T,2]`` = (linear.x, angular.z) through B agents.
 
     ``match_threshold``, ``global_inhibition`` and ``inject_energy`` (None = no injection, else a finite energy >= 0)
@@ -944,10 +1457,15 @@ def replay_ensemble(frames, odom, n_agents=None, match_threshold=MATCH_THRESHOLD
     ``activity_entry(out, b, t)`` returns one entry as ``(index, value)``.  Off by default; off, nothing changes.
 
     This is one ``EnsembleSession`` fed once, with libraries reserved for every frame up front; a session fed in
-    pieces replays recordings that do not fit in host memory, or longer than 65535 frames."""
+    pieces replays recordings that do not fit in host memory, or longer than 65535 frames.
+
+    ``devices`` (None: the current device) is a sequence of CUDA device indices to split the agents over: one
+    ``ShardedEnsembleSession`` fed once, with the same result; ``agents`` and ``maps`` are then its ``ShardedAgents``
+    and ``ShardedMaps``."""
     if not (isinstance(experience_map, (bool, np.bool_))
             or (isinstance(experience_map, str) and experience_map == "device")):
         raise ValueError("experience_map must be False, True or 'device', got %r" % (experience_map,))
+    devices = None if devices is None else _device_list(devices)
     several = isinstance(frames, (list, tuple)) and (len(frames) == 0 or np.ndim(frames[0]) == 3)
     if several:
         R = len(frames)
@@ -977,7 +1495,7 @@ def replay_ensemble(frames, odom, n_agents=None, match_threshold=MATCH_THRESHOLD
     out, rec_of = _replay_once("replay_ensemble", _frame_ticks(fr, od), n_agents, recording, match_threshold,
                                global_inhibition, inject_energy, pose_size, dtype, active_set,
                                "device" if experience_map == "device" else False, experience_links, mode,
-                               activity_threshold, max_active_cells)
+                               activity_threshold, max_active_cells, devices)
     if isinstance(experience_map, (bool, np.bool_)) and experience_map:
         moved, tw = np.zeros((T, R), np.uint8), np.zeros((T, R, 2))
         for r in range(R):
@@ -998,7 +1516,7 @@ def replay_ensemble(frames, odom, n_agents=None, match_threshold=MATCH_THRESHOLD
 def replay_ensemble_events(events, n_agents=None, match_threshold=MATCH_THRESHOLD, global_inhibition=PC_GLOBAL_INHIB,
                            inject_energy=None, pose_size=POSE_SIZE, dtype=np.float32, active_set=0, experience_map=False,
                            experience_links=False, mode="ref", recording=0, activity_threshold=None,
-                           max_active_cells=128):
+                           max_active_cells=128, devices=None):
     """``replay_ensemble`` over message streams (``rosbag_io.read_events``) instead of paired frames and twists: agent b
     is the node's message loop, ``ros_simulate.replay_events(events, match_threshold=..., inject_energy=...,
     experience_links=...)`` with ``pcn.global_inhibition`` set to its own value, so every gated odometry message is its
@@ -1010,23 +1528,27 @@ def replay_ensemble_events(events, n_agents=None, match_threshold=MATCH_THRESHOL
     ``agents`` and, with ``experience_map="device"``, ``maps``.  On a stream in which odometry and images alternate it equals
     ``replay_ensemble`` on ``rosbag_io.events_to_arrays(events)[:2]``.  The activity capture (``activity_threshold``,
     ``max_active_cells``) is ``replay_ensemble``'s, per image: odometry-only ticks capture nothing (there is no
-    per-update capture of message streams).  This is one ``EnsembleSession`` fed once."""
+    per-update capture of message streams).  This is one ``EnsembleSession`` fed once; ``devices`` splits the agents
+    over several devices as ``replay_ensemble``'s does."""
     if not (isinstance(experience_map, (bool, np.bool_)) and not experience_map
             or (isinstance(experience_map, str) and experience_map == "device")):
         raise ValueError("replay_ensemble_events: experience_map must be False or 'device' (the host maps need the "
                          "paired frames of replay_ensemble), got %r" % (experience_map,))
+    devices = None if devices is None else _device_list(devices)
     several = (isinstance(events, (list, tuple)) and len(events) > 0 and not _is_event(events[0]))
     streams = [event_ticks(st) for st in events] if several else [event_ticks(events)]
     return _replay_once("replay_ensemble_events", streams, n_agents, recording, match_threshold, global_inhibition,
                         inject_energy, pose_size, dtype, active_set, experience_map, experience_links, mode,
-                        activity_threshold, max_active_cells)[0]
+                        activity_threshold, max_active_cells, devices)[0]
 
 
 def _replay_once(who, streams, n_agents, recording, match_threshold, global_inhibition, inject_energy, pose_size,
-                 dtype, active_set, experience_map, experience_links, mode, activity_threshold=None, max_active_cells=128):
+                 dtype, active_set, experience_map, experience_links, mode, activity_threshold=None, max_active_cells=128,
+                 devices=None):
     """``replay_ensemble`` and ``replay_ensemble_events`` after their inputs are validated: the agents' parameters and
     recordings are broadcast and validated and the device memory is checked before any other CUDA call, then one
-    ``EnsembleSession`` with libraries for every image is fed the R tick streams once.  Returns the feed's result with
+    ``EnsembleSession`` with libraries for every image is fed the R tick streams once -- a ``ShardedEnsembleSession``
+    over ``devices`` when given, with the memory checked per physical device.  Returns the feed's result with
     ``agents`` (and ``maps`` for ``experience_map="device"``), and the agents' recordings."""
     B, thr, gi, energies = agent_parameters(n_agents if n_agents is not None else _recording_count(recording),
                                             match_threshold, global_inhibition, inject_energy)
@@ -1042,18 +1564,32 @@ def _replay_once(who, streams, n_agents, recording, match_threshold, global_inhi
     for r, st in enumerate(streams):
         img[:len(st[3]), r] = st[3]
     cap = min(capacity_for(int(img.any(axis=1).sum())), MAX_CAPACITY)
-    # what the session allocates: per agent its library, template locations, network, the network's snapshot of a
-    # mixed tick (R > 1 only), a chunk of records and a few scalars; one chunk of every recording's images
-    frame_bytes = IM_SIZE[0] * IM_SIZE[1]
-    chunk = _ens_chunk(R, frame_bytes)
-    net_bytes = int(np.prod(pose_size)) * np.dtype(np_dtype).itemsize
-    need = (B * ((cap // 32) * 34816 + cap * 8 + (2 if R > 1 else 1) * net_bytes + chunk * 32 + 128)
-            + R * chunk * frame_bytes)
-    if experience_map == "device" and experience_links:
-        need += xens.work_bytes(B, K, cap) + xens.record_bytes(B, K)
-    if act_thr is not None:     # the capture's counts, slots and packed cells of one chunk (prs_ens_activity_bytes)
-        rows = chunk * B
-        need += rows * 4 + 2 * rows * act_k * (4 + np.dtype(np_dtype).itemsize) + (rows + 1) * 8 + 6 * 256
+    linked = experience_map == "device" and experience_links
+    if devices is not None:
+        if len(devices) > B:
+            raise ValueError("devices: %d shards for %d agents; a shard holds at least one agent" % (len(devices), B))
+        nat.require_cuda()
+        _check_devices(devices)
+        need = {}
+        for d, (a, recs) in zip(devices, _split(rec_of, len(devices))):
+            need[d] = need.get(d, 0) + _session_bytes(len(a), len(recs), cap, K, pose_size, np_dtype, linked,
+                                                      None if act_thr is None else act_k)
+        for d in sorted(need):
+            free, _ = torch.cuda.mem_get_info(torch.device("cuda", d))
+            if need[d] > free:
+                raise ValueError("%s: the agents on cuda:%d need %.2f GB of device memory (%d templates each), "
+                                 "%.2f GB are free" % (who, d, need[d] / 1e9, cap, free / 1e9))
+        session = ShardedEnsembleSession(devices, B, thr, gi, energies, pose_size, np_dtype, active_set, experience_map,
+                                         experience_links, R, rec_of, cap, act_thr, act_k)
+        try:
+            out = session._feed_ticks(streams)
+            out["agents"] = session.agents
+            if experience_map == "device":
+                out["maps"] = session.maps
+        finally:
+            session.close()
+        return out, rec_of
+    need = _session_bytes(B, R, cap, K, pose_size, np_dtype, linked, None if act_thr is None else act_k)
     nat.require_cuda()
     dev = torch.device("cuda", torch.cuda.current_device())
     free, _ = torch.cuda.mem_get_info(dev)
@@ -1070,6 +1606,24 @@ def _replay_once(who, streams, n_agents, recording, match_threshold, global_inhi
     finally:
         session.close()
     return out, rec_of
+
+
+def _session_bytes(B, R, cap, K, pose_size, np_dtype, linked, act_k):
+    """Device bytes an ``EnsembleSession`` of B agents and R recordings allocates for a replay of K ticks with
+    libraries of ``cap`` templates (``act_k`` None: no activity capture)."""
+    # per agent its library, template locations, network, the network's snapshot of a mixed tick (R > 1 only), a chunk
+    # of records and a few scalars; one chunk of every recording's images
+    frame_bytes = IM_SIZE[0] * IM_SIZE[1]
+    chunk = _ens_chunk(R, frame_bytes)
+    net_bytes = int(np.prod(pose_size)) * np.dtype(np_dtype).itemsize
+    need = (B * ((cap // 32) * 34816 + cap * 8 + (2 if R > 1 else 1) * net_bytes + chunk * 32 + 128)
+            + R * chunk * frame_bytes)
+    if linked:
+        need += xens.work_bytes(B, K, cap) + xens.record_bytes(B, K)
+    if act_k is not None:       # the capture's counts, slots and packed cells of one chunk (prs_ens_activity_bytes)
+        rows = chunk * B
+        need += rows * 4 + 2 * rows * act_k * (4 + np.dtype(np_dtype).itemsize) + (rows + 1) * 8 + 6 * 256
+    return need
 
 
 def _experience_maps(out, moved, tw, pose_size, linked, rec_of=None):
@@ -1119,13 +1673,18 @@ def _activity_stats(out, acc):
         np.maximum(acc[2], c.max(axis=1), out=acc[2])
 
 
-def _replay_chunked(bags, chunk, image_topic, odom_topic, recording, acc=None, **kw):
+def _session(devices, **kw):
+    """An ``EnsembleSession``, or a ``ShardedEnsembleSession`` over ``devices``."""
+    return EnsembleSession(**kw) if devices is None else ShardedEnsembleSession(devices, **kw)
+
+
+def _replay_chunked(bags, chunk, image_topic, odom_topic, recording, acc=None, devices=None, **kw):
     """The bags fed through one ``EnsembleSession`` ``chunk`` frames per bag at a time: per agent the templates, the
     frames created on, its bag's frame count and final arg-max (None for an empty bag), and the session's maps."""
     from . import rosbag_io as rb
     R = len(bags)
     its = [rb.iter_frames(bag, chunk, image_topic=image_topic, odom_topic=odom_topic) for bag in bags]
-    s = EnsembleSession(n_recordings=R, recording=recording if R > 1 else 0, capacity=capacity_for(chunk), **kw)
+    s = _session(devices, n_recordings=R, recording=recording if R > 1 else 0, capacity=capacity_for(chunk), **kw)
     try:
         B = len(s.n_templates)
         created = np.zeros(B, np.int64)
@@ -1147,7 +1706,7 @@ def _replay_chunked(bags, chunk, image_topic, odom_topic, recording, acc=None, *
         s.close()
 
 
-def _replay_all_messages(bags, chunk, image_topic, odom_topic, recording, acc=None, **kw):
+def _replay_all_messages(bags, chunk, image_topic, odom_topic, recording, acc=None, devices=None, **kw):
     """``--all-messages``: the bags' message streams fed through one ``EnsembleSession`` with ``feed_events``, ``chunk``
     images per bag at a time (each bag whole without it): per agent the templates, the images created on, its bag's
     image count and final arg-max, and the experience and loop-closure counts of its map."""
@@ -1157,8 +1716,8 @@ def _replay_all_messages(bags, chunk, image_topic, odom_topic, recording, acc=No
         its = [iter([rb.read_events(bag, image_topic=image_topic, odom_topic=odom_topic)]) for bag in bags]
     else:
         its = [rb.iter_events(bag, chunk, image_topic=image_topic, odom_topic=odom_topic) for bag in bags]
-    s = EnsembleSession(n_recordings=R, recording=recording if R > 1 else 0,
-                        capacity=capacity_for(chunk) if chunk is not None else None, **kw)
+    s = _session(devices, n_recordings=R, recording=recording if R > 1 else 0,
+                 capacity=capacity_for(chunk) if chunk is not None else None, **kw)
     try:
         B = len(s.n_templates)
         created = np.zeros(B, np.int64)
@@ -1204,6 +1763,8 @@ def main(argv=None):
                     help="capture every agent's pose cells above T at each image on the device (0.002 is what the "
                          "viewers draw) and print each agent's mean and max active-cell count; only the counts come "
                          "back from the device")
+    ap.add_argument("--devices", metavar="D1,D2,...",
+                    help="split the agents over these CUDA devices (ShardedEnsembleSession); the output is the same")
     a = ap.parse_args(argv)
     from . import rosbag_io as rb
     thr = _list(a.match_threshold, float)
@@ -1217,6 +1778,8 @@ def main(argv=None):
               experience_map="device" if a.experience_links or a.all_messages else False,
               experience_links=a.experience_links)
     acc, extra = None, {}
+    if a.devices is not None:
+        kw["devices"] = _list(a.devices, int)
     if a.activity_threshold is not None:
         kw.update(activity_threshold=a.activity_threshold, max_active_cells=0)
         acc = [np.zeros(len(agents), np.int64), np.zeros(len(agents), np.int64), np.full(len(agents), -1, np.int64)]
